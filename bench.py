@@ -33,6 +33,10 @@ configs[4] sub-record keeps its batch fixed.  Every rank runs on the host cores 
 
 `--impl reference` times the reference's own CPU path (oracle port; one process per sample on all host cores, the way the
 reference is deployed) for the same metric and config.
+
+`--dump-outputs DIR` writes what the headline's last timed step computed, the arrays a caller of the path receives
+(Batch.fetch() and the per-sample guard counts), as DIR/<name>.npy in float64; the inputs are a function of the arguments
+only, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -47,6 +51,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the benchmark leaves the tree as it found it (no __pycache__ next to the sources)
 
 N_ROWS = 10_700_000
 N_ACC = 1135
@@ -80,7 +85,14 @@ def parse_args():
                          "2 GPUs, and NCCL reduces inside the NVSwitch beyond), none = timing experiment only (totals stay per rank)")
     ap.add_argument("--cpu-markers", type=int, default=0, help="bound the CPU sample (0 = one whole sample)")
     ap.add_argument("--no-numa-bind", action="store_true", help="leave the process on whatever cores it was started on (default: the cores next to its GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline's results of its last timed step as DIR/<name>.npy (float64: score, matches, ninfo, m, prob, L, "
+                         "LR, guard; sample_index = the samples they belong to, a fixed seeded subset when all would exceed 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 arm")
     if args.reduce == "auto":
         args.reduce = "nccl"
     return args
@@ -399,9 +411,18 @@ def all_sum(ctx, vals):
     return [float(x) for x in t]
 
 
-def measure_inbred(ctx, g, samples, positions, regions, r0, r1, n_acc, steps, warmup, chunk, e2e=True, exact=True, hard=False):
+def last_step_outputs(b):
+    """What a caller of the resident path receives from batch `b` after its step: Batch.fetch() and the guard counts."""
+    out = b.fetch()
+    out["guard"] = b.guard_counts()
+    return out
+
+
+def measure_inbred(ctx, g, samples, positions, regions, r0, r1, n_acc, steps, warmup, chunk, e2e=True, exact=True, hard=False,
+                   keep_last=False):
     """Resident and end-to-end arms of inbred scoring of `samples` against this rank's shard.  Returns a dict of numbers plus
-    `res`: the last step's results of this rank's share (for the parity checks)."""
+    `res`: the last step's results of this rank's share (for the parity checks), and with keep_last `last_step`: the results
+    of the last timed step of the resident arm, read from the batch that ran it."""
     from snpmatch_b200 import lib
     torch = ctx.torch
     db = g.db
@@ -474,10 +495,14 @@ def measure_inbred(ctx, g, samples, positions, regions, r0, r1, n_acc, steps, wa
                 gb.wait()
                 gb2.wait()
             dev_ms = timed_steps(ctx, piped_step, wait_both, warmup, steps, flush=flush_step)
+            if keep_last:
+                r["last_step"] = last_step_outputs(pair[(count[0] - 1) % 2])
             gb2.close()
             r["resident_loop"] = "two batches alternate; the NCCL reduce-scatter of a step overlaps the join and grouping kernels of the next"
         else:
             dev_ms = timed_steps(ctx, device_step, gb.wait, warmup, steps)
+            if keep_last:
+                r["last_step"] = last_step_outputs(gb)
         stage = {}
         for _ in range(steps):                                   # one more pass that reads the library's own events each step
             device_step()
@@ -602,6 +627,33 @@ def measure_inbred(ctx, g, samples, positions, regions, r0, r1, n_acc, steps, wa
     return r
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(ctx, res, n_samples, out_dir):
+    """--dump-outputs: `res` (this rank's share of the samples, rows rank * S_loc ...) as out_dir/<name>.npy in float64 (the
+    counts are exact in it).  All samples, or a fixed seeded subset of them when they would take more than DUMP_BYTES;
+    sample_index.npy names the samples either way.  Every rank sends its rows; rank 0 writes."""
+    per_sample = 8 * (1 + sum(int(np.prod(v.shape[1:])) for v in res.values()))
+    keep = np.arange(n_samples)
+    if n_samples * per_sample > DUMP_BYTES:
+        if per_sample > DUMP_BYTES:
+            raise SystemExit("--dump-outputs: the results of one sample exceed %d bytes" % DUMP_BYTES)
+        keep = np.sort(np.random.default_rng(0).choice(n_samples, size=DUMP_BYTES // per_sample, replace=False))
+    s_loc = n_samples // ctx.world
+    mine = keep[(keep >= ctx.rank * s_loc) & (keep < (ctx.rank + 1) * s_loc)] - ctx.rank * s_loc
+    part = {k: v[mine] for k, v in res.items()}
+    if ctx.world > 1:
+        box = [None] * ctx.world
+        ctx.dist.all_gather_object(box, part, group=ctx.host_pg)
+        part = {k: np.concatenate([p[k] for p in box]) for k in part}
+    if ctx.rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        part["sample_index"] = keep
+        for k, v in part.items():
+            np.save(os.path.join(out_dir, k + ".npy"), v.astype(np.float64))
+
+
 def gather_last_rank_sample(ctx, res, i_local):
     """Rank 0 receives (matches, ninfo, score) of local sample i_local of the LAST rank (host collective over gloo)."""
     payload = None
@@ -713,8 +765,11 @@ def run_b200_arm(args):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    h = measure_inbred(ctx, g, samples, positions, regions, r0, r1, n_acc, args.steps, args.warmup, args.group_chunk)
+    h = measure_inbred(ctx, g, samples, positions, regions, r0, r1, n_acc, args.steps, args.warmup, args.group_chunk,
+                       keep_last=bool(args.dump_outputs))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(ctx, h["last_step"], S, args.dump_outputs)
     comps = h["m_total"] * n_acc
     line = None
     if rank == 0:

@@ -118,27 +118,60 @@ def test_pack_reference_layout():
     assert int(packed[0, 3]) == 2**64 - 1 and (int(packed[0, 2]) >> 6) & 1 == 1    # padding = missing
 
 
-REF_SAMPLES = "/root/reference/sample_files"
+def _write_sample_vcf(path, g):
+    """The kept records of the reference's sample file 701_501.filter.vcf, as the reference parsed them (golden
+    vcf701_sample.npz), written back as VCF text: integer PL = -10 ln(wei) (exact for every record), INFO/DP and FORMAT
+    GT:AD:DP:GQ:PL of that file.  After every third record a no-call record (three spellings) that the parser must drop.
+    Returns the number of no-call records written."""
+    with np.errstate(divide="ignore"):
+        pl = np.rint(-10.0 * np.log(g["wei"])).astype(np.int64)
+    dp = g["dp"].astype(np.int64)
+    no_calls = ["./.:0,0:0:.:.", ".|.:.:.:.:.", "."]
+    dropped = 0
+    with open(path, "w") as fh:
+        fh.write("##fileformat=VCFv4.2\n"
+                 "##INFO=<ID=DP,Number=1,Type=Integer,Description=\"Approximate read depth\">\n"
+                 "##FORMAT=<ID=GT,Number=1,Type=String,Description=\"Genotype\">\n"
+                 "##FORMAT=<ID=AD,Number=R,Type=Integer,Description=\"Allelic depths\">\n"
+                 "##FORMAT=<ID=DP,Number=1,Type=Integer,Description=\"Read depth\">\n"
+                 "##FORMAT=<ID=GQ,Number=1,Type=Integer,Description=\"Genotype quality\">\n"
+                 "##FORMAT=<ID=PL,Number=G,Type=Integer,Description=\"Phred-scaled genotype likelihoods\">\n"
+                 "#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\t701_501\n")
+        n = len(g["pos"])
+        for i in range(n):
+            c, p = str(g["chrs"][i]), int(g["pos"][i])
+            fh.write("%s\t%d\t.\tA\tT\t.\t.\tDP=%d\tGT:AD:DP:GQ:PL\t%s:.:%d:.:%d,%d,%d\n" % (c, p, dp[i], g["gt"][i], dp[i], *pl[i]))
+            nxt = (str(g["chrs"][i + 1]), int(g["pos"][i + 1])) if i + 1 < n else None
+            if i % 3 == 2 and nxt != (c, p + 1):
+                fh.write("%s\t%d\t.\tA\tT\t.\t.\tDP=0\tGT:AD:DP:GQ:PL\t%s\n" % (c, p + 1, no_calls[dropped % 3]))
+                dropped += 1
+    return dropped
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SAMPLES), reason="reference sample files are only in the build container")
 def test_parsers_on_the_reference_sample_files(tmp_path, golden_outputs):
-    import shutil
+    """VCF and BED readers on the records of the reference's sample file, against the reference's own parse of it."""
     from snpmatch_b200.core import parsers
-    vcf = tmp_path / "701_501.filter.vcf"
-    bed = tmp_path / "701_502.filter.bed"
-    shutil.copy(os.path.join(REF_SAMPLES, "701_501.filter.vcf"), vcf)      # the parser writes next to its input
-    shutil.copy(os.path.join(REF_SAMPLES, "701_502.filter.bed"), bed)
+    g = load_golden("vcf701_sample.npz")
+    vcf = tmp_path / "701_501.filter.vcf"                                    # the parser writes next to its input
+    bed = tmp_path / "701_501.filter.bed"
+    assert _write_sample_vcf(str(vcf), g) > 2000
     v = parsers.ParseInputs(str(vcf))
     facts = golden_outputs["facts"]
     assert len(v.chrs) == 7545 == facts["vcf_kept"]                          # tests/test_inbred.py:9-12
     assert v.chrs[0] == "Chr1" and v.gt[0] == "0/0" and int(v.pos[0]) == 13226
     np.testing.assert_allclose(v.wei.sum(axis=0), [6582.58869952, 3247.44885746, 903.85454402], rtol=1e-9)
     np.testing.assert_allclose(v.wei[0], [1.0, 0.40656966, 1.66585811e-04], rtol=1e-7)
-    g = load_golden("vcf701_sample.npz")
     assert np.array_equal(v.pos, g["pos"]) and np.array_equal(v.wei, g["wei"]) and np.array_equal(v.gt, g["gt"])
+    assert np.array_equal(v.chrs, g["chrs"]) and np.array_equal(v.dp, g["dp"])
+    np.testing.assert_allclose(parsers.mean_depth(v.dp), facts["vcf_dp_mean"], rtol=1e-12)
+    # the same records as a three-column BED with bare chromosome numbers (the layout of the reference's 701_502.filter.bed)
+    chrs = np.char.replace(g["chrs"], "Chr", "")
+    with open(str(bed), "w") as fh:
+        fh.writelines("%s\t%d\t%s\n" % r for r in zip(chrs, g["pos"], g["gt"]))
     b = parsers.ParseInputs(str(bed))
-    assert len(b.chrs) == 10000 and b.chrs[0] == "1" and b.gt[0] == "0/0" and int(b.pos[1]) == 51103   # tests/test_inbred.py:14-18
+    assert len(b.chrs) == 7545 and b.chrs[0] == "1" and b.gt[0] == "0/0" and int(b.pos[1]) == 21006
+    assert np.array_equal(b.chrs, chrs) and np.array_equal(b.pos, g["pos"]) and np.array_equal(b.gt, g["gt"])
+    assert np.array_equal(b.wei, parsers.ParseInputs.get_wei_from_GT(g["gt"])) and b.wei.sum() == 7545
     assert os.path.isfile(str(bed) + ".snpmatch.npz") and os.path.isfile(str(bed) + ".snpmatch.stats.json")
     again = parsers.ParseInputs(str(bed))                                    # npz cache path
     assert np.array_equal(again.pos, b.pos) and np.array_equal(again.wei, b.wei)
