@@ -274,11 +274,13 @@ int snpm_score(snpm_db *db, const int32_t *s_chrom_id, const int32_t *s_pos, con
 
 /* ---- A5+A6: CrossIdentifier.window_genotyper ----------------------------------------------
  * Replaces csmatch.py:64-104 + get_window_data (:44-61) + genomes.get_bins_* (genomes.py:73-127)
- * for sample 0 of the batch.  Per database chromosome c: win_count[c] windows of bin_len bp
+ * for every sample of the batch (S >= 1).  Per database chromosome c: win_count[c] windows of bin_len bp
  * (0 when the chromosome is not in the genome JSON), first global window number win_off[c]
- * (0-based, in genome-JSON order).  n_windows = total.  kmax int32[kmax_len]: identity table,
+ * (0-based, in genome-JSON order).  n_windows = W = total per sample; window w of sample s sits in
+ * slot s*W + w of every per-window array below.  kmax int32[kmax_len]: identity table,
  * identical <=> floor(n - x - 1) + 1 <= kmax[n] (built by the host with scipy.stats.binom.sf,
- * snpmatch.py:57-72).  Device work is queued; fetch waits. */
+ * snpmatch.py:57-72).  Per sample, every result equals a run of that sample alone; totals (snpm_batch_fetch)
+ * hold one row per sample, m = matched markers inside the sample's windows.  Device work is queued; fetch waits. */
 int snpm_batch_run_windows(snpm_batch *b, int skip_db_hets, int64_t bin_len,
                            const int32_t *win_count, const int32_t *win_off, int32_t n_windows,
                            const int32_t *kmax, int64_t kmax_len, double lr_thres);
@@ -289,22 +291,22 @@ int snpm_batch_run_windows(snpm_batch *b, int skip_db_hets, int64_t bin_len,
  * two ranks contribute); _finish unpacks the sums and runs totals, per-window likelihoods, identity calls and the compaction on
  * them.  Fetches then return the window rows of ALL ranks' markers; matched_s_idx stays this rank's (the caller concatenates).
  * fp64 window scores of the boundary windows are sums of two in-order partial sums (last bits may differ from the reference's
- * single in-order sum; integers do not). */
+ * single in-order sum; integers do not).  Single-sample batches only. */
 int snpm_batch_run_windows_begin(snpm_batch *b, int skip_db_hets, int64_t bin_len, const int32_t *win_count, const int32_t *win_off,
                                  int32_t n_windows, const int32_t *kmax, int64_t kmax_len, double lr_thres, void **dev_ptr,
                                  int64_t *n_doubles);
 int snpm_batch_run_windows_finish(snpm_batch *b);
-/* win_score f64[W,A], win_ninfo int32[W,A], win_L f64[W,A], win_LR f64[W,A],
- * win_identical uint8[W,A], win_num_amb int32[W], win_nrows int32[W] (matched markers per window),
- * matched_s_idx int64[capacity] in window order (matchedTarInd, csmatch.py:90) with *n_matched;
- * totals come from snpm_batch_fetch. */
+/* With SW = S * W window slots: win_score f64[SW,A], win_ninfo int32[SW,A], win_L f64[SW,A], win_LR f64[SW,A],
+ * win_identical uint8[SW,A], win_num_amb int32[SW], win_nrows int32[SW] (matched markers per window),
+ * matched_s_idx int64[capacity] in slot order (matchedTarInd, csmatch.py:90: sample 0's windows, then sample 1's, ...;
+ * indices into the concatenated upload) with *n_matched; totals come from snpm_batch_fetch. */
 int snpm_batch_fetch_windows(snpm_batch *b, double *win_score, int32_t *win_ninfo, double *win_L, double *win_LR,
                              uint8_t *win_identical, int32_t *win_num_amb, int32_t *win_nrows,
                              int64_t *matched_s_idx, int64_t capacity, int64_t *n_matched);
 /* The rows of windowscore.txt exactly as the reference keeps them (get_window_data, csmatch.py:57-60), compacted on the
  * device: for every window with 1 <= num_amb < n_acc its accessions with LR < lr_thres, in accession order.
- * win_row_off int32 [W+1] cuts the row arrays (accession index, float score, informative sites, likelihood, identity
- * call) into windows; win_num_amb / win_nrows int32 [W] and matched_s_idx as in snpm_batch_fetch_windows.  capacity in
+ * win_row_off int32 [S*W+1] cuts the row arrays (accession index, float score, informative sites, likelihood, identity
+ * call) into window slots; win_num_amb / win_nrows int32 [S*W] and matched_s_idx as in snpm_batch_fetch_windows.  capacity in
  * rows, *n_rows receives the row count (call with NULL row arrays to learn it).  A few KB instead of the 21 bytes x W x A of
  * the full arrays cross the bus. */
 int snpm_batch_fetch_window_rows(snpm_batch *b, int32_t *win_row_off, int32_t *win_num_amb, int32_t *win_nrows,
@@ -313,9 +315,10 @@ int snpm_batch_fetch_window_rows(snpm_batch *b, int32_t *win_row_off, int32_t *w
                                  int64_t matched_capacity, int64_t *n_matched);
 
 /* ---- A7: simulated F1 pass ----------------------------------------------------------------
- * Replaces the loop body of CrossIdentifier.match_insilico_f1s (csmatch.py:115-126) for sample 0
- * of the batch over its whole-genome join: all n_top*(n_top-1)/2 pairs (i<j in list order) of the
- * given accession columns.  pair_score f64[P], pair_ninfo int64[P]. */
+ * Replaces the loop body of CrossIdentifier.match_insilico_f1s (csmatch.py:115-126) for every sample
+ * of the batch over its whole-genome join: all P = n_top*(n_top-1)/2 pairs (i<j in list order) of the
+ * sample's accession columns.  acc_idx int32[S, n_top] row-major, pair_score f64[S, P], pair_ninfo int64[S, P];
+ * a sample's sums are the ones a single-sample batch of it gives, bit for bit. */
 int snpm_batch_f1_pairs(snpm_batch *b, const int32_t *acc_idx, int32_t n_top,
                         double *pair_score, int64_t *pair_ninfo);
 

@@ -46,9 +46,41 @@ def snpmatch_inbred(args):
 
 
 def snpmatch_cross(args):
+    if args.get('samples'):
+        samples = read_sample_list(args['samples'], args['outFile'])
+        from .core import csmatch
+        csmatch.potatoCrossIdentifierMany(args, samples)
+        return
     check_file(args['inFile'])
     from .core import csmatch
     csmatch.potatoCrossIdentifier(args)
+
+
+def read_sample_list(list_file, out_prefix):
+    """`cross --samples`: one sample file per line, optionally a tab and the sample's output prefix (default
+    <out_prefix>.<file name up to its first '.'>).  Blank lines are skipped.  Returns [(path, prefix)]; dies on a missing
+    file, an empty list or two samples with the same prefix."""
+    check_file(list_file)
+    samples = []
+    with open(list_file) as fh:
+        for line in fh:
+            line = line.rstrip("\r\n")
+            if not line.strip():
+                continue
+            cols = line.split("\t")
+            path = cols[0].strip()
+            prefix = cols[1].strip() if len(cols) > 1 and cols[1].strip() else out_prefix + "." + os.path.basename(path).split(".")[0]
+            samples.append((path, prefix))
+    if not samples:
+        die("sample list is empty: " + list_file)
+    for path, _ in samples:
+        check_file(path)
+    seen = {}
+    for path, prefix in samples:
+        if prefix in seen:
+            die("samples %s and %s have the same output prefix %s" % (seen[prefix], path, prefix))
+        seen[prefix] = path
+    return samples
 
 
 def snpmatch_parser(args):
@@ -100,7 +132,11 @@ def get_options(description, version_message):
     inbred.set_defaults(func=snpmatch_inbred)
 
     cross = sub.add_parser('cross', help="identify the parents of a cross (F2, F3): window scores and simulated F1s")
-    cross.add_argument("-i", "--input_file", dest="inFile", help="sample variants: VCF (GT, optional PL), BED (chr, pos, GT) or a parser .npz")
+    cross_in = cross.add_mutually_exclusive_group()
+    cross_in.add_argument("-i", "--input_file", dest="inFile", help="sample variants: VCF (GT, optional PL), BED (chr, pos, GT) or a parser .npz")
+    cross_in.add_argument("--samples", dest="samples", default=None,
+                          help="text file listing many samples, one path per line (VCF/BED/npz), optionally a tab and that sample's output "
+                               "prefix (default <-o>.<file name up to its first '.'>); all samples are scored together on the GPU")
     cross.add_argument("-d", "--hdf5_file", default=None, dest="hdf5File", help=db_help)
     cross.add_argument("-e", "--hdf5_acc_file", default=None, dest="hdf5accFile", help="Column-chunked hdf5 file of the reference (accepted for compatibility)")
     cross.add_argument("-b", "--binLength", dest="binLen", help="window length in bp", default=300000, type=int)

@@ -1991,32 +1991,35 @@ int snpm_score_shared_panel(snpm_db *db, const int64_t *panel_rows, int64_t K, c
 }
 
 // ---- A5 + A6 ----------------------------------------------------------------------------------------
-// phase 1 of `cross` on this device's rows: join, window bounds, one order-exact segment per window
+// phase 1 of `cross` on this device's rows: join, window bounds, one order-exact segment per window of every sample
+// (window w of sample s in slot s*W + w)
 static int windows_begin(snpm_batch *b, int skip_db_hets, int64_t bin_len, const int32_t *win_count, const int32_t *win_off,
                          int32_t n_windows, const int32_t *kmax, int64_t kmax_len, double lr_thres) {
     if (!b || bin_len <= 0 || n_windows < 0 || !win_count || !win_off || !kmax || kmax_len < 1)
         return fail(SNPM_E_ARG, "snpm_batch_run_windows: bad arguments");
-    if (b->S != 1) return fail(SNPM_E_ARG, "snpm_batch_run_windows: windows are scored for a single-sample batch");
+    if (b->S < 1) return fail(SNPM_E_ARG, "snpm_batch_run_windows: the batch holds no sample");
+    if (b->S * int64_t(n_windows) > INT32_MAX / 2)
+        return fail(SNPM_E_ARG, "snpm_batch_run_windows: %lld samples x %d windows is too many window slots for one run", (long long)b->S, n_windows);
     if (b->grouped) return fail(SNPM_E_STATE, "snpm_batch_run_windows: windows need the batch in position order (snpm_batch_upload)");
     snpm_db *db = b->db;
     SNPM_CUDA(cudaSetDevice(db->device));
     cudaStream_t st = db->stream;
-    const int32_t W = n_windows;
+    const int32_t W = n_windows, SW = int32_t(b->S) * n_windows;
     b->launches = 0;
     for (int i = 0; i < SNPM_N_EVENTS; ++i) b->ev_rec[i] = false;
-    SNPM_TRY(batch_alloc_outputs(b, std::max<int64_t>(W, 1)));
-    const size_t WA = size_t(std::max(W, 1)) * db->n_acc;
+    SNPM_TRY(batch_alloc_outputs(b, std::max<int64_t>(SW, 1)));
+    const size_t WA = size_t(std::max(SW, 1)) * db->n_acc;
     SNPM_TRY(b->d_win_count.ensure(size_t(std::max(db->n_chr, 1)) * 4));
     SNPM_TRY(b->d_win_off.ensure(size_t(std::max(db->n_chr, 1)) * 4));
-    SNPM_TRY(b->d_win_begin.ensure(size_t(std::max(W, 1)) * 4));
-    SNPM_TRY(b->d_win_end.ensure(size_t(std::max(W, 1)) * 4));
-    SNPM_TRY(b->d_win_nrows.ensure(size_t(std::max(W, 1)) * 4));
-    SNPM_TRY(b->d_win_zero.ensure(size_t(std::max(W, 1)) * 4));
+    SNPM_TRY(b->d_win_begin.ensure(size_t(std::max(SW, 1)) * 4));
+    SNPM_TRY(b->d_win_end.ensure(size_t(std::max(SW, 1)) * 4));
+    SNPM_TRY(b->d_win_nrows.ensure(size_t(std::max(SW, 1)) * 4));
+    SNPM_TRY(b->d_win_zero.ensure(size_t(std::max(SW, 1)) * 4));
     SNPM_TRY(b->d_kmax.ensure(size_t(kmax_len) * 4));
     SNPM_TRY(b->d_win_L.ensure(WA * 8));
     SNPM_TRY(b->d_win_LR.ensure(WA * 8));
     SNPM_TRY(b->d_win_ident.ensure(WA));
-    SNPM_TRY(b->d_win_amb.ensure(size_t(std::max(W, 1)) * 4));
+    SNPM_TRY(b->d_win_amb.ensure(size_t(std::max(SW, 1)) * 4));
     if (db->n_chr) {
         SNPM_CUDA(cudaMemcpyAsync(b->d_win_count.p, win_count, size_t(db->n_chr) * 4, cudaMemcpyHostToDevice, st));
         SNPM_CUDA(cudaMemcpyAsync(b->d_win_off.p, win_off, size_t(db->n_chr) * 4, cudaMemcpyHostToDevice, st));
@@ -2025,16 +2028,16 @@ static int windows_begin(snpm_batch *b, int skip_db_hets, int64_t bin_len, const
     b->kmax_len = kmax_len;
     rec(b, SNPM_EV_START);
     SNPM_TRY(batch_join(b, 0));
-    SNPM_CUDA(cudaMemsetAsync(b->d_win_begin.p, 0, size_t(std::max(W, 1)) * 4, st));
-    SNPM_CUDA(cudaMemsetAsync(b->d_win_end.p, 0, size_t(std::max(W, 1)) * 4, st));
-    SNPM_CUDA(cudaMemsetAsync(b->d_win_zero.p, 0, size_t(std::max(W, 1)) * 4, st));
-    SNPM_CUDA(cudaMemsetAsync(b->d_win_nrows.p, 0, size_t(std::max(W, 1)) * 4, st));
+    SNPM_CUDA(cudaMemsetAsync(b->d_win_begin.p, 0, size_t(std::max(SW, 1)) * 4, st));
+    SNPM_CUDA(cudaMemsetAsync(b->d_win_end.p, 0, size_t(std::max(SW, 1)) * 4, st));
+    SNPM_CUDA(cudaMemsetAsync(b->d_win_zero.p, 0, size_t(std::max(SW, 1)) * 4, st));
+    SNPM_CUDA(cudaMemsetAsync(b->d_win_nrows.p, 0, size_t(std::max(SW, 1)) * 4, st));
     if (b->n > 0 && W > 0) {
-        k_window_bounds<<<int(ceil_div64(b->n, 256)), 256, 0, st>>>(b->d_pair_s.as<int32_t>(), b->d_prefix.as<int32_t>() + b->n,
+        k_window_bounds<<<int(ceil_div64(b->n, 256)), 256, 0, st>>>(b->d_pair_s.as<int32_t>(), b->d_mstart.as<int32_t>(), int32_t(b->S), W,
                                                                  b->d_chrom.as<int32_t>(), b->d_pos.as<int32_t>(), b->d_win_count.as<int32_t>(),
                                                                  b->d_win_off.as<int32_t>(), bin_len, b->d_win_begin.as<int32_t>(),
                                                                  b->d_win_end.as<int32_t>());
-        k_window_nrows<<<(W + 255) / 256, 256, 0, st>>>(b->d_win_begin.as<int32_t>(), b->d_win_end.as<int32_t>(), W, b->d_win_nrows.as<int32_t>());
+        k_window_nrows<<<(SW + 255) / 256, 256, 0, st>>>(b->d_win_begin.as<int32_t>(), b->d_win_end.as<int32_t>(), SW, b->d_win_nrows.as<int32_t>());
         SNPM_KERNEL_CHECK();
         b->launches += 2;
     }
@@ -2045,14 +2048,14 @@ static int windows_begin(snpm_batch *b, int skip_db_hets, int64_t bin_len, const
     a.pair_db = b->d_pair_db.as<int32_t>();
     a.pair_w = b->d_pair_w.as<double>();
     a.table = 1;
-    a.nseg = W;
+    a.nseg = SW;
     a.seg_begin = b->d_win_begin.as<int32_t>();
     a.seg_end = b->d_win_end.as<int32_t>();
     a.part_score = b->d_part_score.as<double>();
     a.part_ninfo = b->d_part_ninfo.as<int32_t>();
     a.a_pad = db->stride * 32;
-    SNPM_TRY(launch_score(st, a, W, skip_db_hets != 0));
-    if (W > 0) b->launches += 1;
+    SNPM_TRY(launch_score(st, a, SW, skip_db_hets != 0));
+    if (SW > 0) b->launches += 1;
     rec(b, SNPM_EV_SCORE);
     b->n_windows = W;
     b->bin_len = bin_len;
@@ -2067,32 +2070,33 @@ static int windows_begin(snpm_batch *b, int skip_db_hets, int64_t bin_len, const
 static int windows_finish(snpm_batch *b) {
     snpm_db *db = b->db;
     cudaStream_t st = db->stream;
-    const int32_t W = b->n_windows;
-    const size_t WA = size_t(std::max(W, 1)) * db->n_acc;
+    const int32_t W = b->n_windows, SW = int32_t(b->S) * W;
+    const size_t WA = size_t(std::max(SW, 1)) * db->n_acc;
     const int32_t a_pad = db->stride * 32;
     const double *part_score = b->d_part_score.as<double>();
     const int32_t *part_ninfo = b->d_part_ninfo.as<int32_t>();
     const int32_t *zero = b->d_win_zero.as<int32_t>(), *nrows = b->d_win_nrows.as<int32_t>();
-    dim3 cgrid((db->n_acc + 31) / 32, 1);
+    // per sample: totals over its W windows in window order; m = the pairs inside its windows (sum of the rows per window)
+    dim3 cgrid((db->n_acc + 31) / 32, unsigned(b->S));
     k_combine<<<cgrid, 32, 0, st>>>(part_score, part_ninfo, a_pad, db->n_acc, nullptr, nullptr, W, zero, nrows, b->d_red.as<double>());
     SNPM_KERNEL_CHECK();
     b->launches += 1;
-    if (W > 0) {
-        k_window_epilogue<<<W, 256, 0, st>>>(part_score, part_ninfo, a_pad, db->n_acc, zero, nrows, b->d_kmax.as<int32_t>(), b->kmax_len,
+    if (SW > 0) {
+        k_window_epilogue<<<SW, 256, 0, st>>>(part_score, part_ninfo, a_pad, db->n_acc, zero, nrows, b->d_kmax.as<int32_t>(), b->kmax_len,
                                              b->lr_thres, b->d_win_L.as<double>(), b->d_win_LR.as<double>(), b->d_win_ident.as<uint8_t>(),
                                              b->d_win_amb.as<int32_t>(), b->d_status.as<int>());
         SNPM_KERNEL_CHECK();
         b->launches += 1;
         // the rows the reference keeps, compacted on the device (what snpm_batch_fetch_window_rows reads back)
-        SNPM_TRY(b->d_win_row_off.ensure(size_t(W + 1) * 4));
+        SNPM_TRY(b->d_win_row_off.ensure(size_t(SW + 1) * 4));
         SNPM_TRY(b->d_row_acc.ensure(WA * 4));
         SNPM_TRY(b->d_row_score.ensure(WA * 8));
         SNPM_TRY(b->d_row_ninfo.ensure(WA * 4));
         SNPM_TRY(b->d_row_L.ensure(WA * 8));
         SNPM_TRY(b->d_row_ident.ensure(WA));
-        k_window_row_offsets<<<1, 1024, 0, st>>>(b->d_win_amb.as<int32_t>(), W, db->n_acc, b->d_win_row_off.as<int32_t>());
+        k_window_row_offsets<<<1, 1024, 0, st>>>(b->d_win_amb.as<int32_t>(), SW, db->n_acc, b->d_win_row_off.as<int32_t>());
         SNPM_KERNEL_CHECK();
-        k_window_compact<<<W, 256, 0, st>>>(part_score, part_ninfo, a_pad, db->n_acc, b->d_win_L.as<double>(), b->d_win_LR.as<double>(),
+        k_window_compact<<<SW, 256, 0, st>>>(part_score, part_ninfo, a_pad, db->n_acc, b->d_win_L.as<double>(), b->d_win_LR.as<double>(),
                                             b->d_win_ident.as<uint8_t>(), b->d_win_row_off.as<int32_t>(), b->lr_thres, b->d_row_acc.as<int32_t>(),
                                             b->d_row_score.as<double>(), b->d_row_ninfo.as<int32_t>(), b->d_row_L.as<double>(),
                                             b->d_row_ident.as<uint8_t>());
@@ -2118,6 +2122,7 @@ int snpm_batch_run_windows(snpm_batch *b, int skip_db_hets, int64_t bin_len, con
 int snpm_batch_run_windows_begin(snpm_batch *b, int skip_db_hets, int64_t bin_len, const int32_t *win_count, const int32_t *win_off,
                                  int32_t n_windows, const int32_t *kmax, int64_t kmax_len, double lr_thres, void **dev_ptr, int64_t *n_doubles) {
     if (!dev_ptr || !n_doubles) return fail(SNPM_E_ARG, "snpm_batch_run_windows_begin: NULL output");
+    if (b && b->S != 1) return fail(SNPM_E_ARG, "snpm_batch_run_windows_begin: windows on a sharded panel are scored for a single-sample batch");
     SNPM_TRY(windows_begin(b, skip_db_hets, bin_len, win_count, win_off, n_windows, kmax, kmax_len, lr_thres));
     snpm_db *db = b->db;
     const int64_t cells = int64_t(std::max(n_windows, 1)) * db->stride * 32;
@@ -2151,7 +2156,7 @@ int snpm_batch_fetch_windows(snpm_batch *b, double *win_score, int32_t *win_ninf
     snpm_db *db = b->db;
     SNPM_CUDA(cudaSetDevice(db->device));
     cudaStream_t st = db->stream;
-    const size_t W = size_t(b->n_windows), A = size_t(db->n_acc), a_pad = size_t(db->stride) * 32;
+    const size_t W = size_t(b->S) * size_t(b->n_windows), A = size_t(db->n_acc), a_pad = size_t(db->stride) * 32;     // all window slots
     std::vector<int32_t> wb(W + 1), we(W + 1), nr(W + 1), ps;
     if (W) {
         if (win_score) SNPM_CUDA(cudaMemcpy2DAsync(win_score, A * 8, b->d_part_score.p, a_pad * 8, A * 8, W, cudaMemcpyDeviceToHost, st));
@@ -2198,7 +2203,7 @@ int snpm_batch_fetch_window_rows(snpm_batch *b, int32_t *win_row_off, int32_t *w
     snpm_db *db = b->db;
     SNPM_CUDA(cudaSetDevice(db->device));
     cudaStream_t st = db->stream;
-    const size_t W = size_t(b->n_windows);
+    const size_t W = size_t(b->S) * size_t(b->n_windows);      // all window slots
     std::vector<int32_t> off(W + 1, 0), wb(W + 1), we(W + 1), nr(W + 1), ps;
     if (W) {
         SNPM_CUDA(cudaMemcpyAsync(off.data(), b->d_win_row_off.p, (W + 1) * 4, cudaMemcpyDeviceToHost, st));
@@ -2245,32 +2250,38 @@ int snpm_batch_fetch_window_rows(snpm_batch *b, int32_t *win_row_off, int32_t *w
 int snpm_batch_f1_pairs(snpm_batch *b, const int32_t *acc_idx, int32_t n_top, double *pair_score, int64_t *pair_ninfo) {
     if (!b || !acc_idx || n_top < 2 || n_top > 4096 || !pair_score || !pair_ninfo) return fail(SNPM_E_ARG, "snpm_batch_f1_pairs: bad arguments");
     if (!b->ran) return fail(SNPM_E_STATE, "snpm_batch_f1_pairs: run the batch first");
-    if (b->S != 1) return fail(SNPM_E_ARG, "snpm_batch_f1_pairs: single-sample batch expected");
+    if (b->S < 1 || b->S > 65535) return fail(SNPM_E_ARG, "snpm_batch_f1_pairs: %lld samples (1 to 65535 per call)", (long long)b->S);
     if (b->grouped) return fail(SNPM_E_STATE, "snpm_batch_f1_pairs: needs the batch in position order (snpm_batch_upload)");
     snpm_db *db = b->db;
-    for (int i = 0; i < n_top; ++i)
-        if (acc_idx[i] < 0 || acc_idx[i] >= db->n_acc) return fail(SNPM_E_ARG, "snpm_batch_f1_pairs: accession index %d out of range", acc_idx[i]);
+    const int64_t S = b->S, SK = S * n_top;
+    for (int64_t i = 0; i < SK; ++i)
+        if (acc_idx[i] < 0 || acc_idx[i] >= db->n_acc)
+            return fail(SNPM_E_ARG, "snpm_batch_f1_pairs: accession index %d of sample %lld out of range", acc_idx[i], (long long)(i / n_top));
     SNPM_CUDA(cudaSetDevice(db->device));
     cudaStream_t st = db->stream;
     const int n_pairs = n_top * (n_top - 1) / 2;
-    const int n_blocks = int(std::max<int64_t>(1, ceil_div64(b->n, F1_ROWS_PER_BLOCK)));
-    SNPM_TRY(b->d_f1_acc.ensure(size_t(n_top) * 4));
-    SNPM_TRY(b->d_f1_part.ensure(size_t(n_pairs) * n_blocks * 32));
-    SNPM_TRY(b->d_f1_out.ensure(size_t(n_pairs) * 16));
-    SNPM_CUDA(cudaMemcpyAsync(b->d_f1_acc.p, acc_idx, size_t(n_top) * 4, cudaMemcpyHostToDevice, st));
-    dim3 grid(n_blocks, n_pairs);
+    const size_t SP = size_t(S) * size_t(n_pairs);
+    // row blocks of the largest sample (a sample's matched pairs never outnumber its markers); the other samples' surplus blocks add zeros
+    int64_t n_max = 0;
+    for (int64_t s = 0; s < S; ++s) n_max = std::max(n_max, b->h_off[size_t(s) + 1] - b->h_off[size_t(s)]);
+    const int n_blocks = int(std::max<int64_t>(1, ceil_div64(n_max, F1_ROWS_PER_BLOCK)));
+    SNPM_TRY(b->d_f1_acc.ensure(size_t(SK) * 4));
+    SNPM_TRY(b->d_f1_part.ensure(SP * n_blocks * 32));
+    SNPM_TRY(b->d_f1_out.ensure(SP * 16));
+    SNPM_CUDA(cudaMemcpyAsync(b->d_f1_acc.p, acc_idx, size_t(SK) * 4, cudaMemcpyHostToDevice, st));
+    dim3 grid(n_blocks, n_pairs, unsigned(S));
     k_f1_partial<<<grid, F1_THREADS, 0, st>>>(db->d_packed, db->stride, b->d_pair_db.as<int32_t>(), b->d_pair_w.as<double>(),
-                                              b->d_prefix.as<int32_t>() + b->n, b->d_f1_acc.as<int32_t>(), n_top, b->d_f1_part.as<double>());
+                                              b->d_mstart.as<int32_t>(), b->d_f1_acc.as<int32_t>(), n_top, b->d_f1_part.as<double>());
     SNPM_KERNEL_CHECK();
-    k_f1_final<<<(n_pairs + 127) / 128, 128, 0, st>>>(b->d_f1_part.as<double>(), n_blocks, n_pairs, b->d_f1_out.as<double>());
+    k_f1_final<<<int((SP + 127) / 128), 128, 0, st>>>(b->d_f1_part.as<double>(), n_blocks, int(SP), b->d_f1_out.as<double>());
     SNPM_KERNEL_CHECK();
     b->launches += 2;
-    std::vector<double> out(size_t(n_pairs) * 2);
-    SNPM_CUDA(cudaMemcpyAsync(out.data(), b->d_f1_out.p, size_t(n_pairs) * 16, cudaMemcpyDeviceToHost, st));
+    std::vector<double> out(SP * 2);
+    SNPM_CUDA(cudaMemcpyAsync(out.data(), b->d_f1_out.p, SP * 16, cudaMemcpyDeviceToHost, st));
     SNPM_CUDA(cudaStreamSynchronize(st));
-    for (int p = 0; p < n_pairs; ++p) {
-        pair_score[p] = out[size_t(2 * p)];
-        pair_ninfo[p] = int64_t(out[size_t(2 * p + 1)]);
+    for (size_t p = 0; p < SP; ++p) {
+        pair_score[p] = out[2 * p];
+        pair_ninfo[p] = int64_t(out[2 * p + 1]);
     }
     return SNPM_OK;
 }

@@ -17,10 +17,13 @@ __device__ __forceinline__ uint32_t code_at(const uint64_t *__restrict__ rowp, i
     return lo | (hi << 1);
 }
 
-// grid (row blocks, pairs); partial[pair][block] = (sum_alt, sum_ref, sum_het, count)
+// grid (row blocks, pairs, samples); partial[sample][pair][block] = (sum_alt, sum_ref, sum_het, count).  Sample s owns the
+// matched pairs [mstart[s], mstart[s+1]) and the accession list acc_idx[s * n_top ...]; its row blocks start at its first pair,
+// so a sample's sums do not depend on the other samples of the batch.  Blocks past a sample's pairs write zeros (the grid is
+// sized for the largest sample).
 __global__ void __launch_bounds__(F1_THREADS) k_f1_partial(const uint64_t *__restrict__ packed, int32_t stride,
                                                            const int32_t *__restrict__ pair_db, const double *__restrict__ pair_w,
-                                                           const int32_t *__restrict__ m_ptr, const int32_t *__restrict__ acc_idx,
+                                                           const int32_t *__restrict__ mstart, const int32_t *__restrict__ acc_idx,
                                                            int32_t n_top, double *__restrict__ partial) {
     __shared__ double s_sum[3][F1_THREADS / 32];
     __shared__ long long s_cnt[F1_THREADS / 32];
@@ -28,9 +31,10 @@ __global__ void __launch_bounds__(F1_THREADS) k_f1_partial(const uint64_t *__res
     int pi = blockIdx.y, i = 0;
     while (pi >= n_top - 1 - i) { pi -= n_top - 1 - i; ++i; }
     const int j = i + 1 + pi;
-    const int32_t a1 = acc_idx[i], a2 = acc_idx[j];
-    const int64_t m = *m_ptr;
-    const int64_t r0 = int64_t(blockIdx.x) * F1_ROWS_PER_BLOCK;
+    const int s = blockIdx.z;
+    const int32_t a1 = acc_idx[int64_t(s) * n_top + i], a2 = acc_idx[int64_t(s) * n_top + j];
+    const int64_t m = mstart[s + 1];
+    const int64_t r0 = mstart[s] + int64_t(blockIdx.x) * F1_ROWS_PER_BLOCK;
     const int64_t r1 = min(m, r0 + F1_ROWS_PER_BLOCK);
     double alt = 0.0, ref = 0.0, het = 0.0;
     long long cnt = 0;
@@ -57,12 +61,13 @@ __global__ void __launch_bounds__(F1_THREADS) k_f1_partial(const uint64_t *__res
         double A = 0.0, R = 0.0, H = 0.0;
         long long C = 0;
         for (int k = 0; k < F1_THREADS / 32; ++k) { A += s_sum[0][k]; R += s_sum[1][k]; H += s_sum[2][k]; C += s_cnt[k]; }
-        double *o = partial + (int64_t(blockIdx.y) * gridDim.x + blockIdx.x) * 4;
+        double *o = partial + ((int64_t(s) * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * 4;
         o[0] = A; o[1] = R; o[2] = H; o[3] = double(C);
     }
 }
 
-// one thread per pair sums the block partials in order: out[pair] = (score, count)
+// one thread per (sample, pair) sums the block partials in order: out[sample][pair] = (score, count); n_pairs here counts the
+// pairs of all samples
 __global__ void k_f1_final(const double *__restrict__ partial, int n_blocks, int n_pairs, double *__restrict__ out) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n_pairs) return;

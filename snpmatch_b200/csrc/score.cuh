@@ -370,8 +370,9 @@ __global__ void __launch_bounds__(256) k_combine(const double *__restrict__ part
                                                  double *__restrict__ red) {
     const int s = blockIdx.y;
     const int acc = blockIdx.x * blockDim.x + threadIdx.x;
+    // without seg_off the segments are windows: sample s owns the slots [s * nseg_table, (s+1) * nseg_table)
     int j0, j1;
-    if (seg_off) { j0 = seg_off[s]; j1 = seg_off[s + 1]; } else { j0 = 0; j1 = nseg_table; }
+    if (seg_off) { j0 = seg_off[s]; j1 = seg_off[s + 1]; } else { j0 = s * nseg_table; j1 = j0 + nseg_table; }
     double *row = red + int64_t(s) * (2 * int64_t(n_acc) + 2);
     if (acc < n_acc) {
         double tot = 0.0;
@@ -403,7 +404,7 @@ __global__ void __launch_bounds__(256) k_combine(const double *__restrict__ part
     if (acc == 0) {
         long long m = 0;
         if (seg_off) m = mstart[s + 1] - mstart[s];
-        else for (int j = 0; j < nseg_table; ++j) m += seg_end[j] - seg_begin[j];
+        else for (int j = j0; j < j1; ++j) m += seg_end[j] - seg_begin[j];
         row[2 * n_acc] = double(m);
         row[2 * n_acc + 1] = 0.0;
     }

@@ -21,22 +21,29 @@ __device__ __forceinline__ int32_t window_of_pair(const int32_t *__restrict__ pa
     return win_off[c] + int32_t(k);
 }
 
-// matched pairs are ordered by (panel chromosome, position), so the pairs of one window are contiguous:
-// record [begin, end) per window (zero-initialised -> empty windows stay [0,0))
-__global__ void __launch_bounds__(256) k_window_bounds(const int32_t *__restrict__ pair_s, const int32_t *__restrict__ m_ptr,
-                                                       const int32_t *__restrict__ chrom, const int32_t *__restrict__ pos,
+// matched pairs of sample s are [mstart[s], mstart[s+1]), ordered by (panel chromosome, position), so the pairs of one window
+// of one sample are contiguous: record [begin, end) in slot s*W + w (zero-initialised -> empty windows stay [0,0)).  A pair
+// opening a sample never continues the previous pair's window: the previous sample closes its own last window.
+__global__ void __launch_bounds__(256) k_window_bounds(const int32_t *__restrict__ pair_s, const int32_t *__restrict__ mstart, int32_t S,
+                                                       int32_t W, const int32_t *__restrict__ chrom, const int32_t *__restrict__ pos,
                                                        const int32_t *__restrict__ win_count, const int32_t *__restrict__ win_off,
                                                        int64_t bin_len, int32_t *__restrict__ win_begin, int32_t *__restrict__ win_end) {
-    const int64_t m = *m_ptr;
     const int64_t r = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-    if (r >= m) return;
-    const int32_t w = window_of_pair(pair_s, chrom, pos, win_count, win_off, bin_len, r);
-    const int32_t wp = r > 0 ? window_of_pair(pair_s, chrom, pos, win_count, win_off, bin_len, r - 1) : -2;
-    if (w != wp) {
-        if (w >= 0) win_begin[w] = int32_t(r);
-        if (wp >= 0) win_end[wp] = int32_t(r);
+    if (r >= mstart[S]) return;
+    int lo = 0, hi = S;                                   // the sample: last s with mstart[s] <= r (empty samples are skipped)
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (mstart[mid] <= r) lo = mid; else hi = mid;
     }
-    if (r == m - 1 && w >= 0) win_end[w] = int32_t(m);
+    const int64_t first = mstart[lo], last = int64_t(mstart[lo + 1]) - 1;
+    const int64_t slot0 = int64_t(lo) * W;
+    const int32_t w = window_of_pair(pair_s, chrom, pos, win_count, win_off, bin_len, r);
+    const int32_t wp = r > first ? window_of_pair(pair_s, chrom, pos, win_count, win_off, bin_len, r - 1) : -2;
+    if (w != wp) {
+        if (w >= 0) win_begin[slot0 + w] = int32_t(r);
+        if (wp >= 0) win_end[slot0 + wp] = int32_t(r);
+    }
+    if (r == last && w >= 0) win_end[slot0 + w] = int32_t(r + 1);
 }
 
 // rows of every window on this device, and the packing of the per-window partials into ONE f64 buffer for a cross-GPU sum
@@ -123,8 +130,8 @@ __global__ void __launch_bounds__(256) k_window_epilogue(const double *__restric
 
 // ---- compaction of the rows the reference keeps (csmatch.py:57-60) -------------------------------------------------
 // A window contributes its accessions with LR < lr_thres, and only when at least one but not all pass.  win_row_off =
-// exclusive scan of those counts (single CTA); k_window_compact then writes the surviving rows of every window in
-// accession order: accession index, float score, informative sites, likelihood, identity call.
+// exclusive scan of those counts over the S*W window slots (single CTA); k_window_compact then writes the surviving rows of
+// every window in accession order: accession index, float score, informative sites, likelihood, identity call.
 __global__ void __launch_bounds__(1024) k_window_row_offsets(const int32_t *__restrict__ win_amb, int32_t n_windows, int32_t n_acc,
                                                              int32_t *__restrict__ win_row_off) {
     __shared__ int s_warp[33];

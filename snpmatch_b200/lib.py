@@ -742,24 +742,38 @@ class Batch(object):
         check(load().snpm_batch_run_windows_finish(self._h))
 
     def fetch_windows(self):
-        W, A = self.n_windows, self.db.n_acc
-        n = int(self.offsets[1])
-        r = {"score": np.empty((W, A), np.float64), "ninfo": np.empty((W, A), np.int32), "L": np.empty((W, A), np.float64),
-             "LR": np.empty((W, A), np.float64), "identical": np.empty((W, A), np.uint8), "num_amb": np.empty(W, np.int32),
-             "nrows": np.empty(W, np.int32)}
+        """Every window's arrays: score, L, LR f64, ninfo int32, identical uint8 [W, A]; num_amb, nrows int32 [W]; matched_s_idx
+        int64 (the sample's matched markers in window order).  A batch of S > 1 samples gets a leading sample axis ([S, W, A],
+        [S, W]) and matched_s_idx as a list of S arrays (indices into the concatenated upload)."""
+        S, W, A = self.n_samples, self.n_windows, self.db.n_acc
+        SW = S * W
+        n = int(self.offsets[-1])
+        r = {"score": np.empty((SW, A), np.float64), "ninfo": np.empty((SW, A), np.int32), "L": np.empty((SW, A), np.float64),
+             "LR": np.empty((SW, A), np.float64), "identical": np.empty((SW, A), np.uint8), "num_amb": np.empty(SW, np.int32),
+             "nrows": np.empty(SW, np.int32)}
         tar = np.empty(max(n, 1), dtype=np.int64)
         m = C.c_int64(0)
         check(load().snpm_batch_fetch_windows(self._h, ptr(r["score"]), ptr(r["ninfo"]), ptr(r["L"]), ptr(r["LR"]),
                                               ptr(r["identical"]), ptr(r["num_amb"]), ptr(r["nrows"]), ptr(tar), n, C.byref(m)))
-        r["matched_s_idx"] = tar[:m.value].copy()
+        tar = tar[:m.value].copy()
+        if S == 1:
+            r["matched_s_idx"] = tar
+            return r
+        for k in ("score", "ninfo", "L", "LR", "identical"):
+            r[k] = r[k].reshape(S, W, A)
+        r["num_amb"], r["nrows"] = r["num_amb"].reshape(S, W), r["nrows"].reshape(S, W)
+        cut = np.concatenate([[0], np.cumsum(r["nrows"].sum(axis=1, dtype=np.int64))])
+        r["matched_s_idx"] = [tar[cut[i]:cut[i + 1]] for i in range(S)]
         return r
 
     def fetch_window_rows(self):
         """The surviving rows of every window (csmatch.py:57-60), compacted on the device.  Returns dict(row_off int32 [W+1],
         num_amb, nrows int32 [W], acc int32 [R], score f64 [R], ninfo int32 [R], L f64 [R], identical uint8 [R],
-        matched_s_idx)."""
-        W = self.n_windows
-        n = int(self.offsets[1])
+        matched_s_idx).  A batch of S > 1 samples gets a list of S such dicts, one per sample (row_off starting at 0,
+        matched_s_idx indexing the concatenated upload)."""
+        S = self.n_samples
+        W = S * self.n_windows
+        n = int(self.offsets[-1])
         r = {"row_off": np.zeros(W + 1, np.int32), "num_amb": np.zeros(max(W, 1), np.int32), "nrows": np.zeros(max(W, 1), np.int32)}
         tar = np.empty(max(n, 1), dtype=np.int64)
         n_rows, m = C.c_int64(0), C.c_int64(0)
@@ -776,16 +790,34 @@ class Batch(object):
             r[k] = r[k][:R]
         r["num_amb"], r["nrows"] = r["num_amb"][:W], r["nrows"][:W]
         r["matched_s_idx"] = tar[:m.value].copy()
-        return r
+        if S == 1:
+            return r
+        Wn, out, at = self.n_windows, [], 0
+        for i in range(S):
+            lo, hi = i * Wn, (i + 1) * Wn
+            r0, r1 = int(r["row_off"][lo]), int(r["row_off"][hi])
+            nrows = r["nrows"][lo:hi]
+            k = int(nrows.sum(dtype=np.int64))
+            d = {"row_off": r["row_off"][lo:hi + 1] - r0, "num_amb": r["num_amb"][lo:hi], "nrows": nrows,
+                 "matched_s_idx": r["matched_s_idx"][at:at + k]}
+            for key in ("acc", "score", "ninfo", "L", "identical"):
+                d[key] = r[key][r0:r1]
+            out.append(d)
+            at += k
+        return out
 
     def f1_pairs(self, acc_idx):
+        """Simulated F1 sums of the accession pairs (i < j in list order): acc_idx [k] -> (score f64, ninfo int64) [P]; on a batch
+        of S samples acc_idx [S, k] (one list per sample) -> [S, P]."""
         acc_idx = as_c(acc_idx, np.int32)
-        k = len(acc_idx)
+        multi = acc_idx.ndim == 2
+        assert (acc_idx.shape[0] == self.n_samples) if multi else self.n_samples == 1
+        k = acc_idx.shape[-1]
         n_pairs = k * (k - 1) // 2
-        score = np.empty(n_pairs, dtype=np.float64)
-        ninfo = np.empty(n_pairs, dtype=np.int64)
+        score = np.empty((self.n_samples, n_pairs), dtype=np.float64)
+        ninfo = np.empty((self.n_samples, n_pairs), dtype=np.int64)
         check(load().snpm_batch_f1_pairs(self._h, ptr(acc_idx), k, ptr(score), ptr(ninfo)))
-        return score, ninfo
+        return (score, ninfo) if multi else (score[0], ninfo[0])
 
 
 def match_gts_accs(wei, snps, skip_hets_db=False, device=0):
