@@ -112,6 +112,12 @@ int snpm_match_gts_accs(int device, const double *wei, const int8_t *snps, int64
  * (nan when n <= 0).  amin_is_calc != 0 -> nanmin, else use amin.  SNPM_E_ASSERT if any y > n. */
 int snpm_calculate_likelihoods(int device, const double *scores, const double *ninfo, int64_t n_acc,
                                int amin_is_calc, double amin, double *prob, double *L, double *LR);
+/* the same for S tables of K entries in one call (GenotyperOutput.calculate_likelihoods of many `--refine` tables, snpmatch.py:106-117
+ * called from :218-219): scores / ninfo / prob / L / LR f64 [S,K], one nanmin per row.  Rows shorter than K are padded with
+ * ninfo = 0 (L = nan there, which leaves the row's minimum as it is); every row gets the bits snpm_calculate_likelihoods gives
+ * for it alone.  SNPM_E_ASSERT if any y > n. */
+int snpm_calculate_likelihoods_many(int device, const double *scores, const double *ninfo, int64_t S, int64_t K,
+                                    int amin_is_calc, double amin, double *prob, double *L, double *LR);
 
 /* ---- A1+A2+A3+A4: Genotyper.genotyper for one or many samples ------------------------------
  * Replaces Genotyper.genotyper (snpmatch.py:207-233) + GenotyperOutput (:94-120).
@@ -210,6 +216,20 @@ int snpm_batch_destroy(snpm_batch *b);
  * GLOBAL database row is in the sorted list (applies to every sample of the batch).  sorted_rows == NULL clears the filter;
  * a non-NULL list with n = 0 is an empty filter: no pair is kept (scores 0, as the reference with an empty filter_pos_ix) */
 int snpm_batch_set_row_filter(snpm_batch *b, const int64_t *sorted_rows, int64_t n);
+/* --refine for many samples at once (snpmatch.py:189-205 with Genotype.identify_segregating_snps, snp_genotype.py:188-211): a
+ * per-sample accession selection.  sel uint32 [S, words] with words == snpm_db_row_words(db); bit j of sel[s][w] selects
+ * accession 32w + j (the bit layout of a packed row; bits at or beyond n_acc: SNPM_E_ARG).  A marker of sample s that the join
+ * matched to row r keeps its pair only when r segregates among s's selected accessions: at least two of the called classes
+ * ref, alt, het occur there (missing calls do not count, het counts whatever skip_db_hets says), the predicate of
+ * snpm_db_segregating_rows.  A selection of fewer than two accessions keeps no pair.  Kept pairs and their order are those of
+ * snpm_batch_set_row_filter(segregating rows of sel[s]) on sample s alone, so mode-0 scores are bit-identical to that.  ANDs with
+ * the row filter.  Honoured by snpm_batch_run modes 0 and 1; S must equal the batch's sample count at run time (SNPM_E_ARG
+ * otherwise); mode 2 and the window runs answer SNPM_E_STATE while it is set.  sel == NULL clears it.  Copies, then returns. */
+int snpm_batch_set_segregation_filter(snpm_batch *b, const uint32_t *sel, int64_t S, int32_t words);
+/* after snpm_batch_run: counts int64[S] = pairs of sample s the run kept whose marker has flags[i] != 0; flags uint8 [n], one per
+ * marker in upload order.  With flags = heterozygous calls this is getHeterozygosity's count (snpmatch.py:244-253) of every
+ * sample at once.  Waits for the result. */
+int snpm_batch_count_flagged_pairs(snpm_batch *b, const uint8_t *flags, int64_t *counts);
 /* join + chunked scoring + per-sample totals; device work is queued on the db's stream and the
  * call returns without waiting (inputs already resident).
  * mode bits 0-7: scoring kernel — 0 = fp64 kernel in the reference's summation order (any weights);

@@ -40,6 +40,11 @@ def check_file(inFile):
 
 
 def snpmatch_inbred(args):
+    if args.get('samples'):
+        samples = read_sample_list(args['samples'], args['outFile'])
+        from .core import snpmatch
+        snpmatch.potatoGenotyperMany(args, samples)
+        return
     check_file(args['inFile'])
     from .core import snpmatch
     snpmatch.potatoGenotyper(args)
@@ -57,7 +62,7 @@ def snpmatch_cross(args):
 
 
 def read_sample_list(list_file, out_prefix):
-    """`cross --samples`: one sample file per line, optionally a tab and the sample's output prefix (default
+    """`inbred --samples` / `cross --samples`: one sample file per line, optionally a tab and the sample's output prefix (default
     <out_prefix>.<file name up to its first '.'>).  Blank lines are skipped.  Returns [(path, prefix)]; dies on a missing
     file, an empty list or two samples with the same prefix."""
     check_file(list_file)
@@ -122,7 +127,12 @@ def get_options(description, version_message):
     sub = p.add_subparsers(title='commands', description='one of', help='what each does')
     db_help = "Path to the SNP database: the reference's row-chunked hdf5 file (needs h5py) or a packed .npz written by Genotype.save_packed"
     inbred = sub.add_parser('inbred', help="identify the accession an inbred sample comes from")
-    inbred.add_argument("-i", "--input_file", dest="inFile", help="sample variants: VCF (GT, optional PL), BED (chr, pos, GT) or a parser .npz")
+    inbred_in = inbred.add_mutually_exclusive_group()
+    inbred_in.add_argument("-i", "--input_file", dest="inFile", help="sample variants: VCF (GT, optional PL), BED (chr, pos, GT) or a parser .npz")
+    inbred_in.add_argument("--samples", dest="samples", default=None,
+                           help="text file listing many samples, one path per line (VCF/BED/npz), optionally a tab and that sample's output "
+                                "prefix (default <-o>.<file name up to its first '.'>); all samples are scored together on the GPU; exit "
+                                "status 1 when --refine finds a sample without top hits")
     inbred.add_argument("-d", "--hdf5_file", default=None, dest="hdf5File", help=db_help)
     inbred.add_argument("-e", "--hdf5_acc_file", default=None, dest="hdf5accFile", help="Column-chunked hdf5 file of the reference (accepted for compatibility; one resident copy serves both)")
     inbred.add_argument("--refine", action="store_true", dest="refine", default=False, help="re-score the accessions that cannot be told apart on the SNPs that segregate among them")

@@ -53,15 +53,17 @@ def _is_identity(order):
     return n == 0 or (order[0] == 0 and order[-1] == n - 1 and bool(np.all(order[1:] > order[:-1])))
 
 
-def coded_batch(g, samples, with_weights=True):
+def coded_batch(g, samples, with_weights=True, prepared=None):
     """lib.CodedSamples of a list of ParseInputs: every sample's markers in the order the join wants (database chromosome
     order, position), chromosome id + position in one word, weights as dictionary codes (ParseInputs.coded_weights: the
     integer PLs of a VCF, or a one-off np.unique for other inputs) into ONE table for the batch.  Returns (CodedSamples or
     None, offsets, chrom ids, positions, weights) — the last three in upload order, for re-scoring flagged samples (weights:
-    None unless `with_weights` or the samples cannot be coded; table[codes] gives them back bit for bit).
+    None unless `with_weights` or the samples cannot be coded; table[codes] gives them back bit for bit).  `prepared`: the
+    samples' g.prepare_markers results when the caller has them already.
     Per-marker work is skipped wherever the input allows it: a file that is already in the join's order is not permuted, and
     samples whose tables are prefixes of one table (VCFs: code = PL, table = exp(-PL/10)) keep their codes as they are."""
-    prepared = [g.prepare_markers(inp.chrs, inp.pos) for inp in samples]
+    if prepared is None:
+        prepared = [g.prepare_markers(inp.chrs, inp.pos) for inp in samples]
     ident = [_is_identity(p[0]) for p in prepared]
     offs = np.concatenate([[0], np.cumsum([len(p[2]) for p in prepared])]).astype(np.int64)
     cid = np.concatenate([p[1] for p in prepared]) if samples else np.zeros(0, np.int32)

@@ -298,6 +298,9 @@ class Genotype(object):
         if getattr(self, "_many_batch", None) is not None:      # the batch of core.batch.genotype_many
             self._many_batch.close()
             self._many_batch = None
+        if getattr(self, "_inbred_batch", None) is not None:    # the batch of core.snpmatch.inbred_identify_many
+            self._inbred_batch.close()
+            self._inbred_batch = None
         if getattr(self, "_cross_batch", None) is not None:     # the batch of core.csmatch.cross_identify_many
             self._cross_batch.close()
             self._cross_batch = None

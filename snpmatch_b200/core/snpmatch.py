@@ -202,20 +202,11 @@ class Genotyper(object):
         indistinguishable accessions."""
         self.result = self.genotyper()
         self.write_genotyper_output(self.result)
-        self.result.get_likelihoods()
-        with np.errstate(invalid="ignore"):
-            topHits = np.where(self.result.lrts < lr_thres)[0]
-        if len(topHits) == 1:
-            log.info("a single accession is left: perfect hit, nothing to refine")
-            return None
-        log.info("%s accessions cannot be told apart at LR < %s", len(topHits), lr_thres)
-        if len(topHits) > (self.num_lines / 2):
-            log.info("more than half of the panel is indistinguishable: not refining")
+        topHits = refine_tophits(self.result, self.num_lines)
+        if topHits is None:
             return None
         seg_ix = identify_segregating_snps(self.g, topHits)
-        with np.errstate(invalid="ignore"):
-            mask = np.where(self.result.lrts >= lr_thres)[0]
-        self.result_fine = self.genotyper(filter_pos_ix=seg_ix, mask_acc_ix=mask)
+        self.result_fine = self.genotyper(filter_pos_ix=seg_ix, mask_acc_ix=refine_mask(self.result))
         self.result_fine.print_out_table(self.outFile + ".refined.scores.txt")
 
     def genotyper(self, filter_pos_ix=None, mask_acc_ix=None):
@@ -242,24 +233,57 @@ class Genotyper(object):
         if filter_pos_ix is not None and len(db_idx) < 100:
             log.info("#positions in segregating sites are are too little: %s" % len(db_idx))
         self.commonSNPs = (db_idx, order[s_idx])
-        NumMatSNPs = int(r["m"][0])
-        overlap = get_fraction(NumMatSNPs, len(self.inputs.pos))
-        accs = g.g.accessions
-        if mask_acc_ix is not None:
-            assert type(mask_acc_ix) is np.ndarray, "provide a numpy array of accessions indices to mask"
-            keep = np.setdiff1d(np.arange(self.num_lines), mask_acc_ix)
-            return GenotyperOutput(accs[keep], r["score"][0][keep], r["ninfo"][0][keep], overlap, NumMatSNPs, self.inputs.dp)
-        out = GenotyperOutput(accs, r["score"][0], r["ninfo"][0], overlap, NumMatSNPs, self.inputs.dp)
-        out._attach_fused(r["prob"][0], r["L"][0], r["LR"][0])
+        out = genotyper_output(g.g.accessions, r["score"][0], r["ninfo"][0], len(self.inputs.pos), int(r["m"][0]), self.inputs.dp,
+                               mask_acc_ix)
+        if mask_acc_ix is None:
+            out._attach_fused(r["prob"][0], r["L"][0], r["LR"][0])
         return out
 
     def write_genotyper_output(self, result):
-        log.info("writing %s.scores.txt and %s.matches.json", self.outFile, self.outFile)
-        result.get_likelihoods()
-        result.print_out_table(self.outFile + '.scores.txt')
-        result.print_json_output(self.outFile + ".matches.json")
+        write_scores_and_matches(result, self.outFile)
         getHeterozygosity(self.inputs.gt[self.commonSNPs[1]], self.outFile + ".matches.json")
         return result
+
+
+# ---- host steps of `inbred` shared by Genotyper and inbred_identify_many --------------------------------------------------
+def genotyper_output(accs, score, ninfo, n_markers, NumMatSNPs, dp, mask_acc_ix=None):
+    """GenotyperOutput of one sample's totals (snpmatch.py:228-233); mask_acc_ix drops those accessions (the refined table)."""
+    overlap = get_fraction(NumMatSNPs, n_markers)
+    if mask_acc_ix is not None:
+        assert type(mask_acc_ix) is np.ndarray, "provide a numpy array of accessions indices to mask"
+        keep = np.setdiff1d(np.arange(len(accs)), mask_acc_ix)
+        return GenotyperOutput(accs[keep], score[keep], ninfo[keep], overlap, NumMatSNPs, dp)
+    return GenotyperOutput(accs, score, ninfo, overlap, NumMatSNPs, dp)
+
+
+def write_scores_and_matches(result, outFile):
+    """<outFile>.scores.txt and <outFile>.matches.json without the heterozygosity (snpmatch.py:235-241)."""
+    log.info("writing %s.scores.txt and %s.matches.json", outFile, outFile)
+    result.get_likelihoods()
+    result.print_out_table(outFile + '.scores.txt')
+    result.print_json_output(outFile + ".matches.json")
+
+
+def refine_tophits(result, num_lines):
+    """The accessions `--refine` re-scores (snpmatch.py:193-202), or None when there is nothing to refine: a single top hit, or
+    more than half of the panel's `num_lines` accessions.  An empty array means no top hit at all (every ratio nan)."""
+    result.get_likelihoods()
+    with np.errstate(invalid="ignore"):
+        topHits = np.where(result.lrts < lr_thres)[0]
+    if len(topHits) == 1:
+        log.info("a single accession is left: perfect hit, nothing to refine")
+        return None
+    log.info("%s accessions cannot be told apart at LR < %s", len(topHits), lr_thres)
+    if len(topHits) > (num_lines / 2):
+        log.info("more than half of the panel is indistinguishable: not refining")
+        return None
+    return topHits
+
+
+def refine_mask(result):
+    """Accessions the refined table leaves out (snpmatch.py:203): LR >= lr_thres; nan ratios stay in."""
+    with np.errstate(invalid="ignore"):
+        return np.where(result.lrts >= lr_thres)[0]
 
 
 def identify_segregating_snps(g, accs_ix):
@@ -276,8 +300,12 @@ def identify_segregating_snps(g, accs_ix):
 def getHeterozygosity(snpGT, outFile='default'):
     """Fraction of heterozygous calls among the matched markers; added to the JSON (snpmatch.py:244-253)."""
     snpBinary = parsers.parseGT(snpGT)
-    numHets = int(np.count_nonzero(snpBinary == 2))
-    frac = get_fraction(numHets, len(snpGT))
+    return write_heterozygosity(int(np.count_nonzero(snpBinary == 2)), len(snpGT), outFile)
+
+
+def write_heterozygosity(numHets, numSNPs, outFile='default'):
+    """percent_heterozygosity = numHets / numSNPs, added to the JSON `outFile` (snpmatch.py:249-253)."""
+    frac = get_fraction(numHets, numSNPs)
     if outFile != 'default':
         with open(outFile) as fh:
             report = json.load(fh)
@@ -295,6 +323,189 @@ def potatoGenotyper(args):
     genotyper = Genotyper(inputs, g, args['outFile'], run_genotyper=not args['refine'], skip_db_hets=args['skip_db_hets'])
     if args['refine']:                       # --refine: score, then re-score the indistinguishable accessions on their segregating SNPs
         genotyper.filter_tophits()
+    log.info("finished!")
+
+
+# Device memory one launch of inbred_identify_many may take, and what a sample takes of it: per marker the join, key, pair and
+# weight arrays of both passes (~128 bytes), per segment of the counting kernel (320 markers) and of the order-exact kernel
+# (chunk_size markers) the partial sums over the padded panel row (16 and 12 bytes per column), and per sample the key and group
+# tables of the device grouping (~192 KB), the reduce buffer and the result arrays.  ~10 MB per 50 k-marker sample at 1135
+# accessions, ~7x that at 20 000.
+INBRED_BUDGET_BYTES = 8 << 30
+
+
+def inbred_bytes_per_sample(n_markers, n_acc, row_words, chunk_size=1000):
+    n, a_pad = int(n_markers), 32 * int(row_words)
+    segs = -(-n // 320) * 16 + -(-n // int(chunk_size)) * 12
+    return n * 128 + segs * a_pad + (192 << 10) + (8 * int(n_acc) + 2) * 8
+
+
+def _het_flags(gt):
+    """parseGT(gt) == 2 per marker, or None when the calls mix formats: parseGT sniffs its format from the first call it is
+    given, so the heterozygous count of a subset (the matched markers) equals the flags' count only when every call has the
+    format of the first."""
+    gt = np.asarray(gt)
+    if len(gt) == 0:
+        return np.zeros(0, dtype=bool)
+    first = str(gt[0])
+    text = gt.astype("str")
+    if "|" in first:
+        same = np.char.find(text, "|") >= 0
+    elif "/" in first:
+        same = (np.char.find(text, "/") >= 0) & (np.char.find(text, "|") < 0)
+    elif first.isdigit():
+        same = np.char.isdigit(text)
+    else:
+        return None
+    return parsers.parseGT(gt) == 2 if bool(np.all(same)) else None
+
+
+def inbred_identify_many(inputs_list, g, output_ids, refine=False, skip_db_hets=False, chunk_size=1000, samples_per_launch=None):
+    """`inbred` (and `inbred --refine`) for many samples: every sample's files (<id>.scores.txt, <id>.matches.json and, when it
+    refines, <id>.refined.scores.txt) are byte for byte the ones Genotyper (+ filter_tophits) writes for it alone.
+    Per launch of samples: one coded counting pass for all of them (core.batch.coded_batch, lib.score_coded) with their
+    heterozygous counts from the same run; the refine decisions on the host; one order-exact pass of every refining sample
+    with a per-sample segregation filter on the device (Batch.set_segregation_filter) instead of a full-panel scan each; and
+    the likelihoods of all refined tables in one call.  The host waits a fixed number of times per launch (plus one re-score
+    per sample whose truncated score depends on the summation order, as in genotype_many).  Launches hold as many samples
+    as fit INBRED_BUDGET_BYTES (`samples_per_launch` overrides).
+    Returns one Genotyper per sample with `result`, `num_matched`, `num_hets` and, when it refined, `result_fine`.  A sample
+    without any top hit (every ratio nan, e.g. no marker in the panel) cannot refine: the single path stops there with an
+    assertion; here its `no_top_hits` is set, its scores and matches files are written, and the other samples go on."""
+    from . import batch as batch_mod
+    inputs_list, output_ids = list(inputs_list), list(output_ids)
+    assert len(inputs_list) == len(output_ids), "one output prefix per sample"
+    assert len(set(output_ids)) == len(output_ids), "output prefixes must differ"
+    assert int(chunk_size) >= 1, "chunk_size must be a positive number of SNPs"
+    if g.db.row0_global != 0 or g.db.n_rows != int(np.max(getattr(g, "global_chr_regions", [[0, g.db.n_rows]]))):
+        raise ValueError("inbred_identify_many needs the whole panel on one device; this one holds a shard of its rows")
+    # every sample's chromosome names are mapped to the panel's before any device work; a bad sample is named
+    gts, prepared = [], []
+    for i, (inp, out) in enumerate(zip(inputs_list, output_ids)):
+        try:
+            assert len(inp.chrs) == len(inp.pos), "%d chromosome names for %d positions" % (len(inp.chrs), len(inp.pos))
+            gts.append(Genotyper(inp, g, out, run_genotyper=False, skip_db_hets=skip_db_hets, chunk_size=chunk_size))
+            prepared.append(g.prepare_markers(inp.chrs, inp.pos))
+        except Exception as e:
+            raise ValueError("sample %d (%s): %s" % (i, out, e)) from e
+    if not gts:
+        return gts
+    per = samples_per_launch
+    if per is None:
+        biggest = max(inbred_bytes_per_sample(len(inp.pos), g.db.n_acc, g.db.row_words, chunk_size) for inp in inputs_list)
+        per = max(1, INBRED_BUDGET_BYTES // biggest)
+    assert int(per) >= 1, "samples_per_launch must be at least 1"
+    # one batch lives with the panel: its device buffers are allocated once, not per call
+    if getattr(g, "_inbred_batch", None) is None:
+        g._inbred_batch = lib.Batch(g.db, [0, 0], np.zeros(0, np.int32), np.zeros(0, np.int32), np.zeros((0, 3)))
+    g._inbred_batch.set_chunk_rows(int(chunk_size))         # the order-exact passes sum in Genotyper's chunks
+    for c0 in range(0, len(gts), int(per)):
+        _inbred_launch(gts[c0:c0 + int(per)], prepared[c0:c0 + int(per)], g._inbred_batch, batch_mod, refine)
+    skipped = [gt.outFile for gt in gts if gt.no_top_hits]
+    if skipped:
+        log.error("no top hits, not refined: %s", ", ".join(skipped))
+    return gts
+
+
+def _inbred_launch(gts, prepared, batch, batch_mod, refine):
+    g, skip = gts[0].g, gts[0]._skip_db_hets
+    accs = g.g.accessions
+    samples = [gt.inputs for gt in gts]
+    flags = [_het_flags(inp.gt) for inp in samples]
+    up_flags = np.concatenate([f[p[0]] if f is not None else np.zeros(len(p[0]), bool) for f, p in zip(flags, prepared)])
+    # first pass: the coded counting path of genotype_many (position-order f64 weights when the weights cannot be coded)
+    cs, offs, cid, pos, _ = batch_mod.coded_batch(g, samples, with_weights=False, prepared=prepared)
+    if cs is not None:
+        r = lib.score_coded(g.db, cs, cid, pos, None, skip_db_hets=skip, batch=batch, flags=up_flags)
+    else:
+        batch.upload(offs, cid, pos, _ordered_weights(samples, prepared))
+        batch.run(skip, kernel_mode=lib.KERNEL_FP64)
+        batch.epilogue()
+        r = batch.fetch()
+        r["flagged"] = batch.count_flagged_pairs(up_flags)
+    for i, gt in enumerate(gts):
+        m = int(r["m"][i])
+        gt.result = genotyper_output(accs, r["score"][i], r["ninfo"][i], len(gt.inputs.pos), m, gt.inputs.dp)
+        gt.result._attach_fused(r["prob"][i], r["L"][i], r["LR"][i])
+        gt.num_matched, gt.num_hets, gt.no_top_hits = m, int(r["flagged"][i]), False
+        write_scores_and_matches(gt.result, gt.outFile)
+        if flags[i] is None:                                # calls in mixed formats: the single path's own count
+            gt.get_common_positions()
+            getHeterozygosity(gt.inputs.gt[gt.commonSNPs[1]], gt.outFile + ".matches.json")
+        else:
+            write_heterozygosity(gt.num_hets, m, gt.outFile + ".matches.json")
+    if not refine:
+        return
+    todo = []
+    for i, gt in enumerate(gts):
+        top = refine_tophits(gt.result, gt.num_lines)
+        if top is not None and len(top) == 0:
+            gt.no_top_hits = True
+        elif top is not None:
+            todo.append((i, top))
+    if todo:
+        _refine_launch([gts[i] for i, _ in todo], [prepared[i] for i, _ in todo], [top for _, top in todo], batch)
+
+
+def _ordered_weights(samples, prepared):
+    return np.concatenate([np.asarray(inp.wei, dtype=np.float64).reshape(-1, 3)[p[0]] for inp, p in zip(samples, prepared)])
+
+
+def _refine_launch(gts, prepared, tops, batch):
+    """The refine pass of the samples of one launch that refine: one order-exact run with the segregation filter of every
+    sample's top hits (the pairs and the summation order of Genotyper.genotyper(filter_pos_ix=...)), one fetch, one likelihood
+    call for all refined tables."""
+    g = gts[0].g
+    accs = g.g.accessions
+    r = _refine_scores(g, batch, [gt.inputs for gt in gts], prepared, tops, gts[0]._skip_db_hets)
+    fine = []
+    for i, gt in enumerate(gts):
+        m = int(r["m"][i])
+        if m < 100:
+            log.info("#positions in segregating sites are are too little: %s" % m)
+        fine.append(genotyper_output(accs, r["score"][i], r["ninfo"][i], len(gt.inputs.pos), m, gt.inputs.dp, refine_mask(gt.result)))
+    K = max(len(f.accs) for f in fine)
+    sc, ni = np.zeros((len(fine), K)), np.zeros((len(fine), K))
+    for i, f in enumerate(fine):
+        sc[i, :len(f.accs)], ni[i, :len(f.accs)] = f.scores, f.ninfo
+    prob, lik, lrt = lib.calculate_likelihoods_many(sc, ni)
+    for i, (gt, f) in enumerate(zip(gts, fine)):
+        k = len(f.accs)
+        f._attach_fused(prob[i, :k], lik[i, :k], lrt[i, :k])
+        gt.result_fine = f
+        f.print_out_table(gt.outFile + ".refined.scores.txt")
+
+
+def _refine_scores(g, batch, samples, prepared, tops, skip_db_hets):
+    """Device part of the refine pass: the samples in position order with f64 weights, each scored over the pairs whose row
+    segregates among its top hits `tops[i]`.  Returns Batch.fetch()."""
+    offs = np.concatenate([[0], np.cumsum([len(p[2]) for p in prepared])]).astype(np.int64)
+    batch.upload(offs, np.concatenate([p[1] for p in prepared]), np.concatenate([p[2] for p in prepared]),
+                 _ordered_weights(samples, prepared))
+    batch.set_segregation_filter(lib.selection_masks(tops, g.db.n_acc))
+    try:
+        # on one-hot weights the order-exact kernel gives the popcount kernel's integers: one launch serves every sample
+        batch.run(skip_db_hets, kernel_mode=lib.KERNEL_FP64)
+        batch.epilogue()
+        return batch.fetch()
+    finally:
+        batch.set_segregation_filter(None)
+
+
+def potatoGenotyperMany(args, samples):
+    """`inbred --samples`: samples = [(input file, output prefix)].  Exits with status 1, after every other sample is written,
+    when a sample had no top hit to refine."""
+    inputs = [parsers.ParseInputs(inFile=path, logDebug=args['logDebug']) for path, _ in samples]
+    log.info("packing the database into HBM")
+    g = snp_genotype.Genotype(args['hdf5File'], args['hdf5accFile'])
+    try:
+        log.info("matching %d samples against %s accessions", len(samples), len(g.accessions))
+        gts = inbred_identify_many(inputs, g, [prefix for _, prefix in samples], refine=args['refine'], skip_db_hets=args['skip_db_hets'])
+    finally:
+        g.close()
+    skipped = [path for (path, _), gt in zip(samples, gts) if gt.no_top_hits]
+    if skipped:
+        die("no top hits to refine (no marker shared with the panel?): " + ", ".join(skipped))
     log.info("finished!")
 
 

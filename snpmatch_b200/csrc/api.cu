@@ -912,7 +912,7 @@ int snpm_batch_destroy(snpm_batch *b) {
                       &b->d_chrom8, &b->d_gid, &b->d_gtable, &b->d_pair_gid, &b->d_part_int, &b->d_guard, &b->d_runs,
                       &b->d_codes, &b->d_wtable, &b->d_key_a, &b->d_key_b, &b->d_idx_a, &b->d_idx_b, &b->d_pair_db_tmp, &b->d_pair_s_tmp,
                       &b->d_tile_sample, &b->d_tile_first, &b->d_tile_hist, &b->d_blk_chg, &b->d_seg_order, &b->d_work_counter, &b->d_hash, &b->d_slot_gid, &b->d_ngroups,
-                      &b->d_group_overflow, &b->d_gkeys, &b->d_gw, &b->d_goff};
+                      &b->d_group_overflow, &b->d_gkeys, &b->d_gw, &b->d_goff, &b->d_segsel, &b->d_segsel_off, &b->d_flags, &b->d_flag_counts};
     for (DevBuf *d : bufs) d->release();
     for (int i = 0; i < SNPM_N_EVENTS; ++i)
         if (b->ev[i]) cudaEventDestroy(b->ev[i]);
@@ -939,6 +939,65 @@ int snpm_batch_set_row_filter(snpm_batch *b, const int64_t *sorted_rows, int64_t
         SNPM_CUDA(cudaMemcpyAsync(b->d_filter.p, sorted_rows, size_t(n) * 8, cudaMemcpyHostToDevice, b->db->stream));
         SNPM_CUDA(cudaStreamSynchronize(b->db->stream));
     }
+    return SNPM_OK;
+}
+
+int snpm_batch_set_segregation_filter(snpm_batch *b, const uint32_t *sel, int64_t S, int32_t words) {
+    if (!b) return fail(SNPM_E_ARG, "snpm_batch_set_segregation_filter: NULL batch");
+    if (!sel) {
+        b->has_seg = false;
+        b->seg_S = 0;
+        return SNPM_OK;
+    }
+    snpm_db *db = b->db;
+    if (S < 1 || words != db->stride)
+        return fail(SNPM_E_ARG, "snpm_batch_set_segregation_filter: need S >= 1 selections of snpm_db_row_words() = %d words (got S = %lld, %d words)",
+                    db->stride, (long long)S, words);
+    std::vector<int32_t> off(size_t(S) + 1, 0);
+    std::vector<uint32_t> pairs;                                // (word, mask) of every touched word, sample by sample
+    for (int64_t s = 0; s < S; ++s) {
+        for (int32_t w = 0; w < words; ++w) {
+            const uint32_t m = sel[size_t(s) * words + w];
+            const int64_t first = int64_t(w) * 32;
+            const uint32_t valid = first >= db->n_acc ? 0u : (db->n_acc - first >= 32 ? 0xffffffffu : (1u << (db->n_acc - first)) - 1u);
+            if (m & ~valid) return fail(SNPM_E_ARG, "snpm_batch_set_segregation_filter: sample %lld selects accessions beyond the panel's %d", (long long)s, db->n_acc);
+            if (m) {
+                pairs.push_back(uint32_t(w));
+                pairs.push_back(m);
+            }
+        }
+        if (pairs.size() / 2 > size_t(INT32_MAX)) return fail(SNPM_E_ARG, "snpm_batch_set_segregation_filter: selections too large");
+        off[size_t(s) + 1] = int32_t(pairs.size() / 2);
+    }
+    SNPM_CUDA(cudaSetDevice(db->device));
+    SNPM_TRY(b->d_segsel.ensure(std::max<size_t>(pairs.size(), 2) * 4));
+    SNPM_TRY(b->d_segsel_off.ensure(off.size() * 4));
+    // the copies queue behind the runs that may still read the previous selections; the host arrays are gone on return
+    if (!pairs.empty()) SNPM_CUDA(cudaMemcpyAsync(b->d_segsel.p, pairs.data(), pairs.size() * 4, cudaMemcpyHostToDevice, db->stream));
+    SNPM_CUDA(cudaMemcpyAsync(b->d_segsel_off.p, off.data(), off.size() * 4, cudaMemcpyHostToDevice, db->stream));
+    SNPM_CUDA(cudaStreamSynchronize(db->stream));
+    b->has_seg = true;
+    b->seg_S = S;
+    return SNPM_OK;
+}
+
+int snpm_batch_count_flagged_pairs(snpm_batch *b, const uint8_t *flags, int64_t *counts) {
+    if (!b || !counts || (b->n > 0 && !flags)) return fail(SNPM_E_ARG, "snpm_batch_count_flagged_pairs: bad arguments");
+    if (!b->ran) return fail(SNPM_E_STATE, "snpm_batch_count_flagged_pairs: run the batch first");
+    snpm_db *db = b->db;
+    SNPM_CUDA(cudaSetDevice(db->device));
+    cudaStream_t st = db->stream;
+    SNPM_TRY(b->d_flag_counts.ensure(size_t(b->S) * 8));
+    SNPM_CUDA(cudaMemsetAsync(b->d_flag_counts.p, 0, size_t(b->S) * 8, st));
+    if (b->n > 0) {
+        SNPM_TRY(b->d_flags.ensure(size_t(b->n)));
+        SNPM_CUDA(cudaMemcpyAsync(b->d_flags.p, flags, size_t(b->n), cudaMemcpyHostToDevice, st));
+        k_count_flagged_pairs<<<int(ceil_div64(b->n, 256)), 256, 0, st>>>(b->d_match_row.as<int32_t>(), b->d_flags.as<uint8_t>(), b->n,
+                                                                          b->d_off.as<int64_t>(), b->S, b->d_flag_counts.as<unsigned long long>());
+        SNPM_KERNEL_CHECK();
+    }
+    SNPM_CUDA(cudaMemcpyAsync(counts, b->d_flag_counts.p, size_t(b->S) * 8, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaStreamSynchronize(st));
     return SNPM_OK;
 }
 
@@ -998,6 +1057,13 @@ static int batch_join(snpm_batch *b, int algo) {
                                                             db->d_bitmap, db->d_bm_first_row, db->d_bm_off,
                                                             (b->grouped && (b->pending_expand & 2)) ? b->d_wei_idx.as<uint32_t>() : nullptr);
         SNPM_KERNEL_CHECK();
+        if (b->has_seg) {
+            static_assert(SEGP_THREADS == JOIN_TILE, "the segregation filter recounts the join's tiles");
+            k_segregating_pairs<<<int(n_tiles), SEGP_THREADS, 0, st>>>(db->d_packed, db->stride, b->d_off.as<int64_t>(), S, n, b->d_segsel.as<uint2>(),
+                                                                      b->d_segsel_off.as<int32_t>(), b->d_match_row.as<int32_t>(), b->d_tile_cnt.as<int32_t>());
+            SNPM_KERNEL_CHECK();
+            b->launches += 1;
+        }
         k_scan_tiles<<<1, 1024, 0, st>>>(b->d_tile_cnt.as<int32_t>(), n_tiles, b->d_tile_off.as<int32_t>(), b->d_prefix.as<int32_t>() + n);
         SNPM_KERNEL_CHECK();
         if (b->coded) {
@@ -1197,6 +1263,10 @@ int snpm_batch_run(snpm_batch *b, int skip_db_hets, int mode) {
     if ((kernel_mode == 2) != b->grouped)
         return fail(SNPM_E_STATE, "snpm_batch_run: kernel mode 2 scores batches uploaded with snpm_batch_upload_grouped, and only those");
     if (algo > 2) return fail(SNPM_E_ARG, "snpm_batch_run: unknown join algorithm %d", algo);
+    if (b->has_seg && kernel_mode == 2)
+        return fail(SNPM_E_STATE, "snpm_batch_run: the segregation filter is honoured by kernel modes 0 and 1 only; clear it first");
+    if (b->has_seg && b->seg_S != b->S)
+        return fail(SNPM_E_ARG, "snpm_batch_run: the segregation filter holds %lld selections for %lld samples", (long long)b->seg_S, (long long)b->S);
     b->launches = 0;
     for (int i = 0; i < SNPM_N_EVENTS; ++i) b->ev_rec[i] = false;
     SNPM_TRY(batch_alloc_outputs(b, b->nseg_cap));
@@ -1784,6 +1854,48 @@ int snpm_calculate_likelihoods(int device, const double *scores, const double *n
     return rc;
 }
 
+int snpm_calculate_likelihoods_many(int device, const double *scores, const double *ninfo, int64_t S, int64_t K, int amin_is_calc, double amin,
+                                    double *prob, double *L, double *LR) {
+    if (S < 0 || K <= 0 || K >= (int64_t(1) << 30) || S > (int64_t(1) << 31) / 8 || (S > 0 && (!scores || !ninfo)))
+        return fail(SNPM_E_ARG, "snpm_calculate_likelihoods_many: bad arguments");
+    int n_dev = 0;
+    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) return fail(SNPM_E_CUDA, "snpm_calculate_likelihoods_many: no CUDA device (there is no CPU fallback)");
+    if (S == 0) return SNPM_OK;
+    SNPM_CUDA(cudaSetDevice(device));
+    // rows of the reduce-buffer layout k_epilogue reads: score[K] | ninfo[K] | m | y > n count
+    const size_t SK = size_t(S) * size_t(K), pitch = 2 * size_t(K) + 2;
+    std::vector<double> red(size_t(S) * pitch, 0.0);
+    for (int64_t s = 0; s < S; ++s) {
+        memcpy(red.data() + size_t(s) * pitch, scores + size_t(s) * K, size_t(K) * 8);
+        memcpy(red.data() + size_t(s) * pitch + K, ninfo + size_t(s) * K, size_t(K) * 8);
+    }
+    DevBuf d_red, d_out;
+    int rc = d_red.ensure(red.size() * 8);
+    if (rc == SNPM_OK) rc = d_out.ensure(3 * SK * 8);
+    cudaError_t e = cudaSuccess;
+    if (rc == SNPM_OK) {
+        e = cudaMemcpy(d_red.p, red.data(), red.size() * 8, cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) {
+            double *o = d_out.as<double>();
+            e = launch_epilogue(nullptr, S, d_red.as<double>(), int64_t(pitch), int32_t(K), 0, amin_is_calc ? 0 : 1, amin, nullptr, nullptr, o, o + SK, o + 2 * SK);
+            if (e == cudaSuccess) e = cudaGetLastError();
+        }
+        if (e == cudaSuccess) e = cudaDeviceSynchronize();
+        std::vector<double> viol(size_t(S), 0.0);
+        if (e == cudaSuccess) e = cudaMemcpy2D(viol.data(), 8, d_red.as<double>() + 2 * K + 1, pitch * 8, 8, size_t(S), cudaMemcpyDeviceToHost);
+        if (e == cudaSuccess && prob) e = cudaMemcpy(prob, d_out.p, SK * 8, cudaMemcpyDeviceToHost);
+        if (e == cudaSuccess && L) e = cudaMemcpy(L, d_out.as<double>() + SK, SK * 8, cudaMemcpyDeviceToHost);
+        if (e == cudaSuccess && LR) e = cudaMemcpy(LR, d_out.as<double>() + 2 * SK, SK * 8, cudaMemcpyDeviceToHost);
+        for (int64_t s = 0; s < S && e == cudaSuccess && rc == SNPM_OK; ++s)
+            if (viol[size_t(s)] > 0.0)
+                rc = fail(SNPM_E_ASSERT, "provided y is greater than n (row %lld, %lld accessions; likeliTest, snpmatch.py:43)", (long long)s, (long long)viol[size_t(s)]);
+    }
+    d_red.release();
+    d_out.release();
+    if (e != cudaSuccess) return fail(SNPM_E_CUDA, "snpm_calculate_likelihoods_many: %s", cudaGetErrorString(e));
+    return rc;
+}
+
 // ---- 8(f)-4: genotype_cross window calls -----------------------------------------------------------------
 int snpm_cross_window_genotypes(int device, const int64_t *par_idx, const int64_t *vcf_idx, int64_t m, const int32_t *win_start, int32_t n_windows,
                                 const int8_t *p1, const int8_t *p2, int64_t n_par, const int8_t *gt, int64_t n_vcf, int32_t n_samples,
@@ -2001,6 +2113,7 @@ static int windows_begin(snpm_batch *b, int skip_db_hets, int64_t bin_len, const
     if (b->S * int64_t(n_windows) > INT32_MAX / 2)
         return fail(SNPM_E_ARG, "snpm_batch_run_windows: %lld samples x %d windows is too many window slots for one run", (long long)b->S, n_windows);
     if (b->grouped) return fail(SNPM_E_STATE, "snpm_batch_run_windows: windows need the batch in position order (snpm_batch_upload)");
+    if (b->has_seg) return fail(SNPM_E_STATE, "snpm_batch_run_windows: windows do not honour the segregation filter; clear it first");
     snpm_db *db = b->db;
     SNPM_CUDA(cudaSetDevice(db->device));
     cudaStream_t st = db->stream;

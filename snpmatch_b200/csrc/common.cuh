@@ -123,6 +123,11 @@ struct snpm_batch {
     snpm::DevBuf d_off, d_chrom, d_pos, d_wei, d_filter;
     int64_t n_filter = 0;
     bool has_filter = false;  // snpm_batch_set_row_filter: a filter is set (possibly an empty one, which keeps nothing)
+    // snpm_batch_set_segregation_filter: per sample the (word, mask) pairs its accession selection touches, cut by d_segsel_off
+    snpm::DevBuf d_segsel, d_segsel_off;
+    int64_t seg_S = 0;
+    bool has_seg = false;
+    snpm::DevBuf d_flags, d_flag_counts;   // snpm_batch_count_flagged_pairs
     // join products
     snpm::DevBuf d_match_row, d_tile_cnt, d_tile_off, d_prefix, d_pair_db, d_pair_s, d_pair_w;
     snpm::DevBuf d_mstart, d_seg_off;

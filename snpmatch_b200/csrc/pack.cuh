@@ -70,6 +70,85 @@ __global__ void __launch_bounds__(256) k_segregating_rows(const uint64_t *__rest
     }
 }
 
+// Sample of marker i of a batch: the last s in [0, S) with off[s] <= i (empty samples share their offset with the next one).
+__device__ __forceinline__ int64_t sample_of_marker(const int64_t *__restrict__ off, int64_t S, int64_t i) {
+    int64_t lo = 0, hi = S;
+    while (hi - lo > 1) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (__ldg(off + mid) <= i) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+
+// Per-sample segregation filter of a batch (snpm_batch_set_segregation_filter), between the join and the compaction: a marker of
+// sample s that the join matched to row r keeps it only when r segregates among s's selected accessions, with the predicate of
+// k_segregating_rows.  The host compacts every selection to the words it touches (sel[sel_off[s] .. sel_off[s+1]) = (word,
+// mask)), so a marker reads one 8-byte word (one 32-byte sector) per touched word, not its whole row.  Selections of more than
+// SEGP_NARROW words are taken by the marker's whole warp after the per-thread pass, lanes sweeping the words.  CTAs are the
+// join's tiles (JOIN_TILE markers): the tile's kept count replaces its tile_cnt, so scan, scatter and the sample ranges run as
+// they do after a plain join.
+constexpr int SEGP_THREADS = 1024;     // = JOIN_TILE
+constexpr int SEGP_NARROW = 8;
+
+__device__ __forceinline__ void seg_classes(uint64_t v, uint32_t m, uint32_t &has_ref, uint32_t &has_alt, uint32_t &has_het) {
+    const uint32_t lo = uint32_t(v), hi = uint32_t(v >> 32);
+    has_ref |= ~(lo | hi) & m;
+    has_alt |= lo & ~hi & m;
+    has_het |= hi & ~lo & m;
+}
+
+__global__ void __launch_bounds__(SEGP_THREADS) k_segregating_pairs(const uint64_t *__restrict__ packed, int32_t stride, const int64_t *__restrict__ off,
+                                                                    int64_t S, int64_t n, const uint2 *__restrict__ sel,
+                                                                    const int32_t *__restrict__ sel_off, int32_t *__restrict__ match_row,
+                                                                    int32_t *__restrict__ tile_cnt) {
+    const int lane = threadIdx.x & 31;
+    const int64_t i = int64_t(blockIdx.x) * SEGP_THREADS + threadIdx.x;
+    const int32_t matched = i < n ? match_row[i] : -1;
+    int32_t row = matched, w0 = 0, w1 = 0;
+    if (row >= 0) {
+        const int64_t s = sample_of_marker(off, S, i);
+        w0 = __ldg(sel_off + s);
+        w1 = __ldg(sel_off + s + 1);
+    }
+    const bool wide = row >= 0 && w1 - w0 > SEGP_NARROW;
+    if (row >= 0 && !wide) {
+        uint32_t r = 0u, a = 0u, h = 0u;
+        const uint64_t *p = packed + int64_t(row) * stride;
+        for (int32_t k = w0; k < w1; ++k) {
+            const uint2 wm = __ldg(sel + k);
+            seg_classes(__ldg(p + wm.x), wm.y, r, a, h);
+        }
+        if ((r != 0u) + (a != 0u) + (h != 0u) < 2) row = -1;
+    }
+    for (unsigned pend = __ballot_sync(0xffffffffu, wide); pend; pend &= pend - 1u) {
+        const int src = __ffs(pend) - 1;
+        const int32_t r_src = __shfl_sync(0xffffffffu, row, src);
+        const int32_t a0 = __shfl_sync(0xffffffffu, w0, src), a1 = __shfl_sync(0xffffffffu, w1, src);
+        const uint64_t *p = packed + int64_t(r_src) * stride;
+        uint32_t r = 0u, a = 0u, h = 0u;
+        for (int32_t k = a0 + lane; k < a1; k += 32) {
+            const uint2 wm = __ldg(sel + k);
+            seg_classes(__ldg(p + wm.x), wm.y, r, a, h);
+        }
+        const int classes = (__any_sync(0xffffffffu, r != 0u) ? 1 : 0) + (__any_sync(0xffffffffu, a != 0u) ? 1 : 0) +
+                            (__any_sync(0xffffffffu, h != 0u) ? 1 : 0);
+        if (lane == src && classes < 2) row = -1;
+    }
+    if (row != matched) match_row[i] = -1;
+    const int cnt = __syncthreads_count(row >= 0);
+    if (threadIdx.x == 0) tile_cnt[blockIdx.x] = cnt;
+}
+
+// counts[s] += matched markers of sample s whose flag is set (snpm_batch_count_flagged_pairs); lanes of one sample add once
+__global__ void __launch_bounds__(256) k_count_flagged_pairs(const int32_t *__restrict__ match_row, const uint8_t *__restrict__ flags, int64_t n,
+                                                             const int64_t *__restrict__ off, int64_t S, unsigned long long *__restrict__ counts) {
+    const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+    const bool hit = i < n && match_row[i] >= 0 && flags[i] != 0;
+    const int64_t s = hit ? sample_of_marker(off, S, i) : -1;
+    const unsigned peers = __match_any_sync(0xffffffffu, s);
+    if (hit && __ffs(peers) - 1 == int(threadIdx.x & 31)) atomicAdd(counts + s, (unsigned long long)__popc(peers));
+}
+
 // ---- synthetic panel: the integer hash of snpmatch_b200/synth.py --------------------------------
 __host__ __device__ __forceinline__ uint64_t mix64(uint64_t key, uint64_t seed) {
     uint64_t z = key + (seed + 1ull) * 0x9E3779B97F4A7C15ull;

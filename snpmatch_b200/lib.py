@@ -221,6 +221,7 @@ SIGNATURES = {
     "snpm_intersect": (C.c_int, [_p, _p, _p, _i64, C.c_int, _p, _p, _p]),
     "snpm_match_gts_accs": (C.c_int, [C.c_int, _p, _p, _i64, _i32, C.c_int, _p, _p]),
     "snpm_calculate_likelihoods": (C.c_int, [C.c_int, _p, _p, _i64, C.c_int, _f64, _p, _p, _p]),
+    "snpm_calculate_likelihoods_many": (C.c_int, [C.c_int, _p, _p, _i64, _i64, C.c_int, _f64, _p, _p, _p]),
     "snpm_batch_create": (C.c_int, [_p, _i64, _p, _p, _p, _p, _p]),
     "snpm_batch_upload": (C.c_int, [_p, _i64, _p, _p, _p, _p]),
     "snpm_batch_upload_indexed": (C.c_int, [_p, _i64, _p, _p, _p, _p, _p, _i32]),
@@ -240,6 +241,8 @@ SIGNATURES = {
     "snpm_batch_set_track_pairs": (C.c_int, [_p, C.c_int]),
     "snpm_batch_set_result_range": (C.c_int, [_p, _i64, _i64]),
     "snpm_batch_set_row_filter": (C.c_int, [_p, _p, _i64]),
+    "snpm_batch_set_segregation_filter": (C.c_int, [_p, _p, _i64, _i32]),
+    "snpm_batch_count_flagged_pairs": (C.c_int, [_p, _p, _p]),
     "snpm_batch_run": (C.c_int, [_p, C.c_int, C.c_int]),
     "snpm_batch_epilogue": (C.c_int, [_p]),
     "snpm_batch_wait": (C.c_int, [_p, _p]),
@@ -637,6 +640,24 @@ class Batch(object):
         self._filter_keep = rows if len(rows) else np.zeros(1, np.int64)      # a valid pointer for the empty list
         check(load().snpm_batch_set_row_filter(self._h, ptr(self._filter_keep), len(rows)))
 
+    def set_segregation_filter(self, sel):
+        """Per-sample `--refine` filter: sel uint32 [S, row_words] accession bit masks (selection_masks()), one row per sample of
+        the next run; a sample keeps only the pairs whose row segregates among its selected accessions.  None clears it."""
+        if sel is None:
+            check(load().snpm_batch_set_segregation_filter(self._h, None, 0, 0))
+            return
+        sel = as_c(sel, np.uint32)
+        assert sel.ndim == 2
+        check(load().snpm_batch_set_segregation_filter(self._h, ptr(sel), sel.shape[0], sel.shape[1]))
+
+    def count_flagged_pairs(self, flags):
+        """After run(): per sample, the kept pairs whose marker is flagged (flags: one per uploaded marker, upload order)."""
+        flags = as_c(np.asarray(flags, dtype=bool).view(np.uint8), np.uint8)
+        assert len(flags) == int(self.offsets[-1])
+        counts = np.zeros(self.n_samples, dtype=np.int64)
+        check(load().snpm_batch_count_flagged_pairs(self._h, ptr(flags) if len(flags) else None, ptr(counts)))
+        return counts
+
     def run(self, skip_db_hets=False, kernel_mode=0, join_algo=JOIN_AUTO):
         check(load().snpm_batch_run(self._h, int(bool(skip_db_hets)), int(kernel_mode) | (int(join_algo) << 8)))
 
@@ -871,6 +892,31 @@ def calculate_likelihoods(scores, ninfo, amin="calc", device=0):
     return prob, lik, lr
 
 
+def calculate_likelihoods_many(scores, ninfo, amin="calc", device=0):
+    """calculate_likelihoods for every row of scores / ninfo [S, K] in one device call; pad short rows with ninfo = 0."""
+    scores = as_c(scores, np.float64)
+    ninfo = as_c(ninfo, np.float64)
+    assert scores.ndim == 2 and scores.shape == ninfo.shape
+    S, K = scores.shape
+    prob, lik, lr = (np.empty((S, K), dtype=np.float64) for _ in range(3))
+    calc = amin == "calc"
+    check(load().snpm_calculate_likelihoods_many(device, ptr(scores), ptr(ninfo), S, K, int(calc), 0.0 if calc else float(amin),
+                                                 ptr(prob), ptr(lik), ptr(lr)))
+    return prob, lik, lr
+
+
+def selection_masks(acc_lists, n_acc):
+    """uint32 [len(acc_lists), row words] accession bit masks for Batch.set_segregation_filter: bit j of word w selects
+    accession 32w + j, the layout of a packed row (rows padded to an even number of words)."""
+    words = 2 * ((int(n_acc) + 63) // 64)
+    sel = np.zeros((len(acc_lists), words), dtype=np.uint32)
+    for s, acc in enumerate(acc_lists):
+        acc = np.asarray(acc, dtype=np.int64)
+        assert acc.size == 0 or (acc.min() >= 0 and acc.max() < n_acc), "accession index outside the panel"
+        np.bitwise_or.at(sel[s], acc >> 5, (np.uint32(1) << (acc & 31).astype(np.uint32)))
+    return sel
+
+
 def score_grouped(db, offsets, s_chrom_id, s_pos, wei, skip_db_hets=False, grouped=None, batch=None):
     """Throughput scoring of many samples (Genotyper.genotyper per sample, snpmatch.py:207-233) with the grouped kernel:
     returns the dict of Batch.fetch().  Samples whose truncated score would depend on the reference's summation order
@@ -911,13 +957,14 @@ def score_grouped(db, offsets, s_chrom_id, s_pos, wei, skip_db_hets=False, group
             b.close()
 
 
-def score_coded(db, cs, s_chrom_id=None, s_pos=None, wei=None, skip_db_hets=False, batch=None):
+def score_coded(db, cs, s_chrom_id=None, s_pos=None, wei=None, skip_db_hets=False, batch=None, flags=None):
     """Throughput scoring of many samples (Genotyper.genotyper per sample, snpmatch.py:207-233) from CodedSamples: join,
     grouping by weight triple and counting all on the device.  Returns the dict of Batch.fetch() plus "rescored".  Samples
     whose truncated score would depend on the reference's summation order (guard_counts > 0) are re-scored with the
     order-exact fp64 kernel when their position-order arrays (s_chrom_id, s_pos, wei of the whole batch) are given (else from
     the codes: table[codes] gives the weights back bit for bit).  Pass a `batch` to keep its device buffers between calls: a
-    fresh batch costs 0.3 - 1 s of cudaMalloc / cudaFree per call on a loaded device (core.batch.genotype_many keeps one)."""
+    fresh batch costs 0.3 - 1 s of cudaMalloc / cudaFree per call on a loaded device (core.batch.genotype_many keeps one).
+    flags (optional, one per marker of cs in upload order): r["flagged"] = Batch.count_flagged_pairs of the coded run."""
     own = batch is None
     b = batch if batch is not None else Batch(db, [0, 0], np.zeros(0, np.int32), np.zeros(0, np.int32), np.zeros((0, 3)))
     try:
@@ -926,6 +973,8 @@ def score_coded(db, cs, s_chrom_id=None, s_pos=None, wei=None, skip_db_hets=Fals
         b.run(skip_db_hets, kernel_mode=KERNEL_GROUPED)
         b.epilogue()
         r = b.fetch()
+        if flags is not None:                       # before the re-scores below replace the run's pairs
+            r["flagged"] = b.count_flagged_pairs(flags)
         flagged = np.flatnonzero(b.guard_counts())
         r["rescored"] = flagged
         offsets = cs.offsets
