@@ -239,7 +239,8 @@ int snpm_batch_count_flagged_pairs(snpm_batch *b, const uint8_t *flags, int64_t 
  *                    integers bit-exact, fp64 scores within a few ulp of the reference; see snpm_batch_guard_counts.
  * mode bits 8-15: join algorithm (0 auto, 1 binary search, 2 merge-path). */
 int snpm_batch_run(snpm_batch *b, int skip_db_hets, int mode);
-/* likelihood epilogue on the (possibly all-reduced) totals; queued, not waited for */
+/* likelihood epilogue on the (possibly all-reduced) totals; queued, not waited for.  Grouped batches finalise their totals in
+ * place, so their epilogue runs once per snpm_batch_run (a second call answers SNPM_E_STATE); position-order batches may repeat it. */
 int snpm_batch_epilogue(snpm_batch *b);
 /* wait for the queued work; ms_device = GPU time of the last run+epilogue measured with CUDA
  * events on the db's stream (may be NULL) */
@@ -251,7 +252,8 @@ int snpm_batch_set_result_range(snpm_batch *b, int64_t first_sample, int64_t n_s
 /* device address of the f64 reduce buffer [S, 2*n_acc+2]: per sample score[n_acc],
  * ninfo[n_acc] (as f64, exact), m, y>n violation count — the payload of the cross-GPU sum (8e).
  * Grouped batches: [S, 3*n_acc+2] = fractional part F | ninfo | m | violations | integer part I; the epilogue
- * turns F into the score after the reduce. */
+ * turns F into the score after the reduce.  Until then the violation slot of a coded batch holds the grouping's overflow flag
+ * (0 or 1 per shard): summed with the rest, it flags the sample on whichever rank finishes it. */
 int snpm_batch_reduce_buffer(snpm_batch *b, void **dev_ptr, int64_t *n_doubles);
 /* ---- 8(e): the cross-GPU sum as a one-shot reduce over peer memory (NVLink / NVSwitch), one process per GPU -------------
  * Every rank exports the reduce buffer of its batch (snpm_batch_ipc_export: a 64-byte CUDA IPC handle; the buffer holds

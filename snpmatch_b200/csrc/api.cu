@@ -1044,6 +1044,8 @@ static int batch_join(snpm_batch *b, int algo) {
     if (algo == 0) algo = (n / S) * 8 >= db->n_rows ? 2 : 1;
     if (b->grouped) algo = 1;                                    // markers are not in position order
     const int64_t *filter = b->has_filter ? b->d_filter.as<int64_t>() : nullptr;
+    // the grouping's overflow flags, read by k_combine_grouped: zero also for a batch without markers
+    if (b->coded && S > 0) SNPM_CUDA(cudaMemsetAsync(b->d_group_overflow.p, 0, size_t(S) * 4, st));
     if (n_tiles > 0) {
         if (algo == 2)
             k_join_mergepath<<<int(n_tiles), 256, 0, st>>>(b->d_chrom.as<int32_t>(), b->d_pos.as<int32_t>(), n, b->d_off.as<int64_t>(), S,
@@ -1068,7 +1070,6 @@ static int batch_join(snpm_batch *b, int algo) {
         SNPM_KERNEL_CHECK();
         if (b->coded) {
             unsigned long long *hash = b->d_hash.as<unsigned long long>();
-            SNPM_CUDA(cudaMemsetAsync(b->d_group_overflow.p, 0, size_t(S) * 4, st));
             SNPM_CUDA(cudaMemsetAsync(hash, 0, size_t(S) * GH_SLOTS * 8, st));
             if (b->key_bits <= 32)
                 k_scatter_pairs_coded<uint32_t><<<int(n_tiles), SC_THREADS, 0, st>>>(b->d_match_row.as<int32_t>(), n, b->d_tile_off.as<int32_t>(), b->d_codes.as<uint16_t>(),
@@ -1296,7 +1297,7 @@ int snpm_batch_run(snpm_batch *b, int skip_db_hets, int mode) {
         rec(b, SNPM_EV_SCORE);
         dim3 cgrid((a.a_pad + 31) / 32, unsigned(b->S));
         k_combine_grouped<<<cgrid, 32 * CG_PARTS, 0, st>>>(a.part_score, b->d_part_int.as<int32_t>(), a.a_pad, db->stride, db->n_acc, a.seg_off, a.mstart,
-                                                 b->d_red.as<double>());
+                                                 b->d_group_overflow.as<int>(), b->d_red.as<double>());
         SNPM_KERNEL_CHECK();
         b->launches += 1;
         rec(b, SNPM_EV_COMBINE);
@@ -1342,7 +1343,7 @@ int snpm_batch_run(snpm_batch *b, int skip_db_hets, int mode) {
         rec(b, SNPM_EV_SCORE);
         dim3 cgrid((a.a_pad + 31) / 32, unsigned(b->S));
         k_combine_grouped<<<cgrid, 32 * CG_PARTS, 0, st>>>(a.part_score, b->d_part_int.as<int32_t>(), a.a_pad, db->stride, db->n_acc, a.seg_off, a.mstart,
-                                                 b->d_red.as<double>());
+                                                 nullptr, b->d_red.as<double>());
         SNPM_KERNEL_CHECK();
         b->launches += 1;
         rec(b, SNPM_EV_COMBINE);
@@ -1399,6 +1400,8 @@ int snpm_batch_run(snpm_batch *b, int skip_db_hets, int mode) {
 int snpm_batch_epilogue(snpm_batch *b) {
     if (!b) return fail(SNPM_E_ARG, "snpm_batch_epilogue: NULL batch");
     if (!b->ran) return fail(SNPM_E_STATE, "snpm_batch_epilogue: run the batch first");
+    // k_grouped_finalize turns F into I + F in place: a second pass over the same totals would add I again
+    if (b->grouped && b->epilogue_done) return fail(SNPM_E_STATE, "snpm_batch_epilogue: the epilogue of a grouped batch runs once per run");
     snpm_db *db = b->db;
     SNPM_CUDA(cudaSetDevice(db->device));
     const int64_t r0 = b->range0(), rn = b->rangen();
@@ -1411,8 +1414,7 @@ int snpm_batch_epilogue(snpm_batch *b) {
             SNPM_TRY(b->d_guard.ensure(size_t(b->S) * 4));
             SNPM_CUDA(cudaMemsetAsync(b->d_guard.as<int32_t>() + r0, 0, size_t(rn) * 4, db->stream));
             dim3 fgrid((db->n_acc + 255) / 256, unsigned(rn));
-            k_grouped_finalize<<<fgrid, 256, 0, db->stream>>>(b->d_red.as<double>() + r0 * pitch, db->n_acc, b->d_guard.as<int32_t>() + r0,
-                                                              b->coded ? b->d_group_overflow.as<int>() + r0 : nullptr);
+            k_grouped_finalize<<<fgrid, 256, 0, db->stream>>>(b->d_red.as<double>() + r0 * pitch, db->n_acc, b->d_guard.as<int32_t>() + r0);
             SNPM_KERNEL_CHECK();
             b->launches += 1;
         }

@@ -473,13 +473,16 @@ __global__ void __launch_bounds__(256) k_expand_runs(const uint32_t *__restrict_
 }
 
 // ---- combine: totals of the segment partials of one sample ----------------------------------------------
-// red row layout in grouped mode [3*n_acc + 2]: F[n_acc] | ninfo[n_acc] | matched pairs | y>n violations | I[n_acc]
-// (the first 2*n_acc + 2 entries are laid out as in k_combine; k_grouped_finalize turns F into the score in place)
+// red row layout in grouped mode [3*n_acc + 2]: F[n_acc] | ninfo[n_acc] | matched pairs | overflow, then y>n violations | I[n_acc]
+// (the first 2*n_acc + 2 entries are laid out as in k_combine; k_grouped_finalize turns F into the score in place).  Slot
+// 2*n_acc + 1 carries the grouping's overflow flag of this shard (coded batches; 0 otherwise) until k_grouped_finalize has read
+// it; k_epilogue then stores the y>n count there.  The flag travels through the cross-GPU sum with the totals, so the rank that
+// finishes a sample sees an overflow of any rank.
 constexpr int CG_PARTS = 8;           // warps of a CTA = contiguous parts of a sample's segments, summed in part order at the end
 __global__ void __launch_bounds__(32 * CG_PARTS) k_combine_grouped(const double *__restrict__ part_score, const int32_t *__restrict__ part_int,
                                                                    int32_t a_pad, int32_t stride, int32_t n_acc,
                                                                    const int32_t *__restrict__ seg_off, const int32_t *__restrict__ mstart,
-                                                                   double *__restrict__ red) {
+                                                                   const int *__restrict__ overflow, double *__restrict__ red) {
     // thread (x, y) -> position p = 32 * blockIdx.x + x of the lane-major segment partials ([lane b][word w], p = b * stride + w:
     // coalesced reads), part y of the segments.  The order of the fp64 adds is fixed (segments in order inside a part, parts in
     // order), so results are reproducible run to run.
@@ -539,7 +542,7 @@ __global__ void __launch_bounds__(32 * CG_PARTS) k_combine_grouped(const double 
         }
         if (p == 0) {
             row[2 * n_acc] = double(mstart[s + 1] - mstart[s]);
-            row[2 * n_acc + 1] = 0.0;
+            row[2 * n_acc + 1] = (overflow != nullptr && overflow[s]) ? 1.0 : 0.0;
         }
     }
 }
@@ -651,15 +654,15 @@ __global__ void __launch_bounds__(32) k_wait_peers_done(const uint32_t *own_flag
 // stored so that the epilogue's int(score) gives exactly that, and cells whose F lies within the summation-error bound of
 // an integer k >= 1 are counted in guard[s]: for them the reference's own rounding decides, so the caller re-scores the
 // sample in reference order.  Runs after the cross-GPU reduce, on totals.
-__global__ void __launch_bounds__(256) k_grouped_finalize(double *__restrict__ red, int32_t n_acc, int32_t *__restrict__ guard,
-                                                          const int *__restrict__ overflow = nullptr) {
+__global__ void __launch_bounds__(256) k_grouped_finalize(double *__restrict__ red, int32_t n_acc, int32_t *__restrict__ guard) {
     const int s = blockIdx.y;
     const int acc = blockIdx.x * blockDim.x + threadIdx.x;
     if (acc >= n_acc) return;
-    // a sample whose weight triples did not fit the dense ids of the device grouping (group_sort.cuh) was scored with ids
-    // folded together: flag it like a guard hit, the caller re-scores it in reference order
-    if (acc == 0 && overflow != nullptr && overflow[s]) atomicAdd(guard + s, 1);
     double *row = red + int64_t(s) * (3 * int64_t(n_acc) + 2);
+    // a sample whose weight triples did not fit the dense ids of the device grouping (group_sort.cuh) on some shard was scored
+    // with ids folded together: flag it like a guard hit, the caller re-scores it in reference order.  The flag is the sum
+    // over the shards of slot 2*n_acc + 1 (k_combine_grouped), not this rank's own.
+    if (acc == 0 && row[2 * n_acc + 1] > 0.0) atomicAdd(guard + s, 1);
     const double f = row[acc], ii = row[2 * n_acc + 2 + acc], m = row[2 * n_acc];
     // |reference - exact| <= (1000 + 2 + m/1000) u (I+F) for its chunked sequential sums (SURVEY A.2), the same bound holds
     // for the sums above; u = 2^-53.  Factor 4 covers both plus slack.

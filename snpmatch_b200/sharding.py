@@ -104,7 +104,8 @@ def allreduce_batch(batch, dist, device):
 
 # ---- grouped counting kernel (csrc/grouped.cuh): the score travels as an exact integer part I and a fractional part F ----
 def grouped_row_len(n_acc):
-    """f64 per sample in the reduce buffer of a grouped batch: F[n_acc] | ninfo[n_acc] | matched pairs | y>n count | I[n_acc]."""
+    """f64 per sample in the reduce buffer of a grouped batch: F[n_acc] | ninfo[n_acc] | matched pairs | overflow flag (the y>n
+    count after the epilogue) | I[n_acc]."""
     return 3 * n_acc + 2
 
 
@@ -129,13 +130,15 @@ def grouped_partials(wei, codes, skip_db_hets=False):
     return F, I, (codes >= 0).sum(axis=0).astype(np.int64)
 
 
-def pack_grouped_rows(F, ninfo, m, I):
+def pack_grouped_rows(F, ninfo, m, I, overflow=0):
+    """overflow: per sample, 1 when this shard's device grouping ran out of dense ids (csrc/group_sort.cuh), else 0."""
     F = np.atleast_2d(np.asarray(F, dtype=np.float64))
     S, A = F.shape
     out = np.zeros((S, grouped_row_len(A)), dtype=np.float64)
     out[:, :A] = F
     out[:, A:2 * A] = np.atleast_2d(ninfo)
     out[:, 2 * A] = np.asarray(m).reshape(S)
+    out[:, 2 * A + 1] = np.broadcast_to(np.asarray(overflow, dtype=np.float64), (S,))
     out[:, 2 * A + 2:] = np.atleast_2d(I)
     return out
 
@@ -144,13 +147,14 @@ def finalize_grouped(buf, n_acc):
     """NumPy restatement of k_grouped_finalize on (all-reduced) totals: returns (score f64[S,A], matches int64[S,A],
     ninfo int64[S,A], m int64[S], guard bool[S,A]).  matches = I + floor(F): the reference's fp64 sum is >= I (monotone
     rounding of non-negative terms) and < I + F + eps, so its truncation can only differ where F lies within the summation
-    error bound of an integer k >= 1 — those cells are flagged for re-scoring in reference order."""
+    error bound of an integer k >= 1 — those cells are flagged for re-scoring in reference order.  A sample whose summed overflow
+    slot is > 0 (some shard folded its weight triples together) is unreliable as a whole: all its cells are flagged."""
     buf = np.asarray(buf, dtype=np.float64).reshape(-1, grouped_row_len(n_acc))
     F, ninfo, m, I = buf[:, :n_acc], buf[:, n_acc:2 * n_acc], buf[:, 2 * n_acc], buf[:, 2 * n_acc + 2:]
     depth = 1010.0 + m[:, None] / 500.0
     g = 4.0 * depth * 1.1102230246251565e-16 * (I + F + 1.0)
     k = np.rint(F)
-    guard = (k >= 1.0) & (np.abs(F - k) <= g)
+    guard = ((k >= 1.0) & (np.abs(F - k) <= g)) | (buf[:, 2 * n_acc + 1] > 0.0)[:, None]
     want = I + np.floor(F)
     v = I + F
     bump = np.floor(v) != want
