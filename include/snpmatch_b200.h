@@ -366,10 +366,12 @@ int snpm_cross_window_genotypes(int device, const int64_t *par_idx, const int64_
 
 /* ---- A9: batched scoring on a shared marker panel (tensor cores) ------------------------------
  * No reference symbol: the reference scores many samples as one process per sample (README.md:9).  S samples of CALLED
- * genotypes that share K markers (panel_rows int64[K], global rows; codes uint8 [S,K]: 0 ref, 1 alt, 2 het, 3 = sample
+ * genotypes that share K markers (panel_rows int64[K], global rows; codes uint8 [S,K]: 0 ref, 1 alt, 2 het, 3 or more = sample
  * lacks the marker) are scored against every accession as one one-hot int8 GEMM on tcgen05 (int32 accumulation, exact):
  * score/ninfo int64 [S,A] equal what snpm_score returns per sample with one-hot weights; prob/L/LR f64 [S,A] optional.
+ * 1 <= S <= SNPM_PANEL_MAX_SAMPLES (one launch row per 64 samples, at most 65 535 rows); more is SNPM_E_ARG.
  * ms_gemm (optional) receives the device time of the GEMM kernel. */
+#define SNPM_PANEL_MAX_SAMPLES (65535 * 64)
 int snpm_score_shared_panel(snpm_db *db, const int64_t *panel_rows, int64_t K, const uint8_t *codes, int64_t S, int skip_db_hets,
                             int64_t *score, int64_t *ninfo, double *prob, double *L, double *LR, float *ms_gemm);
 

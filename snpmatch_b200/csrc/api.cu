@@ -1,5 +1,6 @@
 // C ABI of libsnpmatch_b200 (include/snpmatch_b200.h): handle lifecycle, uploads, kernel launches.
 #include "common.cuh"
+#include <atomic>
 #include <memory>
 #include <new>
 #include "pack.cuh"
@@ -36,13 +37,25 @@ struct DeviceGuard {
     }
 };
 
+// A kernel's dynamic shared-memory limit is an attribute of the function in the CURRENT device's context, so a kernel that asks
+// for more than 48 KB needs it set on every device it runs on (a Database per GPU in one process).  Set once per (kernel,
+// device): bit d of `done` = set on device d (devices past 63 set it on every call).
+template <auto Kernel>
+static cudaError_t smem_attr(int bytes) {
+    static std::atomic<uint64_t> done{0};
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    const uint64_t bit = dev < 64 ? uint64_t(1) << dev : 0;
+    if (done.load(std::memory_order_acquire) & bit) return cudaSuccess;
+    e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e == cudaSuccess) done.fetch_or(bit, std::memory_order_release);
+    return e;
+}
+
 template <bool SKIP, int NW, int MINB>
 static int launch_score_t(cudaStream_t st, const ScoreArgs &a, dim3 grid, dim3 block, size_t smem) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        SNPM_CUDA(cudaFuncSetAttribute(k_score_segments<SKIP, NW, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        attr_set = true;
-    }
+    SNPM_CUDA((smem_attr<k_score_segments<SKIP, NW, MINB>>(200 * 1024)));
     k_score_segments<SKIP, NW, MINB><<<grid, block, smem, st>>>(a);
     SNPM_KERNEL_CHECK();
     return SNPM_OK;
@@ -1114,11 +1127,7 @@ static int batch_group_sort_t(snpm_batch *b) {
     const int32_t *mstart = b->d_mstart.as<int32_t>(), *tsample = b->d_tile_sample.as<int32_t>(), *tfirst = b->d_tile_first.as<int32_t>();
     uint32_t *hist = b->d_tile_hist.as<uint32_t>();
     int2 *range = reinterpret_cast<int2 *>(hist + (size_t(tiles) << 11));
-    static bool gattr = false;
-    if (!gattr) {
-        SNPM_CUDA(cudaFuncSetAttribute(k_group_place, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-        gattr = true;
-    }
+    SNPM_CUDA(smem_attr<k_group_place>(64 * 1024));
     KeyT *gkeys = b->d_gkeys.as<KeyT>();
     k_group_rank<KeyT><<<int(b->S), 1024, 0, st>>>(b->d_hash.as<unsigned long long>(), b->d_wtable.as<double>(), b->code_bits, b->d_slot_gid.as<uint16_t>(),
                                                    b->d_ngroups.as<int32_t>(), gkeys, b->d_gw.as<double4>(), b->d_group_overflow.as<int>());
@@ -1135,12 +1144,7 @@ static int batch_group_sort_t(snpm_batch *b) {
     const bool want = force ? !strcmp(force, "sample") : (n_max <= 32768 || b->S >= 128);
     if (fits && want) {
         // every sample's counters fit shared memory: ids, offsets, placement, block words and segment costs in one kernel per sample
-        static bool sattr = false;
-        if (!sattr) {
-            SNPM_CUDA(cudaFuncSetAttribute(k_group_sample<uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(GP_SMEM)));
-            SNPM_CUDA(cudaFuncSetAttribute(k_group_sample<uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(GP_SMEM)));
-            sattr = true;
-        }
+        SNPM_CUDA(smem_attr<k_group_sample<KeyT>>(int(GP_SMEM)));
         const size_t ncap = size_t(std::max<int64_t>(b->nseg_cap, 1));
         int32_t *cost = reinterpret_cast<int32_t *>(b->d_blk_chg.as<unsigned long long>() + ncap * size_t(b->gchunk / GR_BLOCK));
         int32_t *buckets = cost + ncap;
@@ -1211,11 +1215,7 @@ static int launch_grouped2(snpm_batch *b, bool skip_db_hets) {
     const int grid = int(std::min<int64_t>(db->n_sm, ceil_div64(n_items, g.teams)));
 #define G2_LAUNCH(SK, WXV)                                                                                                        \
     do {                                                                                                                          \
-        static bool attr_ = false;                                                                                                \
-        if (!attr_) {                                                                                                             \
-            SNPM_CUDA(cudaFuncSetAttribute(k_score_grouped2<SK, WXV, ring>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024)); \
-            attr_ = true;                                                                                                         \
-        }                                                                                                                         \
+        SNPM_CUDA((smem_attr<k_score_grouped2<SK, WXV, ring>>(226 * 1024)));                                                    \
         k_score_grouped2<SK, WXV, ring><<<grid, G2_THREADS, smem, st>>>(g);                                                       \
     } while (0)
     if (g.wx == G2_WX) {
@@ -1317,26 +1317,22 @@ int snpm_batch_run(snpm_batch *b, int skip_db_hets, int mode) {
             g.wx = ((db->stride + nsl - 1) / nsl + 1) & ~1;          // even: neighbouring threads copy 16-byte pairs of columns
             g.spc = std::min(GR_THREADS / g.wx, GR_MAX_TEAMS);
             const size_t gsmem = size_t(g.spc) * grouped_team_smem(g.wx, g.chunk);
-            static bool gr_attr = false;
-            if (!gr_attr) {
-                SNPM_CUDA(cudaFuncSetAttribute(k_score_grouped<true, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-                SNPM_CUDA(cudaFuncSetAttribute(k_score_grouped<false, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-                SNPM_CUDA(cudaFuncSetAttribute(k_score_grouped<true, GR_MAX_WX>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-                SNPM_CUDA(cudaFuncSetAttribute(k_score_grouped<false, GR_MAX_WX>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-                gr_attr = true;
-            }
             int64_t jmax = 0;
             for (int64_t smp = 0; smp < b->S; ++smp)
                 jmax = std::max(jmax, ceil_div64(b->h_off[size_t(smp) + 1] - b->h_off[size_t(smp)], b->gchunk));
             g.jmax = int32_t(jmax);
             dim3 ggrid(unsigned(ceil_div64(b->S * jmax, g.spc)), unsigned((db->stride + g.wx - 1) / g.wx));
+#define GR_LAUNCH(SK, WXV)                                                     \
+    do {                                                                       \
+        SNPM_CUDA((smem_attr<k_score_grouped<SK, WXV>>(220 * 1024)));          \
+        k_score_grouped<SK, WXV><<<ggrid, GR_THREADS, gsmem, st>>>(g);         \
+    } while (0)
             if (g.wx == GR_MAX_WX) {       // the 1135-accession row: addresses known at compile time
-                if (skip_db_hets) k_score_grouped<true, GR_MAX_WX><<<ggrid, GR_THREADS, gsmem, st>>>(g);
-                else k_score_grouped<false, GR_MAX_WX><<<ggrid, GR_THREADS, gsmem, st>>>(g);
+                if (skip_db_hets) GR_LAUNCH(true, GR_MAX_WX); else GR_LAUNCH(false, GR_MAX_WX);
             } else {
-                if (skip_db_hets) k_score_grouped<true, 0><<<ggrid, GR_THREADS, gsmem, st>>>(g);
-                else k_score_grouped<false, 0><<<ggrid, GR_THREADS, gsmem, st>>>(g);
+                if (skip_db_hets) GR_LAUNCH(true, 0); else GR_LAUNCH(false, 0);
             }
+#undef GR_LAUNCH
             SNPM_KERNEL_CHECK();
             b->launches += 1;
         }
@@ -1369,14 +1365,13 @@ int snpm_batch_run(snpm_batch *b, int skip_db_hets, int mode) {
         h.spc = spc;
         dim3 hgrid(unsigned(ceil_div64(b->nseg_cap, spc)), unsigned((db->stride + wx - 1) / wx));
         const size_t hsmem = size_t(spc) * SNPM_CHUNK_ROWS * 5;
-        static bool hc_attr = false;
-        if (!hc_attr) {
-            SNPM_CUDA(cudaFuncSetAttribute(k_score_hard<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-            SNPM_CUDA(cudaFuncSetAttribute(k_score_hard<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-            hc_attr = true;
+        if (skip_db_hets) {
+            SNPM_CUDA(smem_attr<k_score_hard<true>>(64 * 1024));
+            k_score_hard<true><<<hgrid, HC_THREADS, hsmem, st>>>(h);
+        } else {
+            SNPM_CUDA(smem_attr<k_score_hard<false>>(64 * 1024));
+            k_score_hard<false><<<hgrid, HC_THREADS, hsmem, st>>>(h);
         }
-        if (skip_db_hets) k_score_hard<true><<<hgrid, HC_THREADS, hsmem, st>>>(h);
-        else k_score_hard<false><<<hgrid, HC_THREADS, hsmem, st>>>(h);
         SNPM_KERNEL_CHECK();
         b->launches += 2;
     } else {
@@ -2009,7 +2004,7 @@ void snpm_panel_destroy(snpm_panel *p) {
 
 int snpm_panel_score(snpm_panel *p, const uint8_t *codes, int packed, int64_t S, int32_t *score, int32_t *ninfo, double *prob, double *L,
                      double *LR, float *ms) {
-    if (!p || S < 1 || S > (1 << 22) || (p->K > 0 && !codes) || !score || !ninfo) return fail(SNPM_E_ARG, "snpm_panel_score: bad arguments");
+    if (!p || S < 1 || S > SNPM_PANEL_MAX_SAMPLES || (p->K > 0 && !codes) || !score || !ninfo) return fail(SNPM_E_ARG, "snpm_panel_score: bad arguments");
     snpm_db *db = p->db;
     SNPM_CUDA(cudaSetDevice(db->device));
     cudaStream_t st = db->stream;
@@ -2045,15 +2040,14 @@ int snpm_panel_score(snpm_panel *p, const uint8_t *codes, int packed, int64_t S,
     g.a_tiled = p->d_at.as<unsigned char>(); g.b_tiled = p->d_bt.as<unsigned char>(); g.n_kb = p->n_kb; g.m_blocks = m_blocks; g.n_blocks = p->n_blocks;
     g.S = int32_t(S); g.out_score = p->d_os.as<int32_t>(); g.out_ninfo = p->d_on.as<int32_t>(); g.ld_out = ld_out;
     const size_t smem = size_t(OG_STAGES) * (OG_A_TILE + OG_B_TILE) + 1024;
-    static bool og_attr = false;
-    if (!og_attr) { SNPM_CUDA(cudaFuncSetAttribute(k_onehot_gemm, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem))); og_attr = true; }
+    SNPM_CUDA(smem_attr<k_onehot_gemm>(int(smem)));
     dim3 grid((unsigned)std::min(m_blocks * p->n_blocks, db->n_sm));      // persistent: one CTA per SM walks the tiles
     SNPM_CUDA(cudaEventRecord(p->ev[1], st));
     k_onehot_gemm<<<grid, OG_THREADS, smem, st>>>(g);
     SNPM_KERNEL_CHECK();
     SNPM_CUDA(cudaEventRecord(p->ev[2], st));
     if (like) {
-        dim3 tgrid((A + 255) / 256, unsigned(S));
+        dim3 tgrid(unsigned(S), unsigned(std::min((A + 255) / 256, 65535)));      // samples on x: any S the API takes
         k_onehot_totals<<<tgrid, 256, 0, st>>>(g.out_score, g.out_ninfo, ld_out, A, int32_t(K), p->d_red.as<double>());
         SNPM_CUDA(launch_epilogue(st, S, p->d_red.as<double>(), 2 * int64_t(A) + 2, A, 1, 0, 0.0, p->d_m.as<int64_t>(), p->d_n64.as<int64_t>(),
                                   p->d_p.as<double>(), p->d_l.as<double>(), p->d_lr.as<double>()));
@@ -2079,7 +2073,7 @@ int snpm_panel_score(snpm_panel *p, const uint8_t *codes, int packed, int64_t S,
 // one-shot form: panel operand, scoring, int64 results
 int snpm_score_shared_panel(snpm_db *db, const int64_t *panel_rows, int64_t K, const uint8_t *codes, int64_t S, int skip_db_hets,
                             int64_t *score, int64_t *ninfo, double *prob, double *L, double *LR, float *ms_gemm) {
-    if (!db || K < 0 || S < 1 || S > (1 << 22) || (K > 0 && (!panel_rows || !codes)) || !score || !ninfo)
+    if (!db || K < 0 || S < 1 || S > SNPM_PANEL_MAX_SAMPLES || (K > 0 && (!panel_rows || !codes)) || !score || !ninfo)
         return fail(SNPM_E_ARG, "snpm_score_shared_panel: bad arguments");
     snpm_panel *p = nullptr;
     SNPM_TRY(snpm_panel_create(db, panel_rows, K, skip_db_hets, &p));

@@ -253,17 +253,17 @@ __global__ void k_onehot_mask_tail(uint8_t *__restrict__ codes, int64_t S, int64
     if (s < S) codes[s * pitch + (K >> 2)] |= uint8_t(0xFFu << (2 * (K & 3)));
 }
 
-// int32 GEMM outputs -> the f64 reduce rows the likelihood epilogue reads (score | ninfo | markers | 0)
+// int32 GEMM outputs -> the f64 reduce rows the likelihood epilogue reads (score | ninfo | markers | 0).  Sample = blockIdx.x (grid
+// x takes 2^31 - 1, grid y only 65 535); the CTAs along y stride over the accessions.
 __global__ void __launch_bounds__(256) k_onehot_totals(const int32_t *__restrict__ out_score, const int32_t *__restrict__ out_ninfo,
                                                        int32_t ld_out, int32_t n_acc, int32_t k_markers, double *__restrict__ red) {
-    const int s = blockIdx.y;
-    const int acc = blockIdx.x * blockDim.x + threadIdx.x;
+    const int s = blockIdx.x;
     double *row = red + int64_t(s) * (2 * int64_t(n_acc) + 2);
-    if (acc < n_acc) {
+    for (int acc = blockIdx.y * blockDim.x + threadIdx.x; acc < n_acc; acc += gridDim.y * blockDim.x) {
         row[acc] = double(out_score[int64_t(s) * ld_out + acc]);
         row[n_acc + acc] = double(out_ninfo[int64_t(s) * ld_out + acc]);
     }
-    if (acc == 0) {
+    if (blockIdx.y == 0 && threadIdx.x == 0) {
         row[2 * n_acc] = double(k_markers);
         row[2 * n_acc + 1] = 0.0;
     }

@@ -450,14 +450,14 @@ class Database(object):
 
 
 def pack_codes2(codes):
-    """uint8 codes [S,K] (0 ref, 1 alt, 2 het, 3 absent) -> 2-bit packed rows uint8 [S, ceil(K/4)] (marker k in bits 2(k&3) of
-    byte k >> 2; the spare bits of the last byte read as absent)."""
+    """uint8 codes [S,K] (0 ref, 1 alt, 2 het, 3 or more absent, as in the unpacked form) -> 2-bit packed rows uint8
+    [S, ceil(K/4)] (marker k in bits 2(k&3) of byte k >> 2; the spare bits of the last byte read as absent)."""
     codes = np.asarray(codes, dtype=np.uint8)
     S, K = codes.shape
     pad = (-K) % 4
     if pad:
         codes = np.concatenate([codes, np.full((S, pad), 3, np.uint8)], axis=1)
-    c = (codes & 3).reshape(S, -1, 4)
+    c = np.minimum(codes, 3).reshape(S, -1, 4)
     return np.ascontiguousarray(c[:, :, 0] | (c[:, :, 1] << 2) | (c[:, :, 2] << 4) | (c[:, :, 3] << 6))
 
 
