@@ -352,6 +352,25 @@ int snpm_batch_f1_pairs(snpm_batch *b, const int32_t *acc_idx, int32_t n_top,
 int snpm_pair_match_counts(int device, const int64_t *idx1, const int64_t *idx2, int64_t m, const int32_t *chrom1, const int32_t *gt1,
                            int64_t n1, const int32_t *gt2, int64_t n2, int32_t n_chr, int64_t *common, int64_t *matches);
 
+/* ---- 8(f)-3 for many samples: every pair's shared-marker identity in one tensor-core pass -------------------------
+ * pairwiseScore (snpmatch.py:270-309) for all S x S pairs at once: its counting loop (:291-297) over the markers two
+ * samples share becomes one-hot int8 GEMMs (tcgen05, int32 accumulation, exact) over the columns of the union of all
+ * samples' markers.  Sample s has the markers offsets[s] .. offsets[s+1]-1 (offsets int64[S+1], offsets[0] = 0); col
+ * int32[n] = the union column of each (strictly ascending inside a sample, < K), cls uint8[n] = the id of its GT string
+ * (< n_cls, 1 <= n_cls <= 8: identical strings, identical ids).  chr_start int64[C+1] = the column range of each chromosome
+ * (non-decreasing from 0 to K).  Out: common / same int32 [C,S,S] = per chromosome the columns samples i and j both have,
+ * and how many of those carry the same class in both.
+ * The columns are walked chromosome by chromosome in chunks of chunk_markers columns (0 = as many as fit
+ * SNPM_PAIR_CHUNK_BYTES of operand tiles); a chunk never spans two chromosomes.  Only the CSR crosses PCIe (about 5 bytes
+ * per marker); the operands of a chunk are expanded from it on the device.  Refused before any allocation: S outside
+ * 1..SNPM_PAIR_MAX_SAMPLES, K >= 2^31, a chromosome of 2^31 columns or more (the counts are int32), and malformed input
+ * (the error names the sample).  ms (optional) float[3]: device time of the operand expansion with its memsets, of the
+ * GEMMs, and of the whole call including the copies. */
+#define SNPM_PAIR_MAX_SAMPLES 8192          /* bounds the [C,S,S] outputs: 512 MB of both counts per chromosome at 8192 */
+#define SNPM_PAIR_CHUNK_BYTES ((int64_t)1 << 30)
+int snpm_pair_matrix(int device, int64_t S, const int64_t *offsets, const int32_t *col, const uint8_t *cls, int32_t n_cls, int64_t K,
+                     const int64_t *chr_start, int32_t C, int64_t chunk_markers, int32_t *common, int32_t *same, float *ms);
+
 /* ---- 8(f)-4: genotype_cross -----------------------------------------------------------------
  * The window loop of GenotypeCross.genotype_cross (genotype_cross.py:210-241): for every genome window w and every sample s
  * of a multi-sample VCF, over the matched pairs k in [win_start[w], win_start[w+1]) (par_idx into the parents' segregating

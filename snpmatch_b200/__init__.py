@@ -61,10 +61,11 @@ def snpmatch_cross(args):
     csmatch.potatoCrossIdentifier(args)
 
 
-def read_sample_list(list_file, out_prefix):
+def read_sample_list(list_file, out_prefix, default_name=None):
     """`inbred --samples` / `cross --samples`: one sample file per line, optionally a tab and the sample's output prefix (default
     <out_prefix>.<file name up to its first '.'>).  Blank lines are skipped.  Returns [(path, prefix)]; dies on a missing
-    file, an empty list or two samples with the same prefix."""
+    file, an empty list or two samples with the same prefix.  `pairsnp --samples` reads the second column as the sample's
+    label: default_name(path) gives it when the line has none."""
     check_file(list_file)
     samples = []
     with open(list_file) as fh:
@@ -74,7 +75,10 @@ def read_sample_list(list_file, out_prefix):
                 continue
             cols = line.split("\t")
             path = cols[0].strip()
-            prefix = cols[1].strip() if len(cols) > 1 and cols[1].strip() else out_prefix + "." + os.path.basename(path).split(".")[0]
+            if len(cols) > 1 and cols[1].strip():
+                prefix = cols[1].strip()
+            else:
+                prefix = default_name(path) if default_name else out_prefix + "." + os.path.basename(path).split(".")[0]
             samples.append((path, prefix))
     if not samples:
         die("sample list is empty: " + list_file)
@@ -83,7 +87,7 @@ def read_sample_list(list_file, out_prefix):
     seen = {}
     for path, prefix in samples:
         if prefix in seen:
-            die("samples %s and %s have the same output prefix %s" % (seen[prefix], path, prefix))
+            die("samples %s and %s have the same %s %s" % (seen[prefix], path, "label" if default_name else "output prefix", prefix))
         seen[prefix] = path
     return samples
 
@@ -97,6 +101,13 @@ def snpmatch_parser(args):
 
 
 def snpmatch_paircomparions(args):
+    if args.get('samples'):
+        if args['inFile_1'] or args['inFile_2']:
+            die("--samples compares every pair of the list; it cannot be combined with -i / -j")
+        samples = read_sample_list(args['samples'], args['outFile'], default_name=os.path.basename)
+        from .core import snpmatch
+        snpmatch.pairwiseScoreMany(args, samples)
+        return
     check_file(args['inFile_1'])
     check_file(args['inFile_2'])
     from .core import snpmatch
@@ -177,9 +188,14 @@ def get_options(description, version_message):
     gc.add_argument("-v", "--verbose", action="store_true", dest="logDebug", default=False, help="log at DEBUG level")
     gc.set_defaults(func=genotype_cross)
 
-    pair = sub.add_parser('pairsnp', help="agreement of the genotype calls two samples share")
+    pair = sub.add_parser('pairsnp', help="agreement of the genotype calls two samples (or every pair of many samples) share")
     pair.add_argument("-i", "--input_file_1", dest="inFile_1", help="first sample (VCF/BED/npz)")
     pair.add_argument("-j", "--input_file_2", dest="inFile_2", help="second sample (VCF/BED/npz)")
+    pair.add_argument("--samples", dest="samples", default=None,
+                      help="text file listing many samples, one path per line (VCF/BED/npz), optionally a tab and that sample's label "
+                           "(default: the file name); every pair is compared in one GPU pass: <-o>.identity.tsv, <-o>.common.tsv")
+    pair.add_argument("--pairs_json", action="store_true", dest="pairs_json", default=False,
+                      help="with --samples: also <-o>.pairs.jsonl, one line per pair with the statistics -i/-j writes to .matches.json")
     pair.add_argument("-d", "--hdf5_file", dest="hdf5File", default=None, help=db_help)
     pair.add_argument("-v", "--verbose", action="store_true", dest="logDebug", default=False, help="log at DEBUG level")
     pair.add_argument("-o", "--output", dest="outFile", default="pairsnp", help="output prefix (<prefix>.matches.json)")

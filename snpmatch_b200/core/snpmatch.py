@@ -554,3 +554,226 @@ def pairwiseScore(inFile_1, inFile_2, logDebug, outFile=None, hdf5File=None, dev
         with open(outFile + ".matches.json", "w") as fh:
             json.dump(snpmatch_stats, fh, sort_keys=True, indent=4)
     return snpmatch_stats
+
+
+# ---- pairsnp for many samples ----------------------------------------------------------------------------------------------
+def _chromosome_codes(inp):
+    """(raw names, codes into them, normalised names) of a sample's markers: every 'chr' deleted, any case (parsers.py:161)."""
+    codes, raw = labels.factorize(np.asarray(inp.chrs))
+    norm = np.array([snp_genotype._CHR_RE.sub("", str(u)) for u in raw], dtype="str") if len(raw) else np.zeros(0, dtype="U1")
+    return raw, codes, norm
+
+
+def _no_repeats(cid, pos, n_names):
+    """True when no (chromosome, position) repeats: the common case (one run per chromosome, ascending positions) in O(n)."""
+    if len(cid) < 2:
+        return True
+    run = cid[1:] == cid[:-1]
+    if np.count_nonzero(~run) + 1 == n_names and bool(np.all(pos[1:][run] > pos[:-1][run])):
+        return True
+    key = np.sort((cid.astype(np.int64) << 32) | (pos + 2**31))
+    return not bool(np.any(key[1:] == key[:-1]))
+
+
+def gt_classes(gts):
+    """Class of every GT string (equal strings, equal classes) and the distinct strings, for the concatenated calls of all
+    samples.  Strings of up to three characters are compared as one integer each (21 bits per character)."""
+    gts = np.asarray(gts)
+    if gts.dtype.kind != "U":
+        gts = gts.astype("U")
+    if len(gts) and gts.dtype.itemsize <= 12:
+        v = np.ascontiguousarray(gts).view(np.uint32).reshape(len(gts), -1)
+        key = v[:, 0].astype(np.uint64)
+        for k in range(1, v.shape[1]):
+            key |= v[:, k].astype(np.uint64) << np.uint64(21 * k)
+        codes, uniq = pd.factorize(key)
+        first = np.full(len(uniq), len(gts), np.int64)
+        np.minimum.at(first, codes, np.arange(len(gts)))
+        return codes.astype(np.int64), gts[first]
+    return labels.factorize(gts)
+
+
+def build_pair_columns(keys, counts, cls, device, restrict=None):
+    """The union of all samples' markers and each marker's column in it, sorted on `device` (a torch device).
+    keys int64[n] = chromosome index << 32 | (position + 2^31), sample after sample (counts[s] markers each, no key twice in a
+    sample); cls uint8[n] the marker's GT-string class.  restrict(union keys) -> bool mask keeps only those columns (the
+    positions of a database).  Returns (offsets int64[S+1], col int32[m], cls uint8[m], union keys int64[K]) with every
+    sample's markers in column order; columns are ordered by (chromosome, position)."""
+    import torch
+    counts = np.asarray(counts, dtype=np.int64)
+    kt = torch.as_tensor(np.ascontiguousarray(keys, dtype=np.int64)).to(device)
+    ct = torch.as_tensor(np.ascontiguousarray(cls, dtype=np.uint8)).to(device)
+    sample = torch.repeat_interleave(torch.arange(len(counts), device=device), torch.as_tensor(counts).to(device))
+    uniq, inv = torch.unique(kt, sorted=True, return_inverse=True)
+    if restrict is not None:
+        keep_col = torch.as_tensor(np.ascontiguousarray(restrict(uniq.cpu().numpy()), dtype=bool)).to(device)
+        keep = keep_col[inv]
+        inv = (torch.cumsum(keep_col.to(torch.int64), 0) - 1)[inv[keep]]
+        sample, ct, uniq = sample[keep], ct[keep], uniq[keep_col]
+    K = len(uniq)
+    order = torch.argsort(sample * max(K, 1) + inv)
+    col = inv[order].to(torch.int32)
+    offsets = np.zeros(len(counts) + 1, np.int64)
+    offsets[1:] = np.cumsum(torch.bincount(sample, minlength=len(counts)).cpu().numpy())
+    return offsets, col.cpu().numpy(), ct[order].cpu().numpy(), uniq.cpu().numpy()
+
+
+class PairMatrix(object):
+    """Result of pairwise_score_many: common / same int64 [C,S,S] = per normalised chromosome (`chromosomes`) the markers
+    samples i and j share and how many of those carry identical GT strings."""
+
+    def __init__(self, common, same, chromosomes, chr_ids, n_markers, names, hdf5=None):
+        self.common, self.same = common, same
+        self.chromosomes = chromosomes
+        self._chr_ids = chr_ids              # per sample: sorted indices into `chromosomes` of its g_chrs_ids
+        self.n_markers = n_markers
+        self.names = names
+        self.hdf5 = hdf5
+        self.timings = {}
+
+    def identity(self):
+        """[S,S] same / common over all chromosomes, nan where the pair shares no marker."""
+        c, s = self.common.sum(axis=0), self.same.sum(axis=0)
+        with np.errstate(invalid="ignore", divide="ignore"):
+            return np.where(c > 0, s / np.maximum(c, 1), np.nan)
+
+    def stats(self, i, j):
+        """The dict pairwiseScore(names[i], names[j], ..., hdf5File) returns."""
+        d = {}
+        if self.hdf5 is not None:
+            d['hdf5'] = self.hdf5
+        for c in np.intersect1d(self._chr_ids[i], self._chr_ids[j]):
+            n = int(self.common[c, i, j])
+            d[str(self.chromosomes[c])] = [get_fraction(int(self.same[c, i, j]), n), n]
+        tc, ts = int(self.common[:, i, j].sum()), int(self.same[:, i, j].sum())
+        d['matches'] = [get_fraction(ts, tc), tc]
+        ni, nj = int(self.n_markers[i]), int(self.n_markers[j])
+        d['unique'] = {"%s" % os.path.basename(self.names[i]): [get_fraction(ni - tc, ni), ni],
+                       "%s" % os.path.basename(self.names[j]): [get_fraction(nj - tc, nj), nj]}
+        return d
+
+    def write(self, prefix, pairs_json=False, labels=None):
+        """<prefix>.identity.tsv and <prefix>.common.tsv (S x S, the sample labels as header row and first column; labels
+        default to the names' basenames) and, with pairs_json, <prefix>.pairs.jsonl: one line per pair i < j,
+        {"sample_1", "sample_2", "stats": stats(i, j)}."""
+        import time
+        t0 = time.perf_counter()
+        labels = [os.path.basename(n) for n in self.names] if labels is None else [str(x) for x in labels]
+        check_labels(labels, len(self.names))
+        write_matrix_tsv(prefix + ".identity.tsv", labels, self.identity())
+        write_matrix_tsv(prefix + ".common.tsv", labels, self.common.sum(axis=0))
+        if pairs_json:
+            with open(prefix + ".pairs.jsonl", "w") as fh:
+                S = len(self.names)
+                for i in range(S):
+                    for j in range(i + 1, S):
+                        fh.write(json.dumps({"sample_1": self.names[i], "sample_2": self.names[j], "stats": self.stats(i, j)},
+                                            sort_keys=True) + "\n")
+        self.timings["write"] = time.perf_counter() - t0
+
+
+def check_labels(labels, n):
+    """Labels of the TSV header: one per sample, distinct, without tabs or line breaks."""
+    if len(labels) != n:
+        raise ValueError("%d labels for %d samples" % (len(labels), n))
+    seen = {}
+    for i, lab in enumerate(labels):
+        if "\t" in lab or "\n" in lab or "\r" in lab or not lab:
+            raise ValueError("sample %d: label %r is empty or holds a tab or line break" % (i, lab))
+        if lab in seen:
+            raise ValueError("samples %d and %d have the same label %s" % (seen[lab], i, lab))
+        seen[lab] = i
+
+
+def write_matrix_tsv(path, labels, matrix):
+    """S x S matrix as TSV: header 'sample' + labels, then per row its label and the values (floats round-trip, nan as nan)."""
+    with open(path, "w") as fh:
+        fh.write("\t".join(["sample"] + list(labels)) + "\n")
+        for lab, row in zip(labels, matrix):
+            fh.write(lab + "\t" + "\t".join(map(str, row.tolist())) + "\n")
+
+
+def pairwise_score_many(samples, hdf5File=None, device=0, names=None, chunk_markers=0, logDebug=False):
+    """`pairsnp` for every pair of many samples in one device pass.  samples: sample files (VCF/BED/npz) or ParseInputs;
+    names: what stands for each sample in stats() (default: its path, or sample<i> for a ParseInputs).  For every pair,
+    PairMatrix.stats(i, j) is the dict pairwiseScore(names[i], names[j], ..., hdf5File) returns.
+    Markers join on (normalised chromosome, position); with a database (path or Genotype, loaded once) only its positions
+    count.  The columns are the union of all samples' markers, built by a device sort; the counts of all pairs come from
+    lib.pair_matrix (one-hot tensor-core GEMMs over that union).  Refused before any device work: an empty list, more than
+    lib.PAIR_MAX_SAMPLES samples, a sample with a repeated (chromosome, position), a position outside int32, and more than 8
+    distinct GT strings.  `timings` of the result holds the host seconds of every stage and the library's device times."""
+    import time
+    t0 = time.perf_counter()
+    samples = list(samples)
+    if not samples:
+        raise ValueError("pairwise_score_many: the sample list is empty")
+    if len(samples) > lib.PAIR_MAX_SAMPLES:
+        raise ValueError("pairwise_score_many: %d samples; one call takes at most %d" % (len(samples), lib.PAIR_MAX_SAMPLES))
+    names = [s if isinstance(s, str) else "sample%d" % i for i, s in enumerate(samples)] if names is None else [str(n) for n in names]
+    assert len(names) == len(samples), "one name per sample"
+    inputs = [parsers.ParseInputs(inFile=s, logDebug=logDebug) if isinstance(s, str) else s for s in samples]
+    t1 = time.perf_counter()
+    # chromosomes: every normalised name any sample has, sorted (the order of np.intersect1d in pairwiseScore)
+    chr_codes = [_chromosome_codes(inp) for inp in inputs]
+    chromosomes = np.unique(np.concatenate([n for _, _, n in chr_codes])) if any(len(n) for _, _, n in chr_codes) else np.zeros(0, "U1")
+    rep = np.empty(len(chromosomes), dtype=object)           # one raw name per chromosome, for the database join
+    keys, chr_ids = [], []
+    for i, ((raw, codes, norm), inp) in enumerate(zip(chr_codes, inputs)):
+        gid = np.searchsorted(chromosomes, norm).astype(np.int64)
+        rep[gid] = raw
+        chr_ids.append(np.unique(gid))
+        cid = gid[codes] if len(codes) else np.zeros(0, np.int64)
+        pos = np.asarray(inp.pos, dtype=np.int64)
+        if len(cid) != len(pos):
+            raise ValueError("sample %d (%s): %d chromosome names for %d positions" % (i, names[i], len(cid), len(pos)))
+        bad = pos[(pos < -2**31) | (pos >= 2**31 - 1)]
+        if len(bad):
+            raise ValueError("sample %d (%s): position %d is outside the int32 range of the join" % (i, names[i], int(bad[0])))
+        if not _no_repeats(cid, pos, len(chr_ids[-1])):
+            key = np.sort((cid << 32) | (pos + 2**31))
+            k = key[1:][key[1:] == key[:-1]][0]
+            raise ValueError("sample %d (%s): marker %s:%d appears more than once; compare such a sample with `pairsnp -i -j`"
+                             % (i, names[i], chromosomes[k >> 32], (k & 0xFFFFFFFF) - 2**31))
+        keys.append((cid << 32) | (pos + 2**31))
+    counts = np.array([len(k) for k in keys], dtype=np.int64)
+    cls, strings = gt_classes(np.concatenate([np.asarray(inp.gt).astype("U") for inp in inputs]))
+    if len(strings) > 8:
+        raise ValueError("the samples hold %d distinct GT strings (%s); at most 8 are compared in one call"
+                         % (len(strings), ", ".join(map(str, strings[:9]))))
+    t2 = time.perf_counter()
+    g, hdf5 = None, None
+    if hdf5File is not None:
+        g = hdf5File if isinstance(hdf5File, snp_genotype.Genotype) else snp_genotype.Genotype(hdf5File, None, device=device)
+        hdf5 = hdf5File if not isinstance(hdf5File, snp_genotype.Genotype) else "resident"
+    try:
+        restrict = None
+        if g is not None:
+            def restrict(u):
+                in_db = np.zeros(len(u), dtype=bool)
+                if len(u):
+                    in_db[g.get_positions_idxs(rep[u >> 32].astype("U"), (u & 0xFFFFFFFF) - 2**31)[1]] = True
+                return in_db
+        offsets, col, mcls, union = build_pair_columns(np.concatenate(keys), counts, cls.astype(np.uint8), "cuda:%d" % device, restrict)
+    finally:
+        if g is not None and g is not hdf5File:
+            g.close()
+    chr_start = np.searchsorted(union >> 32, np.arange(len(chromosomes) + 1)).astype(np.int64)
+    t3 = time.perf_counter()
+    common, same, ms = lib.pair_matrix(offsets, col, mcls, max(len(strings), 1), len(union), chr_start, chunk_markers, device=device)
+    t4 = time.perf_counter()
+    pm = PairMatrix(common.astype(np.int64), same.astype(np.int64), chromosomes, chr_ids, counts, names, hdf5)
+    pm.n_columns, pm.n_classes = len(union), len(strings)
+    pm.timings = {"parse": t1 - t0, "prepare": t2 - t1, "union": t3 - t2, "device": t4 - t3, "build": time.perf_counter() - t4,
+                  "expand_ms": ms[0], "gemm_ms": ms[1], "device_ms": ms[2]}
+    return pm
+
+
+def pairwiseScoreMany(args, samples):
+    """`pairsnp --samples`: samples = [(file, label)]; writes <-o>.identity.tsv, <-o>.common.tsv and, with --pairs_json,
+    <-o>.pairs.jsonl."""
+    paths = [p for p, _ in samples]
+    log.info("comparing %d samples, %d pairs", len(paths), len(paths) * (len(paths) - 1) // 2)
+    pm = pairwise_score_many(paths, hdf5File=args['hdf5File'], names=paths, logDebug=args['logDebug'])
+    log.info("writing %s.identity.tsv and %s.common.tsv", args['outFile'], args['outFile'])
+    pm.write(args['outFile'], pairs_json=args.get('pairs_json', False), labels=[lab for _, lab in samples])
+    return pm

@@ -14,6 +14,7 @@
 #include "group_sort.cuh"
 #include "grouped2.cuh"
 #include "pairs.cuh"
+#include "pair_matrix.cuh"
 #include "cross_geno.cuh"
 #include <unordered_map>
 
@@ -406,6 +407,144 @@ int snpm_pair_match_counts(int device, const int64_t *idx1, const int64_t *idx2,
     for (int32_t c = 0; c < n_chr; ++c) {
         common[c] = int64_t(cnt[size_t(c)]);
         matches[c] = int64_t(cnt[size_t(n_chr) + c]);
+    }
+    return SNPM_OK;
+}
+
+// ---- all-against-all pairsnp -----------------------------------------------------------------
+int snpm_pair_matrix(int device, int64_t S, const int64_t *offsets, const int32_t *col, const uint8_t *cls, int32_t n_cls, int64_t K,
+                     const int64_t *chr_start, int32_t C, int64_t chunk_markers, int32_t *common, int32_t *same, float *ms) {
+    // every check runs on the host, before anything is allocated
+    if (S < 1 || S > SNPM_PAIR_MAX_SAMPLES) return fail(SNPM_E_ARG, "snpm_pair_matrix: %lld samples; 1 to %d are allowed", (long long)S, SNPM_PAIR_MAX_SAMPLES);
+    if (!offsets || n_cls < 1 || n_cls > 8 || K < 0 || C < 0 || !chr_start || chunk_markers < 0 || (C > 0 && (!common || !same)))
+        return fail(SNPM_E_ARG, "snpm_pair_matrix: bad arguments");
+    if (K > INT32_MAX) return fail(SNPM_E_ARG, "snpm_pair_matrix: %lld columns; column indices are int32", (long long)K);
+    if (chr_start[0] != 0 || chr_start[C] != K) return fail(SNPM_E_ARG, "snpm_pair_matrix: chr_start must run from 0 to K = %lld", (long long)K);
+    for (int32_t c = 0; c < C; ++c) {
+        if (chr_start[c + 1] < chr_start[c]) return fail(SNPM_E_ARG, "snpm_pair_matrix: chr_start decreases at chromosome %d", c);
+        if (chr_start[c + 1] - chr_start[c] >= (int64_t(1) << 31))
+            return fail(SNPM_E_RANGE, "snpm_pair_matrix: chromosome %d has 2^31 columns or more; the counts are int32", c);
+    }
+    if (offsets[0] != 0) return fail(SNPM_E_ARG, "snpm_pair_matrix: offsets[0] must be 0");
+    if (offsets[S] > 0 && (!col || !cls)) return fail(SNPM_E_ARG, "snpm_pair_matrix: bad arguments");
+    for (int64_t s = 0; s < S; ++s) {
+        if (offsets[s + 1] < offsets[s]) return fail(SNPM_E_ARG, "snpm_pair_matrix: offsets decrease at sample %lld", (long long)s);
+        for (int64_t i = offsets[s]; i < offsets[s + 1]; ++i) {
+            if (col[i] < 0 || col[i] >= K) return fail(SNPM_E_ARG, "snpm_pair_matrix: sample %lld: column %d is outside 0..K-1", (long long)s, col[i]);
+            if (i > offsets[s] && col[i] <= col[i - 1]) return fail(SNPM_E_ARG, "snpm_pair_matrix: sample %lld: columns are not strictly ascending", (long long)s);
+            if (cls[i] >= n_cls) return fail(SNPM_E_ARG, "snpm_pair_matrix: sample %lld: class %d is not below n_cls = %d", (long long)s, int(cls[i]), n_cls);
+        }
+    }
+    const int64_t n = offsets[S];
+    const int slots = n_cls <= 4 ? 4 : 8, mk = 128 / slots;
+    const int m_blocks = int(ceil_div64(S, 64)), n_blocks = int(ceil_div64(S, OG_BN)), ld_out = n_blocks * OG_BN;
+    const int64_t kb_bytes = int64_t(m_blocks) * OG_A_TILE + int64_t(n_blocks) * OG_B_TILE;
+    int64_t widest = 0;
+    for (int32_t c = 0; c < C; ++c) widest = std::max(widest, chr_start[c + 1] - chr_start[c]);
+    int64_t step = chunk_markers > 0 ? chunk_markers : std::max<int64_t>(1, SNPM_PAIR_CHUNK_BYTES / kb_bytes) * mk;
+    step = std::max<int64_t>(1, std::min(step, widest));
+    const int64_t max_kb = ceil_div64(step, mk);
+    const size_t cells = size_t(C) * size_t(S) * size_t(S);
+
+    SNPM_CUDA(cudaSetDevice(device));
+    int n_sm = 0;
+    SNPM_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device));
+    struct Res {
+        DevBuf off, col, cls, at, bt, ps, pc, same, common;
+        cudaStream_t st = nullptr;
+        std::vector<cudaEvent_t> ev;
+        ~Res() {
+            for (DevBuf *d : {&off, &col, &cls, &at, &bt, &ps, &pc, &same, &common}) d->release();
+            for (cudaEvent_t e : ev) cudaEventDestroy(e);
+            if (st) cudaStreamDestroy(st);
+        }
+    } r;
+    // events: call start / end, then per chunk of a ring of RING: start, operands ready, GEMM done
+    constexpr int RING = 64;
+    r.ev.assign(2 + 3 * RING, nullptr);
+    for (cudaEvent_t &e : r.ev) SNPM_CUDA(cudaEventCreate(&e));
+    SNPM_CUDA(cudaStreamCreateWithFlags(&r.st, cudaStreamNonBlocking));
+    cudaStream_t st = r.st;
+    SNPM_TRY(r.off.ensure(size_t(S + 1) * 8));
+    SNPM_TRY(r.col.ensure(size_t(n) * 4));
+    SNPM_TRY(r.cls.ensure(size_t(n)));
+    SNPM_TRY(r.same.ensure(cells * 4));
+    SNPM_TRY(r.common.ensure(cells * 4));
+    if (K > 0) {
+        SNPM_TRY(r.at.ensure(size_t(m_blocks) * max_kb * OG_A_TILE));
+        SNPM_TRY(r.bt.ensure(size_t(n_blocks) * max_kb * OG_B_TILE));
+        SNPM_TRY(r.ps.ensure(size_t(S) * ld_out * 4));
+        SNPM_TRY(r.pc.ensure(size_t(S) * ld_out * 4));
+    }
+    const size_t smem = size_t(OG_STAGES) * (OG_A_TILE + OG_B_TILE) + 1024;
+    SNPM_CUDA(smem_attr<k_onehot_gemm>(int(smem)));
+
+    SNPM_CUDA(cudaEventRecord(r.ev[0], st));
+    SNPM_CUDA(cudaMemcpyAsync(r.off.p, offsets, size_t(S + 1) * 8, cudaMemcpyHostToDevice, st));
+    if (n > 0) {
+        SNPM_CUDA(cudaMemcpyAsync(r.col.p, col, size_t(n) * 4, cudaMemcpyHostToDevice, st));
+        SNPM_CUDA(cudaMemcpyAsync(r.cls.p, cls, size_t(n), cudaMemcpyHostToDevice, st));
+    }
+    if (cells) {
+        SNPM_CUDA(cudaMemsetAsync(r.same.p, 0, cells * 4, st));
+        SNPM_CUDA(cudaMemsetAsync(r.common.p, 0, cells * 4, st));
+    }
+    float t_expand = 0.f, t_gemm = 0.f;
+    auto collect = [&](int q) -> int {                          // the times of the chunk in ring slot q
+        cudaEvent_t *e = &r.ev[2 + 3 * q];
+        float a = 0.f, b = 0.f;
+        SNPM_CUDA(cudaEventSynchronize(e[2]));
+        SNPM_CUDA(cudaEventElapsedTime(&a, e[0], e[1]));
+        SNPM_CUDA(cudaEventElapsedTime(&b, e[1], e[2]));
+        t_expand += a;
+        t_gemm += b;
+        return SNPM_OK;
+    };
+    const int warps = 8;
+    const dim3 acc_grid(unsigned(ceil_div64(S, 256)), unsigned(S));
+    int64_t chunk = 0;
+    for (int32_t c = 0; c < C; ++c) {
+        for (int64_t c0 = chr_start[c]; c0 < chr_start[c + 1]; c0 += step, ++chunk) {  // a chunk never spans two chromosomes
+            const int64_t c1 = std::min(c0 + step, chr_start[c + 1]);
+            const int32_t n_kb = int32_t(ceil_div64(c1 - c0, mk));
+            const int q = int(chunk % RING);
+            if (chunk >= RING) SNPM_TRY(collect(q));
+            cudaEvent_t *e = &r.ev[2 + 3 * q];
+            SNPM_CUDA(cudaEventRecord(e[0], st));
+            SNPM_CUDA(cudaMemsetAsync(r.at.p, 0, size_t(m_blocks) * n_kb * OG_A_TILE, st));
+            SNPM_CUDA(cudaMemsetAsync(r.bt.p, 0, size_t(n_blocks) * n_kb * OG_B_TILE, st));
+            const unsigned eg = unsigned(ceil_div64(S, warps));
+            if (slots == 4)
+                k_pair_expand<4><<<eg, 32 * warps, 0, st>>>(r.off.as<int64_t>(), r.col.as<int32_t>(), r.cls.as<uint8_t>(), int32_t(S), int32_t(c0),
+                                                           int32_t(c1), n_kb, r.at.as<unsigned char>(), r.bt.as<unsigned char>());
+            else
+                k_pair_expand<8><<<eg, 32 * warps, 0, st>>>(r.off.as<int64_t>(), r.col.as<int32_t>(), r.cls.as<uint8_t>(), int32_t(S), int32_t(c0),
+                                                           int32_t(c1), n_kb, r.at.as<unsigned char>(), r.bt.as<unsigned char>());
+            SNPM_KERNEL_CHECK();
+            SNPM_CUDA(cudaEventRecord(e[1], st));
+            OneHotGemmArgs g = {};
+            g.a_tiled = r.at.as<unsigned char>(); g.b_tiled = r.bt.as<unsigned char>(); g.n_kb = n_kb; g.m_blocks = m_blocks; g.n_blocks = n_blocks;
+            g.S = int32_t(S); g.out_score = r.ps.as<int32_t>(); g.out_ninfo = r.pc.as<int32_t>(); g.ld_out = ld_out;
+            k_onehot_gemm<<<unsigned(std::min(m_blocks * n_blocks, n_sm)), OG_THREADS, smem, st>>>(g);
+            SNPM_KERNEL_CHECK();
+            SNPM_CUDA(cudaEventRecord(e[2], st));
+            const size_t at = size_t(c) * S * S;
+            k_pair_accumulate<<<acc_grid, 256, 0, st>>>(g.out_score, g.out_ninfo, ld_out, int32_t(S), r.same.as<int32_t>() + at, r.common.as<int32_t>() + at);
+            SNPM_KERNEL_CHECK();
+        }
+    }
+    for (int64_t k = std::max<int64_t>(0, chunk - RING); k < chunk; ++k) SNPM_TRY(collect(int(k % RING)));
+    if (cells) {
+        SNPM_CUDA(cudaMemcpyAsync(same, r.same.p, cells * 4, cudaMemcpyDeviceToHost, st));
+        SNPM_CUDA(cudaMemcpyAsync(common, r.common.p, cells * 4, cudaMemcpyDeviceToHost, st));
+    }
+    SNPM_CUDA(cudaEventRecord(r.ev[1], st));
+    SNPM_CUDA(cudaStreamSynchronize(st));
+    if (ms) {
+        ms[0] = t_expand;
+        ms[1] = t_gemm;
+        ms[2] = 0.f;
+        SNPM_CUDA(cudaEventElapsedTime(&ms[2], r.ev[0], r.ev[1]));
     }
     return SNPM_OK;
 }

@@ -23,6 +23,7 @@ SNPM_E_ASSERT = -5
 SNPM_E_RANGE = -6
 
 CHUNK_ROWS = 1000
+PAIR_MAX_SAMPLES = 8192        # SNPM_PAIR_MAX_SAMPLES
 
 JOIN_AUTO, JOIN_SEARCH, JOIN_MERGEPATH = 0, 1, 2
 KERNEL_FP64, KERNEL_POPCOUNT, KERNEL_GROUPED = 0, 1, 2
@@ -212,6 +213,7 @@ SIGNATURES = {
     "snpm_db_segregating_rows": (C.c_int, [_p, _p, _i32, _p]),
     "snpm_db_read_columns": (C.c_int, [_p, _p, _i32, _p]),
     "snpm_pair_match_counts": (C.c_int, [C.c_int, _p, _p, _i64, _p, _p, _i64, _p, _i64, _i32, _p, _p]),
+    "snpm_pair_matrix": (C.c_int, [C.c_int, _i64, _p, _p, _p, _i32, _i64, _p, _i32, _i64, _p, _p, _p]),
     "snpm_cross_window_genotypes": (C.c_int, [C.c_int, _p, _p, _i64, _p, _i32, _p, _p, _i64, _p, _i64, _i32, _f64, _i32, _p, _p, _p]),
     "snpm_db_n_rows": (_i64, [_p]),
     "snpm_db_n_acc": (_i32, [_p]),
@@ -861,6 +863,22 @@ def pair_match_counts(idx1, idx2, chrom1, gt1, gt2, n_chr, device=0):
     check(load().snpm_pair_match_counts(device, ptr(idx1), ptr(idx2), len(idx1), ptr(chrom1), ptr(gt1), len(gt1), ptr(gt2), len(gt2),
                                         n_chr, ptr(common), ptr(matches)))
     return common, matches
+
+
+def pair_matrix(offsets, col, cls, n_cls, K, chr_start, chunk_markers=0, device=0):
+    """All-against-all counts of pairsnp on the device (snpm_pair_matrix): samples as CSR (offsets int64[S+1]; col int32 union
+    column of each marker, strictly ascending inside a sample; cls uint8 GT-string class < n_cls <= 8), chr_start int64[C+1]
+    column range of each chromosome.  Returns (common int32 [C,S,S], same int32 [C,S,S], (expand_ms, gemm_ms, device_ms))."""
+    offsets, col, cls = as_c(offsets, np.int64), as_c(col, np.int32), as_c(cls, np.uint8)
+    chr_start = as_c(chr_start, np.int64)
+    S, C_ = len(offsets) - 1, len(chr_start) - 1
+    assert S >= 0 and C_ >= 0 and len(col) == len(cls)
+    shape = (C_, max(S, 0), max(S, 0)) if S <= PAIR_MAX_SAMPLES else (0, 0, 0)     # an S past the limit is refused by the library
+    common, same = np.empty(shape, np.int32), np.empty(shape, np.int32)
+    ms = (C.c_float * 3)()
+    check(load().snpm_pair_matrix(device, S, ptr(offsets), ptr(col), ptr(cls), int(n_cls), int(K), ptr(chr_start), C_, int(chunk_markers),
+                                  ptr(common), ptr(same), ms))
+    return common, same, (ms[0], ms[1], ms[2])
 
 
 def cross_window_genotypes(par_idx, vcf_idx, win_start, p1, p2, gt, lr_thres, n_marker_thres=5, device=0):
