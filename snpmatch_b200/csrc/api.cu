@@ -216,7 +216,6 @@ int snpm_db_destroy(snpm_db *db) {
     if (db->d_bm_first_row) cudaFree(db->d_bm_first_row);
     if (db->d_bm_off) cudaFree(db->d_bm_off);
     if (db->scratch_batch_) { snpm_batch_destroy(db->scratch_batch_); db->scratch_batch_ = nullptr; }
-    db->scratch.release();
     if (db->own_stream && db->stream) cudaStreamDestroy(db->stream);
     delete db;
     return SNPM_OK;
@@ -283,18 +282,12 @@ int snpm_db_read_rows_int8(snpm_db *db, const int64_t *rows, int64_t k, int8_t *
     SNPM_CUDA(cudaSetDevice(db->device));
     DevBuf d_rows, d_out;
     SNPM_TRY(d_rows.ensure(size_t(k) * 8));
-    int rc = d_out.ensure(size_t(k) * db->n_acc);
-    if (rc) { d_rows.release(); return rc; }
-    cudaError_t e = cudaMemcpyAsync(d_rows.p, rows, size_t(k) * 8, cudaMemcpyHostToDevice, db->stream);
-    if (e == cudaSuccess) {
-        k_unpack_rows<<<grid_for(k * db->n_acc, 256, db->n_sm), 256, 0, db->stream>>>(db->d_packed, db->stride, db->n_acc, d_rows.as<int64_t>(), k, d_out.as<int8_t>());
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_out.p, size_t(k) * db->n_acc, cudaMemcpyDeviceToHost, db->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(db->stream);
-    d_rows.release();
-    d_out.release();
-    if (e != cudaSuccess) return fail(SNPM_E_CUDA, "snpm_db_read_rows_int8: %s", cudaGetErrorString(e));
+    SNPM_TRY(d_out.ensure(size_t(k) * db->n_acc));
+    SNPM_CUDA(cudaMemcpyAsync(d_rows.p, rows, size_t(k) * 8, cudaMemcpyHostToDevice, db->stream));
+    k_unpack_rows<<<grid_for(k * db->n_acc, 256, db->n_sm), 256, 0, db->stream>>>(db->d_packed, db->stride, db->n_acc, d_rows.as<int64_t>(), k, d_out.as<int8_t>());
+    SNPM_CUDA(cudaGetLastError());
+    SNPM_CUDA(cudaMemcpyAsync(out, d_out.p, size_t(k) * db->n_acc, cudaMemcpyDeviceToHost, db->stream));
+    SNPM_CUDA(cudaStreamSynchronize(db->stream));
     return SNPM_OK;
 }
 
@@ -318,22 +311,14 @@ int snpm_db_segregating_rows(snpm_db *db, const int32_t *acc_idx, int32_t n_sel,
     SNPM_CUDA(cudaSetDevice(db->device));
     DevBuf d_sel, d_flags;
     SNPM_TRY(d_sel.ensure(size_t(db->stride) * 4));
-    int rc = d_flags.ensure(size_t(db->n_rows));
-    cudaError_t e = cudaSuccess;
-    if (rc == SNPM_OK) {
-        e = cudaMemcpyAsync(d_sel.p, sel.data(), size_t(db->stride) * 4, cudaMemcpyHostToDevice, db->stream);
-        if (e == cudaSuccess) {
-            k_segregating_rows<<<grid_for(db->n_rows * 32, 256, db->n_sm, 32), 256, 0, db->stream>>>(db->d_packed, db->n_rows, db->stride,
-                                                                                                  d_sel.as<uint32_t>(), d_flags.as<uint8_t>());
-            e = cudaGetLastError();
-        }
-        if (e == cudaSuccess) e = cudaMemcpyAsync(flags, d_flags.p, size_t(db->n_rows), cudaMemcpyDeviceToHost, db->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(db->stream);
-    }
-    d_sel.release();
-    d_flags.release();
-    if (e != cudaSuccess) return fail(SNPM_E_CUDA, "snpm_db_segregating_rows: %s", cudaGetErrorString(e));
-    return rc;
+    SNPM_TRY(d_flags.ensure(size_t(db->n_rows)));
+    SNPM_CUDA(cudaMemcpyAsync(d_sel.p, sel.data(), size_t(db->stride) * 4, cudaMemcpyHostToDevice, db->stream));
+    k_segregating_rows<<<grid_for(db->n_rows * 32, 256, db->n_sm, 32), 256, 0, db->stream>>>(db->d_packed, db->n_rows, db->stride,
+                                                                                          d_sel.as<uint32_t>(), d_flags.as<uint8_t>());
+    SNPM_CUDA(cudaGetLastError());
+    SNPM_CUDA(cudaMemcpyAsync(flags, d_flags.p, size_t(db->n_rows), cudaMemcpyDeviceToHost, db->stream));
+    SNPM_CUDA(cudaStreamSynchronize(db->stream));
+    return SNPM_OK;
 }
 
 int snpm_db_read_columns(snpm_db *db, const int32_t *acc_idx, int32_t n_sel, int8_t *out) {
@@ -345,8 +330,7 @@ int snpm_db_read_columns(snpm_db *db, const int32_t *acc_idx, int32_t n_sel, int
     DevBuf d_out;
     const int32_t per = std::min<int32_t>(n_sel, RC_MAX_COLS);
     SNPM_TRY(d_out.ensure(size_t(per) * size_t(db->n_rows)));
-    cudaError_t e = cudaSuccess;
-    for (int32_t c0 = 0; c0 < n_sel && e == cudaSuccess; c0 += RC_MAX_COLS) {
+    for (int32_t c0 = 0; c0 < n_sel; c0 += RC_MAX_COLS) {
         ColumnSel sel;
         sel.n = std::min<int32_t>(RC_MAX_COLS, n_sel - c0);
         for (int32_t c = 0; c < RC_MAX_COLS; ++c) {
@@ -355,12 +339,10 @@ int snpm_db_read_columns(snpm_db *db, const int32_t *acc_idx, int32_t n_sel, int
             sel.bit[c] = a & 31;
         }
         k_read_columns<<<grid_for(db->n_rows, 256, db->n_sm, 32), 256, 0, db->stream>>>(db->d_packed, db->n_rows, db->stride, sel, d_out.as<int8_t>());
-        e = cudaGetLastError();
-        if (e == cudaSuccess) e = cudaMemcpyAsync(out + size_t(c0) * size_t(db->n_rows), d_out.p, size_t(sel.n) * size_t(db->n_rows), cudaMemcpyDeviceToHost, db->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(db->stream);
+        SNPM_CUDA(cudaGetLastError());
+        SNPM_CUDA(cudaMemcpyAsync(out + size_t(c0) * size_t(db->n_rows), d_out.p, size_t(sel.n) * size_t(db->n_rows), cudaMemcpyDeviceToHost, db->stream));
+        SNPM_CUDA(cudaStreamSynchronize(db->stream));
     }
-    d_out.release();
-    if (e != cudaSuccess) return fail(SNPM_E_CUDA, "snpm_db_read_columns: %s", cudaGetErrorString(e));
     return SNPM_OK;
 }
 
@@ -375,35 +357,27 @@ int snpm_pair_match_counts(int device, const int64_t *idx1, const int64_t *idx2,
     if (n_chr == 0) return SNPM_OK;
     SNPM_CUDA(cudaSetDevice(device));
     DevBuf d_i1, d_i2, d_c1, d_g1, d_g2, d_cnt;
-    int rc = SNPM_OK;
-    cudaError_t e = cudaSuccess;
     std::vector<unsigned long long> cnt(size_t(2) * n_chr, 0ull);
-    if ((rc = d_cnt.ensure(size_t(2) * n_chr * 8)) == SNPM_OK) e = cudaMemset(d_cnt.p, 0, size_t(2) * n_chr * 8);
-    if (rc == SNPM_OK && e == cudaSuccess && m > 0) {
-        if (rc == SNPM_OK) rc = d_i1.ensure(size_t(m) * 8);
-        if (rc == SNPM_OK) rc = d_i2.ensure(size_t(m) * 8);
-        if (rc == SNPM_OK) rc = d_c1.ensure(size_t(n1) * 4);
-        if (rc == SNPM_OK) rc = d_g1.ensure(size_t(n1) * 4);
-        if (rc == SNPM_OK) rc = d_g2.ensure(size_t(n2) * 4);
-        if (rc == SNPM_OK) {
-            e = cudaMemcpy(d_i1.p, idx1, size_t(m) * 8, cudaMemcpyHostToDevice);
-            if (e == cudaSuccess) e = cudaMemcpy(d_i2.p, idx2, size_t(m) * 8, cudaMemcpyHostToDevice);
-            if (e == cudaSuccess) e = cudaMemcpy(d_c1.p, chrom1, size_t(n1) * 4, cudaMemcpyHostToDevice);
-            if (e == cudaSuccess) e = cudaMemcpy(d_g1.p, gt1, size_t(n1) * 4, cudaMemcpyHostToDevice);
-            if (e == cudaSuccess) e = cudaMemcpy(d_g2.p, gt2, size_t(n2) * 4, cudaMemcpyHostToDevice);
-            if (e == cudaSuccess) {
-                const int grid = int(std::min<int64_t>(ceil_div64(m, 256), 1184));
-                k_pair_counts<<<grid, 256>>>(d_i1.as<int64_t>(), d_i2.as<int64_t>(), m, d_c1.as<int32_t>(), d_g1.as<int32_t>(), d_g2.as<int32_t>(), n_chr,
-                                             d_cnt.as<unsigned long long>());
-                e = cudaGetLastError();
-            }
-            if (e == cudaSuccess) e = cudaDeviceSynchronize();
-        }
+    SNPM_TRY(d_cnt.ensure(size_t(2) * n_chr * 8));
+    SNPM_CUDA(cudaMemset(d_cnt.p, 0, size_t(2) * n_chr * 8));
+    if (m > 0) {
+        SNPM_TRY(d_i1.ensure(size_t(m) * 8));
+        SNPM_TRY(d_i2.ensure(size_t(m) * 8));
+        SNPM_TRY(d_c1.ensure(size_t(n1) * 4));
+        SNPM_TRY(d_g1.ensure(size_t(n1) * 4));
+        SNPM_TRY(d_g2.ensure(size_t(n2) * 4));
+        SNPM_CUDA(cudaMemcpy(d_i1.p, idx1, size_t(m) * 8, cudaMemcpyHostToDevice));
+        SNPM_CUDA(cudaMemcpy(d_i2.p, idx2, size_t(m) * 8, cudaMemcpyHostToDevice));
+        SNPM_CUDA(cudaMemcpy(d_c1.p, chrom1, size_t(n1) * 4, cudaMemcpyHostToDevice));
+        SNPM_CUDA(cudaMemcpy(d_g1.p, gt1, size_t(n1) * 4, cudaMemcpyHostToDevice));
+        SNPM_CUDA(cudaMemcpy(d_g2.p, gt2, size_t(n2) * 4, cudaMemcpyHostToDevice));
+        const int grid = int(std::min<int64_t>(ceil_div64(m, 256), 1184));
+        k_pair_counts<<<grid, 256>>>(d_i1.as<int64_t>(), d_i2.as<int64_t>(), m, d_c1.as<int32_t>(), d_g1.as<int32_t>(), d_g2.as<int32_t>(), n_chr,
+                                     d_cnt.as<unsigned long long>());
+        SNPM_CUDA(cudaGetLastError());
+        SNPM_CUDA(cudaDeviceSynchronize());
     }
-    if (rc == SNPM_OK && e == cudaSuccess) e = cudaMemcpy(cnt.data(), d_cnt.p, size_t(2) * n_chr * 8, cudaMemcpyDeviceToHost);
-    for (DevBuf *d : {&d_i1, &d_i2, &d_c1, &d_g1, &d_g2, &d_cnt}) d->release();
-    if (e != cudaSuccess) return fail(SNPM_E_CUDA, "snpm_pair_match_counts: %s", cudaGetErrorString(e));
-    if (rc != SNPM_OK) return rc;
+    SNPM_CUDA(cudaMemcpy(cnt.data(), d_cnt.p, size_t(2) * n_chr * 8, cudaMemcpyDeviceToHost));
     for (int32_t c = 0; c < n_chr; ++c) {
         common[c] = int64_t(cnt[size_t(c)]);
         matches[c] = int64_t(cnt[size_t(n_chr) + c]);
@@ -454,7 +428,6 @@ int snpm_pair_matrix(int device, int64_t S, const int64_t *offsets, const int32_
         cudaStream_t st = nullptr;
         std::vector<cudaEvent_t> ev;
         ~Res() {
-            for (DevBuf *d : {&off, &col, &cls, &at, &bt, &ps, &pc, &same, &common}) d->release();
             for (cudaEvent_t e : ev) cudaEventDestroy(e);
             if (st) cudaStreamDestroy(st);
         }
@@ -555,15 +528,27 @@ int32_t snpm_db_row_words(const snpm_db *db) { return db ? db->stride : -1; }
 int64_t snpm_db_packed_bytes(const snpm_db *db) { return db ? db->n_rows * int64_t(db->stride) * 8 : -1; }
 
 // ---- batches --------------------------------------------------------------------------------------
+// the sample offsets of every upload: S >= 1 samples, offsets from 0, non-decreasing, fewer than 2^31 - 2048 markers in all
+static int check_offsets(const char *fn, int64_t S, const int64_t *offsets) {
+    if (S < 1 || !offsets) return fail(SNPM_E_ARG, "%s: need at least one sample and its offsets", fn);
+    if (offsets[0] != 0) return fail(SNPM_E_ARG, "%s: offsets[0] must be 0", fn);
+    for (int64_t s = 0; s < S; ++s)
+        if (offsets[s + 1] < offsets[s]) return fail(SNPM_E_ARG, "%s: offsets must be non-decreasing", fn);
+    if (offsets[S] >= (int64_t(1) << 31) - 2048) return fail(SNPM_E_ARG, "%s: %lld markers exceed the 2^31 limit", fn, (long long)offsets[S]);
+    return SNPM_OK;
+}
+
+// the end of every upload: the next run waits for the copies, and the results of the last run are no longer the batch's
+static int upload_done(snpm_batch *b) {
+    SNPM_CUDA(cudaEventRecord(b->ev_uploaded, b->copy_stream));
+    b->ran = b->ran_windows = b->epilogue_done = false;
+    return SNPM_OK;
+}
+
 static int batch_upload(snpm_batch *b, int64_t S, const int64_t *offsets, const int32_t *chrom, const int32_t *pos, const double *wei,
                         const uint16_t *wei_idx = nullptr, const double *table = nullptr, int32_t n_table = 0) {
-    snpm_db *db = b->db;
-    if (S < 1 || !offsets) return fail(SNPM_E_ARG, "batch: need at least one sample and its offsets");
-    if (offsets[0] != 0) return fail(SNPM_E_ARG, "batch: offsets[0] must be 0");
-    for (int64_t s = 0; s < S; ++s)
-        if (offsets[s + 1] < offsets[s]) return fail(SNPM_E_ARG, "batch: offsets must be non-decreasing");
+    SNPM_TRY(check_offsets("batch", S, offsets));
     const int64_t n = offsets[S];
-    if (n >= (int64_t(1) << 31) - 2048) return fail(SNPM_E_ARG, "batch: %lld markers exceed the 2^31 limit", (long long)n);
     if (n > 0 && (!chrom || !pos || (!wei && !wei_idx))) return fail(SNPM_E_ARG, "batch: NULL marker arrays");
     if (wei_idx && (!table || n_table < 1 || n_table > 65536)) return fail(SNPM_E_ARG, "batch: weight table must hold 1..65536 entries");
     b->S = S;
@@ -598,9 +583,7 @@ static int batch_upload(snpm_batch *b, int64_t S, const int64_t *offsets, const 
             SNPM_CUDA(cudaMemcpyAsync(b->d_wei.p, wei, size_t(n) * 24, cudaMemcpyHostToDevice, st));
         }
     }
-    SNPM_CUDA(cudaEventRecord(b->ev_uploaded, st));
-    b->ran = b->ran_windows = b->epilogue_done = false;
-    return SNPM_OK;
+    return upload_done(b);
 }
 
 static int batch_new(snpm_db *db, snpm_batch **out) {
@@ -771,11 +754,8 @@ static int upload_grouped(snpm_batch *b, int64_t n_samples, const int64_t *offse
                           const uint16_t *run_gid = nullptr, const uint32_t *run_end = nullptr, int64_t n_runs = 0) {
     if (!b) return fail(SNPM_E_ARG, "snpm_batch_upload_grouped: NULL batch");
     snpm_db *db = b->db;
-    if (n_samples < 1 || !offsets || offsets[0] != 0) return fail(SNPM_E_ARG, "snpm_batch_upload_grouped: need samples and offsets starting at 0");
-    for (int64_t s = 0; s < n_samples; ++s)
-        if (offsets[s + 1] < offsets[s]) return fail(SNPM_E_ARG, "snpm_batch_upload_grouped: offsets must be non-decreasing");
+    SNPM_TRY(check_offsets("snpm_batch_upload_grouped", n_samples, offsets));
     const int64_t n = offsets[n_samples];
-    if (n >= (int64_t(1) << 31) - 2048) return fail(SNPM_E_ARG, "snpm_batch_upload_grouped: %lld markers exceed the 2^31 limit", (long long)n);
     if (n > 0 && ((!gid && !run_gid) || (!packed_cp && (!chrom_u8 || !s_pos)))) return fail(SNPM_E_ARG, "snpm_batch_upload_grouped: NULL marker arrays");
     if (run_gid && n > 0) {
         if (!run_end || n_runs < 1 || n_runs > n) return fail(SNPM_E_ARG, "snpm_batch_upload_grouped_runs: need 1..n runs");
@@ -842,9 +822,7 @@ static int upload_grouped(snpm_batch *b, int64_t n_samples, const int64_t *offse
             b->pending_expand |= 4;
         }
     }
-    SNPM_CUDA(cudaEventRecord(b->ev_uploaded, st));
-    b->ran = b->ran_windows = b->epilogue_done = false;
-    return SNPM_OK;
+    return upload_done(b);
 }
 
 int snpm_batch_upload_grouped(snpm_batch *b, int64_t n_samples, const int64_t *offsets, const uint8_t *chrom_u8, const int32_t *s_pos,
@@ -867,11 +845,8 @@ static int upload_coded(snpm_batch *b, int64_t n_samples, const int64_t *offsets
     if (!b) return fail(SNPM_E_ARG, "snpm_batch_upload_coded: NULL batch");
     if (codes32 && n_wtable > 1024) return fail(SNPM_E_ARG, "snpm_batch_upload_coded32: three codes share one word only up to 1024 weight values (%d given)", n_wtable);
     snpm_db *db = b->db;
-    if (n_samples < 1 || !offsets || offsets[0] != 0) return fail(SNPM_E_ARG, "snpm_batch_upload_coded: need samples and offsets starting at 0");
-    for (int64_t s = 0; s < n_samples; ++s)
-        if (offsets[s + 1] < offsets[s]) return fail(SNPM_E_ARG, "snpm_batch_upload_coded: offsets must be non-decreasing");
+    SNPM_TRY(check_offsets("snpm_batch_upload_coded", n_samples, offsets));
     const int64_t n = offsets[n_samples];
-    if (n >= (int64_t(1) << 31) - 2048) return fail(SNPM_E_ARG, "snpm_batch_upload_coded: %lld markers exceed the 2^31 limit", (long long)n);
     if (n > 0 && (!chrom_pos || (!codes && !codes32))) return fail(SNPM_E_ARG, "snpm_batch_upload_coded: NULL marker arrays");
     if (!wtable || n_wtable < 1 || n_wtable > 65536) return fail(SNPM_E_ARG, "snpm_batch_upload_coded: the weight table must hold 1..65536 values");
     for (int32_t t = 0; t < n_wtable; ++t)
@@ -950,9 +925,7 @@ static int upload_coded(snpm_batch *b, int64_t n_samples, const int64_t *offsets
         if (codes32) SNPM_CUDA(cudaMemcpyAsync(b->d_codes.p, codes32, size_t(n) * 4, cudaMemcpyHostToDevice, st));
         else SNPM_CUDA(cudaMemcpyAsync(b->d_codes.p, codes, size_t(n) * 6, cudaMemcpyHostToDevice, st));
     }
-    SNPM_CUDA(cudaEventRecord(b->ev_uploaded, st));
-    b->ran = b->ran_windows = b->epilogue_done = false;
-    return SNPM_OK;
+    return upload_done(b);
 }
 
 int snpm_batch_upload_coded(snpm_batch *b, int64_t n_samples, const int64_t *offsets, const uint32_t *chrom_pos, const uint16_t *codes,
@@ -1056,16 +1029,6 @@ int snpm_batch_destroy(snpm_batch *b) {
     if (b->ev_joined) cudaEventDestroy(b->ev_joined);
     if (b->ev_fork) cudaEventDestroy(b->ev_fork);
     if (b->ev_join) cudaEventDestroy(b->ev_join);
-    DevBuf *bufs[] = {&b->d_off, &b->d_chrom, &b->d_pos, &b->d_wei, &b->d_filter, &b->d_match_row, &b->d_tile_cnt, &b->d_tile_off,
-                      &b->d_prefix, &b->d_pair_db, &b->d_pair_s, &b->d_pair_w, &b->d_mstart, &b->d_seg_off, &b->d_part_score,
-                      &b->d_part_ninfo, &b->d_red, &b->d_matches, &b->d_ninfo64, &b->d_prob, &b->d_L, &b->d_LR, &b->d_status,
-                      &b->d_win_count, &b->d_win_off, &b->d_win_begin, &b->d_win_end, &b->d_kmax, &b->d_win_L, &b->d_win_LR,
-                      &b->d_win_ident, &b->d_win_amb, &b->d_win_row_off, &b->d_row_acc, &b->d_row_score, &b->d_row_ninfo, &b->d_row_L, &b->d_row_ident, &b->d_f1_acc, &b->d_f1_part, &b->d_f1_out, &b->d_pair_code, &b->d_wei_idx, &b->d_wei_table,
-                      &b->d_chrom8, &b->d_gid, &b->d_gtable, &b->d_pair_gid, &b->d_part_int, &b->d_guard, &b->d_runs,
-                      &b->d_codes, &b->d_wtable, &b->d_key_a, &b->d_key_b, &b->d_idx_a, &b->d_idx_b, &b->d_pair_db_tmp, &b->d_pair_s_tmp,
-                      &b->d_tile_sample, &b->d_tile_first, &b->d_tile_hist, &b->d_blk_chg, &b->d_seg_order, &b->d_work_counter, &b->d_hash, &b->d_slot_gid, &b->d_ngroups,
-                      &b->d_group_overflow, &b->d_gkeys, &b->d_gw, &b->d_goff, &b->d_segsel, &b->d_segsel_off, &b->d_flags, &b->d_flag_counts};
-    for (DevBuf *d : bufs) d->release();
     for (int i = 0; i < SNPM_N_EVENTS; ++i)
         if (b->ev[i]) cudaEventDestroy(b->ev[i]);
     if (b->h_status) cudaFreeHost(b->h_status);
@@ -1393,6 +1356,16 @@ static void rec(snpm_batch *b, int which) {
     b->ev_rec[which] = true;
 }
 
+// the end of every run: the next upload may overwrite the inputs behind its kernels, and the epilogue is still to come
+static int run_done(snpm_batch *b) {
+    rec(b, SNPM_EV_COMBINE);
+    SNPM_CUDA(cudaEventRecord(b->ev_inputs_free, b->db->stream));
+    b->ran = true;
+    b->ran_windows = false;
+    b->epilogue_done = false;
+    return SNPM_OK;
+}
+
 int snpm_batch_run(snpm_batch *b, int skip_db_hets, int mode) {
     if (!b) return fail(SNPM_E_ARG, "snpm_batch_run: NULL batch");
     snpm_db *db = b->db;
@@ -1439,12 +1412,7 @@ int snpm_batch_run(snpm_batch *b, int skip_db_hets, int mode) {
                                                  b->d_group_overflow.as<int>(), b->d_red.as<double>());
         SNPM_KERNEL_CHECK();
         b->launches += 1;
-        rec(b, SNPM_EV_COMBINE);
-        SNPM_CUDA(cudaEventRecord(b->ev_inputs_free, st));
-        b->ran = true;
-        b->ran_windows = false;
-        b->epilogue_done = false;
-        return SNPM_OK;
+        return run_done(b);
     }
     if (kernel_mode == 2) {
         if (b->nseg_cap > 0) {
@@ -1481,12 +1449,7 @@ int snpm_batch_run(snpm_batch *b, int skip_db_hets, int mode) {
                                                  nullptr, b->d_red.as<double>());
         SNPM_KERNEL_CHECK();
         b->launches += 1;
-        rec(b, SNPM_EV_COMBINE);
-        SNPM_CUDA(cudaEventRecord(b->ev_inputs_free, st));
-        b->ran = true;
-        b->ran_windows = false;
-        b->epilogue_done = false;
-        return SNPM_OK;
+        return run_done(b);
     }
     if (kernel_mode == 1 && b->chunk_rows != SNPM_CHUNK_ROWS)
         return fail(SNPM_E_STATE, "snpm_batch_run: the popcount kernel works in %d-row chunks (its sums are exact in any chunking); set the chunk back", SNPM_CHUNK_ROWS);
@@ -1523,12 +1486,7 @@ int snpm_batch_run(snpm_batch *b, int skip_db_hets, int mode) {
     k_combine<<<cgrid, 32, 0, st>>>(a.part_score, a.part_ninfo, a.a_pad, db->n_acc, a.seg_off, a.mstart, 0, nullptr, nullptr, b->d_red.as<double>());
     SNPM_KERNEL_CHECK();
     b->launches += 1;
-    rec(b, SNPM_EV_COMBINE);
-    SNPM_CUDA(cudaEventRecord(b->ev_inputs_free, st));
-    b->ran = true;
-    b->ran_windows = false;
-    b->epilogue_done = false;
-    return SNPM_OK;
+    return run_done(b);
 }
 
 int snpm_batch_epilogue(snpm_batch *b) {
@@ -1563,6 +1521,23 @@ int snpm_batch_epilogue(snpm_batch *b) {
     return SNPM_OK;
 }
 
+// the argument and state errors the kernels count in the status slots (read back into h_status), in their order of precedence
+static int status_error(const int *h_status) {
+    if (h_status[0] > 0)
+        return fail(SNPM_E_ARG, "sample markers are not sorted by (database chromosome order, position) or repeat a position (%d places)", h_status[0]);
+    if (h_status[1] > 0)
+        return fail(SNPM_E_ASSERT, "provided y is greater than n (%d window cells; likeliTest, snpmatch.py:43)", h_status[1]);
+    if (h_status[2] > 0)
+        return fail(SNPM_E_ARG, "identity table too short for %d window cells", h_status[2]);
+    if (h_status[3] > 0)
+        return fail(SNPM_E_ARG, "kernel mode 1 needs one-hot weights (called genotypes); %d matched markers are not", h_status[3]);
+    if (h_status[4] > 0)
+        return fail(SNPM_E_ARG, "%d matched markers carry a weight-triple id outside the table (or run-length coded ids do not ascend)", h_status[4]);
+    if (h_status[5] > 0)
+        return fail(SNPM_E_STATE, "peer reduce: a rank did not arrive within thirty seconds (every rank must run and reduce the same batches in the same order)");
+    return SNPM_OK;
+}
+
 int snpm_batch_wait(snpm_batch *b, float *ms_device) {
     if (!b) return fail(SNPM_E_ARG, "snpm_batch_wait: NULL batch");
     snpm_db *db = b->db;
@@ -1583,19 +1558,7 @@ int snpm_batch_wait(snpm_batch *b, float *ms_device) {
             *ms_device += t;
         }
     }
-    if (b->h_status[0] > 0)
-        return fail(SNPM_E_ARG, "sample markers are not sorted by (database chromosome order, position) or repeat a position (%d places)", b->h_status[0]);
-    if (b->h_status[1] > 0)
-        return fail(SNPM_E_ASSERT, "provided y is greater than n (%d window cells; likeliTest, snpmatch.py:43)", b->h_status[1]);
-    if (b->h_status[2] > 0)
-        return fail(SNPM_E_ARG, "identity table too short for %d window cells", b->h_status[2]);
-    if (b->h_status[3] > 0)
-        return fail(SNPM_E_ARG, "kernel mode 1 needs one-hot weights (called genotypes); %d matched markers are not", b->h_status[3]);
-    if (b->h_status[4] > 0)
-        return fail(SNPM_E_ARG, "%d matched markers carry a weight-triple id outside the table (or run-length coded ids do not ascend)", b->h_status[4]);
-    if (b->h_status[5] > 0)
-        return fail(SNPM_E_STATE, "peer reduce: a rank did not arrive within thirty seconds (every rank must run and reduce the same batches in the same order)");
-    return SNPM_OK;
+    return status_error(b->h_status);
 }
 
 int snpm_batch_timings(snpm_batch *b, float *ms, int n) {
@@ -1719,35 +1682,45 @@ int snpm_batch_reduce_peers(snpm_batch *b) {
     return SNPM_OK;
 }
 
+// queues on `st` the read-back of the result range: the (m, y > n count) pair of every sample into `tail` (2 doubles a sample),
+// and whichever of the scores and the epilogue's outputs the caller asks for
+static int queue_result_copies(snpm_batch *b, cudaStream_t st, double *tail, double *score, int64_t *matches, int64_t *ninfo, double *prob,
+                               double *L, double *LR) {
+    const size_t A = size_t(b->db->n_acc), S = size_t(b->rangen()), R0 = size_t(b->range0()), pitch = size_t(b->red_pitch()) * 8;
+    const double *red = b->d_red.as<double>() + R0 * size_t(b->red_pitch());
+    if (score) SNPM_CUDA(cudaMemcpy2DAsync(score, A * 8, red, pitch, A * 8, S, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaMemcpy2DAsync(tail, 16, red + 2 * A, pitch, 16, S, cudaMemcpyDeviceToHost, st));
+    if (matches) SNPM_CUDA(cudaMemcpyAsync(matches, b->d_matches.as<int64_t>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
+    if (ninfo) SNPM_CUDA(cudaMemcpyAsync(ninfo, b->d_ninfo64.as<int64_t>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
+    if (prob) SNPM_CUDA(cudaMemcpyAsync(prob, b->d_prob.as<double>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
+    if (L) SNPM_CUDA(cudaMemcpyAsync(L, b->d_L.as<double>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
+    if (LR) SNPM_CUDA(cudaMemcpyAsync(LR, b->d_LR.as<double>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
+    return SNPM_OK;
+}
+
+// m of each of the S samples from the read-back tail; with `check` (after the epilogue) an accession with y > n fails the fetch
+static int decode_tail(const double *tail, int64_t S, int64_t *m, bool check) {
+    long long viol = 0;
+    for (int64_t s = 0; s < S; ++s) {
+        if (m) m[s] = int64_t(tail[2 * s]);
+        viol += (long long)tail[2 * s + 1];
+    }
+    if (viol > 0 && check) return fail(SNPM_E_ASSERT, "provided y is greater than n (%lld accessions; likeliTest, snpmatch.py:43)", viol);
+    return SNPM_OK;
+}
+
 int snpm_batch_fetch(snpm_batch *b, double *score, int64_t *matches, int64_t *ninfo, int64_t *m, double *prob, double *L, double *LR) {
     if (!b) return fail(SNPM_E_ARG, "snpm_batch_fetch: NULL batch");
     if (!b->ran) return fail(SNPM_E_STATE, "snpm_batch_fetch: run the batch first");
     if ((matches || ninfo || prob || L || LR) && !b->epilogue_done) return fail(SNPM_E_STATE, "snpm_batch_fetch: run the epilogue first");
-    snpm_db *db = b->db;
-    SNPM_CUDA(cudaSetDevice(db->device));
-    cudaStream_t st = db->stream;
-    const size_t A = size_t(db->n_acc), S = size_t(b->rangen()), R0 = size_t(b->range0()), pitch = size_t(b->red_pitch()) * 8;
+    SNPM_CUDA(cudaSetDevice(b->db->device));
+    const size_t S = size_t(b->rangen()), R0 = size_t(b->range0());
     if (R0 + S > size_t(b->S)) return fail(SNPM_E_ARG, "snpm_batch_fetch: result range outside the batch");
     if (b->grouped && score && !b->epilogue_done) return fail(SNPM_E_STATE, "snpm_batch_fetch: grouped batches finalise their scores in the epilogue; run it first");
-    const double *red = b->d_red.as<double>() + R0 * size_t(b->red_pitch());
     std::vector<double> tail(2 * S + 2);
-    if (S > 0) {
-        if (score) SNPM_CUDA(cudaMemcpy2DAsync(score, A * 8, red, pitch, A * 8, S, cudaMemcpyDeviceToHost, st));
-        SNPM_CUDA(cudaMemcpy2DAsync(tail.data(), 16, red + 2 * A, pitch, 16, S, cudaMemcpyDeviceToHost, st));
-        if (matches) SNPM_CUDA(cudaMemcpyAsync(matches, b->d_matches.as<int64_t>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
-        if (ninfo) SNPM_CUDA(cudaMemcpyAsync(ninfo, b->d_ninfo64.as<int64_t>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
-        if (prob) SNPM_CUDA(cudaMemcpyAsync(prob, b->d_prob.as<double>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
-        if (L) SNPM_CUDA(cudaMemcpyAsync(L, b->d_L.as<double>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
-        if (LR) SNPM_CUDA(cudaMemcpyAsync(LR, b->d_LR.as<double>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
-    }
+    if (S > 0) SNPM_TRY(queue_result_copies(b, b->db->stream, tail.data(), score, matches, ninfo, prob, L, LR));
     SNPM_TRY(snpm_batch_wait(b, nullptr));
-    long long viol = 0;
-    for (size_t s = 0; s < S; ++s) {
-        if (m) m[s] = int64_t(tail[2 * s]);
-        viol += (long long)tail[2 * s + 1];
-    }
-    if (viol > 0 && b->epilogue_done) return fail(SNPM_E_ASSERT, "provided y is greater than n (%lld accessions; likeliTest, snpmatch.py:43)", viol);
-    return SNPM_OK;
+    return decode_tail(tail.data(), int64_t(S), m, b->epilogue_done);
 }
 
 
@@ -1764,7 +1737,7 @@ int snpm_batch_fetch_async(snpm_batch *b, double *score, int64_t *matches, int64
     // the copies run on the batch's copy stream, behind an event that marks the end of its kernels: the read-back does not
     // hold up whatever is queued next on the compute stream
     cudaStream_t st = b->copy_stream;
-    const size_t A = size_t(db->n_acc), S = size_t(b->rangen()), R0 = size_t(b->range0()), pitch = size_t(b->red_pitch()) * 8;
+    const size_t S = size_t(b->rangen()), R0 = size_t(b->range0());
     if (R0 + S > size_t(b->S) || S == 0) return fail(SNPM_E_ARG, "snpm_batch_fetch_async: empty result range or outside the batch");
     if (!b->ev_fetched) SNPM_CUDA(cudaEventCreateWithFlags(&b->ev_fetched, cudaEventDisableTiming));
     if (!b->ev_results) SNPM_CUDA(cudaEventCreateWithFlags(&b->ev_results, cudaEventDisableTiming));
@@ -1776,14 +1749,7 @@ int snpm_batch_fetch_async(snpm_batch *b, double *score, int64_t *matches, int64
         SNPM_CUDA(cudaMallocHost(reinterpret_cast<void **>(&b->h_tail), S * 16));
         b->h_tail_cap = int64_t(S);
     }
-    const double *red = b->d_red.as<double>() + R0 * size_t(b->red_pitch());
-    if (score) SNPM_CUDA(cudaMemcpy2DAsync(score, A * 8, red, pitch, A * 8, S, cudaMemcpyDeviceToHost, st));
-    SNPM_CUDA(cudaMemcpy2DAsync(b->h_tail, 16, red + 2 * A, pitch, 16, S, cudaMemcpyDeviceToHost, st));
-    if (matches) SNPM_CUDA(cudaMemcpyAsync(matches, b->d_matches.as<int64_t>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
-    if (ninfo) SNPM_CUDA(cudaMemcpyAsync(ninfo, b->d_ninfo64.as<int64_t>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
-    if (prob) SNPM_CUDA(cudaMemcpyAsync(prob, b->d_prob.as<double>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
-    if (L) SNPM_CUDA(cudaMemcpyAsync(L, b->d_L.as<double>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
-    if (LR) SNPM_CUDA(cudaMemcpyAsync(LR, b->d_LR.as<double>() + R0 * A, S * A * 8, cudaMemcpyDeviceToHost, st));
+    SNPM_TRY(queue_result_copies(b, st, b->h_tail, score, matches, ninfo, prob, L, LR));
     if (guard) {
         if (b->grouped) SNPM_CUDA(cudaMemcpyAsync(guard, b->d_guard.as<int32_t>() + R0, S * 4, cudaMemcpyDeviceToHost, st));
         else memset(guard, 0, S * 4);
@@ -1802,21 +1768,8 @@ int snpm_batch_fetch_wait(snpm_batch *b) {
     SNPM_CUDA(cudaSetDevice(b->db->device));
     SNPM_CUDA(cudaEventSynchronize(b->ev_fetched));
     b->fetch_pending = false;
-    if (b->h_status[0] > 0)
-        return fail(SNPM_E_ARG, "sample markers are not sorted by (database chromosome order, position) or repeat a position (%d places)", b->h_status[0]);
-    if (b->h_status[3] > 0)
-        return fail(SNPM_E_ARG, "kernel mode 1 needs one-hot weights (called genotypes); %d matched markers are not", b->h_status[3]);
-    if (b->h_status[4] > 0)
-        return fail(SNPM_E_ARG, "%d matched markers carry a weight-triple id outside the table (or run-length coded ids do not ascend)", b->h_status[4]);
-    if (b->h_status[5] > 0)
-        return fail(SNPM_E_STATE, "peer reduce: a rank did not arrive within thirty seconds (every rank must run and reduce the same batches in the same order)");
-    long long viol = 0;
-    for (int64_t s = 0; s < b->rangen(); ++s) {
-        if (b->pend_m) b->pend_m[s] = int64_t(b->h_tail[2 * s]);
-        viol += (long long)b->h_tail[2 * s + 1];
-    }
-    if (viol > 0) return fail(SNPM_E_ASSERT, "provided y is greater than n (%lld accessions; likeliTest, snpmatch.py:43)", viol);
-    return SNPM_OK;
+    SNPM_TRY(status_error(b->h_status));
+    return decode_tail(b->h_tail, b->rangen(), b->pend_m, true);
 }
 
 int snpm_batch_fetch_pairs(snpm_batch *b, int64_t s, int64_t *db_idx, int64_t *s_idx, int64_t capacity, int64_t *m) {
@@ -1897,40 +1850,34 @@ int snpm_match_gts_accs(int device, const double *wei, const int8_t *snps, int64
         w4[size_t(4 * r + 3)] = 0.0;
     }
     const int32_t seg[2] = {0, int32_t(k)};
+    struct Stream {
+        cudaStream_t s = nullptr;
+        ~Stream() { if (s) cudaStreamDestroy(s); }
+    } own;
+    SNPM_CUDA(cudaStreamCreateWithFlags(&own.s, cudaStreamNonBlocking));
+    cudaStream_t st = own.s;
     DevBuf d_snps, d_packed, d_rows, d_w, d_seg, d_ps, d_pn;
-    int rc = SNPM_OK;
-    cudaStream_t st = nullptr;
-    auto cleanup = [&]() {
-        d_snps.release(); d_packed.release(); d_rows.release(); d_w.release(); d_seg.release(); d_ps.release(); d_pn.release();
-        if (st) cudaStreamDestroy(st);
-    };
-#define MG_TRY(x) do { rc = (x); if (rc != SNPM_OK) { cleanup(); return rc; } } while (0)
-#define MG_CUDA(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { cleanup(); return fail(SNPM_E_CUDA, "snpm_match_gts_accs: %s -> %s", #x, cudaGetErrorString(e_)); } } while (0)
-    MG_CUDA(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-    MG_TRY(d_snps.ensure(size_t(k) * n_acc));
-    MG_TRY(d_packed.ensure(size_t(k) * stride * 8));
-    MG_TRY(d_rows.ensure(size_t(k) * 4));
-    MG_TRY(d_w.ensure(size_t(k) * 32));
-    MG_TRY(d_seg.ensure(8));
-    MG_TRY(d_ps.ensure(size_t(a_pad) * 8));
-    MG_TRY(d_pn.ensure(size_t(a_pad) * 4));
+    SNPM_TRY(d_snps.ensure(size_t(k) * n_acc));
+    SNPM_TRY(d_packed.ensure(size_t(k) * stride * 8));
+    SNPM_TRY(d_rows.ensure(size_t(k) * 4));
+    SNPM_TRY(d_w.ensure(size_t(k) * 32));
+    SNPM_TRY(d_seg.ensure(8));
+    SNPM_TRY(d_ps.ensure(size_t(a_pad) * 8));
+    SNPM_TRY(d_pn.ensure(size_t(a_pad) * 4));
     if (k > 0) {
-        MG_CUDA(cudaMemcpyAsync(d_snps.p, snps, size_t(k) * n_acc, cudaMemcpyHostToDevice, st));
-        MG_CUDA(cudaMemcpyAsync(d_rows.p, iota.data(), size_t(k) * 4, cudaMemcpyHostToDevice, st));
-        MG_CUDA(cudaMemcpyAsync(d_w.p, w4.data(), size_t(k) * 32, cudaMemcpyHostToDevice, st));
+        SNPM_CUDA(cudaMemcpyAsync(d_snps.p, snps, size_t(k) * n_acc, cudaMemcpyHostToDevice, st));
+        SNPM_CUDA(cudaMemcpyAsync(d_rows.p, iota.data(), size_t(k) * 4, cudaMemcpyHostToDevice, st));
+        SNPM_CUDA(cudaMemcpyAsync(d_w.p, w4.data(), size_t(k) * 32, cudaMemcpyHostToDevice, st));
         int *d_bad = d_seg.as<int>() + 4;            // DevBuf allocations hold at least 256 bytes
-        MG_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
+        SNPM_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
         k_pack_int8<<<grid_for(k * stride * 32, 256, 148), 256, 0, st>>>(d_snps.as<int8_t>(), k, n_acc, stride, d_packed.as<uint64_t>(), d_bad);
-        MG_CUDA(cudaGetLastError());
+        SNPM_CUDA(cudaGetLastError());
         int bad = 0;
-        MG_CUDA(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
-        MG_CUDA(cudaStreamSynchronize(st));
-        if (bad > 0) {
-            cleanup();
-            return fail(SNPM_E_RANGE, "snpm_match_gts_accs: %d genotype codes above 2 (codes are 0 ref, 1 alt, 2 het, negative = missing)", bad);
-        }
+        SNPM_CUDA(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+        SNPM_CUDA(cudaStreamSynchronize(st));
+        if (bad > 0) return fail(SNPM_E_RANGE, "snpm_match_gts_accs: %d genotype codes above 2 (codes are 0 ref, 1 alt, 2 het, negative = missing)", bad);
     }
-    MG_CUDA(cudaMemcpyAsync(d_seg.p, seg, 8, cudaMemcpyHostToDevice, st));
+    SNPM_CUDA(cudaMemcpyAsync(d_seg.p, seg, 8, cudaMemcpyHostToDevice, st));
     ScoreArgs a = {};
     a.packed = d_packed.as<uint64_t>();
     a.stride = stride;
@@ -1943,51 +1890,18 @@ int snpm_match_gts_accs(int device, const double *wei, const int8_t *snps, int64
     a.part_score = d_ps.as<double>();
     a.part_ninfo = d_pn.as<int32_t>();
     a.a_pad = int32_t(a_pad);
-    MG_TRY(launch_score(st, a, 1, skip_hets_db != 0));
+    SNPM_TRY(launch_score(st, a, 1, skip_hets_db != 0));
     std::vector<int32_t> ni(static_cast<size_t>(n_acc), 0);
-    MG_CUDA(cudaMemcpyAsync(score, d_ps.p, size_t(n_acc) * 8, cudaMemcpyDeviceToHost, st));
-    MG_CUDA(cudaMemcpyAsync(ni.data(), d_pn.p, size_t(n_acc) * 4, cudaMemcpyDeviceToHost, st));
-    MG_CUDA(cudaStreamSynchronize(st));
+    SNPM_CUDA(cudaMemcpyAsync(score, d_ps.p, size_t(n_acc) * 8, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaMemcpyAsync(ni.data(), d_pn.p, size_t(n_acc) * 4, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaStreamSynchronize(st));
     for (int32_t i = 0; i < n_acc; ++i) ninfo[i] = ni[size_t(i)];
-    cleanup();
-#undef MG_TRY
-#undef MG_CUDA
     return SNPM_OK;
 }
 
 int snpm_calculate_likelihoods(int device, const double *scores, const double *ninfo, int64_t n_acc, int amin_is_calc, double amin,
                                double *prob, double *L, double *LR) {
-    if (n_acc <= 0 || n_acc >= (int64_t(1) << 30) || !scores || !ninfo) return fail(SNPM_E_ARG, "snpm_calculate_likelihoods: bad arguments");
-    int n_dev = 0;
-    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) return fail(SNPM_E_CUDA, "snpm_calculate_likelihoods: no CUDA device (there is no CPU fallback)");
-    SNPM_CUDA(cudaSetDevice(device));
-    const size_t A = size_t(n_acc);
-    std::vector<double> red(2 * A + 2, 0.0);
-    memcpy(red.data(), scores, A * 8);
-    memcpy(red.data() + A, ninfo, A * 8);
-    DevBuf d_red, d_out;
-    int rc = d_red.ensure((2 * A + 2) * 8);
-    if (rc == SNPM_OK) rc = d_out.ensure(3 * A * 8);
-    cudaError_t e = cudaSuccess;
-    if (rc == SNPM_OK) {
-        e = cudaMemcpy(d_red.p, red.data(), (2 * A + 2) * 8, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) {
-            double *o = d_out.as<double>();
-            e = launch_epilogue(nullptr, 1, d_red.as<double>(), 2 * int64_t(n_acc) + 2, int32_t(n_acc), 0, amin_is_calc ? 0 : 1, amin, nullptr, nullptr, o, o + A, o + 2 * A);
-            if (e == cudaSuccess) e = cudaGetLastError();
-        }
-        if (e == cudaSuccess) e = cudaDeviceSynchronize();
-        double viol = 0.0;
-        if (e == cudaSuccess) e = cudaMemcpy(&viol, d_red.as<double>() + 2 * A + 1, 8, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess && prob) e = cudaMemcpy(prob, d_out.p, A * 8, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess && L) e = cudaMemcpy(L, d_out.as<double>() + A, A * 8, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess && LR) e = cudaMemcpy(LR, d_out.as<double>() + 2 * A, A * 8, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess && viol > 0.0) rc = fail(SNPM_E_ASSERT, "provided y is greater than n (%lld accessions; likeliTest, snpmatch.py:43)", (long long)viol);
-    }
-    d_red.release();
-    d_out.release();
-    if (e != cudaSuccess) return fail(SNPM_E_CUDA, "snpm_calculate_likelihoods: %s", cudaGetErrorString(e));
-    return rc;
+    return snpm_calculate_likelihoods_many(device, scores, ninfo, 1, n_acc, amin_is_calc, amin, prob, L, LR);
 }
 
 int snpm_calculate_likelihoods_many(int device, const double *scores, const double *ninfo, int64_t S, int64_t K, int amin_is_calc, double amin,
@@ -2006,30 +1920,22 @@ int snpm_calculate_likelihoods_many(int device, const double *scores, const doub
         memcpy(red.data() + size_t(s) * pitch + K, ninfo + size_t(s) * K, size_t(K) * 8);
     }
     DevBuf d_red, d_out;
-    int rc = d_red.ensure(red.size() * 8);
-    if (rc == SNPM_OK) rc = d_out.ensure(3 * SK * 8);
-    cudaError_t e = cudaSuccess;
-    if (rc == SNPM_OK) {
-        e = cudaMemcpy(d_red.p, red.data(), red.size() * 8, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) {
-            double *o = d_out.as<double>();
-            e = launch_epilogue(nullptr, S, d_red.as<double>(), int64_t(pitch), int32_t(K), 0, amin_is_calc ? 0 : 1, amin, nullptr, nullptr, o, o + SK, o + 2 * SK);
-            if (e == cudaSuccess) e = cudaGetLastError();
-        }
-        if (e == cudaSuccess) e = cudaDeviceSynchronize();
-        std::vector<double> viol(size_t(S), 0.0);
-        if (e == cudaSuccess) e = cudaMemcpy2D(viol.data(), 8, d_red.as<double>() + 2 * K + 1, pitch * 8, 8, size_t(S), cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess && prob) e = cudaMemcpy(prob, d_out.p, SK * 8, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess && L) e = cudaMemcpy(L, d_out.as<double>() + SK, SK * 8, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess && LR) e = cudaMemcpy(LR, d_out.as<double>() + 2 * SK, SK * 8, cudaMemcpyDeviceToHost);
-        for (int64_t s = 0; s < S && e == cudaSuccess && rc == SNPM_OK; ++s)
-            if (viol[size_t(s)] > 0.0)
-                rc = fail(SNPM_E_ASSERT, "provided y is greater than n (row %lld, %lld accessions; likeliTest, snpmatch.py:43)", (long long)s, (long long)viol[size_t(s)]);
-    }
-    d_red.release();
-    d_out.release();
-    if (e != cudaSuccess) return fail(SNPM_E_CUDA, "snpm_calculate_likelihoods_many: %s", cudaGetErrorString(e));
-    return rc;
+    SNPM_TRY(d_red.ensure(red.size() * 8));
+    SNPM_TRY(d_out.ensure(3 * SK * 8));
+    SNPM_CUDA(cudaMemcpy(d_red.p, red.data(), red.size() * 8, cudaMemcpyHostToDevice));
+    double *o = d_out.as<double>();
+    SNPM_CUDA(launch_epilogue(nullptr, S, d_red.as<double>(), int64_t(pitch), int32_t(K), 0, amin_is_calc ? 0 : 1, amin, nullptr, nullptr, o, o + SK, o + 2 * SK));
+    SNPM_CUDA(cudaGetLastError());
+    SNPM_CUDA(cudaDeviceSynchronize());
+    std::vector<double> viol(size_t(S), 0.0);
+    SNPM_CUDA(cudaMemcpy2D(viol.data(), 8, d_red.as<double>() + 2 * K + 1, pitch * 8, 8, size_t(S), cudaMemcpyDeviceToHost));
+    if (prob) SNPM_CUDA(cudaMemcpy(prob, d_out.p, SK * 8, cudaMemcpyDeviceToHost));
+    if (L) SNPM_CUDA(cudaMemcpy(L, d_out.as<double>() + SK, SK * 8, cudaMemcpyDeviceToHost));
+    if (LR) SNPM_CUDA(cudaMemcpy(LR, d_out.as<double>() + 2 * SK, SK * 8, cudaMemcpyDeviceToHost));
+    for (int64_t s = 0; s < S; ++s)
+        if (viol[size_t(s)] > 0.0)
+            return fail(SNPM_E_ASSERT, "provided y is greater than n (row %lld, %lld accessions; likeliTest, snpmatch.py:43)", (long long)s, (long long)viol[size_t(s)]);
+    return SNPM_OK;
 }
 
 // ---- 8(f)-4: genotype_cross window calls -----------------------------------------------------------------
@@ -2052,36 +1958,32 @@ int snpm_cross_window_genotypes(int device, const int64_t *par_idx, const int64_
     if (cells == 0) return SNPM_OK;
     SNPM_CUDA(cudaSetDevice(device));
     DevBuf d_pi, d_vi, d_ws, d_p1, d_p2, d_gt, d_cnt, d_geno, d_border;
-    int rc = SNPM_OK;
-    cudaError_t e = cudaSuccess;
-    auto up = [&](DevBuf &d, const void *src, size_t bytes) {
-        if (rc != SNPM_OK || e != cudaSuccess) return;
-        rc = d.ensure(bytes);
-        if (rc == SNPM_OK && bytes) e = cudaMemcpy(d.p, src, bytes, cudaMemcpyHostToDevice);
-    };
-    up(d_pi, par_idx, size_t(m) * 8);
-    up(d_vi, vcf_idx, size_t(m) * 8);
-    up(d_ws, win_start, (size_t(n_windows) + 1) * 4);
-    up(d_p1, p1, size_t(n_par));
-    up(d_p2, p2, size_t(n_par));
-    up(d_gt, gt, size_t(n_vcf) * size_t(n_samples));
-    if (rc == SNPM_OK) rc = d_cnt.ensure(cells * 12);
-    if (rc == SNPM_OK) rc = d_geno.ensure(cells);
-    if (rc == SNPM_OK) rc = d_border.ensure(cells);
-    if (rc == SNPM_OK && e == cudaSuccess) {
-        dim3 grid(unsigned(n_windows), unsigned((n_samples + GC_THREADS - 1) / GC_THREADS));
-        k_gc_window_calls<<<grid, GC_THREADS>>>(d_pi.as<int64_t>(), d_vi.as<int64_t>(), d_ws.as<int32_t>(), d_p1.as<int8_t>(), d_p2.as<int8_t>(),
-                                                d_gt.as<int8_t>(), n_samples, lr_thres, n_marker_thres, d_cnt.as<int32_t>(), d_geno.as<int8_t>(),
-                                                d_border.as<uint8_t>());
-        e = cudaGetLastError();
-        if (e == cudaSuccess) e = cudaDeviceSynchronize();
-        if (e == cudaSuccess) e = cudaMemcpy(counts, d_cnt.p, cells * 12, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(geno, d_geno.p, cells, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess && borderline) e = cudaMemcpy(borderline, d_border.p, cells, cudaMemcpyDeviceToHost);
-    }
-    for (DevBuf *d : {&d_pi, &d_vi, &d_ws, &d_p1, &d_p2, &d_gt, &d_cnt, &d_geno, &d_border}) d->release();
-    if (e != cudaSuccess) return fail(SNPM_E_CUDA, "snpm_cross_window_genotypes: %s", cudaGetErrorString(e));
-    return rc;
+    const size_t n_gt = size_t(n_vcf) * size_t(n_samples);
+    SNPM_TRY(d_pi.ensure(size_t(m) * 8));
+    if (m) SNPM_CUDA(cudaMemcpy(d_pi.p, par_idx, size_t(m) * 8, cudaMemcpyHostToDevice));
+    SNPM_TRY(d_vi.ensure(size_t(m) * 8));
+    if (m) SNPM_CUDA(cudaMemcpy(d_vi.p, vcf_idx, size_t(m) * 8, cudaMemcpyHostToDevice));
+    SNPM_TRY(d_ws.ensure((size_t(n_windows) + 1) * 4));
+    SNPM_CUDA(cudaMemcpy(d_ws.p, win_start, (size_t(n_windows) + 1) * 4, cudaMemcpyHostToDevice));
+    SNPM_TRY(d_p1.ensure(size_t(n_par)));
+    if (n_par) SNPM_CUDA(cudaMemcpy(d_p1.p, p1, size_t(n_par), cudaMemcpyHostToDevice));
+    SNPM_TRY(d_p2.ensure(size_t(n_par)));
+    if (n_par) SNPM_CUDA(cudaMemcpy(d_p2.p, p2, size_t(n_par), cudaMemcpyHostToDevice));
+    SNPM_TRY(d_gt.ensure(n_gt));
+    if (n_gt) SNPM_CUDA(cudaMemcpy(d_gt.p, gt, n_gt, cudaMemcpyHostToDevice));
+    SNPM_TRY(d_cnt.ensure(cells * 12));
+    SNPM_TRY(d_geno.ensure(cells));
+    SNPM_TRY(d_border.ensure(cells));
+    dim3 grid(unsigned(n_windows), unsigned((n_samples + GC_THREADS - 1) / GC_THREADS));
+    k_gc_window_calls<<<grid, GC_THREADS>>>(d_pi.as<int64_t>(), d_vi.as<int64_t>(), d_ws.as<int32_t>(), d_p1.as<int8_t>(), d_p2.as<int8_t>(),
+                                            d_gt.as<int8_t>(), n_samples, lr_thres, n_marker_thres, d_cnt.as<int32_t>(), d_geno.as<int8_t>(),
+                                            d_border.as<uint8_t>());
+    SNPM_CUDA(cudaGetLastError());
+    SNPM_CUDA(cudaDeviceSynchronize());
+    SNPM_CUDA(cudaMemcpy(counts, d_cnt.p, cells * 12, cudaMemcpyDeviceToHost));
+    SNPM_CUDA(cudaMemcpy(geno, d_geno.p, cells, cudaMemcpyDeviceToHost));
+    if (borderline) SNPM_CUDA(cudaMemcpy(borderline, d_border.p, cells, cudaMemcpyDeviceToHost));
+    return SNPM_OK;
 }
 
 // ---- A9 ------------------------------------------------------------------------------------------------
@@ -2093,12 +1995,9 @@ struct snpm_panel {
     int32_t n_kb = 0, n_blocks = 0, ld_out = 0;
     DevBuf d_rows, d_bt, d_codes, d_at, d_os, d_on, d_red, d_m, d_n64, d_p, d_l, d_lr;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
-    void release() {
-        for (DevBuf *d : {&d_rows, &d_bt, &d_codes, &d_at, &d_os, &d_on, &d_red, &d_m, &d_n64, &d_p, &d_l, &d_lr}) d->release();
-        for (cudaEvent_t &e : ev) {
+    ~snpm_panel() {
+        for (cudaEvent_t e : ev)
             if (e) cudaEventDestroy(e);
-            e = nullptr;
-        }
     }
 };
 
@@ -2108,7 +2007,7 @@ int snpm_panel_create(snpm_db *db, const int64_t *panel_rows, int64_t K, int ski
     *out = nullptr;
     SNPM_CUDA(cudaSetDevice(db->device));
     cudaStream_t st = db->stream;
-    std::unique_ptr<snpm_panel, void (*)(snpm_panel *)> p(new (std::nothrow) snpm_panel, [](snpm_panel *q) { q->release(); delete q; });
+    std::unique_ptr<snpm_panel> p(new (std::nothrow) snpm_panel);
     if (!p) return fail(SNPM_E_NOMEM, "snpm_panel_create: out of host memory");
     p->db = db;
     p->K = K;
@@ -2137,7 +2036,6 @@ int snpm_panel_create(snpm_db *db, const int64_t *panel_rows, int64_t K, int ski
 void snpm_panel_destroy(snpm_panel *p) {
     if (!p) return;
     cudaSetDevice(p->db->device);
-    p->release();
     delete p;
 }
 
@@ -2351,12 +2249,9 @@ static int windows_finish(snpm_batch *b) {
         SNPM_KERNEL_CHECK();
         b->launches += 2;
     }
-    rec(b, SNPM_EV_COMBINE);
-    SNPM_CUDA(cudaEventRecord(b->ev_inputs_free, st));
+    SNPM_TRY(run_done(b));
     b->win_pending = false;
-    b->ran = true;
     b->ran_windows = true;
-    b->epilogue_done = false;
     return SNPM_OK;
 }
 
@@ -2397,6 +2292,49 @@ int snpm_batch_run_windows_finish(snpm_batch *b) {
     return windows_finish(b);
 }
 
+// the matched-marker ranges of all window slots of the last windows run, shared by the two window fetches
+struct WindowBounds {
+    std::vector<int32_t> begin, end;
+    int32_t m_all = 0;       // matched pairs of the batch
+    int64_t total = 0;       // of them inside the windows
+};
+
+// Queues the read-back of the bounds behind the caller's copies on the batch's stream, then waits for the batch; win_nrows (when
+// given) receives the rows of every window, on all ranks after a sharded run.
+static int read_window_bounds(snpm_batch *b, int32_t *win_nrows, WindowBounds &wb) {
+    cudaStream_t st = b->db->stream;
+    const size_t W = size_t(b->S) * size_t(b->n_windows);
+    std::vector<int32_t> nr(W + 1);
+    wb.begin.resize(W + 1);
+    wb.end.resize(W + 1);
+    if (W) {
+        SNPM_CUDA(cudaMemcpyAsync(wb.begin.data(), b->d_win_begin.p, W * 4, cudaMemcpyDeviceToHost, st));
+        SNPM_CUDA(cudaMemcpyAsync(wb.end.data(), b->d_win_end.p, W * 4, cudaMemcpyDeviceToHost, st));
+        SNPM_CUDA(cudaMemcpyAsync(nr.data(), b->d_win_nrows.p, W * 4, cudaMemcpyDeviceToHost, st));
+    }
+    SNPM_CUDA(cudaMemcpyAsync(&wb.m_all, b->d_prefix.as<int32_t>() + b->n, 4, cudaMemcpyDeviceToHost, st));
+    SNPM_TRY(snpm_batch_wait(b, nullptr));
+    for (size_t w = 0; w < W; ++w) {
+        if (win_nrows) win_nrows[w] = nr[w];
+        wb.total += wb.end[w] - wb.begin[w];
+    }
+    return SNPM_OK;
+}
+
+// matched_s_idx (when given): the sample index of every matched marker inside the windows, in window order
+static int gather_window_markers(snpm_batch *b, const WindowBounds &wb, const char *fn, int64_t *matched_s_idx, int64_t capacity) {
+    if (!matched_s_idx || wb.total == 0) return SNPM_OK;
+    if (wb.total > capacity) return fail(SNPM_E_ARG, "%s: capacity %lld < %lld matched markers", fn, (long long)capacity, (long long)wb.total);
+    cudaStream_t st = b->db->stream;
+    std::vector<int32_t> ps(size_t(wb.m_all));
+    SNPM_CUDA(cudaMemcpyAsync(ps.data(), b->d_pair_s.p, size_t(wb.m_all) * 4, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaStreamSynchronize(st));
+    int64_t o = 0;
+    for (size_t w = 0; w + 1 < wb.begin.size(); ++w)
+        for (int32_t r = wb.begin[w]; r < wb.end[w]; ++r) matched_s_idx[o++] = ps[size_t(r)];
+    return SNPM_OK;
+}
+
 int snpm_batch_fetch_windows(snpm_batch *b, double *win_score, int32_t *win_ninfo, double *win_L, double *win_LR, uint8_t *win_identical,
                              int32_t *win_num_amb, int32_t *win_nrows, int64_t *matched_s_idx, int64_t capacity, int64_t *n_matched) {
     if (!b) return fail(SNPM_E_ARG, "snpm_batch_fetch_windows: NULL batch");
@@ -2405,7 +2343,6 @@ int snpm_batch_fetch_windows(snpm_batch *b, double *win_score, int32_t *win_ninf
     SNPM_CUDA(cudaSetDevice(db->device));
     cudaStream_t st = db->stream;
     const size_t W = size_t(b->S) * size_t(b->n_windows), A = size_t(db->n_acc), a_pad = size_t(db->stride) * 32;     // all window slots
-    std::vector<int32_t> wb(W + 1), we(W + 1), nr(W + 1), ps;
     if (W) {
         if (win_score) SNPM_CUDA(cudaMemcpy2DAsync(win_score, A * 8, b->d_part_score.p, a_pad * 8, A * 8, W, cudaMemcpyDeviceToHost, st));
         if (win_ninfo) SNPM_CUDA(cudaMemcpy2DAsync(win_ninfo, A * 4, b->d_part_ninfo.p, a_pad * 4, A * 4, W, cudaMemcpyDeviceToHost, st));
@@ -2413,29 +2350,11 @@ int snpm_batch_fetch_windows(snpm_batch *b, double *win_score, int32_t *win_ninf
         if (win_LR) SNPM_CUDA(cudaMemcpyAsync(win_LR, b->d_win_LR.p, W * A * 8, cudaMemcpyDeviceToHost, st));
         if (win_identical) SNPM_CUDA(cudaMemcpyAsync(win_identical, b->d_win_ident.p, W * A, cudaMemcpyDeviceToHost, st));
         if (win_num_amb) SNPM_CUDA(cudaMemcpyAsync(win_num_amb, b->d_win_amb.p, W * 4, cudaMemcpyDeviceToHost, st));
-        SNPM_CUDA(cudaMemcpyAsync(wb.data(), b->d_win_begin.p, W * 4, cudaMemcpyDeviceToHost, st));
-        SNPM_CUDA(cudaMemcpyAsync(we.data(), b->d_win_end.p, W * 4, cudaMemcpyDeviceToHost, st));
-        SNPM_CUDA(cudaMemcpyAsync(nr.data(), b->d_win_nrows.p, W * 4, cudaMemcpyDeviceToHost, st));     // rows of the window on ALL ranks after a sharded run
     }
-    int32_t m_all = 0;
-    SNPM_CUDA(cudaMemcpyAsync(&m_all, b->d_prefix.as<int32_t>() + b->n, 4, cudaMemcpyDeviceToHost, st));
-    SNPM_TRY(snpm_batch_wait(b, nullptr));
-    int64_t total = 0;
-    for (size_t w = 0; w < W; ++w) {
-        if (win_nrows) win_nrows[w] = nr[w];
-        total += we[w] - wb[w];
-    }
-    if (n_matched) *n_matched = total;
-    if (matched_s_idx && total > 0) {
-        if (total > capacity) return fail(SNPM_E_ARG, "snpm_batch_fetch_windows: capacity %lld < %lld", (long long)capacity, (long long)total);
-        ps.resize(size_t(m_all));
-        SNPM_CUDA(cudaMemcpyAsync(ps.data(), b->d_pair_s.p, size_t(m_all) * 4, cudaMemcpyDeviceToHost, st));
-        SNPM_CUDA(cudaStreamSynchronize(st));
-        int64_t o = 0;
-        for (size_t w = 0; w < W; ++w)
-            for (int32_t r = wb[w]; r < we[w]; ++r) matched_s_idx[o++] = ps[size_t(r)];
-    }
-    return SNPM_OK;
+    WindowBounds wb;
+    SNPM_TRY(read_window_bounds(b, win_nrows, wb));
+    if (n_matched) *n_matched = wb.total;
+    return gather_window_markers(b, wb, "snpm_batch_fetch_windows", matched_s_idx, capacity);
 }
 
 
@@ -2452,26 +2371,17 @@ int snpm_batch_fetch_window_rows(snpm_batch *b, int32_t *win_row_off, int32_t *w
     SNPM_CUDA(cudaSetDevice(db->device));
     cudaStream_t st = db->stream;
     const size_t W = size_t(b->S) * size_t(b->n_windows);      // all window slots
-    std::vector<int32_t> off(W + 1, 0), wb(W + 1), we(W + 1), nr(W + 1), ps;
+    std::vector<int32_t> off(W + 1, 0);
     if (W) {
         SNPM_CUDA(cudaMemcpyAsync(off.data(), b->d_win_row_off.p, (W + 1) * 4, cudaMemcpyDeviceToHost, st));
-        SNPM_CUDA(cudaMemcpyAsync(wb.data(), b->d_win_begin.p, W * 4, cudaMemcpyDeviceToHost, st));
-        SNPM_CUDA(cudaMemcpyAsync(we.data(), b->d_win_end.p, W * 4, cudaMemcpyDeviceToHost, st));
-        SNPM_CUDA(cudaMemcpyAsync(nr.data(), b->d_win_nrows.p, W * 4, cudaMemcpyDeviceToHost, st));     // rows of the window on ALL ranks after a sharded run
         if (win_num_amb) SNPM_CUDA(cudaMemcpyAsync(win_num_amb, b->d_win_amb.p, W * 4, cudaMemcpyDeviceToHost, st));
     }
-    int32_t m_all = 0;
-    SNPM_CUDA(cudaMemcpyAsync(&m_all, b->d_prefix.as<int32_t>() + b->n, 4, cudaMemcpyDeviceToHost, st));
-    SNPM_TRY(snpm_batch_wait(b, nullptr));
+    WindowBounds wb;
+    SNPM_TRY(read_window_bounds(b, win_nrows, wb));
     const int64_t R = off[W];
     *n_rows = R;
     if (win_row_off) memcpy(win_row_off, off.data(), (W + 1) * 4);
-    int64_t total = 0;
-    for (size_t w = 0; w < W; ++w) {
-        if (win_nrows) win_nrows[w] = nr[w];
-        total += we[w] - wb[w];
-    }
-    if (n_matched) *n_matched = total;
+    if (n_matched) *n_matched = wb.total;
     if (R > 0 && (row_acc || row_score || row_ninfo || row_L || row_identical)) {
         if (R > capacity) return fail(SNPM_E_ARG, "snpm_batch_fetch_window_rows: capacity %lld < %lld rows", (long long)capacity, (long long)R);
         if (row_acc) SNPM_CUDA(cudaMemcpyAsync(row_acc, b->d_row_acc.p, size_t(R) * 4, cudaMemcpyDeviceToHost, st));
@@ -2480,17 +2390,8 @@ int snpm_batch_fetch_window_rows(snpm_batch *b, int32_t *win_row_off, int32_t *w
         if (row_L) SNPM_CUDA(cudaMemcpyAsync(row_L, b->d_row_L.p, size_t(R) * 8, cudaMemcpyDeviceToHost, st));
         if (row_identical) SNPM_CUDA(cudaMemcpyAsync(row_identical, b->d_row_ident.p, size_t(R), cudaMemcpyDeviceToHost, st));
     }
-    if (matched_s_idx && total > 0) {
-        if (total > matched_capacity) return fail(SNPM_E_ARG, "snpm_batch_fetch_window_rows: capacity %lld < %lld matched markers", (long long)matched_capacity, (long long)total);
-        ps.resize(size_t(m_all));
-        SNPM_CUDA(cudaMemcpyAsync(ps.data(), b->d_pair_s.p, size_t(m_all) * 4, cudaMemcpyDeviceToHost, st));
-    }
-    SNPM_CUDA(cudaStreamSynchronize(st));
-    if (matched_s_idx && total > 0) {
-        int64_t o = 0;
-        for (size_t w = 0; w < W; ++w)
-            for (int32_t r = wb[w]; r < we[w]; ++r) matched_s_idx[o++] = ps[size_t(r)];
-    }
+    SNPM_TRY(gather_window_markers(b, wb, "snpm_batch_fetch_window_rows", matched_s_idx, matched_capacity));
+    SNPM_CUDA(cudaStreamSynchronize(st));                       // the row copies
     return SNPM_OK;
 }
 

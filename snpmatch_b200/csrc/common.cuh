@@ -55,10 +55,14 @@ static inline bool snpm_sync_debug() {
         if (snpm_sync_debug()) SNPM_CUDA(cudaDeviceSynchronize());       \
     } while (0)
 
-// Grow-only device allocation.
+// Grow-only device allocation, freed with its owner.  The owner makes the buffer's device current before it destroys it.
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { release(); }
     int ensure(size_t bytes) {
         if (bytes <= cap && p) return SNPM_OK;
         if (p) { cudaFree(p); p = nullptr; cap = 0; }
@@ -159,7 +163,7 @@ struct snpm_batch {
     bool codes_packed = false;         // the three codes of a marker in one uint32 (snpm_batch_upload_coded32)
     int32_t n_wtable = 0, code_bits = 0, key_bits = 0;
     int64_t n_sort_tiles = 0;
-    snpm::DevBuf d_codes, d_wtable, d_key_a, d_key_b, d_idx_a, d_idx_b, d_pair_db_tmp, d_pair_s_tmp, d_tile_sample, d_tile_first,
+    snpm::DevBuf d_codes, d_wtable, d_key_a, d_pair_db_tmp, d_pair_s_tmp, d_tile_sample, d_tile_first,
                  d_tile_hist, d_blk_chg, d_seg_order, d_work_counter, d_hash, d_slot_gid, d_ngroups, d_group_overflow, d_gkeys, d_gw, d_goff;
     bool track_pairs = true;           // coded runs: also move the marker index of every pair into grouped order (snpm_batch_fetch_pairs)
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;   // coded runs: block words + work order on the copy stream next to the partition pass
