@@ -371,6 +371,26 @@ int snpm_pair_match_counts(int device, const int64_t *idx1, const int64_t *idx2,
 int snpm_pair_matrix(int device, int64_t S, const int64_t *offsets, const int32_t *col, const uint8_t *cls, int32_t n_cls, int64_t K,
                      const int64_t *chr_start, int32_t C, int64_t chunk_markers, int32_t *common, int32_t *same, float *ms);
 
+/* ---- accession against accession: every pair of panel accessions in one tensor-core pass --------------------------
+ * pairwiseScore's statistic for two accession columns of the resident panel, for every pair of the selection acc_idx
+ * int32[n_sel] (indices into the panel's accessions, in output order), over the rows this handle holds:
+ *   common[i, j] = rows on which accessions acc_idx[i] and acc_idx[j] are both called (code 0, 1 or 2),
+ *   same[i, j]   = those of them with equal codes (het equals het).
+ * With skip_db_hets, code 2 counts as missing.  Out: common / same int32 [n_sel, n_sel], full and symmetric; common[i, i] is the
+ * number of called rows of accession i.  Two row shards of one panel give counts that sum to the whole panel's.
+ * Both one-hot operands of a chunk of rows are expanded from the packed panel on the device (nothing but acc_idx crosses
+ * PCIe on the way in) and multiplied with k_onehot_gemm: 12 n_sel operand bytes per row, and 16 n_i n_j int8 operations per
+ * row for a block pair of n_i and n_j accessions (16 n_sel^2 when the selection is one block).
+ * The rows are walked in chunks of chunk_rows rows (0 = as many as fit SNPM_PAIR_CHUNK_BYTES of operand tiles; a chunk may
+ * span chromosomes).  The output is computed in blocks of block_acc accessions (0 = SNPM_ACC_BLOCK; a positive multiple of
+ * 256): block pairs bi <= bj, the blocks below the diagonal mirrored from the ones above, so a selection of 20 000 runs as
+ * 3 blocks and 6 block pairs.  Refused before any allocation, with the value named: n_sel < 1, an index outside 0..A-1,
+ * block_acc not a positive multiple of 256, chunk_rows < 0, and a handle of 2^31 rows or more (the counts are int32).
+ * ms (optional) float[3]: device time of the operand expansion, of the GEMMs, and of the whole call including the copies. */
+#define SNPM_ACC_BLOCK 8192
+int snpm_db_acc_pairs(snpm_db *db, const int32_t *acc_idx, int32_t n_sel, int skip_db_hets, int64_t chunk_rows, int32_t block_acc,
+                      int32_t *common, int32_t *same, float *ms);
+
 /* ---- 8(f)-4: genotype_cross -----------------------------------------------------------------
  * The window loop of GenotypeCross.genotype_cross (genotype_cross.py:210-241): for every genome window w and every sample s
  * of a multi-sample VCF, over the matched pairs k in [win_start[w], win_start[w+1]) (par_idx into the parents' segregating

@@ -100,7 +100,38 @@ def snpmatch_parser(args):
     parsers.potatoParser(inFile=args['inFile'], logDebug=args['logDebug'], outFile=args['outFile'])
 
 
+def read_accession_list(list_file):
+    """`pairsnp --accessions ids.txt`: one accession id per line, in output order; blank lines are skipped.  Dies on a
+    missing file, an empty list or an id listed twice."""
+    check_file(list_file)
+    ids, seen = [], {}
+    with open(list_file) as fh:
+        for k, line in enumerate(fh, 1):
+            a = line.strip()
+            if not a:
+                continue
+            if a in seen:
+                die("accession %s is listed twice in %s (lines %d and %d)" % (a, list_file, seen[a], k))
+            seen[a] = k
+            ids.append(a)
+    if not ids:
+        die("accession list is empty: " + list_file)
+    return ids
+
+
 def snpmatch_paircomparions(args):
+    if args.get('accessions'):
+        if args['inFile_1'] or args['inFile_2'] or args.get('samples'):
+            die("--accessions compares accessions of the database; it cannot be combined with -i / -j or --samples")
+        if not args['hdf5File']:
+            die("--accessions compares accessions of the database; give the database with -d")
+        check_file(args['hdf5File'])
+        ids = None if args['accessions'] == "all" else read_accession_list(args['accessions'])
+        from .core import snpmatch
+        snpmatch.panelIdentity(args, ids)
+        return
+    if args.get('skip_db_hets') or args.get('min_identity') is not None:
+        die("--skip_db_hets and --min_identity go with --accessions")
     if args.get('samples'):
         if args['inFile_1'] or args['inFile_2']:
             die("--samples compares every pair of the list; it cannot be combined with -i / -j")
@@ -188,7 +219,7 @@ def get_options(description, version_message):
     gc.add_argument("-v", "--verbose", action="store_true", dest="logDebug", default=False, help="log at DEBUG level")
     gc.set_defaults(func=genotype_cross)
 
-    pair = sub.add_parser('pairsnp', help="agreement of the genotype calls two samples (or every pair of many samples) share")
+    pair = sub.add_parser('pairsnp', help="agreement of the genotype calls two samples (or every pair of many samples, or of database accessions) share")
     pair.add_argument("-i", "--input_file_1", dest="inFile_1", help="first sample (VCF/BED/npz)")
     pair.add_argument("-j", "--input_file_2", dest="inFile_2", help="second sample (VCF/BED/npz)")
     pair.add_argument("--samples", dest="samples", default=None,
@@ -196,6 +227,16 @@ def get_options(description, version_message):
                            "(default: the file name); every pair is compared in one GPU pass: <-o>.identity.tsv, <-o>.common.tsv")
     pair.add_argument("--pairs_json", action="store_true", dest="pairs_json", default=False,
                       help="with --samples: also <-o>.pairs.jsonl, one line per pair with the statistics -i/-j writes to .matches.json")
+    pair.add_argument("--accessions", dest="accessions", default=None,
+                      help="'all', or a text file of database accession ids, one per line, in output order: every pair of those "
+                           "accessions of the -d database is compared over all its rows in one GPU pass: <-o>.identity.tsv, "
+                           "<-o>.common.tsv (n x n, labelled by the ids; at 20 000 accessions each file is several GB, the Python "
+                           "API snpmatch.panel_identity returns the arrays)")
+    pair.add_argument("--skip_db_hets", action="store_true", dest="skip_db_hets", default=False,
+                      help="with --accessions: treat heterozygous database calls as missing")
+    pair.add_argument("--min_identity", dest="min_identity", default=None, type=float,
+                      help="with --accessions: also <-o>.close_pairs.tsv, every pair with identity >= this value (acc_1, acc_2, "
+                           "identity, common, same), most identical first")
     pair.add_argument("-d", "--hdf5_file", dest="hdf5File", default=None, help=db_help)
     pair.add_argument("-v", "--verbose", action="store_true", dest="logDebug", default=False, help="log at DEBUG level")
     pair.add_argument("-o", "--output", dest="outFile", default="pairsnp", help="output prefix (<prefix>.matches.json)")

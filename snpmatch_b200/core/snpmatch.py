@@ -777,3 +777,112 @@ def pairwiseScoreMany(args, samples):
     log.info("writing %s.identity.tsv and %s.common.tsv", args['outFile'], args['outFile'])
     pm.write(args['outFile'], pairs_json=args.get('pairs_json', False), labels=[lab for _, lab in samples])
     return pm
+
+
+# ---- accession against accession ------------------------------------------------------------------------------------------
+class PanelIdentity(object):
+    """Result of panel_identity: common / same int32 [n,n] over the selected accessions `accessions` (ids, in output order):
+    the panel rows both accessions have called, and those of them with equal calls.  Symmetric; common[i, i] is the number
+    of called rows of accession i."""
+
+    def __init__(self, common, same, accessions, skip_db_hets=False):
+        self.common, self.same = common, same
+        self.accessions = accessions
+        self.skip_db_hets = skip_db_hets
+        self.timings = {}
+
+    def identity(self):
+        """[n,n] same / common, nan where the pair has no row both have called."""
+        with np.errstate(invalid="ignore", divide="ignore"):
+            return np.where(self.common > 0, self.same / np.maximum(self.common, 1), np.nan)
+
+    def close_pairs(self, min_identity):
+        """Pairs i < j with common > 0 and identity >= min_identity, most identical first (ties in (i, j) order):
+        a list of (acc_1, acc_2, identity, common, same)."""
+        n = len(self.accessions)
+        ii, jj, idents = [], [], []
+        step = max(1, (8 << 20) // max(n, 1))                   # rows at a time: the float matrix is never built whole
+        for r0 in range(0, n, step):
+            c = self.common[r0:r0 + step]
+            with np.errstate(invalid="ignore", divide="ignore"):
+                ident = self.same[r0:r0 + step] / np.maximum(c, 1)
+            i, j = np.nonzero((c > 0) & (ident >= min_identity) & (np.arange(n)[None, :] > np.arange(r0, r0 + len(c))[:, None]))
+            ii.append(i + r0)
+            jj.append(j)
+            idents.append(ident[i, j])
+        ii, jj, idents = np.concatenate(ii), np.concatenate(jj), np.concatenate(idents)
+        order = np.lexsort((jj, ii, -idents))
+        return [(str(self.accessions[i]), str(self.accessions[j]), float(v), int(self.common[i, j]), int(self.same[i, j]))
+                for i, j, v in zip(ii[order], jj[order], idents[order])]
+
+    def write(self, prefix, min_identity=None):
+        """<prefix>.identity.tsv and <prefix>.common.tsv (n x n, the accession ids as header row and first column, the layout
+        of `pairsnp --samples`) and, with min_identity, <prefix>.close_pairs.tsv: acc_1, acc_2, identity, common, same of every
+        close_pairs(min_identity) pair."""
+        import time
+        t0 = time.perf_counter()
+        labels = [str(a) for a in self.accessions]
+        check_labels(labels, len(labels))
+        write_matrix_tsv(prefix + ".identity.tsv", labels, self.identity())
+        write_matrix_tsv(prefix + ".common.tsv", labels, self.common)
+        if min_identity is not None:
+            with open(prefix + ".close_pairs.tsv", "w") as fh:
+                fh.write("acc_1\tacc_2\tidentity\tcommon\tsame\n")
+                for a, b, v, c, s in self.close_pairs(min_identity):
+                    fh.write("%s\t%s\t%s\t%d\t%d\n" % (a, b, str(v), c, s))
+        self.timings["write"] = time.perf_counter() - t0
+
+
+def accession_indices(g, accessions):
+    """Panel indices of the accession ids `accessions` (output order); None = every accession in panel order.  Raises
+    ValueError naming an id the panel lacks or one listed twice."""
+    ids = np.asarray(g.accessions).astype("U")
+    if accessions is None:
+        return np.arange(len(ids), dtype=np.int32)
+    index = {a: k for k, a in enumerate(ids.tolist())}
+    seen = {}
+    out = np.empty(len(accessions), dtype=np.int32)
+    for k, a in enumerate(str(x) for x in accessions):
+        if a in seen:
+            raise ValueError("accession %s is listed twice (entries %d and %d)" % (a, seen[a], k))
+        if a not in index:
+            raise ValueError("accession %s is not in the database" % a)
+        seen[a] = k
+        out[k] = index[a]
+    if not len(out):
+        raise ValueError("the accession list is empty")
+    return out
+
+
+def panel_identity(g, accessions=None, skip_db_hets=False, chunk_rows=0, block_acc=0):
+    """Which accessions of a panel cannot be told apart: pairwiseScore's statistic for every pair of the accessions
+    `accessions` (ids, in output order; default all) over every row of the resident panel g (a Genotype), in one tensor-core
+    pass (lib.Database.acc_pairs).  "Called" is code 0, 1 or 2; skip_db_hets counts hets as missing; het equals het.
+    Returns a PanelIdentity.  A Genotype holding a row shard is refused: its counts would cover part of the genome."""
+    import time
+    if g.db.row0_global != 0 or g.db.n_rows != int(np.max(getattr(g, "global_chr_regions", [[0, g.db.n_rows]]))):
+        raise ValueError("panel_identity needs the whole panel on one device; this one holds a shard of its rows")
+    idx = accession_indices(g, accessions)
+    t0 = time.perf_counter()
+    common, same, ms = g.db.acc_pairs(idx, skip_db_hets=skip_db_hets, chunk_rows=chunk_rows, block_acc=block_acc)
+    res = PanelIdentity(common, same, np.asarray(g.accessions).astype("U")[idx], skip_db_hets=skip_db_hets)
+    res.timings = {"device": time.perf_counter() - t0, "expand_ms": ms[0], "gemm_ms": ms[1], "device_ms": ms[2]}
+    return res
+
+
+def panelIdentity(args, accessions):
+    """`pairsnp --accessions`: accessions = ids in output order or None (all); writes <-o>.identity.tsv, <-o>.common.tsv and,
+    with --min_identity, <-o>.close_pairs.tsv.  Dies naming an id the database lacks."""
+    g = snp_genotype.Genotype(args['hdf5File'], None)
+    try:
+        try:
+            accession_indices(g, accessions)
+        except ValueError as e:
+            die(str(e))
+        log.info("comparing %d accessions over %d rows", len(g.accessions) if accessions is None else len(accessions), g.g.num_snps)
+        res = panel_identity(g, accessions, skip_db_hets=args.get('skip_db_hets', False))
+    finally:
+        g.close()
+    log.info("writing %s.identity.tsv and %s.common.tsv", args['outFile'], args['outFile'])
+    res.write(args['outFile'], min_identity=args.get('min_identity'))
+    return res

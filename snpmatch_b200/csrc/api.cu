@@ -15,6 +15,7 @@
 #include "grouped2.cuh"
 #include "pairs.cuh"
 #include "pair_matrix.cuh"
+#include "acc_pairs.cuh"
 #include "cross_geno.cuh"
 #include <unordered_map>
 
@@ -516,6 +517,141 @@ int snpm_pair_matrix(int device, int64_t S, const int64_t *offsets, const int32_
     if (ms) {
         ms[0] = t_expand;
         ms[1] = t_gemm;
+        ms[2] = 0.f;
+        SNPM_CUDA(cudaEventElapsedTime(&ms[2], r.ev[0], r.ev[1]));
+    }
+    return SNPM_OK;
+}
+
+// ---- accession against accession ----------------------------------------------------------------
+int snpm_db_acc_pairs(snpm_db *db, const int32_t *acc_idx, int32_t n_sel, int skip_db_hets, int64_t chunk_rows, int32_t block_acc,
+                      int32_t *common, int32_t *same, float *ms) {
+    // every check runs on the host, before anything is allocated
+    if (!db) return fail(SNPM_E_ARG, "snpm_db_acc_pairs: db is NULL");
+    if (n_sel < 1) return fail(SNPM_E_ARG, "snpm_db_acc_pairs: n_sel = %d; select at least one accession", n_sel);
+    if (!acc_idx || !common || !same) return fail(SNPM_E_ARG, "snpm_db_acc_pairs: bad arguments");
+    for (int32_t i = 0; i < n_sel; ++i)
+        if (acc_idx[i] < 0 || acc_idx[i] >= db->n_acc)
+            return fail(SNPM_E_ARG, "snpm_db_acc_pairs: accession index %d (entry %d) is outside 0..%d", acc_idx[i], i, db->n_acc - 1);
+    if (block_acc < 0 || block_acc % OG_BN)
+        return fail(SNPM_E_ARG, "snpm_db_acc_pairs: block_acc = %d is not a positive multiple of %d", block_acc, OG_BN);
+    if (chunk_rows < 0) return fail(SNPM_E_ARG, "snpm_db_acc_pairs: chunk_rows = %lld is negative", (long long)chunk_rows);
+    if (db->n_rows >= (int64_t(1) << 31))
+        return fail(SNPM_E_RANGE, "snpm_db_acc_pairs: the handle holds %lld rows; the counts are int32", (long long)db->n_rows);
+    const int64_t n = n_sel, rows = db->n_rows;
+    const int64_t nb_acc = block_acc > 0 ? block_acc : SNPM_ACC_BLOCK;
+    const int n_blk = int(ceil_div64(n, nb_acc));
+    const int m_blocks = int(ceil_div64(n, 64)), n_blocks = int(ceil_div64(n, OG_BN));
+    const int64_t widest = std::min(n, nb_acc), ld_part = ceil_div64(widest, OG_BN) * OG_BN;
+    const int64_t kb_bytes = int64_t(m_blocks) * OG_A_TILE + int64_t(n_blocks) * OG_B_TILE;
+    int64_t step = chunk_rows > 0 ? chunk_rows : std::max<int64_t>(1, SNPM_PAIR_CHUNK_BYTES / kb_bytes) * OG_ROWS;
+    step = std::max<int64_t>(1, std::min(step, rows));
+    const int64_t max_kb = ceil_div64(step, OG_ROWS);
+    const size_t cells = size_t(n) * size_t(n);
+
+    SNPM_CUDA(cudaSetDevice(db->device));
+    cudaStream_t st = db->stream;
+    struct Res {
+        DevBuf sel, at, bt, ps, pc, same, common;
+        std::vector<cudaEvent_t> ev;
+        ~Res() {
+            for (cudaEvent_t e : ev) cudaEventDestroy(e);
+        }
+    } r;
+    // events: call start / end, then a ring of RING timed spans (start, end), each an operand expansion or one GEMM
+    constexpr int RING = 128;
+    r.ev.assign(2 + 2 * RING, nullptr);
+    for (cudaEvent_t &e : r.ev) SNPM_CUDA(cudaEventCreate(&e));
+    SNPM_TRY(r.sel.ensure(size_t(n) * 4));
+    SNPM_TRY(r.same.ensure(cells * 4));
+    SNPM_TRY(r.common.ensure(cells * 4));
+    if (rows > 0) {
+        SNPM_TRY(r.at.ensure(size_t(m_blocks) * max_kb * OG_A_TILE));
+        SNPM_TRY(r.bt.ensure(size_t(n_blocks) * max_kb * OG_B_TILE));
+        SNPM_TRY(r.ps.ensure(size_t(widest) * ld_part * 4));
+        SNPM_TRY(r.pc.ensure(size_t(widest) * ld_part * 4));
+    }
+    const size_t smem = size_t(OG_STAGES) * (OG_A_TILE + OG_B_TILE) + 1024;
+    SNPM_CUDA(smem_attr<k_onehot_gemm>(int(smem)));
+
+    SNPM_CUDA(cudaEventRecord(r.ev[0], st));
+    SNPM_CUDA(cudaMemcpyAsync(r.sel.p, acc_idx, size_t(n) * 4, cudaMemcpyHostToDevice, st));
+    SNPM_CUDA(cudaMemsetAsync(r.same.p, 0, cells * 4, st));
+    SNPM_CUDA(cudaMemsetAsync(r.common.p, 0, cells * 4, st));
+    float t_span[2] = {0.f, 0.f};                               // expansion, GEMMs
+    int kind[RING] = {};
+    int64_t spans = 0;
+    auto collect = [&](int q) -> int {                          // the time of the span in ring slot q
+        float t = 0.f;
+        SNPM_CUDA(cudaEventSynchronize(r.ev[2 + 2 * q + 1]));
+        SNPM_CUDA(cudaEventElapsedTime(&t, r.ev[2 + 2 * q], r.ev[2 + 2 * q + 1]));
+        t_span[kind[q]] += t;
+        return SNPM_OK;
+    };
+    auto open_span = [&](int k) -> int {
+        const int q = int(spans % RING);
+        if (spans >= RING) SNPM_TRY(collect(q));
+        kind[q] = k;
+        SNPM_CUDA(cudaEventRecord(r.ev[2 + 2 * q], st));
+        return SNPM_OK;
+    };
+    auto close_span = [&]() -> int {
+        SNPM_CUDA(cudaEventRecord(r.ev[2 + 2 * int(spans % RING) + 1], st));
+        ++spans;
+        return SNPM_OK;
+    };
+    for (int64_t r0 = 0; r0 < rows; r0 += step) {
+        const int64_t r1 = std::min(r0 + step, rows);
+        const int32_t n_kb = int32_t(ceil_div64(r1 - r0, OG_ROWS));
+        SNPM_TRY(open_span(0));
+        k_acc_expand<<<dim3(unsigned(n_kb), unsigned(n_blocks)), 256, 0, st>>>(db->d_packed, db->stride, r.sel.as<int32_t>(), n_sel, r0, r1, n_kb,
+                                                                             m_blocks, skip_db_hets ? 1 : 0, r.at.as<unsigned char>(),
+                                                                             r.bt.as<unsigned char>());
+        SNPM_KERNEL_CHECK();
+        SNPM_TRY(close_span());
+        for (int bi = 0; bi < n_blk; ++bi) {
+            for (int bj = bi; bj < n_blk; ++bj) {
+                const int64_t i0 = bi * nb_acc, j0 = bj * nb_acc;
+                const int32_t ni = int32_t(std::min(nb_acc, n - i0)), nj = int32_t(std::min(nb_acc, n - j0));
+                OneHotGemmArgs g = {};
+                g.a_tiled = r.at.as<unsigned char>() + size_t(i0 / 64) * n_kb * OG_A_TILE;
+                g.b_tiled = r.bt.as<unsigned char>() + size_t(j0 / OG_BN) * n_kb * OG_B_TILE;
+                g.n_kb = n_kb;
+                g.m_blocks = int32_t(ceil_div64(ni, 64));
+                g.n_blocks = int32_t(ceil_div64(nj, OG_BN));
+                g.S = ni;
+                g.out_score = r.ps.as<int32_t>();
+                g.out_ninfo = r.pc.as<int32_t>();
+                g.ld_out = g.n_blocks * OG_BN;
+                SNPM_TRY(open_span(1));
+                k_onehot_gemm<<<unsigned(std::min(g.m_blocks * g.n_blocks, db->n_sm)), OG_THREADS, smem, st>>>(g);
+                SNPM_KERNEL_CHECK();
+                SNPM_TRY(close_span());
+                const size_t at = size_t(i0) * size_t(n) + size_t(j0);
+                const dim3 acc_grid(unsigned(ceil_div64(nj, 256)), unsigned(std::min<int32_t>(ni, 65535)));
+                k_acc_accumulate<<<acc_grid, 256, 0, st>>>(g.out_score, g.out_ninfo, g.ld_out, ni, nj, n, r.same.as<int32_t>() + at,
+                                                           r.common.as<int32_t>() + at);
+                SNPM_KERNEL_CHECK();
+            }
+        }
+    }
+    for (int64_t k = std::max<int64_t>(0, spans - RING); k < spans; ++k) SNPM_TRY(collect(int(k % RING)));
+    for (int bi = 0; bi < n_blk; ++bi) {
+        for (int bj = bi + 1; bj < n_blk; ++bj) {
+            const int64_t i0 = bi * nb_acc, j0 = bj * nb_acc;
+            const int32_t ni = int32_t(std::min(nb_acc, n - i0)), nj = int32_t(std::min(nb_acc, n - j0));
+            k_acc_mirror<<<dim3(unsigned(ceil_div64(nj, 32)), unsigned(ceil_div64(ni, 32))), dim3(32, 8), 0, st>>>(
+                r.same.as<int32_t>(), r.common.as<int32_t>(), n, i0, j0, ni, nj);
+            SNPM_KERNEL_CHECK();
+        }
+    }
+    SNPM_CUDA(cudaMemcpyAsync(same, r.same.p, cells * 4, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaMemcpyAsync(common, r.common.p, cells * 4, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaEventRecord(r.ev[1], st));
+    SNPM_CUDA(cudaStreamSynchronize(st));
+    if (ms) {
+        ms[0] = t_span[0];
+        ms[1] = t_span[1];
         ms[2] = 0.f;
         SNPM_CUDA(cudaEventElapsedTime(&ms[2], r.ev[0], r.ev[1]));
     }

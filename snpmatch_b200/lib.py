@@ -214,6 +214,7 @@ SIGNATURES = {
     "snpm_db_read_columns": (C.c_int, [_p, _p, _i32, _p]),
     "snpm_pair_match_counts": (C.c_int, [C.c_int, _p, _p, _i64, _p, _p, _i64, _p, _i64, _i32, _p, _p]),
     "snpm_pair_matrix": (C.c_int, [C.c_int, _i64, _p, _p, _p, _i32, _i64, _p, _i32, _i64, _p, _p, _p]),
+    "snpm_db_acc_pairs": (C.c_int, [_p, _p, _i32, C.c_int, _i64, _i32, _p, _p, _p]),
     "snpm_cross_window_genotypes": (C.c_int, [C.c_int, _p, _p, _i64, _p, _i32, _p, _p, _i64, _p, _i64, _i32, _f64, _i32, _p, _p, _p]),
     "snpm_db_n_rows": (_i64, [_p]),
     "snpm_db_n_acc": (_i32, [_p]),
@@ -396,6 +397,19 @@ class Database(object):
         flags = np.empty(max(self.n_rows, 1), dtype=np.uint8)
         check(load().snpm_db_segregating_rows(self._h, ptr(acc_idx), len(acc_idx), ptr(flags)))
         return np.flatnonzero(flags[:self.n_rows])
+
+    def acc_pairs(self, acc_idx=None, skip_db_hets=False, chunk_rows=0, block_acc=0):
+        """Every pair of the accessions acc_idx (default: all, in panel order) over the rows this handle holds
+        (snpm_db_acc_pairs): returns (common int32 [n,n], same int32 [n,n], (expand_ms, gemm_ms, device_ms)).  common[i, j] =
+        rows both accessions have called, same[i, j] = those with equal calls; skip_db_hets counts hets as missing.
+        chunk_rows / block_acc: rows per operand chunk and accessions per output block (0 = the library's defaults)."""
+        acc_idx = np.arange(self.n_acc, dtype=np.int32) if acc_idx is None else as_c(np.atleast_1d(acc_idx), np.int32)
+        n = len(acc_idx)
+        common, same = np.empty((n, n), np.int32), np.empty((n, n), np.int32)
+        ms = (C.c_float * 3)()
+        check(load().snpm_db_acc_pairs(self._h, ptr(acc_idx), n, int(bool(skip_db_hets)), int(chunk_rows), int(block_acc),
+                                       ptr(common), ptr(same), ms))
+        return common, same, (ms[0], ms[1], ms[2])
 
     def score_shared_panel(self, panel_rows, codes, skip_db_hets=False, likelihoods=True):
         """Batched tensor-core scoring (A9): codes uint8 [S,K] (0 ref, 1 alt, 2 het, 3 absent) of S called-genotype samples on
