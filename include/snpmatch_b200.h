@@ -340,7 +340,9 @@ int snpm_batch_fetch_window_rows(snpm_batch *b, int32_t *win_row_off, int32_t *w
  * Replaces the loop body of CrossIdentifier.match_insilico_f1s (csmatch.py:115-126) for every sample
  * of the batch over its whole-genome join: all P = n_top*(n_top-1)/2 pairs (i<j in list order) of the
  * sample's accession columns.  acc_idx int32[S, n_top] row-major, pair_score f64[S, P], pair_ninfo int64[S, P];
- * a sample's sums are the ones a single-sample batch of it gives, bit for bit. */
+ * a sample's sums are the ones a single-sample batch of it gives, bit for bit.  Limits (SNPM_E_ARG, the value named):
+ * 2 <= n_top <= 4096, every index in 0..n_acc-1 (a list may repeat one), 1 <= S <= 65535, S * P <= INT32_MAX, and at
+ * most 65535 row blocks of 4096 markers (268 M markers) in the largest sample. */
 int snpm_batch_f1_pairs(snpm_batch *b, const int32_t *acc_idx, int32_t n_top,
                         double *pair_score, int64_t *pair_ninfo);
 

@@ -2533,7 +2533,8 @@ int snpm_batch_fetch_window_rows(snpm_batch *b, int32_t *win_row_off, int32_t *w
 
 // ---- A7 ---------------------------------------------------------------------------------------------
 int snpm_batch_f1_pairs(snpm_batch *b, const int32_t *acc_idx, int32_t n_top, double *pair_score, int64_t *pair_ninfo) {
-    if (!b || !acc_idx || n_top < 2 || n_top > 4096 || !pair_score || !pair_ninfo) return fail(SNPM_E_ARG, "snpm_batch_f1_pairs: bad arguments");
+    if (!b || !acc_idx || !pair_score || !pair_ninfo) return fail(SNPM_E_ARG, "snpm_batch_f1_pairs: bad arguments");
+    if (n_top < 2 || n_top > 4096) return fail(SNPM_E_ARG, "snpm_batch_f1_pairs: n_top %d (2 to 4096)", n_top);
     if (!b->ran) return fail(SNPM_E_STATE, "snpm_batch_f1_pairs: run the batch first");
     if (b->S < 1 || b->S > 65535) return fail(SNPM_E_ARG, "snpm_batch_f1_pairs: %lld samples (1 to 65535 per call)", (long long)b->S);
     if (b->grouped) return fail(SNPM_E_STATE, "snpm_batch_f1_pairs: needs the batch in position order (snpm_batch_upload)");
@@ -2546,15 +2547,22 @@ int snpm_batch_f1_pairs(snpm_batch *b, const int32_t *acc_idx, int32_t n_top, do
     cudaStream_t st = db->stream;
     const int n_pairs = n_top * (n_top - 1) / 2;
     const size_t SP = size_t(S) * size_t(n_pairs);
+    // k_f1_final numbers the (sample, pair) slots with an int
+    if (SP > size_t(INT32_MAX))
+        return fail(SNPM_E_ARG, "snpm_batch_f1_pairs: %lld samples x %d pairs = %zu pair slots (at most %d per call)", (long long)S, n_pairs, SP, INT32_MAX);
     // row blocks of the largest sample (a sample's matched pairs never outnumber its markers); the other samples' surplus blocks add zeros
     int64_t n_max = 0;
     for (int64_t s = 0; s < S; ++s) n_max = std::max(n_max, b->h_off[size_t(s) + 1] - b->h_off[size_t(s)]);
-    const int n_blocks = int(std::max<int64_t>(1, ceil_div64(n_max, F1_ROWS_PER_BLOCK)));
+    const int64_t n_blocks64 = std::max<int64_t>(1, ceil_div64(n_max, F1_ROWS_PER_BLOCK));
+    if (n_blocks64 > 65535)
+        return fail(SNPM_E_ARG, "snpm_batch_f1_pairs: a sample of %lld markers needs %lld row blocks of %d (at most 65535)", (long long)n_max,
+                    (long long)n_blocks64, F1_ROWS_PER_BLOCK);
+    const int n_blocks = int(n_blocks64);
     SNPM_TRY(b->d_f1_acc.ensure(size_t(SK) * 4));
     SNPM_TRY(b->d_f1_part.ensure(SP * n_blocks * 32));
     SNPM_TRY(b->d_f1_out.ensure(SP * 16));
     SNPM_CUDA(cudaMemcpyAsync(b->d_f1_acc.p, acc_idx, size_t(SK) * 4, cudaMemcpyHostToDevice, st));
-    dim3 grid(n_blocks, n_pairs, unsigned(S));
+    const dim3 grid(static_cast<unsigned>(n_pairs), static_cast<unsigned>(n_blocks), static_cast<unsigned>(S));
     k_f1_partial<<<grid, F1_THREADS, 0, st>>>(db->d_packed, db->stride, b->d_pair_db.as<int32_t>(), b->d_pair_w.as<double>(),
                                               b->d_mstart.as<int32_t>(), b->d_f1_acc.as<int32_t>(), n_top, b->d_f1_part.as<double>());
     SNPM_KERNEL_CHECK();

@@ -17,10 +17,11 @@ __device__ __forceinline__ uint32_t code_at(const uint64_t *__restrict__ rowp, i
     return lo | (hi << 1);
 }
 
-// grid (row blocks, pairs, samples); partial[sample][pair][block] = (sum_alt, sum_ref, sum_het, count).  Sample s owns the
+// grid (pairs, row blocks, samples); partial[sample][pair][block] = (sum_alt, sum_ref, sum_het, count).  Sample s owns the
 // matched pairs [mstart[s], mstart[s+1]) and the accession list acc_idx[s * n_top ...]; its row blocks start at its first pair,
 // so a sample's sums do not depend on the other samples of the batch.  Blocks past a sample's pairs write zeros (the grid is
-// sized for the largest sample).
+// sized for the largest sample).  The pairs sit on grid x (up to 2^31 - 1) because n_top = 4096 gives 8 386 560 of them; the
+// row blocks sit on grid y, so a sample may have at most 65 535 * F1_ROWS_PER_BLOCK matched pairs.
 __global__ void __launch_bounds__(F1_THREADS) k_f1_partial(const uint64_t *__restrict__ packed, int32_t stride,
                                                            const int32_t *__restrict__ pair_db, const double *__restrict__ pair_w,
                                                            const int32_t *__restrict__ mstart, const int32_t *__restrict__ acc_idx,
@@ -28,13 +29,13 @@ __global__ void __launch_bounds__(F1_THREADS) k_f1_partial(const uint64_t *__res
     __shared__ double s_sum[3][F1_THREADS / 32];
     __shared__ long long s_cnt[F1_THREADS / 32];
     // pair index -> (i, j), i < j, itertools.combinations order
-    int pi = blockIdx.y, i = 0;
+    int pi = blockIdx.x, i = 0;
     while (pi >= n_top - 1 - i) { pi -= n_top - 1 - i; ++i; }
     const int j = i + 1 + pi;
     const int s = blockIdx.z;
     const int32_t a1 = acc_idx[int64_t(s) * n_top + i], a2 = acc_idx[int64_t(s) * n_top + j];
     const int64_t m = mstart[s + 1];
-    const int64_t r0 = mstart[s] + int64_t(blockIdx.x) * F1_ROWS_PER_BLOCK;
+    const int64_t r0 = mstart[s] + int64_t(blockIdx.y) * F1_ROWS_PER_BLOCK;
     const int64_t r1 = min(m, r0 + F1_ROWS_PER_BLOCK);
     double alt = 0.0, ref = 0.0, het = 0.0;
     long long cnt = 0;
@@ -61,7 +62,7 @@ __global__ void __launch_bounds__(F1_THREADS) k_f1_partial(const uint64_t *__res
         double A = 0.0, R = 0.0, H = 0.0;
         long long C = 0;
         for (int k = 0; k < F1_THREADS / 32; ++k) { A += s_sum[0][k]; R += s_sum[1][k]; H += s_sum[2][k]; C += s_cnt[k]; }
-        double *o = partial + ((int64_t(s) * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * 4;
+        double *o = partial + ((int64_t(s) * gridDim.x + blockIdx.x) * gridDim.y + blockIdx.y) * 4;
         o[0] = A; o[1] = R; o[2] = H; o[3] = double(C);
     }
 }
