@@ -431,6 +431,28 @@ int snpm_panel_score(snpm_panel *p, const uint8_t *codes, int packed, int64_t S,
                      double *LR, float *ms);
 void snpm_panel_destroy(snpm_panel *p);
 
+/* ---- multi-sample VCF text on the device (`inbred --samples_vcf`, `cross --samples_vcf`) ----------------------------------
+ * No reference symbol: the reference reads one sample column per scikit-allel call (parsers.py:184-213).  A handle parses the
+ * genotype columns of the records of one VCF, chunk by chunk, for n_samples sample columns (the #CHROM line's).  The caller
+ * passes whole lines: text [n_bytes] with 1 <= n_bytes <= chunk_bytes <= SNPM_VCF_MAX_CHUNK, ending in a line end; '\n',
+ * "\r\n" and a lone '\r' each end a line (Python's universal newlines).  Lines starting with '#' and lines of fewer than 10
+ * tab-separated fields are not records.
+ * snpm_vcf_parse: info int64[5] = lines, cells of samples 0..n_samples-1 in records, called cells kept, 1 if the chunk holds a
+ * byte >= 0x80, lines starting with "##INFO=<ID=DP,"; ms (optional) float[2] = device time of the copy up and of the kernels.
+ * snpm_vcf_fetch, per line (n = info[0]): line_start int32[n+1] (byte offsets; line k is [line_start[k], line_start[k+1])
+ * with its line end), flags int32[n] (1 record, 2 the device cannot reproduce the Python parser on this record: re-parse it,
+ * 4 FORMAT has a PL key, 8 CHROM may differ from the previous record's), nsf int32[n] sample fields, pos int32[n], dp int32[n]
+ * (INFO DP, -1 none), chrom_len int32[n] bytes of CHROM.  Per sample s, entries sample_off[s] .. sample_off[s+1]-1 (int32
+ * [n_samples+1]) are its called cells in line order, records flagged 2 left out: line int32, cls uint16 = a1 * 111 + a2 of the
+ * rendered GT's two alleles (0 '.', 1 + d for the digit d, 11 + 10x + y for the digits xy), pl int32 [3] (-1 missing). */
+#define SNPM_VCF_MAX_CHUNK (int64_t(1) << 30)
+typedef struct snpm_vcf snpm_vcf;
+int snpm_vcf_create(int device, int32_t n_samples, int64_t chunk_bytes, snpm_vcf **out);
+int snpm_vcf_parse(snpm_vcf *h, const char *text, int64_t n_bytes, int64_t *info, float *ms);
+int snpm_vcf_fetch(snpm_vcf *h, int32_t *line_start, int32_t *flags, int32_t *nsf, int32_t *pos, int32_t *dp, int32_t *chrom_len,
+                   int32_t *sample_off, int32_t *line, uint16_t *cls, int32_t *pl);
+void snpm_vcf_destroy(snpm_vcf *h);
+
 #ifdef __cplusplus
 }
 #endif

@@ -40,6 +40,11 @@ def check_file(inFile):
 
 
 def snpmatch_inbred(args):
+    if args.get('samples_vcf'):
+        prefixes = vcf_sample_prefixes(args['samples_vcf'], args['outFile'])
+        from .core import snpmatch
+        snpmatch.potatoGenotyperVcf(args, prefixes)
+        return
     if args.get('samples'):
         samples = read_sample_list(args['samples'], args['outFile'])
         from .core import snpmatch
@@ -51,6 +56,11 @@ def snpmatch_inbred(args):
 
 
 def snpmatch_cross(args):
+    if args.get('samples_vcf'):
+        prefixes = vcf_sample_prefixes(args['samples_vcf'], args['outFile'])
+        from .core import csmatch
+        csmatch.potatoCrossIdentifierVcf(args, prefixes)
+        return
     if args.get('samples'):
         samples = read_sample_list(args['samples'], args['outFile'])
         from .core import csmatch
@@ -90,6 +100,27 @@ def read_sample_list(list_file, out_prefix, default_name=None):
             die("samples %s and %s have the same %s %s" % (seen[prefix], path, "label" if default_name else "output prefix", prefix))
         seen[prefix] = path
     return samples
+
+
+def vcf_sample_prefixes(vcf, out_prefix):
+    """`inbred --samples_vcf` / `cross --samples_vcf`: the output prefix <out_prefix>.<sample name> of every sample column of
+    the VCF.  Dies on a missing file, a VCF without sample columns and a sample name that is empty, repeated or holds a '/'."""
+    check_file(vcf)
+    from .core import parsers
+    try:
+        names = parsers.vcf_sample_names(vcf)
+    except ValueError as e:
+        die("%s: %s" % (vcf, e))
+    if not names:
+        die("VCF without sample columns: " + vcf)
+    seen = set()
+    for i, name in enumerate(names):
+        if not name or "/" in name:
+            die("sample column %d of %s has the name %r, which cannot be part of an output file name" % (i + 1, vcf, name))
+        if name in seen:
+            die("sample name %s appears twice in %s" % (name, vcf))
+        seen.add(name)
+    return [out_prefix + "." + name for name in names]
 
 
 def snpmatch_parser(args):
@@ -175,6 +206,10 @@ def get_options(description, version_message):
                            help="text file listing many samples, one path per line (VCF/BED/npz), optionally a tab and that sample's output "
                                 "prefix (default <-o>.<file name up to its first '.'>); all samples are scored together on the GPU; exit "
                                 "status 1 when --refine finds a sample without top hits")
+    inbred_in.add_argument("--samples_vcf", dest="samples_vcf", default=None,
+                           help="one VCF (plain or .vcf.gz) with many sample columns: every column is a sample, written under "
+                                "<-o>.<sample name>; its genotype columns are parsed on the GPU and all samples are scored together; "
+                                "exit status as with --samples")
     inbred.add_argument("-d", "--hdf5_file", default=None, dest="hdf5File", help=db_help)
     inbred.add_argument("-e", "--hdf5_acc_file", default=None, dest="hdf5accFile", help="Column-chunked hdf5 file of the reference (accepted for compatibility; one resident copy serves both)")
     inbred.add_argument("--refine", action="store_true", dest="refine", default=False, help="re-score the accessions that cannot be told apart on the SNPs that segregate among them")
@@ -189,6 +224,10 @@ def get_options(description, version_message):
     cross_in.add_argument("--samples", dest="samples", default=None,
                           help="text file listing many samples, one path per line (VCF/BED/npz), optionally a tab and that sample's output "
                                "prefix (default <-o>.<file name up to its first '.'>); all samples are scored together on the GPU")
+    cross_in.add_argument("--samples_vcf", dest="samples_vcf", default=None,
+                          help="one VCF (plain or .vcf.gz) with many sample columns: every column is a sample, written under "
+                               "<-o>.<sample name>; its genotype columns are parsed on the GPU and all samples are scored together; "
+                               "exit status 1, after the other samples are written, when a column's chromosomes do not name the genome's")
     cross.add_argument("-d", "--hdf5_file", default=None, dest="hdf5File", help=db_help)
     cross.add_argument("-e", "--hdf5_acc_file", default=None, dest="hdf5accFile", help="Column-chunked hdf5 file of the reference (accepted for compatibility)")
     cross.add_argument("-b", "--binLength", dest="binLen", help="window length in bp", default=300000, type=int)

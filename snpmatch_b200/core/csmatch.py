@@ -425,3 +425,35 @@ def potatoCrossIdentifierMany(args, samples):
     finally:
         g.close()
     log.info("finished!")
+
+
+def potatoCrossIdentifierVcf(args, prefixes):
+    """`cross --samples_vcf`: every sample column of one VCF, parsed on the device (parsers.read_vcf_many), sample i written
+    under prefixes[i].  Exits with status 1 on a sharded panel or a VCF the parser refuses.  A column whose chromosomes do not
+    name the genome's (no called genotype at all, say; the single path stops there with an assertion) gets no files: every
+    other sample is run and written, then the run exits with status 1 naming those columns."""
+    log.info("loading genotype files!")
+    g = snp_genotype.Genotype(args['hdf5File'], args['hdf5accFile'])
+    try:
+        if not snpmatch.holds_whole_panel(g):
+            parsers.die("--samples_vcf needs the whole panel on one device; this one holds a shard of its rows")
+        try:
+            parsed = parsers.read_vcf_many(args['samples_vcf'], device=g.db.device)
+        except ValueError as e:
+            parsers.die(str(e))
+        keep, refused = [], []
+        for i, (name, inp) in enumerate(parsed):
+            try:
+                CrossIdentifier(inp, g, args['genome'], args['binLen'], prefixes[i], run_identifier=False)._check_genome()
+                keep.append(i)
+            except AssertionError as e:
+                refused.append("%s (%s)" % (name, e))
+        log.info("running cross identifier on %d samples!" % len(keep))
+        cross_identify_many([parsed[i][1] for i in keep], g, args['genome'], args['binLen'], [prefixes[i] for i in keep],
+                            skip_db_hets=args['skip_db_hets'])
+    finally:
+        g.close()
+    if refused:
+        parsers.die("no cross run for %d sample column(s) of %s whose chromosomes do not name the genome's: %s"
+                    % (len(refused), args['samples_vcf'], ", ".join(refused)))
+    log.info("finished!")

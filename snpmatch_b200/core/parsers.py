@@ -16,6 +16,7 @@ in np.nanmean on the first parse (parsers.py:113) — here the depth statistic i
 """
 import gzip
 import json
+import locale
 import logging
 import os
 import re
@@ -77,6 +78,36 @@ def mean_depth(dp):
     return float(np.nanmean(arr))
 
 
+_DP_RE = re.compile(r"(?:^|;)DP=([^;]+)")
+
+
+def vcf_record(f, sample_index=0):
+    """What read_vcf_minimal takes from one record, f = the line's tab-separated fields: (chrom, pos, dp, gt, pl, has_pl) with
+    dp = INFO/DP (-1 when absent or not an integer), gt rendered 'a/b', pl the first three PLs (-1 where missing) and has_pl
+    whether FORMAT has a PL key; None when the line has fewer than 10 + sample_index fields."""
+    if len(f) < 10 + sample_index:
+        return None
+    pos = int(f[1])
+    m = _DP_RE.search(f[7])
+    try:
+        dp = int(m.group(1)) if m else -1
+    except ValueError:
+        dp = -1
+    keys = f[8].split(":")
+    vals = f[9 + sample_index].split(":")
+    rec = dict(zip(keys, vals))
+    alleles = re.split(r"[/|]", rec.get("GT", "."))
+    if len(alleles) == 1:
+        alleles = [alleles[0], "."] if alleles[0] != "." else [".", "."]
+    gt = "/".join(a if a != "" else "." for a in alleles[:2])
+    pl = [-1.0, -1.0, -1.0]
+    if "PL" in rec:
+        for i, v in enumerate(rec["PL"].split(",")[:3]):
+            if v not in (".", ""):
+                pl[i] = float(v)
+    return f[0], pos, dp, gt, pl, "PL" in keys
+
+
 def read_vcf_minimal(inFile, sample_index=0):
     """Minimal VCF reader: CHROM, POS, INFO/DP, and GT + PL of one sample.
 
@@ -89,7 +120,6 @@ def read_vcf_minimal(inFile, sample_index=0):
     chrom, pos, gts, pls, dps = [], [], [], [], []
     has_info_dp = False
     has_pl = False
-    dp_re = re.compile(r"(?:^|;)DP=([^;]+)")
     with opener(inFile, "rt") as fh:
         for line in fh:
             if line.startswith("##"):
@@ -98,32 +128,15 @@ def read_vcf_minimal(inFile, sample_index=0):
                 continue
             if line.startswith("#"):
                 continue
-            f = line.rstrip("\n").split("\t")
-            if len(f) < 10 + sample_index:
+            r = vcf_record(line.rstrip("\n").split("\t"), sample_index)
+            if r is None:
                 continue
-            chrom.append(f[0])
-            pos.append(int(f[1]))
-            m = dp_re.search(f[7])
-            try:
-                dps.append(int(m.group(1)) if m else -1)
-            except ValueError:
-                dps.append(-1)
-            keys = f[8].split(":")
-            vals = f[9 + sample_index].split(":")
-            rec = dict(zip(keys, vals))
-            alleles = re.split(r"[/|]", rec.get("GT", "."))
-            if len(alleles) == 1:
-                alleles = [alleles[0], "."] if alleles[0] != "." else [".", "."]
-            gts.append("/".join(a if a != "" else "." for a in alleles[:2]))
-            pl = [-1.0, -1.0, -1.0]
-            if "PL" in rec:
-                has_pl = True
-                for i, v in enumerate(rec["PL"].split(",")[:3]):
-                    if v not in (".", ""):
-                        pl[i] = float(v)
-            elif "PL" in keys:
-                has_pl = True
-            pls.append(pl)
+            chrom.append(r[0])
+            pos.append(r[1])
+            dps.append(r[2])
+            gts.append(r[3])
+            pls.append(r[4])
+            has_pl |= r[5]
     out = {
         "chr": np.array(chrom, dtype="str"),
         "pos": np.array(pos, dtype=np.int64),
@@ -278,28 +291,8 @@ class ParseInputs(object):
         """First sample; drop no-calls; wei = exp(-PL/10), GT one-hot where PL is absent
         (parsers.py:141-157)."""
         v = import_vcf_file(inFile, logDebug, samples_to_load=[0])
-        gt_all = v['gt'][:, 0]
-        req = np.flatnonzero((gt_all != './.') & (gt_all != '.|.'))
-        gt = gt_all[req]
-        self._pl_codes = None
-        if 'wei' in v:
-            pl = v['wei'][req, 0]
-            no_pl = np.all(pl == -1, axis=1)
-            wei = np.exp(pl / (-10))
-            wei[no_pl, ] = self.get_wei_from_GT(gt[no_pl])
-            # integer PLs are ready-made dictionary codes of the weights: table[k] = exp(k / -10), one extra entry for 0.0
-            if len(pl) and np.all(pl == np.floor(pl)) and pl.min() >= -1 and pl.max() < 65000:
-                top = int(pl.max()) + 1
-                table = np.append(np.exp(np.arange(top) / (-10)), 0.0)
-                codes = np.where(pl < 0, 0, pl).astype(np.uint16)
-                if no_pl.any():
-                    hard = wei[no_pl]
-                    codes[no_pl] = np.where(hard == 1.0, 0, top).astype(np.uint16)
-                if np.array_equal(table[codes.astype(np.int64)], wei):
-                    self._pl_codes = (codes, table)
-        else:
-            wei = self.get_wei_from_GT(gt)
-        return (v['chr'][req], v['pos'][req], gt, wei, v['dp'][req])
+        parsed, self._pl_codes = vcf_called_inputs(v['chr'], v['pos'], v['gt'][:, 0], v['wei'][:, 0] if 'wei' in v else None, v['dp'])
+        return parsed
 
     def filter_chr_names(self):
         """parsers.py:159-163: strip every 'chr' (any case); ids in first-appearance order."""
@@ -311,6 +304,232 @@ class ParseInputs(object):
         with open(outFile, "w") as fh:
             for c, p, g in zip(self.chrs, self.pos, self.gt):
                 fh.write("%s\t%s\t%s\n" % (c, p, g))
+
+
+def vcf_called_inputs(chrs, pos, gt_all, pl, dp):
+    """The step of ParseInputs.read_vcf from one sample's VCF fields to (chrs, pos, gt, wei, dp): drop the no-calls; wei =
+    exp(-PL/10), the called genotype's one-hot where a marker has no PL and everywhere when pl is None (no PL key in the file).
+    pl: float [n,3] with -1 for a missing value, or None.  Returns (those five, pl_codes): pl_codes = (codes uint16 [m,3],
+    table) when the PLs are integers, the dictionary codes of the weights that coded_weights() hands out, else None."""
+    req = np.flatnonzero((gt_all != './.') & (gt_all != '.|.'))
+    gt = gt_all[req]
+    pl_codes = None
+    if pl is not None:
+        pl = pl[req]
+        no_pl = np.all(pl == -1, axis=1)
+        wei = np.exp(pl / (-10))
+        wei[no_pl, ] = ParseInputs.get_wei_from_GT(gt[no_pl])
+        # integer PLs are ready-made dictionary codes of the weights: table[k] = exp(k / -10), one extra entry for 0.0
+        if len(pl) and np.all(pl == np.floor(pl)) and pl.min() >= -1 and pl.max() < 65000:
+            top = int(pl.max()) + 1
+            table = np.append(np.exp(np.arange(top) / (-10)), 0.0)
+            codes = np.where(pl < 0, 0, pl).astype(np.uint16)
+            if no_pl.any():
+                hard = wei[no_pl]
+                codes[no_pl] = np.where(hard == 1.0, 0, top).astype(np.uint16)
+            if np.array_equal(table[codes.astype(np.int64)], wei):
+                pl_codes = (codes, table)
+    else:
+        wei = ParseInputs.get_wei_from_GT(gt)
+    return (chrs[req], pos[req], gt, wei, dp[req]), pl_codes
+
+
+# ---- every sample column of one VCF, the genotype columns parsed on the device (`inbred/cross --samples_vcf`) ----------------
+VCF_CHUNK_BYTES = 64 << 20
+# allele codes of snpm_vcf_fetch: 0 '.', 1 + d for the digit d, 11 + 10x + y for the two digits xy; class = a1 * 111 + a2
+_ALLELES = ["."] + [str(d) for d in range(10)] + ["%d%d" % (x, y) for x in range(10) for y in range(10)]
+VCF_GT_TEXT = np.array([a + "/" + b for a in _ALLELES for b in _ALLELES])
+VCF_GT_LEN = np.array([len(t) for t in VCF_GT_TEXT.tolist()])
+_LINE_END = re.compile(rb"\r\n|\r|\n")
+
+
+def _open_binary(path):
+    return gzip.open(path, "rb") if str(path).endswith(".gz") else open(path, "rb")
+
+
+def read_vcf_header(fh, block=1 << 20):
+    """Header of a VCF opened in binary mode, read up to and including its #CHROM line with the universal-newline rule of the
+    text-mode readers: returns (sample names, has_info_dp, lines read, the bytes read past the #CHROM line).  Raises ValueError
+    when a record (10 fields or more) comes before the #CHROM line, or when there is no #CHROM line."""
+    enc = locale.getpreferredencoding(False)
+    buf, at, n, has_dp, eof = b"", 0, 0, False, False
+    while True:
+        m = _LINE_END.search(buf, at)
+        if m is None or (m.group() == b"\r" and m.end() == len(buf) and not eof):
+            if not eof:
+                piece = fh.read(block)
+                eof = not piece
+                buf, at = buf[at:] + piece, 0
+                continue
+            if at == len(buf):
+                raise ValueError("no #CHROM line")
+            line, at = buf[at:], len(buf)
+        else:
+            line, at = buf[at:m.start()], m.end()
+        n += 1
+        text = line.decode(enc)
+        if text.startswith("##"):
+            has_dp |= text.startswith("##INFO=<ID=DP,")
+        elif text.startswith("#"):
+            return text.split("\t")[9:], has_dp, n, buf[at:]
+        elif len(text.split("\t")) >= 10:
+            raise ValueError("line %d is a record before the #CHROM line" % n)
+
+
+def vcf_sample_names(path):
+    """The sample columns of a VCF's #CHROM line."""
+    with _open_binary(path) as fh:
+        return read_vcf_header(fh)[0]
+
+
+def _whole_lines(buf, limit, eof):
+    """Bytes of buf[:limit] up to its last line end; a trailing '\r' counts only when the byte after it is known."""
+    n = min(len(buf), limit)
+    cut = buf.rfind(b"\n", 0, n) + 1
+    r = buf.rfind(b"\r", cut, n)
+    while r >= 0:
+        if (r + 1 < len(buf) and buf[r + 1] != 10) or (r + 1 == len(buf) and eof):
+            return r + 1
+        r = buf.rfind(b"\r", cut, r)
+    return cut
+
+
+def read_vcf_many(path, device=0, chunk_bytes=VCF_CHUNK_BYTES, timings=None):
+    """Every sample column of a VCF (plain or .vcf.gz): [(sample name, ParseInputs)], where sample s's ParseInputs has the
+    chrs, pos, gt, wei, dp and coded_weights() of ParseInputs on a VCF of the same header, the 9 fixed columns and column s
+    alone (read_vcf_minimal(path, sample_index=s) + ParseInputs.read_vcf).  The host reads (and decompresses) the text after
+    the #CHROM line in chunks of whole lines of at most chunk_bytes; the genotype columns are parsed on CUDA device `device`
+    (lib.VcfParser); records the device flags are re-parsed with vcf_record.  Nothing is written next to the VCF and no parser
+    dump is loaded.  A line longer than chunk_bytes, a record before the #CHROM line and a VCF without sample columns raise
+    ValueError.  timings (optional dict) receives seconds and bytes of the stages and, under "fallback", the indices of the
+    records the Python code parsed."""
+    import time
+    from .. import lib
+    enc = locale.getpreferredencoding(False)
+    tm = timings if timings is not None else {}
+    for k in ("read_s", "device_s", "host_chunk_s", "assemble_s", "h2d_ms", "kernel_ms", "h2d_bytes"):
+        tm[k] = 0
+    tm["fallback"] = []
+    t0 = time.perf_counter()
+    fh = _open_binary(path)
+    try:
+        names, has_info_dp, line_no, head = read_vcf_header(fh)
+        if not names:
+            raise ValueError("%s has no sample columns" % path)
+        S = len(names)
+        name_id, name_list = {}, []
+
+        def chrom_id(text):
+            if text not in name_id:
+                name_id[text] = len(name_list)
+                name_list.append(text)
+            return name_id[text]
+        rec = {k: [] for k in ("cid", "pos", "dp", "nsf", "has_pl")}
+        chunks, fb = [], [[] for _ in range(S)]
+        n_rec = 0
+        buf, eof = bytearray(head), False
+        tm["read_s"] += time.perf_counter() - t0
+        parser = lib.VcfParser(device, S, chunk_bytes)
+        try:
+            while True:
+                t0 = time.perf_counter()
+                while len(buf) < chunk_bytes and not eof:
+                    piece = fh.read(chunk_bytes - len(buf))
+                    eof = not piece
+                    buf += piece
+                if eof and buf and buf[-1] not in (10, 13):
+                    buf += b"\n"
+                tm["read_s"] += time.perf_counter() - t0
+                if not buf:
+                    break
+                cut = _whole_lines(buf, chunk_bytes, eof)
+                if cut == 0:
+                    raise ValueError("%s: line %d is longer than the chunk of %d bytes" % (path, line_no + 1, chunk_bytes))
+                chunk = bytes(memoryview(buf)[:cut])
+                del buf[:cut]
+                t0 = time.perf_counter()
+                r = parser.parse(chunk)
+                tm["device_s"] += time.perf_counter() - t0
+                tm["h2d_ms"] += r["h2d_ms"]
+                tm["kernel_ms"] += r["kernel_ms"]
+                tm["h2d_bytes"] += len(chunk)
+                t0 = time.perf_counter()
+                line_no += r["n_lines"]
+                if r["non_ascii"]:
+                    chunk.decode(enc)                  # the text-mode readers fail on what does not decode
+                has_info_dp |= r["info_dp_lines"] > 0
+                flags, ls = r["flags"], r["line_start"]
+                lines = np.flatnonzero(flags & lib.VcfParser.FLAG_RECORD)
+                fl = flags[lines]
+                pos, dp, nsf = r["pos"][lines].astype(np.int64), r["dp"][lines].astype(np.int64), r["nsf"][lines]
+                has_pl = (fl & lib.VcfParser.FLAG_HAS_PL) != 0
+                # CHROM: decoded where it may differ from the previous record's, carried forward elsewhere
+                new = np.flatnonzero(fl & lib.VcfParser.FLAG_NEW_CHROM)
+                ids = np.zeros(len(lines), np.int32)
+                ids[new] = [chrom_id(chunk[ls[L]:ls[L] + r["chrom_len"][L]].decode(enc)) for L in lines[new].tolist()]
+                src = np.zeros(len(lines), np.int64)
+                src[new] = new
+                cid = ids[np.maximum.accumulate(src)] if len(lines) else ids
+                for k in np.flatnonzero(fl & lib.VcfParser.FLAG_FALLBACK).tolist():
+                    L = int(lines[k])
+                    f = chunk[ls[L]:ls[L + 1]].rstrip(b"\r\n").decode(enc).split("\t")
+                    first = vcf_record(f, 0)
+                    cid[k], pos[k], dp[k], has_pl[k] = chrom_id(first[0]), first[1], first[2], first[5]
+                    for smp in range(min(int(nsf[k]), S)):
+                        one = vcf_record(f, smp)
+                        if one[3] not in ('./.', '.|.'):
+                            fb[smp].append((n_rec + k, one[3], one[4]))
+                    tm["fallback"].append(n_rec + k)
+                for key, v in (("cid", cid), ("pos", pos), ("dp", dp), ("nsf", nsf), ("has_pl", has_pl)):
+                    rec[key].append(v)
+                rec_of_line = np.cumsum(flags & lib.VcfParser.FLAG_RECORD, dtype=np.int64) - 1 + n_rec
+                chunks.append((r["sample_off"], rec_of_line[r["line"]], r["cls"], r["pl"]))
+                n_rec += len(lines)
+                tm["host_chunk_s"] += time.perf_counter() - t0
+        finally:
+            parser.close()
+    finally:
+        fh.close()
+    t0 = time.perf_counter()
+    rec = {k: (np.concatenate(v) if v else np.zeros(0)) for k, v in rec.items()}
+    cid_all, pos_all, dp_all = rec["cid"].astype(np.int64), rec["pos"].astype(np.int64), rec["dp"].astype(np.int64)
+    nsf_all = np.minimum(rec["nsf"].astype(np.int64), S)
+    has_pl_all = rec["has_pl"].astype(bool)
+    names_arr = np.array(name_list, dtype="str")
+    # per sample, the records it has (nsf > s): whether any has a PL key, how many there are, the longest CHROM among them
+    # (read_vcf_minimal's arrays are as wide as their longest entry)
+    pl_upto = int(nsf_all[has_pl_all].max()) if has_pl_all.any() else 0
+    has_rec = np.cumsum(np.bincount(nsf_all, minlength=S + 1)[::-1])[::-1] if len(nsf_all) else np.zeros(S + 1, np.int64)
+    longest = np.zeros(S + 1, np.int64)
+    if len(nsf_all):
+        np.maximum.at(longest, nsf_all, np.array([len(c) for c in name_list], np.int64)[cid_all])
+    longest = np.maximum.accumulate(longest[::-1])[::-1]
+    out = []
+    for smp in range(S):
+        parts = [(c_rec[o[smp]:o[smp + 1]], c_cls[o[smp]:o[smp + 1]], c_pl[o[smp]:o[smp + 1]]) for o, c_rec, c_cls, c_pl in chunks]
+        idx = np.concatenate([p[0] for p in parts]) if parts else np.zeros(0, np.int64)
+        cls = np.concatenate([p[1] for p in parts]) if parts else np.zeros(0, np.uint16)
+        gt = VCF_GT_TEXT[cls]
+        pl = (np.concatenate([p[2] for p in parts]) if parts else np.zeros((0, 3), np.int32)).astype(np.float64)
+        width = int(VCF_GT_LEN[cls].max()) if len(cls) else 3
+        if fb[smp]:
+            idx = np.concatenate([idx, np.array([e[0] for e in fb[smp]], np.int64)])
+            gt = np.concatenate([gt, np.array([e[1] for e in fb[smp]], dtype="str")])
+            pl = np.concatenate([pl, np.array([e[2] for e in fb[smp]], dtype=np.float64).reshape(-1, 3)])
+            width = max(width, max(len(e[1]) for e in fb[smp]))
+            order = np.argsort(idx, kind="stable")
+            idx, gt, pl = idx[order], gt[order], pl[order]
+        n_have = int(has_rec[smp + 1])
+        gt = gt.astype("<U%d" % (max(width, 3) if n_have else 1))
+        chrs = names_arr[cid_all[idx]].astype("<U%d" % max(int(longest[smp + 1]), 1))
+        dp = dp_all[idx] if has_info_dp else np.repeat("NA", len(idx))
+        parsed, pl_codes = vcf_called_inputs(chrs, pos_all[idx], gt, pl if smp < pl_upto else None, dp)
+        inp = object.__new__(ParseInputs)
+        inp._pl_codes = pl_codes
+        inp.load_snp_info(*parsed)
+        out.append((names[smp], inp))
+    tm["assemble_s"] += time.perf_counter() - t0
+    return out
 
 
 def potatoParser(inFile, logDebug, outFile="parser"):

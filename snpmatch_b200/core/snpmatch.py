@@ -360,6 +360,11 @@ def _het_flags(gt):
     return parsers.parseGT(gt) == 2 if bool(np.all(same)) else None
 
 
+def holds_whole_panel(g):
+    """False when the Genotype holds a row shard of its panel (the many-sample paths need every row on one device)."""
+    return g.db.row0_global == 0 and g.db.n_rows == int(np.max(getattr(g, "global_chr_regions", [[0, g.db.n_rows]])))
+
+
 def inbred_identify_many(inputs_list, g, output_ids, refine=False, skip_db_hets=False, chunk_size=1000, samples_per_launch=None):
     """`inbred` (and `inbred --refine`) for many samples: every sample's files (<id>.scores.txt, <id>.matches.json and, when it
     refines, <id>.refined.scores.txt) are byte for byte the ones Genotyper (+ filter_tophits) writes for it alone.
@@ -377,7 +382,7 @@ def inbred_identify_many(inputs_list, g, output_ids, refine=False, skip_db_hets=
     assert len(inputs_list) == len(output_ids), "one output prefix per sample"
     assert len(set(output_ids)) == len(output_ids), "output prefixes must differ"
     assert int(chunk_size) >= 1, "chunk_size must be a positive number of SNPs"
-    if g.db.row0_global != 0 or g.db.n_rows != int(np.max(getattr(g, "global_chr_regions", [[0, g.db.n_rows]]))):
+    if not holds_whole_panel(g):
         raise ValueError("inbred_identify_many needs the whole panel on one device; this one holds a shard of its rows")
     # every sample's chromosome names are mapped to the panel's before any device work; a bad sample is named
     gts, prepared = [], []
@@ -504,6 +509,29 @@ def potatoGenotyperMany(args, samples):
     finally:
         g.close()
     skipped = [path for (path, _), gt in zip(samples, gts) if gt.no_top_hits]
+    if skipped:
+        die("no top hits to refine (no marker shared with the panel?): " + ", ".join(skipped))
+    log.info("finished!")
+
+
+def potatoGenotyperVcf(args, prefixes):
+    """`inbred --samples_vcf`: every sample column of one VCF, parsed on the device (parsers.read_vcf_many), sample i written
+    under prefixes[i].  Exits with status 1 on a sharded panel or a VCF the parser refuses, and, after every other sample is
+    written, when a sample had no top hit to refine."""
+    log.info("packing the database into HBM")
+    g = snp_genotype.Genotype(args['hdf5File'], args['hdf5accFile'])
+    try:
+        if not holds_whole_panel(g):
+            die("--samples_vcf needs the whole panel on one device; this one holds a shard of its rows")
+        try:
+            parsed = parsers.read_vcf_many(args['samples_vcf'], device=g.db.device)
+        except ValueError as e:
+            die(str(e))
+        log.info("matching %d samples against %s accessions", len(parsed), len(g.accessions))
+        gts = inbred_identify_many([inp for _, inp in parsed], g, prefixes, refine=args['refine'], skip_db_hets=args['skip_db_hets'])
+    finally:
+        g.close()
+    skipped = [name for (name, _), gt in zip(parsed, gts) if gt.no_top_hits]
     if skipped:
         die("no top hits to refine (no marker shared with the panel?): " + ", ".join(skipped))
     log.info("finished!")

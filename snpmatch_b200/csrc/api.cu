@@ -17,6 +17,7 @@
 #include "pair_matrix.cuh"
 #include "acc_pairs.cuh"
 #include "cross_geno.cuh"
+#include "vcf.cuh"
 #include <unordered_map>
 
 namespace snpm {
@@ -2576,6 +2577,200 @@ int snpm_batch_f1_pairs(snpm_batch *b, const int32_t *acc_idx, int32_t n_top, do
         pair_score[p] = out[2 * p];
         pair_ninfo[p] = int64_t(out[2 * p + 1]);
     }
+    return SNPM_OK;
+}
+
+}  // extern "C"
+
+// ---- multi-sample VCF text (vcf.cuh) ---------------------------------------------------------------------------------------
+struct snpm_vcf {
+    int device = 0;
+    int32_t S = 0;
+    int64_t chunk = 0;
+    cudaStream_t st = nullptr;
+    char *h_text = nullptr;              // pinned staging of one chunk
+    DevBuf d_text, d_tile_cnt, d_tile_off, d_chunk, d_starts, d_flags, d_nsf, d_pos, d_dp, d_clen, d_samp0, d_fmt, d_ncell,
+        d_cell_off, d_cls, d_pl, d_ccnt, d_coff, d_soff, d_line, d_ocls, d_opl, d_scan;
+    int64_t n_lines = 0, n_cells = 0, n_kept = 0;
+    bool parsed = false;
+    cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
+    ~snpm_vcf() {
+        for (cudaEvent_t e : ev)
+            if (e) cudaEventDestroy(e);
+        if (h_text) cudaFreeHost(h_text);
+        if (st) cudaStreamDestroy(st);
+    }
+    VcfLines lines() const {
+        return VcfLines{d_flags.as<int>(), d_nsf.as<int>(), d_pos.as<int>(), d_dp.as<int>(), d_clen.as<int>(), d_samp0.as<int>(),
+                        d_fmt.as<int>(), d_ncell.as<int>()};
+    }
+};
+
+// exclusive scan of n int32 counts into out[0..n]
+static int vcf_scan(cudaStream_t st, const int *in, int64_t n, int *out, DevBuf &tmp) {
+    const int64_t nb = std::max<int64_t>(1, ceil_div64(n, VCF_SCAN_ITEMS));
+    if (nb > INT32_MAX - 1) return fail(SNPM_E_ARG, "vcf scan: %lld items are too many", (long long)n);
+    SNPM_TRY(tmp.ensure(size_t(nb + 1) * 4));
+    k_vcf_scan_reduce<<<unsigned(nb), 1024, 0, st>>>(in, n, tmp.as<int>());
+    k_vcf_scan_top<<<1, 1024, 0, st>>>(tmp.as<int>(), int(nb));
+    k_vcf_scan_apply<<<unsigned(nb), 1024, 0, st>>>(in, n, tmp.as<int>(), out);
+    SNPM_KERNEL_CHECK();
+    return SNPM_OK;
+}
+
+static int vcf_read_count(cudaStream_t st, const int *d_at, int64_t &out) {
+    int v = 0;
+    SNPM_CUDA(cudaMemcpyAsync(&v, d_at, 4, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaStreamSynchronize(st));
+    out = v;
+    return SNPM_OK;
+}
+
+extern "C" {
+
+int snpm_vcf_create(int device, int32_t n_samples, int64_t chunk_bytes, snpm_vcf **out) {
+    if (!out) return fail(SNPM_E_ARG, "snpm_vcf_create: out is NULL");
+    *out = nullptr;
+    if (n_samples < 1) return fail(SNPM_E_ARG, "snpm_vcf_create: n_samples = %d, need at least 1", n_samples);
+    if (chunk_bytes < 1 || chunk_bytes > SNPM_VCF_MAX_CHUNK)
+        return fail(SNPM_E_ARG, "snpm_vcf_create: chunk_bytes = %lld outside 1..%lld", (long long)chunk_bytes, (long long)SNPM_VCF_MAX_CHUNK);
+    SNPM_CUDA(cudaSetDevice(device));
+    std::unique_ptr<snpm_vcf> h(new (std::nothrow) snpm_vcf);
+    if (!h) return fail(SNPM_E_NOMEM, "snpm_vcf_create: out of host memory");
+    h->device = device;
+    h->S = n_samples;
+    h->chunk = chunk_bytes;
+    SNPM_CUDA(cudaStreamCreateWithFlags(&h->st, cudaStreamNonBlocking));
+    for (cudaEvent_t &e : h->ev) SNPM_CUDA(cudaEventCreate(&e));
+    if (cudaMallocHost(&h->h_text, size_t(chunk_bytes)) != cudaSuccess) {
+        h->h_text = nullptr;
+        return fail(SNPM_E_NOMEM, "snpm_vcf_create: cannot pin %lld bytes of host memory", (long long)chunk_bytes);
+    }
+    SNPM_TRY(h->d_text.ensure(size_t(chunk_bytes) + 16));
+    SNPM_TRY(h->d_chunk.ensure(8));
+    *out = h.release();
+    return SNPM_OK;
+}
+
+void snpm_vcf_destroy(snpm_vcf *h) {
+    if (!h) return;
+    cudaSetDevice(h->device);
+    if (h->st) cudaStreamSynchronize(h->st);
+    delete h;
+}
+
+int snpm_vcf_parse(snpm_vcf *h, const char *text, int64_t n_bytes, int64_t *info, float *ms) {
+    if (!h || !text || !info) return fail(SNPM_E_ARG, "snpm_vcf_parse: bad arguments");
+    if (n_bytes < 1 || n_bytes > h->chunk)
+        return fail(SNPM_E_ARG, "snpm_vcf_parse: %lld bytes for a chunk of %lld", (long long)n_bytes, (long long)h->chunk);
+    if (text[n_bytes - 1] != '\n' && text[n_bytes - 1] != '\r')
+        return fail(SNPM_E_ARG, "snpm_vcf_parse: the chunk must end with a line end");
+    SNPM_CUDA(cudaSetDevice(h->device));
+    cudaStream_t st = h->st;
+    h->parsed = false;
+    const int S = h->S;
+    memcpy(h->h_text, text, size_t(n_bytes));
+    SNPM_CUDA(cudaEventRecord(h->ev[0], st));
+    SNPM_CUDA(cudaMemcpyAsync(h->d_text.p, h->h_text, size_t(n_bytes), cudaMemcpyHostToDevice, st));
+    SNPM_CUDA(cudaEventRecord(h->ev[1], st));
+    const uint8_t *t = h->d_text.as<uint8_t>();
+    // 1. line index
+    const int64_t n_tiles = ceil_div64(n_bytes, VCF_TILE);
+    SNPM_TRY(h->d_tile_cnt.ensure(size_t(n_tiles) * 4));
+    SNPM_TRY(h->d_tile_off.ensure(size_t(n_tiles + 1) * 4));
+    SNPM_CUDA(cudaMemsetAsync(h->d_chunk.p, 0, 8, st));
+    k_vcf_line_count<<<unsigned(n_tiles), 256, 0, st>>>(t, n_bytes, h->d_tile_cnt.as<int>(), h->d_chunk.as<int>());
+    SNPM_KERNEL_CHECK();
+    SNPM_TRY(vcf_scan(st, h->d_tile_cnt.as<int>(), n_tiles, h->d_tile_off.as<int>(), h->d_scan));
+    int64_t n_lines = 0;
+    SNPM_TRY(vcf_read_count(st, h->d_tile_off.as<int>() + n_tiles, n_lines));
+    SNPM_TRY(h->d_starts.ensure(size_t(n_lines + 1) * 4));
+    k_vcf_line_starts<<<unsigned(n_tiles), 256, 0, st>>>(t, n_bytes, h->d_tile_off.as<int>(), h->d_starts.as<int>(), h->d_chunk.as<int>());
+    SNPM_KERNEL_CHECK();
+    // 2. fixed fields
+    for (DevBuf *b : {&h->d_flags, &h->d_nsf, &h->d_pos, &h->d_dp, &h->d_clen, &h->d_samp0, &h->d_fmt, &h->d_ncell})
+        SNPM_TRY(b->ensure(size_t(n_lines) * 4));
+    SNPM_TRY(h->d_cell_off.ensure(size_t(n_lines + 1) * 4));
+    int n_sm = 148;
+    cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, h->device);
+    const int lgrid = grid_for(n_lines, 8, n_sm);
+    const VcfLines o = h->lines();
+    if (n_lines) {
+        k_vcf_records<<<lgrid, 256, 0, st>>>(t, h->d_starts.as<int>(), int(n_lines), S, o);
+        SNPM_KERNEL_CHECK();
+    }
+    SNPM_TRY(vcf_scan(st, o.ncell, n_lines, h->d_cell_off.as<int>(), h->d_scan));
+    int64_t n_cells = 0;
+    SNPM_TRY(vcf_read_count(st, h->d_cell_off.as<int>() + n_lines, n_cells));
+    // 3. cells
+    SNPM_TRY(h->d_cls.ensure(size_t(n_cells) * 2));
+    SNPM_TRY(h->d_pl.ensure(size_t(n_cells) * 12));
+    if (n_lines) {
+        k_vcf_cells<<<lgrid, 256, 0, st>>>(t, h->d_starts.as<int>(), int(n_lines), o, h->d_cell_off.as<int>(), h->d_cls.as<uint16_t>(),
+                                           h->d_pl.as<int>());
+        SNPM_KERNEL_CHECK();
+    }
+    // 5. per-sample compaction
+    const int64_t n_ctiles = std::max<int64_t>(1, ceil_div64(n_lines, VCF_CTILE));
+    const int64_t n_cnt = n_ctiles * S;
+    SNPM_TRY(h->d_ccnt.ensure(size_t(n_cnt) * 4));
+    SNPM_TRY(h->d_coff.ensure(size_t(n_cnt + 1) * 4));
+    SNPM_TRY(h->d_soff.ensure(size_t(S + 1) * 4));
+    const dim3 cgrid(unsigned(n_ctiles), unsigned((S + 127) / 128));
+    k_vcf_count_called<<<cgrid, 128, 0, st>>>(int(n_lines), S, o, h->d_cell_off.as<int>(), h->d_cls.as<uint16_t>(), h->d_ccnt.as<int>());
+    SNPM_KERNEL_CHECK();
+    SNPM_TRY(vcf_scan(st, h->d_ccnt.as<int>(), n_cnt, h->d_coff.as<int>(), h->d_scan));
+    k_vcf_sample_off<<<(S + 256) / 256, 256, 0, st>>>(h->d_coff.as<int>(), S, int(n_ctiles), h->d_soff.as<int>());
+    SNPM_KERNEL_CHECK();
+    int64_t n_kept = 0;
+    SNPM_TRY(vcf_read_count(st, h->d_coff.as<int>() + n_cnt, n_kept));
+    SNPM_TRY(h->d_line.ensure(size_t(n_kept) * 4));
+    SNPM_TRY(h->d_ocls.ensure(size_t(n_kept) * 2));
+    SNPM_TRY(h->d_opl.ensure(size_t(n_kept) * 12));
+    k_vcf_write_called<<<cgrid, 128, 0, st>>>(int(n_lines), S, o, h->d_cell_off.as<int>(), h->d_cls.as<uint16_t>(), h->d_pl.as<int>(),
+                                              h->d_coff.as<int>(), h->d_line.as<int>(), h->d_ocls.as<uint16_t>(), h->d_opl.as<int>());
+    SNPM_KERNEL_CHECK();
+    SNPM_CUDA(cudaEventRecord(h->ev[2], st));
+    int cf[2] = {0, 0};
+    SNPM_CUDA(cudaMemcpyAsync(cf, h->d_chunk.p, 8, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaStreamSynchronize(st));
+    h->n_lines = n_lines;
+    h->n_cells = n_cells;
+    h->n_kept = n_kept;
+    h->parsed = true;
+    info[0] = n_lines;
+    info[1] = n_cells;
+    info[2] = n_kept;
+    info[3] = cf[0];
+    info[4] = cf[1];
+    if (ms) {
+        ms[0] = ms[1] = 0.f;
+        cudaEventElapsedTime(&ms[0], h->ev[0], h->ev[1]);
+        cudaEventElapsedTime(&ms[1], h->ev[1], h->ev[2]);
+    }
+    return SNPM_OK;
+}
+
+int snpm_vcf_fetch(snpm_vcf *h, int32_t *line_start, int32_t *flags, int32_t *nsf, int32_t *pos, int32_t *dp, int32_t *chrom_len,
+                   int32_t *sample_off, int32_t *line, uint16_t *cls, int32_t *pl) {
+    if (!h || !line_start || !flags || !nsf || !pos || !dp || !chrom_len || !sample_off || !line || !cls || !pl)
+        return fail(SNPM_E_ARG, "snpm_vcf_fetch: bad arguments");
+    if (!h->parsed) return fail(SNPM_E_STATE, "snpm_vcf_fetch: no parsed chunk");
+    SNPM_CUDA(cudaSetDevice(h->device));
+    cudaStream_t st = h->st;
+    const size_t nl = size_t(h->n_lines), nk = size_t(h->n_kept);
+    SNPM_CUDA(cudaMemcpyAsync(line_start, h->d_starts.p, (nl + 1) * 4, cudaMemcpyDeviceToHost, st));
+    const std::pair<void *, const DevBuf *> per_line[] = {{flags, &h->d_flags}, {nsf, &h->d_nsf}, {pos, &h->d_pos}, {dp, &h->d_dp},
+                                                          {chrom_len, &h->d_clen}};
+    if (nl)
+        for (const auto &c : per_line) SNPM_CUDA(cudaMemcpyAsync(c.first, c.second->p, nl * 4, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaMemcpyAsync(sample_off, h->d_soff.p, size_t(h->S + 1) * 4, cudaMemcpyDeviceToHost, st));
+    if (nk) {
+        SNPM_CUDA(cudaMemcpyAsync(line, h->d_line.p, nk * 4, cudaMemcpyDeviceToHost, st));
+        SNPM_CUDA(cudaMemcpyAsync(cls, h->d_ocls.p, nk * 2, cudaMemcpyDeviceToHost, st));
+        SNPM_CUDA(cudaMemcpyAsync(pl, h->d_opl.p, nk * 12, cudaMemcpyDeviceToHost, st));
+    }
+    SNPM_CUDA(cudaStreamSynchronize(st));
     return SNPM_OK;
 }
 

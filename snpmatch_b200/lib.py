@@ -270,6 +270,10 @@ SIGNATURES = {
     "snpm_panel_create": (C.c_int, [_p, _p, _i64, C.c_int, _p]),
     "snpm_panel_score": (C.c_int, [_p, _p, C.c_int, _i64, _p, _p, _p, _p, _p, _p]),
     "snpm_panel_destroy": (None, [_p]),
+    "snpm_vcf_create": (C.c_int, [C.c_int, _i32, _i64, _p]),
+    "snpm_vcf_parse": (C.c_int, [_p, C.c_char_p, _i64, _p, _p]),
+    "snpm_vcf_fetch": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
+    "snpm_vcf_destroy": (None, [_p]),
 }
 
 
@@ -520,6 +524,48 @@ class SharedPanel(object):
     def close(self):
         if getattr(self, "_h", None):
             load().snpm_panel_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class VcfParser(object):
+    """The genotype columns of a multi-sample VCF parsed on the device (snpm_vcf_*), one chunk of whole lines at a time.
+    parse(text) returns the chunk's per-line arrays and every sample's called cells (see snpm_vcf_fetch); core.parsers.read_vcf_many
+    turns them into one ParseInputs per sample."""
+
+    FLAG_RECORD, FLAG_FALLBACK, FLAG_HAS_PL, FLAG_NEW_CHROM = 1, 2, 4, 8
+    N_ALLELE_CODES = 111
+
+    def __init__(self, device, n_samples, chunk_bytes):
+        self.device, self.n_samples, self.chunk_bytes = int(device), int(n_samples), int(chunk_bytes)
+        h = C.c_void_p()
+        check(load().snpm_vcf_create(self.device, self.n_samples, self.chunk_bytes, C.byref(h)))
+        self._h = h
+
+    def parse(self, text):
+        """text: bytes of whole lines, ending in a line end.  Returns dict(n_lines, n_cells, non_ascii, info_dp_lines, h2d_ms,
+        kernel_ms, and the arrays line_start, flags, nsf, pos, dp, chrom_len, sample_off, line, cls, pl)."""
+        info = np.zeros(5, np.int64)
+        ms = (C.c_float * 2)()
+        check(load().snpm_vcf_parse(self._h, text, len(text), ptr(info), ms))
+        n, k, S = int(info[0]), int(info[2]), self.n_samples
+        r = dict(n_lines=n, n_cells=int(info[1]), non_ascii=bool(info[3]), info_dp_lines=int(info[4]), h2d_ms=ms[0], kernel_ms=ms[1],
+                 line_start=np.empty(n + 1, np.int32), sample_off=np.empty(S + 1, np.int32), line=np.empty(k, np.int32),
+                 cls=np.empty(k, np.uint16), pl=np.empty((k, 3), np.int32))
+        for key in ("flags", "nsf", "pos", "dp", "chrom_len"):
+            r[key] = np.empty(n, np.int32)
+        check(load().snpm_vcf_fetch(self._h, *[ptr(r[key]) for key in ("line_start", "flags", "nsf", "pos", "dp", "chrom_len",
+                                                                       "sample_off", "line", "cls", "pl")]))
+        return r
+
+    def close(self):
+        if getattr(self, "_h", None):
+            load().snpm_vcf_destroy(self._h)
             self._h = None
 
     def __del__(self):

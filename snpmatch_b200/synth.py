@@ -12,6 +12,8 @@ Shapes follow the 1001 Genomes panel: TAIR10 chromosome lengths
 The sample recipe follows the reference's simulator (simulate.py:10-31) and the PL shape of
 sample_files/701_501.filter.vcf (e.g. `0,9,87` at DP 3).
 """
+import io
+
 import numpy as np
 
 TAIR10_CHRS = ["1", "2", "3", "4", "5"]
@@ -245,3 +247,98 @@ def pl_table(max_pl):
     """exp(-PL/10) for PL = 0..max_pl, computed as parsers.py:147-148 computes it per marker (PL / -10, then exp): the weight
     of a marker IS table[PL], bit for bit, so integer PLs are ready-made dictionary codes of the weights."""
     return np.exp(np.arange(int(max_pl) + 1) / -10.0)
+
+
+# ---- multi-sample VCF text (tests and measurement of parsers.read_vcf_many) -----------------------------------------------
+def multi_sample_vcf(n_records, n_samples, seed=7, line_end="\n", info_dp_header=True, late_info_dp=False, edge_cases=True):
+    """Seeded text of a VCF with n_samples sample columns.  With edge_cases, the records mix every GT form read_vcf_minimal
+    renders (phased, single alleles, '.', empty, multi-digit, more than two alleles, GT missing from FORMAT or from the cell,
+    PL before GT), PL forms (missing key, '.', fewer or more than three values, 3.5, 1e2), INFO DP forms (present, absent,
+    DP=x, DP=1_0, ADP=, an empty DP= before a real one), cells with fewer subfields than FORMAT, records with fewer sample
+    columns than the header (one with exactly 32), '##' and '#' lines, blank and short lines among the records and a non-ASCII chromosome name.
+    late_info_dp puts a '##INFO=<ID=DP,' line among the records.  line_end may also be a list of line ends to cycle through.  Returns (text, fallback): fallback = the 0-based indices of
+    the records the device parser cannot reproduce (lib.VcfParser.FLAG_FALLBACK), i.e. the ones it hands to the Python code."""
+    rng = np.random.default_rng(seed)
+    ends = line_end if isinstance(line_end, (list, tuple)) else [line_end]
+    lines = ["##fileformat=VCFv4.2"]
+    if info_dp_header:
+        lines.append('##INFO=<ID=DP,Number=1,Type=Integer,Description="depth">')
+    lines.append("#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\t" + "\t".join("smp%d" % i for i in range(n_samples)))
+    plain_gt = ["0/0", "0|1", "1/0", "1/1", "./.", ".", "0", "./1", "2/3", "0/0/1", "", "1|1", "10/1", "01/1", "./0", "1"]
+    chroms = ["Chr1", "Chr2", "chr3", "Chr4", "Chr5"]
+    fallback = []
+    pos = 100
+    for r in range(n_records):
+        fb = False
+        if late_info_dp and r == n_records // 2:
+            lines.append('##INFO=<ID=DP,Number=1,Type=Integer,Description="depth">')
+        if edge_cases and rng.random() < 0.03:
+            lines.append(["##INFO=<ID=XX,Number=1>", "#comment", "", "Chr1\t5\t.\tA\tT", "##contig=<ID=Chr1>"][rng.integers(0, 5)])
+        chrom = chroms[min(r * len(chroms) // max(n_records, 1), len(chroms) - 1)]
+        if edge_cases and r % 97 == 13:
+            chrom, fb = "Chrü", True
+        pos += int(rng.integers(1, 400))
+        pos_text = str(pos)
+        if edge_cases and r % 89 == 5:
+            pos_text, fb = "+" + pos_text, True
+        info = "DP=%d" % rng.integers(0, 99)
+        if edge_cases:
+            k = rng.integers(0, 10)
+            info = ["DP=%d" % rng.integers(0, 99), "AC=1;DP=%d;MQ=4" % rng.integers(0, 99), "ADP=3", "ADP=3;DP=9", ".", "DP=;DP=4",
+                    "DP=12", "AC=2", "DP=x", "DP=1_0"][k]
+            fb |= k >= 8
+        fmt = ["GT", "PL"]
+        if edge_cases:
+            k = rng.integers(0, 9)
+            fmt = [["GT", "PL"], ["PL", "GT"], ["GT"], ["GT", "AD", "PL"], ["AD", "DP"], ["GT", "PL"], ["GT", "PL"], ["GT", "GT"],
+                   ["GT", "PL", "PL"]][k]
+            fb |= k >= 7
+        n_fields = n_samples
+        if edge_cases and rng.random() < 0.08:
+            n_fields = int(rng.integers(1, n_samples + 1))
+        if edge_cases and r % 61 == 7:
+            n_fields = min(32, n_samples)              # the last field closes a full warp's batch of cells
+        cells = []
+        for s in range(n_fields):
+            gt = plain_gt[rng.integers(0, len(plain_gt))] if edge_cases else ["0/0", "0/1", "1/1", "./."][rng.integers(0, 4)]
+            bad_gt = edge_cases and rng.random() < 0.002
+            if bad_gt:
+                gt = "A/1"
+            pl = ",".join(str(v) for v in rng.integers(0, 255, 3))
+            bad_pl = False
+            if edge_cases:
+                k = rng.integers(0, 12)
+                pl = [pl, pl, pl, pl, ".", "5,3", "1,2,3,4,5,6", "", ".,.,.", "0,.,7", "3.5,1,2", "1e2,0,3"][k]
+                bad_pl = k >= 10
+            vals = {"GT": gt, "PL": pl, "AD": "3,4", "DP": "7"}
+            sub = [vals[k] for k in fmt]
+            keep = len(sub)
+            if edge_cases and rng.random() < 0.05:
+                keep = int(rng.integers(0, len(sub)))
+            sub = sub[:keep]
+            cells.append(":".join(sub))
+            if s < n_samples and len(set(fmt)) == len(fmt):
+                if bad_gt and "GT" in fmt[:keep]:
+                    fb = True
+                if bad_pl and "PL" in fmt[:keep]:
+                    fb = True
+        lines.append("\t".join([chrom, pos_text, ".", "A", "T", ".", "PASS", info, ":".join(fmt)] + cells))
+        if fb:
+            fallback.append(r)
+    text = "".join(line + ends[i % len(ends)] for i, line in enumerate(lines))
+    return text, fallback
+
+
+def split_vcf_column(text, s):
+    """The single-sample VCF of column s of a multi-sample VCF's text: every header and '#' line, and every other line cut to
+    its 9 fixed fields and field 9 + s (to its first 9 fields when it has no field 9 + s)."""
+    out = []
+    for line in io.StringIO(text, newline=None):
+        f = line.rstrip("\n").split("\t")
+        if line.startswith("##"):
+            out.append(line.rstrip("\n"))
+        elif line.startswith("#") or len(f) >= 10 + s:
+            out.append("\t".join(f[:9] + f[9 + s:10 + s]))
+        else:
+            out.append("\t".join(f[:9]))
+    return "".join(x + "\n" for x in out)
