@@ -451,6 +451,20 @@ int snpm_vcf_create(int device, int32_t n_samples, int64_t chunk_bytes, snpm_vcf
 int snpm_vcf_parse(snpm_vcf *h, const char *text, int64_t n_bytes, int64_t *info, float *ms);
 int snpm_vcf_fetch(snpm_vcf *h, int32_t *line_start, int32_t *flags, int32_t *nsf, int32_t *pos, int32_t *dp, int32_t *chrom_len,
                    int32_t *sample_off, int32_t *line, uint16_t *cls, int32_t *pl);
+/* `makedb --no_csv`: the same handle and chunks, parsed with the rules of the reference's makedb CSV (makedb.py:34-62) into
+ * rows of the packed panel, no per-cell array.  A record's calls are taken from the FIRST GT key of FORMAT; the GT text maps by
+ * exact match: 0/0 0|0 -> 0, 1/1 1|1 -> 1, 0/1 0|1 1/0 1|0 -> 2, ./. .|. . -> missing; a record without GT and a cell without
+ * that subfield are missing; any other text is missing and counted.
+ * snpm_vcf_parse_gt_packed: info int64[4] = lines, rows, the counted calls, 1 if the chunk holds a byte >= 0x80; ms (optional)
+ * float[2] as for snpm_vcf_parse.
+ * snpm_vcf_fetch_gt_packed, per line (n = info[0]): line_start int32[n+1], flags int32[n] (1 record, 2 POS is not 1-9 plain
+ * digits: pos is not set, convert the text on the host; 8 CHROM may differ from the previous record's), nsf int32[n], pos
+ * int32[n], chrom_len int32[n] as for snpm_vcf_fetch; packed uint64 [info[1], stride] with stride = snpm_db_row_words of a
+ * panel of n_samples accessions, in the layout of snpm_db_load_packed: one row per record with exactly n_samples sample fields,
+ * in line order (a record with another count gets no row, and flag 8 is left unset on it). */
+int snpm_vcf_parse_gt_packed(snpm_vcf *h, const char *text, int64_t n_bytes, int64_t *info, float *ms);
+int snpm_vcf_fetch_gt_packed(snpm_vcf *h, int32_t *line_start, int32_t *flags, int32_t *nsf, int32_t *pos, int32_t *chrom_len,
+                             uint64_t *packed);
 void snpm_vcf_destroy(snpm_vcf *h);
 
 #ifdef __cplusplus

@@ -284,7 +284,13 @@ def get_options(description, version_message):
     mk = sub.add_parser('makedb', help="build the packed database (<id>.npz) and the genome JSON from a multi-sample VCF of the known strains, or from the intermediate CSV of the reference")
     mk.add_argument("-i", "--input_vcf", dest="inFile", help="VCF of the known strains (biallelic SNPs), or a CSV with the columns Chromosome,Position,<accession>...")
     mk.add_argument("-p", "--bcftools_path", dest="bcfpath", default='', help="accepted for compatibility: the VCF is read directly, bcftools is not needed")
-    mk.add_argument("-o", "--out_db_id", dest="db_id", help="output id: <id>.npz, <id>.json (and <id>.csv for VCF input)")
+    mk.add_argument("-o", "--out_db_id", dest="db_id", help="output id: <id>.npz, <id>.json (and <id>.csv for VCF input unless --no_csv)")
+    mk.add_argument("--no_csv", action="store_true", dest="no_csv", default=False,
+                    help="VCF input only: build <id>.npz and <id>.json straight from the VCF (plain or .vcf.gz), its genotype columns "
+                         "parsed and packed on the GPU, without writing <id>.csv; the database equals the one built through the CSV. "
+                         "Exit status 1, naming the line or value, on the inputs the CSV cannot hold (a record whose number of sample "
+                         "fields differs from the #CHROM line's, a '#' line after the #CHROM line, a POS that is not an integer, a "
+                         "',' or '\"' in CHROM or a sample name, a non-ASCII sample name)")
     mk.add_argument("-v", "--verbose", action="store_true", dest="logDebug", default=False, help="log at DEBUG level")
     mk.set_defaults(func=makedb_vcf_to_db)
 

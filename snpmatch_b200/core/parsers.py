@@ -347,10 +347,11 @@ def _open_binary(path):
     return gzip.open(path, "rb") if str(path).endswith(".gz") else open(path, "rb")
 
 
-def read_vcf_header(fh, block=1 << 20):
+def read_vcf_header(fh, block=1 << 20, meta_lines=None):
     """Header of a VCF opened in binary mode, read up to and including its #CHROM line with the universal-newline rule of the
     text-mode readers: returns (sample names, has_info_dp, lines read, the bytes read past the #CHROM line).  Raises ValueError
-    when a record (10 fields or more) comes before the #CHROM line, or when there is no #CHROM line."""
+    when a record (10 fields or more) comes before the #CHROM line, or when there is no #CHROM line.  meta_lines (optional
+    list) receives the '##' lines before the #CHROM line, without their line ends."""
     enc = locale.getpreferredencoding(False)
     buf, at, n, has_dp, eof = b"", 0, 0, False, False
     while True:
@@ -370,6 +371,8 @@ def read_vcf_header(fh, block=1 << 20):
         text = line.decode(enc)
         if text.startswith("##"):
             has_dp |= text.startswith("##INFO=<ID=DP,")
+            if meta_lines is not None:
+                meta_lines.append(text)
         elif text.startswith("#"):
             return text.split("\t")[9:], has_dp, n, buf[at:]
         elif len(text.split("\t")) >= 10:

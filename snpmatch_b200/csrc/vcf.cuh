@@ -13,6 +13,14 @@
 //      empty or 1-2 digits, GT or PL twice in FORMAT, a non-ASCII byte in the fixed fields;
 //   5. k_vcf_count_called + scan + k_vcf_write_called: per sample, the called cells (rendered GT != ./.) of the records that
 //      did not fall back, in record order (sample-major CSR).  The dense [cells] arrays stay on the device.
+//
+// `makedb --no_csv` (snpm_vcf_parse_gt_packed) reuses the line index and takes makedb's rules instead of steps 2-5:
+//   2'. k_vcf_records<true>: tab positions, POS, the index of the FIRST GT in FORMAT (vcf_to_csv's keys.index), the number of
+//       sample fields; only a POS that is not 1-9 plain digits flags a record (the host converts that POS text);
+//   3'. scan of the records whose sample-field count equals the header's: each one's row in the chunk's packed panel;
+//   4'. k_vcf_gt_packed, one warp per record: lane j classifies cell 32 w + j by the exact GT text of vcf_to_csv's _GT_CODE and
+//       two ballots write packed word w in k_pack_int8's layout (padding lanes and words missing); calls that are no _GT_CODE
+//       string are counted with one atomic per warp.  No per-cell array exists.
 #pragma once
 #include "common.cuh"
 
@@ -203,6 +211,9 @@ struct VcfLines {
     int *flags, *nsf, *pos, *dp, *chrom_len, *samp0, *fmt, *ncell;
 };
 
+// MAKEDB: vcf_to_csv's rules (first GT of FORMAT, only POS flags a record, ncell = 1 for a record of exactly n_samples sample
+// fields: the rows of the packed panel); otherwise read_vcf_minimal's (see the top of the file)
+template <bool MAKEDB>
 __global__ void __launch_bounds__(256) k_vcf_records(const uint8_t *__restrict__ t, const int *__restrict__ starts, int n_lines,
                                                      int n_samples, VcfLines o) {
     const int lane = threadIdx.x & 31;
@@ -216,8 +227,10 @@ __global__ void __launch_bounds__(256) k_vcf_records(const uint8_t *__restrict__
                 const int p = base + lane;
                 const uint8_t c = p < e ? t[p] : 0;
                 const unsigned m = __ballot_sync(0xffffffffu, c == '\t');
-                const unsigned hm = __ballot_sync(0xffffffffu, c >= 0x80);
-                if (hm && first_high == e) first_high = base + __ffs(hm) - 1;
+                if constexpr (!MAKEDB) {
+                    const unsigned hm = __ballot_sync(0xffffffffu, c >= 0x80);
+                    if (hm && first_high == e) first_high = base + __ffs(hm) - 1;
+                }
                 const int j = lane - ntab;                    // lane k < 9 keeps the position of tab k
                 if (lane < 9 && j >= 0 && j < __popc(m)) tab = base + int(__fns(m, 0, j + 1));
                 ntab += __popc(m);
@@ -230,42 +243,57 @@ __global__ void __launch_bounds__(256) k_vcf_records(const uint8_t *__restrict__
                 nsf = ntab - 8;
                 clen = tb[0] - s;
                 samp0 = tb[8] + 1;
-                bool fb = first_high < tb[8];
-                // INFO: the first (?:^|;)DP= followed by a non-empty value
-                const int i0 = tb[6] + 1, i1 = tb[7];
-                int found = -1;
-                for (int base = i0; base < i1 && found < 0; base += 32) {
-                    const int p = base + lane;
-                    const bool cand = p + 3 < i1 && (p == i0 || t[p - 1] == ';') && t[p] == 'D' && t[p + 1] == 'P' && t[p + 2] == '=' &&
-                                      t[p + 3] != ';';
-                    const unsigned m = __ballot_sync(0xffffffffu, cand);
-                    if (m) found = base + __ffs(m) - 1;
-                }
-                if (lane == 0) {
-                    fb |= !vcf_uint9(t, tb[0] + 1, tb[1], pos);
-                    if (found >= 0) {
-                        int v = found + 3;
-                        while (v < i1 && t[v] != ';' && v - found < 13) ++v;      // 10 characters are already too many
-                        fb |= !vcf_uint9(t, found + 3, v, dp);
-                    }
-                    // FORMAT: indices of GT and PL (1-based, 0 = absent), either one twice falls back (dict(zip()) keeps the last)
-                    int k = 0, ks = tb[7] + 1, gi = 0, pi = 0;
-                    for (int p = tb[7] + 1; p <= tb[8]; ++p) {
-                        if (p < tb[8] && t[p] != ':') continue;
-                        if (p - ks == 2 && t[ks] == 'G' && t[ks + 1] == 'T') {
-                            fb |= gi != 0;
-                            gi = k + 1;
-                        } else if (p - ks == 2 && t[ks] == 'P' && t[ks + 1] == 'L') {
-                            fb |= pi != 0;
-                            pi = k + 1;
+                if constexpr (MAKEDB) {
+                    if (lane == 0) {
+                        if (!vcf_uint9(t, tb[0] + 1, tb[1], pos)) flags |= VCF_FALLBACK;
+                        // FORMAT: the index of the first GT (1-based, 0 = absent)
+                        int k = 0, ks = tb[7] + 1, gi = 0;
+                        for (int p = tb[7] + 1; p <= tb[8] && !gi; ++p) {
+                            if (p < tb[8] && t[p] != ':') continue;
+                            if (p - ks == 2 && t[ks] == 'G' && t[ks + 1] == 'T') gi = k + 1;
+                            ++k;
+                            ks = p + 1;
                         }
-                        ++k;
-                        ks = p + 1;
+                        fmt = gi;
                     }
-                    fb |= k >= 0xffff;
-                    fmt = (gi & 0xffff) | (pi << 16);
-                    if (pi) flags |= VCF_HAS_PL;
-                    if (fb) flags |= VCF_FALLBACK;
+                } else {
+                    bool fb = first_high < tb[8];
+                    // INFO: the first (?:^|;)DP= followed by a non-empty value
+                    const int i0 = tb[6] + 1, i1 = tb[7];
+                    int found = -1;
+                    for (int base = i0; base < i1 && found < 0; base += 32) {
+                        const int p = base + lane;
+                        const bool cand = p + 3 < i1 && (p == i0 || t[p - 1] == ';') && t[p] == 'D' && t[p + 1] == 'P' && t[p + 2] == '=' &&
+                                          t[p + 3] != ';';
+                        const unsigned m = __ballot_sync(0xffffffffu, cand);
+                        if (m) found = base + __ffs(m) - 1;
+                    }
+                    if (lane == 0) {
+                        fb |= !vcf_uint9(t, tb[0] + 1, tb[1], pos);
+                        if (found >= 0) {
+                            int v = found + 3;
+                            while (v < i1 && t[v] != ';' && v - found < 13) ++v;      // 10 characters are already too many
+                            fb |= !vcf_uint9(t, found + 3, v, dp);
+                        }
+                        // FORMAT: indices of GT and PL (1-based, 0 = absent), either one twice falls back (dict(zip()) keeps the last)
+                        int k = 0, ks = tb[7] + 1, gi = 0, pi = 0;
+                        for (int p = tb[7] + 1; p <= tb[8]; ++p) {
+                            if (p < tb[8] && t[p] != ':') continue;
+                            if (p - ks == 2 && t[ks] == 'G' && t[ks + 1] == 'T') {
+                                fb |= gi != 0;
+                                gi = k + 1;
+                            } else if (p - ks == 2 && t[ks] == 'P' && t[ks + 1] == 'L') {
+                                fb |= pi != 0;
+                                pi = k + 1;
+                            }
+                            ++k;
+                            ks = p + 1;
+                        }
+                        fb |= k >= 0xffff;
+                        fmt = (gi & 0xffff) | (pi << 16);
+                        if (pi) flags |= VCF_HAS_PL;
+                        if (fb) flags |= VCF_FALLBACK;
+                    }
                 }
                 flags = __shfl_sync(0xffffffffu, flags, 0);
             }
@@ -278,7 +306,10 @@ __global__ void __launch_bounds__(256) k_vcf_records(const uint8_t *__restrict__
             o.chrom_len[L] = clen;
             o.samp0[L] = samp0;
             o.fmt[L] = fmt;
-            o.ncell[L] = (flags & (VCF_REC | VCF_FALLBACK)) == VCF_REC ? min(nsf, n_samples) : 0;
+            if constexpr (MAKEDB)
+                o.ncell[L] = (flags & VCF_REC) && nsf == n_samples;
+            else
+                o.ncell[L] = (flags & (VCF_REC | VCF_FALLBACK)) == VCF_REC ? min(nsf, n_samples) : 0;
         }
     }
 }
@@ -445,6 +476,92 @@ __global__ void __launch_bounds__(128) k_vcf_write_called(int n_lines, int n_sam
 __global__ void k_vcf_sample_off(const int *__restrict__ coff, int n_samples, int n_ctiles, int *__restrict__ sample_off) {
     const int s = int(blockIdx.x) * blockDim.x + threadIdx.x;
     if (s <= n_samples) sample_off[s] = coff[int64_t(s) * n_ctiles];
+}
+
+// ---- makedb: records -> packed panel rows ------------------------------------------------------------------------------------
+// the code of vcf_to_csv's _GT_CODE for the cell [a, b) whose GT is subfield gi (0-based, -1 absent): 0 for 0/0 0|0, 1 for 1/1
+// 1|1, 2 for 0/1 0|1 1/0 1|0, 3 (missing) for ./. .|. . and for a cell without that subfield; any other text is missing and
+// sets `other`.
+__device__ __forceinline__ uint32_t vcf_gt_code(const uint8_t *__restrict__ t, int a, int b, int gi, bool &other) {
+    if (gi < 0) return 3u;
+    int k = 0, g0 = a;
+    for (int p = a; p < b && k < gi; ++p)
+        if (t[p] == ':') { ++k; g0 = p + 1; }
+    if (k < gi) return 3u;
+    int g1 = g0;
+    while (g1 < b && t[g1] != ':') ++g1;
+    if (g1 - g0 == 1 && t[g0] == '.') return 3u;
+    if (g1 - g0 == 3 && (t[g0 + 1] == '/' || t[g0 + 1] == '|')) {
+        const uint8_t x = t[g0], y = t[g0 + 2];
+        if (x == '.' && y == '.') return 3u;
+        if ((x == '0' || x == '1') && (y == '0' || y == '1')) return x == y ? uint32_t(x - '0') : 2u;
+    }
+    other = true;
+    return 3u;
+}
+
+// one packed word from the warp's 32 cells (lanes without a cell are missing); returns the other calls among them on lane 0
+__device__ __forceinline__ int vcf_pack_word(const uint8_t *__restrict__ t, bool have, int a, int b, int gi, uint64_t *__restrict__ dst) {
+    bool other = false;
+    const uint32_t code = have ? vcf_gt_code(t, a, b, gi, other) : 3u;
+    const uint32_t lo = __ballot_sync(0xffffffffu, code & 1u);
+    const uint32_t hi = __ballot_sync(0xffffffffu, code & 2u);
+    const int n_other = __popc(__ballot_sync(0xffffffffu, other));
+    if ((threadIdx.x & 31) == 0) {
+        *dst = uint64_t(lo) | (uint64_t(hi) << 32);
+        return n_other;
+    }
+    return 0;
+}
+
+// One warp per record of exactly n_samples sample fields (ncell == 1): its row row_off[L] of packed [rows, stride], the cells
+// walked as in k_vcf_cells; VCF_NEW_CHROM as there.  chunk_flags[2] += the calls that are no _GT_CODE string.
+__global__ void __launch_bounds__(256) k_vcf_gt_packed(const uint8_t *__restrict__ t, const int *__restrict__ starts, int n_lines,
+                                                       VcfLines o, const int *__restrict__ row_off, int n_samples, int stride,
+                                                       uint64_t *__restrict__ packed, int *__restrict__ chunk_flags) {
+    const int lane = threadIdx.x & 31;
+    const int n_warps = int(gridDim.x) * (blockDim.x >> 5);
+    int other = 0;
+    for (int L = int(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5); L < n_lines; L += n_warps) {
+        if (!o.ncell[L]) continue;
+        const int s = starts[L];
+        const int clen = o.chrom_len[L];
+        bool same = L > 0 && (o.flags[L - 1] & VCF_REC) && o.chrom_len[L - 1] == clen;
+        if (same) {
+            const int ps = starts[L - 1];
+            for (int b0 = 0; b0 < clen && same; b0 += 32) {
+                const int i = b0 + lane;
+                same = __all_sync(0xffffffffu, i >= clen || t[ps + i] == t[s + i]);
+            }
+        }
+        uint64_t *row = packed + int64_t(row_off[L]) * stride;
+        const int gi = o.fmt[L] - 1;
+        const int nc = gi >= 0 ? n_samples : 0;          // without GT every call is missing: nothing to read
+        const int e = vcf_line_end(t, s, starts[L + 1]);
+        int cell = 0, w = 0, cur = o.samp0[L], my_a = 0, my_b = 0;
+        for (int base = cur; base < e && cell < nc; base += 32) {
+            const int p = base + lane;
+            unsigned m = __ballot_sync(0xffffffffu, p < e && t[p] == '\t');
+            while (m && cell < nc) {
+                const int tp = base + __ffs(m) - 1;
+                m &= m - 1;
+                if (lane == (cell & 31)) { my_a = cur; my_b = tp; }
+                cur = tp + 1;
+                if ((++cell & 31) == 0) other += vcf_pack_word(t, true, my_a, my_b, gi, row + w++);
+            }
+        }
+        bool closed_by_end = false;
+        if (cell < nc) {                                   // the line end closes the last sample field
+            if (lane == (cell & 31)) { my_a = cur; my_b = e; }
+            ++cell;
+            closed_by_end = true;
+        }
+        const int pending = (cell & 31) ? (cell & 31) : (closed_by_end ? 32 : 0);
+        if (pending) other += vcf_pack_word(t, lane < pending, my_a, my_b, gi, row + w++);
+        for (int k = w + lane; k < stride; k += 32) row[k] = ~0ull;     // padding words, or every word without GT
+        if (lane == 0 && !same) atomicOr(o.flags + L, VCF_NEW_CHROM);
+    }
+    if (lane == 0 && other) atomicAdd(chunk_flags + 2, other);
 }
 
 }  // namespace snpm

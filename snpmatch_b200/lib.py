@@ -273,6 +273,8 @@ SIGNATURES = {
     "snpm_vcf_create": (C.c_int, [C.c_int, _i32, _i64, _p]),
     "snpm_vcf_parse": (C.c_int, [_p, C.c_char_p, _i64, _p, _p]),
     "snpm_vcf_fetch": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
+    "snpm_vcf_parse_gt_packed": (C.c_int, [_p, C.c_char_p, _i64, _p, _p]),
+    "snpm_vcf_fetch_gt_packed": (C.c_int, [_p, _p, _p, _p, _p, _p, _p]),
     "snpm_vcf_destroy": (None, [_p]),
 }
 
@@ -536,7 +538,8 @@ class SharedPanel(object):
 class VcfParser(object):
     """The genotype columns of a multi-sample VCF parsed on the device (snpm_vcf_*), one chunk of whole lines at a time.
     parse(text) returns the chunk's per-line arrays and every sample's called cells (see snpm_vcf_fetch); core.parsers.read_vcf_many
-    turns them into one ParseInputs per sample."""
+    turns them into one ParseInputs per sample.  parse_gt_packed(text) returns the chunk's records as rows of the packed panel
+    (snpm_vcf_fetch_gt_packed), which core.makedb.makeDB_from_vcf assembles."""
 
     FLAG_RECORD, FLAG_FALLBACK, FLAG_HAS_PL, FLAG_NEW_CHROM = 1, 2, 4, 8
     N_ALLELE_CODES = 111
@@ -562,6 +565,27 @@ class VcfParser(object):
         check(load().snpm_vcf_fetch(self._h, *[ptr(r[key]) for key in ("line_start", "flags", "nsf", "pos", "dp", "chrom_len",
                                                                        "sample_off", "line", "cls", "pl")]))
         return r
+
+    def parse_gt_packed(self, text):
+        """`makedb --no_csv`: text as for parse(), read with makedb's rules (snpm_vcf_parse_gt_packed).  Returns dict(n_lines,
+        n_rows, other_calls, non_ascii, h2d_ms, kernel_ms, and the arrays line_start, flags, nsf, pos, chrom_len and packed uint64
+        [n_rows, row_words]: the panel rows of the records with n_samples sample fields, in line order)."""
+        info = np.zeros(4, np.int64)
+        ms = (C.c_float * 2)()
+        check(load().snpm_vcf_parse_gt_packed(self._h, text, len(text), ptr(info), ms))
+        n, rows = int(info[0]), int(info[1])
+        r = dict(n_lines=n, n_rows=rows, other_calls=int(info[2]), non_ascii=bool(info[3]), h2d_ms=ms[0], kernel_ms=ms[1],
+                 line_start=np.empty(n + 1, np.int32), packed=np.empty((rows, self.row_words), np.uint64))
+        for key in ("flags", "nsf", "pos", "chrom_len"):
+            r[key] = np.empty(n, np.int32)
+        check(load().snpm_vcf_fetch_gt_packed(self._h, *[ptr(r[key]) for key in ("line_start", "flags", "nsf", "pos", "chrom_len",
+                                                                                 "packed")]))
+        return r
+
+    @property
+    def row_words(self):
+        """Words per packed row: snpm_db_row_words of a panel of n_samples accessions."""
+        return (((self.n_samples + 31) // 32) + 1) & ~1
 
     def close(self):
         if getattr(self, "_h", None):

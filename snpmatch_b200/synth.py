@@ -342,3 +342,27 @@ def split_vcf_column(text, s):
         else:
             out.append("\t".join(f[:9]))
     return "".join(x + "\n" for x in out)
+
+
+_GT_TOKEN = np.array([b"./.", b"0/0", b"1/1", b"0/1"])      # index code + 1
+
+
+def panel_vcf(fh, n_rows, n_acc, seed=SEED_PANEL, block=4096):
+    """A GT-only multi-sample VCF of the synthetic panel, written to the binary file fh: record r is row r at
+    panel_positions(n_rows) on chromosome TAIR10_CHRS[c], sample a (named accession_ids) calls panel_codes(seed, r, a) as
+    0/0, 1/1, 0/1 or ./. (missing).  Built from these codes, `makedb` gives the panel load_int8 would.  Returns (positions,
+    chr_regions)."""
+    positions, regions = panel_positions(n_rows)
+    fh.write(b"##fileformat=VCFv4.2\n")
+    for c, n in zip(TAIR10_CHRS, TAIR10_CHRLEN):
+        fh.write(b"##contig=<ID=%s,length=%d>\n" % (c.encode(), n))
+    fh.write(b"#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\t" + b"\t".join(accession_ids(n_acc).tolist()) + b"\n")
+    chrom = np.searchsorted(regions[:, 1], np.arange(n_rows), side="right")
+    token = np.frombuffer(b"".join(t + b"\t" for t in _GT_TOKEN.tolist()), np.uint8).reshape(4, 4)
+    for r0 in range(0, n_rows, block):
+        rows = np.arange(r0, min(r0 + block, n_rows))
+        cells = token[panel_codes(seed, rows, n_acc).astype(np.int64) + 1].reshape(len(rows), 4 * n_acc)
+        cells[:, -1] = 10
+        fh.write(b"".join(b"%s\t%d\t.\tA\tT\t.\tPASS\t.\tGT\t" % (TAIR10_CHRS[c].encode(), p) + line.tobytes()
+                          for c, p, line in zip(chrom[rows].tolist(), positions[rows].tolist(), cells)))
+    return positions, regions
