@@ -465,6 +465,19 @@ int snpm_vcf_fetch(snpm_vcf *h, int32_t *line_start, int32_t *flags, int32_t *ns
 int snpm_vcf_parse_gt_packed(snpm_vcf *h, const char *text, int64_t n_bytes, int64_t *info, float *ms);
 int snpm_vcf_fetch_gt_packed(snpm_vcf *h, int32_t *line_start, int32_t *flags, int32_t *nsf, int32_t *pos, int32_t *chrom_len,
                              uint64_t *packed);
+/* `genotype_cross --gpu_parse`: the same handle and chunks, every record read into one row of int8 window-call codes, the codes
+ * the reference's parseGT gives the GT strings of its import_vcf_file (parsers.py:12-35, 178-213).  A record's calls are taken
+ * from the FIRST GT key of FORMAT, split at '/' and '|', the first two tokens kept (a missing or empty one is '.'), each matched
+ * exactly: (1,1) -> 1, (0,1) (1,0) -> 2, (.,.) -> -1, any other pair -> 0; a record without GT, a cell without that subfield and
+ * the cells past the record's sample fields are -1; sample fields past n_samples are ignored.  No cell is left to the host.
+ * snpm_vcf_parse_gt_codes: info int64[3] = lines, rows, 1 if the chunk holds a byte >= 0x80; ms (optional) float[2] as for
+ * snpm_vcf_parse.
+ * snpm_vcf_fetch_gt_codes, per line (n = info[0]): line_start, flags, nsf, pos, chrom_len as for snpm_vcf_fetch_gt_packed (flag
+ * 2: POS is not 1-9 plain digits, convert the text on the host); codes int8 [info[1], n_samples]: one row per record, in line
+ * order, whatever its number of sample fields. */
+int snpm_vcf_parse_gt_codes(snpm_vcf *h, const char *text, int64_t n_bytes, int64_t *info, float *ms);
+int snpm_vcf_fetch_gt_codes(snpm_vcf *h, int32_t *line_start, int32_t *flags, int32_t *nsf, int32_t *pos, int32_t *chrom_len,
+                            int8_t *codes);
 void snpm_vcf_destroy(snpm_vcf *h);
 
 #ifdef __cplusplus

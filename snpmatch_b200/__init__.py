@@ -255,6 +255,10 @@ def get_options(description, version_message):
     gc.add_argument("--hmm", dest="hmm", action="store_true", help="HMM Viterbi genotyper of the reference: not part of this package")
     gc.add_argument("--genome", dest="genome", default="athaliana_tair10", help="bundled genome id or path to a genome JSON (chromosome names and lengths)")
     gc.add_argument("-o", "--output", dest="outFile", default="genotype_cross", help="output CSV (R/qtl layout)")
+    gc.add_argument("--gpu_parse", action="store_true", dest="gpu_parse", default=False,
+                    help="parse the genotype columns of the -i VCF (plain or .vcf.gz) on the GPU instead of in Python; the output is the "
+                         "same. Exit status 1, naming the line or value, and no output file on a '#' line after the #CHROM line, a POS "
+                         "that is not an integer, a line longer than 64 MB, no #CHROM line, a record before it or no sample columns")
     gc.add_argument("-v", "--verbose", action="store_true", dest="logDebug", default=False, help="log at DEBUG level")
     gc.set_defaults(func=genotype_cross)
 

@@ -171,14 +171,20 @@ class GenotypeCross(object):
         counts, _, _ = lib.cross_window_genotypes(ix, ix, [0, num_snps], snpsP1_gt, snpsP2_gt, codes, lr_thres)
         return getWindowGenotype(counts[0, 0].tolist(), num_snps, lr_thres)
 
-    def genotype_cross(self, input_file, lr_thres, good_samples_file=None):
+    def genotype_cross(self, input_file, lr_thres, good_samples_file=None, gpu_parse=False):
+        """gpu_parse: the population VCF's genotype columns are parsed on the device (parsers.read_vcf_gt_codes, which raises
+        ValueError on the inputs it refuses); the window calls and the lines are the same."""
         log.info("loading input files!")
-        snpvcf = parsers.import_vcf_file(inFile=input_file, logDebug=self.logDebug, samples_to_load=None)
+        if gpu_parse:
+            snpvcf = parsers.read_vcf_gt_codes(input_file)
+            gt_codes = snpvcf['gt_codes']
+        else:
+            snpvcf = parsers.import_vcf_file(inFile=input_file, logDebug=self.logDebug, samples_to_load=None)
+            gt = snpvcf['gt']
+            gt_codes = parsers.parseGT(gt.ravel()).reshape(gt.shape) if gt.size else np.zeros(gt.shape, dtype=np.int8)
         num_samples = snpvcf['samples'].shape[0]
         log.info("number of samples printed: %s" % num_samples)
         gen = self.genome
-        gt = snpvcf['gt']
-        gt_codes = parsers.parseGT(gt.ravel()).reshape(gt.shape) if gt.size else np.zeros(gt.shape, dtype=np.int8)
         r = window_calls(self.commonSNPsCHR, self.commonSNPsPOS, self.snpsP1, self.snpsP2, snpvcf['chr'], snpvcf['pos'], gt_codes,
                          gen, self.window_size, float(lr_thres))
         self.last_window_calls = r
@@ -208,6 +214,12 @@ class GenotypeCross(object):
 
 def potatoCrossGenotyper(args):
     global genome
+    gpu_parse = bool(args.get('gpu_parse'))
+    if gpu_parse and not args['hmm']:
+        try:
+            parsers.vcf_population_samples(args['inFile'])       # header refusals before the database goes to the device
+        except ValueError as e:
+            snpmatch.die(str(e))
     genome = genomes.Genome(args['genome'])
     log.info("loading database files")
     g = snp_genotype.Genotype(args['hdf5File'], args['hdf5accFile'])
@@ -216,5 +228,10 @@ def potatoCrossGenotyper(args):
     if args['hmm']:
         outfile_str = crossgenotyper.genotype_cross_hmm(args['inFile'])
     else:
-        outfile_str = crossgenotyper.genotype_cross(args['inFile'], float(args['lr_thres']))
+        try:
+            outfile_str = crossgenotyper.genotype_cross(args['inFile'], float(args['lr_thres']), gpu_parse=gpu_parse)
+        except ValueError as e:
+            if not gpu_parse:
+                raise
+            snpmatch.die(str(e))
     crossgenotyper.write_output_genotype_cross(outfile_str, args['outFile'])

@@ -210,32 +210,10 @@ def makeDB_from_vcf(inVCF, outFile, device=0, chunk_bytes=parsers.VCF_CHUNK_BYTE
         label_of, label_id = {}, {}               # CHROM text -> id of the label the CSV route reads from it; label -> id
         ids, positions, rows = [], [], []
         n_rec, other = 0, 0
-        buf, eof = bytearray(head), False
         tm["read_s"] += time.perf_counter() - t0
         parser = lib.VcfParser(device, S, chunk_bytes)
         try:
-            while True:
-                t0 = time.perf_counter()
-                while len(buf) < chunk_bytes and not eof:
-                    piece = fh.read(chunk_bytes - len(buf))
-                    eof = not piece
-                    buf += piece
-                if eof and buf and buf[-1] not in (10, 13):
-                    buf += b"\n"
-                tm["read_s"] += time.perf_counter() - t0
-                if not buf:
-                    break
-                cut = parsers._whole_lines(buf, chunk_bytes, eof)
-                if cut == 0:
-                    raise ValueError("%s: line %d is longer than the chunk of %d bytes" % (inVCF, line_no + 1, chunk_bytes))
-                chunk = bytes(memoryview(buf)[:cut])
-                del buf[:cut]
-                t0 = time.perf_counter()
-                r = parser.parse_gt_packed(chunk)
-                tm["device_s"] += time.perf_counter() - t0
-                tm["h2d_ms"] += r["h2d_ms"]
-                tm["kernel_ms"] += r["kernel_ms"]
-                tm["h2d_bytes"] += len(chunk)
+            for chunk, r, line_no in parsers.vcf_chunks(fh, head, chunk_bytes, inVCF, line_no, parser.parse_gt_packed, tm):
                 t0 = time.perf_counter()
                 if r["non_ascii"]:
                     chunk.decode(enc)                  # the text-mode reader fails on what does not decode
@@ -294,7 +272,6 @@ def makeDB_from_vcf(inVCF, outFile, device=0, chunk_bytes=parsers.VCF_CHUNK_BYTE
                 rows.append(r["packed"])
                 other += r["other_calls"]
                 n_rec += len(lines)
-                line_no += r["n_lines"]
                 tm["host_chunk_s"] += time.perf_counter() - t0
         finally:
             parser.close()

@@ -21,6 +21,7 @@ import logging
 import os
 import re
 import sys
+import time
 
 import numpy as np
 
@@ -397,6 +398,39 @@ def _whole_lines(buf, limit, eof):
     return cut
 
 
+def vcf_chunks(fh, head, chunk_bytes, path, line_no, parse, tm):
+    """The text after the #CHROM line of the VCF fh (binary; head = the bytes the header reader read past that line) in chunks of
+    whole lines of at most chunk_bytes, a line end added after an unterminated last line; each chunk goes through parse (a
+    lib.VcfParser method).  Yields (chunk, parse(chunk), lines of the file before the chunk), line_no counting the header's.  A
+    line longer than chunk_bytes raises ValueError naming it.  Adds to tm: read_s (read and gunzip), device_s, h2d_ms,
+    kernel_ms, h2d_bytes."""
+    buf, eof = bytearray(head), False
+    while True:
+        t0 = time.perf_counter()
+        while len(buf) < chunk_bytes and not eof:
+            piece = fh.read(chunk_bytes - len(buf))
+            eof = not piece
+            buf += piece
+        if eof and buf and buf[-1] not in (10, 13):
+            buf += b"\n"
+        tm["read_s"] += time.perf_counter() - t0
+        if not buf:
+            return
+        cut = _whole_lines(buf, chunk_bytes, eof)
+        if cut == 0:
+            raise ValueError("%s: line %d is longer than the chunk of %d bytes" % (path, line_no + 1, chunk_bytes))
+        chunk = bytes(memoryview(buf)[:cut])
+        del buf[:cut]
+        t0 = time.perf_counter()
+        r = parse(chunk)
+        tm["device_s"] += time.perf_counter() - t0
+        tm["h2d_ms"] += r["h2d_ms"]
+        tm["kernel_ms"] += r["kernel_ms"]
+        tm["h2d_bytes"] += len(chunk)
+        yield chunk, r, line_no
+        line_no += r["n_lines"]
+
+
 def read_vcf_many(path, device=0, chunk_bytes=VCF_CHUNK_BYTES, timings=None):
     """Every sample column of a VCF (plain or .vcf.gz): [(sample name, ParseInputs)], where sample s's ParseInputs has the
     chrs, pos, gt, wei, dp and coded_weights() of ParseInputs on a VCF of the same header, the 9 fixed columns and column s
@@ -406,7 +440,6 @@ def read_vcf_many(path, device=0, chunk_bytes=VCF_CHUNK_BYTES, timings=None):
     dump is loaded.  A line longer than chunk_bytes, a record before the #CHROM line and a VCF without sample columns raise
     ValueError.  timings (optional dict) receives seconds and bytes of the stages and, under "fallback", the indices of the
     records the Python code parsed."""
-    import time
     from .. import lib
     enc = locale.getpreferredencoding(False)
     tm = timings if timings is not None else {}
@@ -430,34 +463,11 @@ def read_vcf_many(path, device=0, chunk_bytes=VCF_CHUNK_BYTES, timings=None):
         rec = {k: [] for k in ("cid", "pos", "dp", "nsf", "has_pl")}
         chunks, fb = [], [[] for _ in range(S)]
         n_rec = 0
-        buf, eof = bytearray(head), False
         tm["read_s"] += time.perf_counter() - t0
         parser = lib.VcfParser(device, S, chunk_bytes)
         try:
-            while True:
+            for chunk, r, _ in vcf_chunks(fh, head, chunk_bytes, path, line_no, parser.parse, tm):
                 t0 = time.perf_counter()
-                while len(buf) < chunk_bytes and not eof:
-                    piece = fh.read(chunk_bytes - len(buf))
-                    eof = not piece
-                    buf += piece
-                if eof and buf and buf[-1] not in (10, 13):
-                    buf += b"\n"
-                tm["read_s"] += time.perf_counter() - t0
-                if not buf:
-                    break
-                cut = _whole_lines(buf, chunk_bytes, eof)
-                if cut == 0:
-                    raise ValueError("%s: line %d is longer than the chunk of %d bytes" % (path, line_no + 1, chunk_bytes))
-                chunk = bytes(memoryview(buf)[:cut])
-                del buf[:cut]
-                t0 = time.perf_counter()
-                r = parser.parse(chunk)
-                tm["device_s"] += time.perf_counter() - t0
-                tm["h2d_ms"] += r["h2d_ms"]
-                tm["kernel_ms"] += r["kernel_ms"]
-                tm["h2d_bytes"] += len(chunk)
-                t0 = time.perf_counter()
-                line_no += r["n_lines"]
                 if r["non_ascii"]:
                     chunk.decode(enc)                  # the text-mode readers fail on what does not decode
                 has_info_dp |= r["info_dp_lines"] > 0
@@ -531,6 +541,106 @@ def read_vcf_many(path, device=0, chunk_bytes=VCF_CHUNK_BYTES, timings=None):
         inp._pl_codes = pl_codes
         inp.load_snp_info(*parsed)
         out.append((names[smp], inp))
+    tm["assemble_s"] += time.perf_counter() - t0
+    return out
+
+
+def _population_header(fh, path):
+    """read_vcf_header for read_vcf_gt_codes: (sample names, lines read, bytes past the #CHROM line); ValueError naming path when
+    there is no #CHROM line, a record comes before it or it names no sample column."""
+    try:
+        names, _, line_no, head = read_vcf_header(fh)
+    except ValueError as e:
+        raise ValueError("%s: %s" % (path, e))
+    if not names:
+        raise ValueError("%s has no sample columns" % path)
+    return names, line_no, head
+
+
+def vcf_population_samples(path):
+    """The sample names read_vcf_gt_codes(path) returns, or the ValueError of its header refusals; reads the header only and
+    needs no device."""
+    with _open_binary(path) as fh:
+        return _population_header(fh, path)[0]
+
+
+def read_vcf_gt_codes(path, device=0, chunk_bytes=VCF_CHUNK_BYTES, timings=None):
+    """What genotype_cross takes from a multi-sample VCF (plain or .vcf.gz), its genotype columns parsed on CUDA device `device`:
+    dict(samples str [S], chr str [n], pos int64 [n], gt_codes int8 [n, S]), equal to read_vcf_samples(path)'s samples, chr and
+    pos and to parseGT of its gt.  The host reads (and decompresses) the text after the #CHROM line in chunks of whole lines of
+    at most chunk_bytes; the device turns each chunk's records into rows of codes (lib.VcfParser.parse_gt_codes); the host decodes
+    CHROM only where it may change and converts a POS that is not 1-9 plain digits with int().  Raises ValueError naming the line
+    or value on the inputs read_vcf_samples gives no usable result for: a '#' line after the #CHROM line, a POS that int()
+    rejects; and on no #CHROM line, a record before it, no sample columns and a line longer than chunk_bytes.  timings (optional
+    dict) receives read_s, device_s, h2d_ms, kernel_ms, host_chunk_s, assemble_s (seconds, ms) and h2d_bytes."""
+    from .. import lib
+    chunk_bytes = int(chunk_bytes)
+    enc = locale.getpreferredencoding(False)
+    tm = timings if timings is not None else {}
+    for k in ("read_s", "device_s", "host_chunk_s", "assemble_s", "h2d_ms", "kernel_ms", "h2d_bytes"):
+        tm[k] = 0
+    t0 = time.perf_counter()
+    fh = _open_binary(path)
+    try:
+        names, line_no, head = _population_header(fh, path)
+        S = len(names)
+        name_id, name_list = {}, []
+
+        def chrom_id(text):
+            if text not in name_id:
+                name_id[text] = len(name_list)
+                name_list.append(text)
+            return name_id[text]
+        cids, positions, codes = [], [], []
+        tm["read_s"] += time.perf_counter() - t0
+        parser = lib.VcfParser(device, S, chunk_bytes)
+        try:
+            for chunk, r, line_no in vcf_chunks(fh, head, chunk_bytes, path, line_no, parser.parse_gt_codes, tm):
+                t0 = time.perf_counter()
+                if r["non_ascii"]:
+                    chunk.decode(enc)                  # the text-mode reader fails on what does not decode
+                flags, ls, clen = r["flags"], r["line_start"], r["chrom_len"]
+                lines = np.flatnonzero(flags & lib.VcfParser.FLAG_RECORD)
+                fl = flags[lines]
+                refuse = []                           # (line in chunk, message): the earliest wins
+                text = np.frombuffer(chunk, np.uint8)
+                first = ls[:-1]
+                hashes = np.flatnonzero((text[first] == 35) & (text[np.minimum(first + 1, len(text) - 1)] != 35))
+                if len(hashes):
+                    refuse.append((int(hashes[0]), "is a '#' line after the #CHROM line"))
+                # POS: converted on the host where the device did not read 1-9 plain digits
+                pos = r["pos"][lines].astype(np.int64)
+                for k in np.flatnonzero(fl & lib.VcfParser.FLAG_FALLBACK).tolist():
+                    L = int(lines[k])
+                    p0 = int(ls[L] + clen[L] + 1)
+                    v = chunk[p0:chunk.index(b"\t", p0)].decode(enc)
+                    try:
+                        pos[k] = int(v)
+                    except (ValueError, OverflowError):
+                        refuse.append((L, "has the POS %r, which does not read as an int64 integer" % v))
+                        break
+                if refuse:
+                    L, msg = min(refuse)
+                    raise ValueError("%s: line %d %s" % (path, line_no + L + 1, msg))
+                # CHROM: decoded where it may differ from the previous record's, carried forward elsewhere
+                new = np.flatnonzero(fl & lib.VcfParser.FLAG_NEW_CHROM)
+                ids = np.zeros(len(lines), np.int32)
+                ids[new] = [chrom_id(chunk[ls[L]:ls[L] + clen[L]].decode(enc)) for L in lines[new].tolist()]
+                src = np.zeros(len(lines), np.int64)
+                src[new] = new
+                cids.append(ids[np.maximum.accumulate(src)] if len(lines) else ids)
+                positions.append(pos)
+                codes.append(r["codes"])
+                tm["host_chunk_s"] += time.perf_counter() - t0
+        finally:
+            parser.close()
+    finally:
+        fh.close()
+    t0 = time.perf_counter()
+    cid = np.concatenate(cids) if cids else np.zeros(0, np.int32)
+    out = {"samples": np.array(names, dtype="str"), "chr": np.array(name_list, dtype="str")[cid],
+           "pos": np.concatenate(positions) if positions else np.zeros(0, np.int64),
+           "gt_codes": np.concatenate(codes) if codes else np.zeros((0, S), np.int8)}
     tm["assemble_s"] += time.perf_counter() - t0
     return out
 

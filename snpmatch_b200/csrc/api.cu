@@ -2590,10 +2590,10 @@ struct snpm_vcf {
     cudaStream_t st = nullptr;
     char *h_text = nullptr;              // pinned staging of one chunk
     DevBuf d_text, d_tile_cnt, d_tile_off, d_chunk, d_starts, d_flags, d_nsf, d_pos, d_dp, d_clen, d_samp0, d_fmt, d_ncell,
-        d_cell_off, d_cls, d_pl, d_ccnt, d_coff, d_soff, d_line, d_ocls, d_opl, d_scan, d_packed;
+        d_cell_off, d_cls, d_pl, d_ccnt, d_coff, d_soff, d_line, d_ocls, d_opl, d_scan, d_packed, d_codes;
     int64_t n_lines = 0, n_cells = 0, n_kept = 0, n_rows = 0;
     int32_t stride = 0;                  // packed words per row of snpm_vcf_parse_gt_packed (snpm_db_row_words for n_samples)
-    bool parsed = false, packed_parsed = false;
+    bool parsed = false, packed_parsed = false, codes_parsed = false;
     cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
     ~snpm_vcf() {
         for (cudaEvent_t e : ev)
@@ -2624,6 +2624,33 @@ static int vcf_read_count(cudaStream_t st, const int *d_at, int64_t &out) {
     SNPM_CUDA(cudaMemcpyAsync(&v, d_at, 4, cudaMemcpyDeviceToHost, st));
     SNPM_CUDA(cudaStreamSynchronize(st));
     out = v;
+    return SNPM_OK;
+}
+
+// every parse call: the chunk's copy up (timed by ev[0], ev[1]), d_chunk cleared, and 1. the line index into d_starts
+static int vcf_line_index(snpm_vcf *h, const char *text, int64_t n_bytes, int64_t &n_lines) {
+    SNPM_CUDA(cudaSetDevice(h->device));
+    cudaStream_t st = h->st;
+    h->parsed = h->packed_parsed = h->codes_parsed = false;
+    memcpy(h->h_text, text, size_t(n_bytes));
+    SNPM_CUDA(cudaEventRecord(h->ev[0], st));
+    SNPM_CUDA(cudaMemcpyAsync(h->d_text.p, h->h_text, size_t(n_bytes), cudaMemcpyHostToDevice, st));
+    SNPM_CUDA(cudaEventRecord(h->ev[1], st));
+    const uint8_t *t = h->d_text.as<uint8_t>();
+    const int64_t n_tiles = ceil_div64(n_bytes, VCF_TILE);
+    SNPM_TRY(h->d_tile_cnt.ensure(size_t(n_tiles) * 4));
+    SNPM_TRY(h->d_tile_off.ensure(size_t(n_tiles + 1) * 4));
+    SNPM_CUDA(cudaMemsetAsync(h->d_chunk.p, 0, 12, st));
+    k_vcf_line_count<<<unsigned(n_tiles), 256, 0, st>>>(t, n_bytes, h->d_tile_cnt.as<int>(), h->d_chunk.as<int>());
+    SNPM_KERNEL_CHECK();
+    SNPM_TRY(vcf_scan(st, h->d_tile_cnt.as<int>(), n_tiles, h->d_tile_off.as<int>(), h->d_scan));
+    SNPM_TRY(vcf_read_count(st, h->d_tile_off.as<int>() + n_tiles, n_lines));
+    SNPM_TRY(h->d_starts.ensure(size_t(n_lines + 1) * 4));
+    k_vcf_line_starts<<<unsigned(n_tiles), 256, 0, st>>>(t, n_bytes, h->d_tile_off.as<int>(), h->d_starts.as<int>(), h->d_chunk.as<int>());
+    SNPM_KERNEL_CHECK();
+    for (DevBuf *b : {&h->d_flags, &h->d_nsf, &h->d_pos, &h->d_dp, &h->d_clen, &h->d_samp0, &h->d_fmt, &h->d_ncell})
+        SNPM_TRY(b->ensure(size_t(n_lines) * 4));
+    SNPM_TRY(h->d_cell_off.ensure(size_t(n_lines + 1) * 4));
     return SNPM_OK;
 }
 
@@ -2667,32 +2694,13 @@ int snpm_vcf_parse(snpm_vcf *h, const char *text, int64_t n_bytes, int64_t *info
         return fail(SNPM_E_ARG, "snpm_vcf_parse: %lld bytes for a chunk of %lld", (long long)n_bytes, (long long)h->chunk);
     if (text[n_bytes - 1] != '\n' && text[n_bytes - 1] != '\r')
         return fail(SNPM_E_ARG, "snpm_vcf_parse: the chunk must end with a line end");
-    SNPM_CUDA(cudaSetDevice(h->device));
-    cudaStream_t st = h->st;
-    h->parsed = h->packed_parsed = false;
-    const int S = h->S;
-    memcpy(h->h_text, text, size_t(n_bytes));
-    SNPM_CUDA(cudaEventRecord(h->ev[0], st));
-    SNPM_CUDA(cudaMemcpyAsync(h->d_text.p, h->h_text, size_t(n_bytes), cudaMemcpyHostToDevice, st));
-    SNPM_CUDA(cudaEventRecord(h->ev[1], st));
-    const uint8_t *t = h->d_text.as<uint8_t>();
     // 1. line index
-    const int64_t n_tiles = ceil_div64(n_bytes, VCF_TILE);
-    SNPM_TRY(h->d_tile_cnt.ensure(size_t(n_tiles) * 4));
-    SNPM_TRY(h->d_tile_off.ensure(size_t(n_tiles + 1) * 4));
-    SNPM_CUDA(cudaMemsetAsync(h->d_chunk.p, 0, 8, st));
-    k_vcf_line_count<<<unsigned(n_tiles), 256, 0, st>>>(t, n_bytes, h->d_tile_cnt.as<int>(), h->d_chunk.as<int>());
-    SNPM_KERNEL_CHECK();
-    SNPM_TRY(vcf_scan(st, h->d_tile_cnt.as<int>(), n_tiles, h->d_tile_off.as<int>(), h->d_scan));
     int64_t n_lines = 0;
-    SNPM_TRY(vcf_read_count(st, h->d_tile_off.as<int>() + n_tiles, n_lines));
-    SNPM_TRY(h->d_starts.ensure(size_t(n_lines + 1) * 4));
-    k_vcf_line_starts<<<unsigned(n_tiles), 256, 0, st>>>(t, n_bytes, h->d_tile_off.as<int>(), h->d_starts.as<int>(), h->d_chunk.as<int>());
-    SNPM_KERNEL_CHECK();
+    SNPM_TRY(vcf_line_index(h, text, n_bytes, n_lines));
+    cudaStream_t st = h->st;
+    const int S = h->S;
+    const uint8_t *t = h->d_text.as<uint8_t>();
     // 2. fixed fields
-    for (DevBuf *b : {&h->d_flags, &h->d_nsf, &h->d_pos, &h->d_dp, &h->d_clen, &h->d_samp0, &h->d_fmt, &h->d_ncell})
-        SNPM_TRY(b->ensure(size_t(n_lines) * 4));
-    SNPM_TRY(h->d_cell_off.ensure(size_t(n_lines + 1) * 4));
     int n_sm = 148;
     cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, h->device);
     const int lgrid = grid_for(n_lines, 8, n_sm);
@@ -2784,32 +2792,13 @@ int snpm_vcf_parse_gt_packed(snpm_vcf *h, const char *text, int64_t n_bytes, int
         return fail(SNPM_E_ARG, "snpm_vcf_parse_gt_packed: n_bytes = %lld outside 1..%lld", (long long)n_bytes, (long long)h->chunk);
     if (text[n_bytes - 1] != '\n' && text[n_bytes - 1] != '\r')
         return fail(SNPM_E_ARG, "snpm_vcf_parse_gt_packed: the chunk ends in byte %d, not in a line end", int(uint8_t(text[n_bytes - 1])));
-    SNPM_CUDA(cudaSetDevice(h->device));
-    cudaStream_t st = h->st;
-    h->parsed = h->packed_parsed = false;
-    const int S = h->S;
-    memcpy(h->h_text, text, size_t(n_bytes));
-    SNPM_CUDA(cudaEventRecord(h->ev[0], st));
-    SNPM_CUDA(cudaMemcpyAsync(h->d_text.p, h->h_text, size_t(n_bytes), cudaMemcpyHostToDevice, st));
-    SNPM_CUDA(cudaEventRecord(h->ev[1], st));
-    const uint8_t *t = h->d_text.as<uint8_t>();
     // 1. line index, as snpm_vcf_parse
-    const int64_t n_tiles = ceil_div64(n_bytes, VCF_TILE);
-    SNPM_TRY(h->d_tile_cnt.ensure(size_t(n_tiles) * 4));
-    SNPM_TRY(h->d_tile_off.ensure(size_t(n_tiles + 1) * 4));
-    SNPM_CUDA(cudaMemsetAsync(h->d_chunk.p, 0, 12, st));
-    k_vcf_line_count<<<unsigned(n_tiles), 256, 0, st>>>(t, n_bytes, h->d_tile_cnt.as<int>(), h->d_chunk.as<int>());
-    SNPM_KERNEL_CHECK();
-    SNPM_TRY(vcf_scan(st, h->d_tile_cnt.as<int>(), n_tiles, h->d_tile_off.as<int>(), h->d_scan));
     int64_t n_lines = 0;
-    SNPM_TRY(vcf_read_count(st, h->d_tile_off.as<int>() + n_tiles, n_lines));
-    SNPM_TRY(h->d_starts.ensure(size_t(n_lines + 1) * 4));
-    k_vcf_line_starts<<<unsigned(n_tiles), 256, 0, st>>>(t, n_bytes, h->d_tile_off.as<int>(), h->d_starts.as<int>(), h->d_chunk.as<int>());
-    SNPM_KERNEL_CHECK();
+    SNPM_TRY(vcf_line_index(h, text, n_bytes, n_lines));
+    cudaStream_t st = h->st;
+    const int S = h->S;
+    const uint8_t *t = h->d_text.as<uint8_t>();
     // 2'. fixed fields with makedb's rules; ncell = 1 marks a record that gets a row
-    for (DevBuf *b : {&h->d_flags, &h->d_nsf, &h->d_pos, &h->d_dp, &h->d_clen, &h->d_samp0, &h->d_fmt, &h->d_ncell})
-        SNPM_TRY(b->ensure(size_t(n_lines) * 4));
-    SNPM_TRY(h->d_cell_off.ensure(size_t(n_lines + 1) * 4));
     int n_sm = 148;
     cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, h->device);
     const int lgrid = grid_for(n_lines, 8, n_sm);
@@ -2864,6 +2853,78 @@ int snpm_vcf_fetch_gt_packed(snpm_vcf *h, int32_t *line_start, int32_t *flags, i
     if (nl)
         for (const auto &c : per_line) SNPM_CUDA(cudaMemcpyAsync(c.first, c.second->p, nl * 4, cudaMemcpyDeviceToHost, st));
     if (nw) SNPM_CUDA(cudaMemcpyAsync(packed, h->d_packed.p, nw * 8, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaStreamSynchronize(st));
+    return SNPM_OK;
+}
+
+int snpm_vcf_parse_gt_codes(snpm_vcf *h, const char *text, int64_t n_bytes, int64_t *info, float *ms) {
+    if (!h) return fail(SNPM_E_ARG, "snpm_vcf_parse_gt_codes: h is NULL");
+    if (!text) return fail(SNPM_E_ARG, "snpm_vcf_parse_gt_codes: text is NULL");
+    if (!info) return fail(SNPM_E_ARG, "snpm_vcf_parse_gt_codes: info is NULL");
+    if (n_bytes < 1 || n_bytes > h->chunk)
+        return fail(SNPM_E_ARG, "snpm_vcf_parse_gt_codes: n_bytes = %lld outside 1..%lld", (long long)n_bytes, (long long)h->chunk);
+    if (text[n_bytes - 1] != '\n' && text[n_bytes - 1] != '\r')
+        return fail(SNPM_E_ARG, "snpm_vcf_parse_gt_codes: the chunk ends in byte %d, not in a line end", int(uint8_t(text[n_bytes - 1])));
+    // 1. line index, as snpm_vcf_parse
+    int64_t n_lines = 0;
+    SNPM_TRY(vcf_line_index(h, text, n_bytes, n_lines));
+    cudaStream_t st = h->st;
+    const int S = h->S;
+    const uint8_t *t = h->d_text.as<uint8_t>();
+    // 2''. fixed fields with makedb's rules; every record gets a row
+    int n_sm = 148;
+    cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, h->device);
+    const int lgrid = grid_for(n_lines, 8, n_sm);
+    const VcfLines o = h->lines();
+    if (n_lines) {
+        k_vcf_records_all<<<lgrid, 256, 0, st>>>(t, h->d_starts.as<int>(), int(n_lines), o);
+        SNPM_KERNEL_CHECK();
+    }
+    // 3''. rows
+    SNPM_TRY(vcf_scan(st, o.ncell, n_lines, h->d_cell_off.as<int>(), h->d_scan));
+    int64_t n_rows = 0;
+    SNPM_TRY(vcf_read_count(st, h->d_cell_off.as<int>() + n_lines, n_rows));
+    // 4''. codes, S bytes per record
+    SNPM_TRY(h->d_codes.ensure(size_t(n_rows) * size_t(S)));
+    if (n_rows) {
+        k_vcf_gt_codes<<<lgrid, 256, 0, st>>>(t, h->d_starts.as<int>(), int(n_lines), o, h->d_cell_off.as<int>(), S,
+                                              h->d_codes.as<int8_t>());
+        SNPM_KERNEL_CHECK();
+    }
+    SNPM_CUDA(cudaEventRecord(h->ev[2], st));
+    int cf = 0;
+    SNPM_CUDA(cudaMemcpyAsync(&cf, h->d_chunk.p, 4, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaStreamSynchronize(st));
+    h->n_lines = n_lines;
+    h->n_rows = n_rows;
+    h->codes_parsed = true;
+    info[0] = n_lines;
+    info[1] = n_rows;
+    info[2] = cf;
+    if (ms) {
+        ms[0] = ms[1] = 0.f;
+        cudaEventElapsedTime(&ms[0], h->ev[0], h->ev[1]);
+        cudaEventElapsedTime(&ms[1], h->ev[1], h->ev[2]);
+    }
+    return SNPM_OK;
+}
+
+int snpm_vcf_fetch_gt_codes(snpm_vcf *h, int32_t *line_start, int32_t *flags, int32_t *nsf, int32_t *pos, int32_t *chrom_len,
+                            int8_t *codes) {
+    if (!h) return fail(SNPM_E_ARG, "snpm_vcf_fetch_gt_codes: h is NULL");
+    const std::pair<const void *, const char *> args[] = {{line_start, "line_start"}, {flags, "flags"}, {nsf, "nsf"}, {pos, "pos"},
+                                                          {chrom_len, "chrom_len"}, {codes, "codes"}};
+    for (const auto &a : args)
+        if (!a.first) return fail(SNPM_E_ARG, "snpm_vcf_fetch_gt_codes: %s is NULL", a.second);
+    if (!h->codes_parsed) return fail(SNPM_E_STATE, "snpm_vcf_fetch_gt_codes: no chunk parsed by snpm_vcf_parse_gt_codes");
+    SNPM_CUDA(cudaSetDevice(h->device));
+    cudaStream_t st = h->st;
+    const size_t nl = size_t(h->n_lines), nc = size_t(h->n_rows) * size_t(h->S);
+    SNPM_CUDA(cudaMemcpyAsync(line_start, h->d_starts.p, (nl + 1) * 4, cudaMemcpyDeviceToHost, st));
+    const std::pair<void *, const DevBuf *> per_line[] = {{flags, &h->d_flags}, {nsf, &h->d_nsf}, {pos, &h->d_pos}, {chrom_len, &h->d_clen}};
+    if (nl)
+        for (const auto &c : per_line) SNPM_CUDA(cudaMemcpyAsync(c.first, c.second->p, nl * 4, cudaMemcpyDeviceToHost, st));
+    if (nc) SNPM_CUDA(cudaMemcpyAsync(codes, h->d_codes.p, nc, cudaMemcpyDeviceToHost, st));
     SNPM_CUDA(cudaStreamSynchronize(st));
     return SNPM_OK;
 }

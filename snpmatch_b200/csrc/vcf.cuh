@@ -21,6 +21,13 @@
 //   4'. k_vcf_gt_packed, one warp per record: lane j classifies cell 32 w + j by the exact GT text of vcf_to_csv's _GT_CODE and
 //       two ballots write packed word w in k_pack_int8's layout (padding lanes and words missing); calls that are no _GT_CODE
 //       string are counted with one atomic per warp.  No per-cell array exists.
+//
+// `genotype_cross --gpu_parse` (snpm_vcf_parse_gt_codes) reuses the line index and 2' with a row for every record:
+//   2''. k_vcf_records_all: k_vcf_records<true>'s fields, ncell = 1 for every record whatever its number of sample fields;
+//   3''. scan of the records: each one's row of the chunk's [rows, n_samples] int8 codes;
+//   4''. k_vcf_gt_codes, one warp per record: lane j writes the code read_vcf_samples + parseGT give cell 32 w + j (1 for 1/1, 2
+//        for 0/1 and 1/0, -1 for ./., a missing GT and a cell past the record's sample fields, 0 otherwise).  The rule is total:
+//        no cell falls back to the host.
 #pragma once
 #include "common.cuh"
 
@@ -212,10 +219,11 @@ struct VcfLines {
 };
 
 // MAKEDB: vcf_to_csv's rules (first GT of FORMAT, only POS flags a record, ncell = 1 for a record of exactly n_samples sample
-// fields: the rows of the packed panel); otherwise read_vcf_minimal's (see the top of the file)
-template <bool MAKEDB>
-__global__ void __launch_bounds__(256) k_vcf_records(const uint8_t *__restrict__ t, const int *__restrict__ starts, int n_lines,
-                                                     int n_samples, VcfLines o) {
+// fields: the rows of the packed panel); otherwise read_vcf_minimal's (see the top of the file).  ALL_ROWS (with MAKEDB): ncell = 1
+// for every record, whatever its number of sample fields (the rows of k_vcf_gt_codes).
+template <bool MAKEDB, bool ALL_ROWS>
+__device__ __forceinline__ void vcf_records(const uint8_t *__restrict__ t, const int *__restrict__ starts, int n_lines, int n_samples,
+                                            VcfLines o) {
     const int lane = threadIdx.x & 31;
     const int n_warps = int(gridDim.x) * (blockDim.x >> 5);
     for (int L = int(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5); L < n_lines; L += n_warps) {
@@ -306,12 +314,26 @@ __global__ void __launch_bounds__(256) k_vcf_records(const uint8_t *__restrict__
             o.chrom_len[L] = clen;
             o.samp0[L] = samp0;
             o.fmt[L] = fmt;
-            if constexpr (MAKEDB)
+            if constexpr (ALL_ROWS)
+                o.ncell[L] = flags & VCF_REC;
+            else if constexpr (MAKEDB)
                 o.ncell[L] = (flags & VCF_REC) && nsf == n_samples;
             else
                 o.ncell[L] = (flags & (VCF_REC | VCF_FALLBACK)) == VCF_REC ? min(nsf, n_samples) : 0;
         }
     }
+}
+
+template <bool MAKEDB>
+__global__ void __launch_bounds__(256) k_vcf_records(const uint8_t *__restrict__ t, const int *__restrict__ starts, int n_lines,
+                                                     int n_samples, VcfLines o) {
+    vcf_records<MAKEDB, false>(t, starts, n_lines, n_samples, o);
+}
+
+// makedb's rules, a row for every record
+__global__ void __launch_bounds__(256) k_vcf_records_all(const uint8_t *__restrict__ t, const int *__restrict__ starts, int n_lines,
+                                                         VcfLines o) {
+    vcf_records<true, true>(t, starts, n_lines, 0, o);
 }
 
 // ---- 3. cells, one warp per record, lanes over its cells --------------------------------------------------------------------
@@ -562,6 +584,85 @@ __global__ void __launch_bounds__(256) k_vcf_gt_packed(const uint8_t *__restrict
         if (lane == 0 && !same) atomicOr(o.flags + L, VCF_NEW_CHROM);
     }
     if (lane == 0 && other) atomicAdd(chunk_flags + 2, other);
+}
+
+// ---- genotype_cross: records -> rows of int8 window-call codes ---------------------------------------------------------------
+// class of the GT token [a, b): 0 '.' or empty, 1 "0", 2 "1", 3 anything else
+__device__ __forceinline__ int vcf_token_class(const uint8_t *__restrict__ t, int a, int b) {
+    if (b == a) return 0;
+    if (b - a > 1) return 3;
+    return t[a] == '.' ? 0 : t[a] == '0' ? 1 : t[a] == '1' ? 2 : 3;
+}
+
+// The code read_vcf_samples + parseGT give the cell [a, b) whose GT is subfield gi (0-based, -1 absent): the GT text split at '/'
+// and '|', the first two tokens kept, a missing or empty one read as '.'; 1 for (1,1), 2 for (0,1) and (1,0), -1 for (.,.), 0 for
+// any other pair; -1 for a cell without that subfield.
+__device__ __forceinline__ int8_t vcf_cross_code(const uint8_t *__restrict__ t, int a, int b, int gi) {
+    if (gi < 0) return -1;
+    int k = 0, g0 = a;
+    for (int p = a; p < b && k < gi; ++p)
+        if (t[p] == ':') { ++k; g0 = p + 1; }
+    if (k < gi) return -1;
+    int c[2] = {0, 0}, n = 0;
+    for (int p = g0, st = g0; n < 2; ++p) {
+        const bool end = p >= b || t[p] == ':';
+        if (!end && t[p] != '/' && t[p] != '|') continue;
+        c[n++] = vcf_token_class(t, st, p);
+        st = p + 1;
+        if (end) break;
+    }
+    if (c[0] == 2 && c[1] == 2) return 1;
+    if (c[0] + c[1] == 3 && c[0] != 3 && c[1] != 3) return 2;
+    return c[0] == 0 && c[1] == 0 ? -1 : 0;
+}
+
+// One warp per record (ncell == 1): row row_off[L] of codes [rows, n_samples], lane j writing the code of cell 32 w + j, so a
+// warp stores 32 consecutive bytes per step; the cells walked as in k_vcf_cells, VCF_NEW_CHROM as there.  Cells past
+// min(nsf, n_samples), and every cell of a record without GT in FORMAT, are -1.
+__global__ void __launch_bounds__(256) k_vcf_gt_codes(const uint8_t *__restrict__ t, const int *__restrict__ starts, int n_lines,
+                                                      VcfLines o, const int *__restrict__ row_off, int n_samples,
+                                                      int8_t *__restrict__ codes) {
+    const int lane = threadIdx.x & 31;
+    const int n_warps = int(gridDim.x) * (blockDim.x >> 5);
+    for (int L = int(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5); L < n_lines; L += n_warps) {
+        if (!o.ncell[L]) continue;
+        const int s = starts[L];
+        const int clen = o.chrom_len[L];
+        bool same = L > 0 && (o.flags[L - 1] & VCF_REC) && o.chrom_len[L - 1] == clen;
+        if (same) {
+            const int ps = starts[L - 1];
+            for (int b0 = 0; b0 < clen && same; b0 += 32) {
+                const int i = b0 + lane;
+                same = __all_sync(0xffffffffu, i >= clen || t[ps + i] == t[s + i]);
+            }
+        }
+        int8_t *row = codes + int64_t(row_off[L]) * n_samples;
+        const int gi = o.fmt[L] - 1;
+        const int nc = gi >= 0 ? min(o.nsf[L], n_samples) : 0;    // without GT every call is missing: nothing to read
+        const int e = vcf_line_end(t, s, starts[L + 1]);
+        int cell = 0, cur = o.samp0[L], my_a = 0, my_b = 0;
+        for (int base = cur; base < e && cell < nc; base += 32) {
+            const int p = base + lane;
+            unsigned m = __ballot_sync(0xffffffffu, p < e && t[p] == '\t');
+            while (m && cell < nc) {
+                const int tp = base + __ffs(m) - 1;
+                m &= m - 1;
+                if (lane == (cell & 31)) { my_a = cur; my_b = tp; }
+                cur = tp + 1;
+                if ((++cell & 31) == 0) row[cell - 32 + lane] = vcf_cross_code(t, my_a, my_b, gi);
+            }
+        }
+        bool closed_by_end = false;
+        if (cell < nc) {                                   // the line end closes the last sample field
+            if (lane == (cell & 31)) { my_a = cur; my_b = e; }
+            ++cell;
+            closed_by_end = true;
+        }
+        const int pending = (cell & 31) ? (cell & 31) : (closed_by_end ? 32 : 0);
+        if (lane < pending) row[cell - pending + lane] = vcf_cross_code(t, my_a, my_b, gi);
+        for (int k = cell + lane; k < n_samples; k += 32) row[k] = -1;
+        if (lane == 0 && !same) atomicOr(o.flags + L, VCF_NEW_CHROM);
+    }
 }
 
 }  // namespace snpm

@@ -275,6 +275,8 @@ SIGNATURES = {
     "snpm_vcf_fetch": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
     "snpm_vcf_parse_gt_packed": (C.c_int, [_p, C.c_char_p, _i64, _p, _p]),
     "snpm_vcf_fetch_gt_packed": (C.c_int, [_p, _p, _p, _p, _p, _p, _p]),
+    "snpm_vcf_parse_gt_codes": (C.c_int, [_p, C.c_char_p, _i64, _p, _p]),
+    "snpm_vcf_fetch_gt_codes": (C.c_int, [_p, _p, _p, _p, _p, _p, _p]),
     "snpm_vcf_destroy": (None, [_p]),
 }
 
@@ -539,7 +541,8 @@ class VcfParser(object):
     """The genotype columns of a multi-sample VCF parsed on the device (snpm_vcf_*), one chunk of whole lines at a time.
     parse(text) returns the chunk's per-line arrays and every sample's called cells (see snpm_vcf_fetch); core.parsers.read_vcf_many
     turns them into one ParseInputs per sample.  parse_gt_packed(text) returns the chunk's records as rows of the packed panel
-    (snpm_vcf_fetch_gt_packed), which core.makedb.makeDB_from_vcf assembles."""
+    (snpm_vcf_fetch_gt_packed), which core.makedb.makeDB_from_vcf assembles.  parse_gt_codes(text) returns them as rows of int8
+    window-call codes (snpm_vcf_fetch_gt_codes), which core.parsers.read_vcf_gt_codes assembles."""
 
     FLAG_RECORD, FLAG_FALLBACK, FLAG_HAS_PL, FLAG_NEW_CHROM = 1, 2, 4, 8
     N_ALLELE_CODES = 111
@@ -580,6 +583,22 @@ class VcfParser(object):
             r[key] = np.empty(n, np.int32)
         check(load().snpm_vcf_fetch_gt_packed(self._h, *[ptr(r[key]) for key in ("line_start", "flags", "nsf", "pos", "chrom_len",
                                                                                  "packed")]))
+        return r
+
+    def parse_gt_codes(self, text):
+        """`genotype_cross --gpu_parse`: text as for parse(), every record read into a row of the codes parseGT gives the GT
+        strings of read_vcf_samples (snpm_vcf_parse_gt_codes).  Returns dict(n_lines, n_rows, non_ascii, h2d_ms, kernel_ms, and
+        the arrays line_start, flags, nsf, pos, chrom_len and codes int8 [n_rows, n_samples]: one row per record, in line order)."""
+        info = np.zeros(3, np.int64)
+        ms = (C.c_float * 2)()
+        check(load().snpm_vcf_parse_gt_codes(self._h, text, len(text), ptr(info), ms))
+        n, rows = int(info[0]), int(info[1])
+        r = dict(n_lines=n, n_rows=rows, non_ascii=bool(info[2]), h2d_ms=ms[0], kernel_ms=ms[1],
+                 line_start=np.empty(n + 1, np.int32), codes=np.empty((rows, self.n_samples), np.int8))
+        for key in ("flags", "nsf", "pos", "chrom_len"):
+            r[key] = np.empty(n, np.int32)
+        check(load().snpm_vcf_fetch_gt_codes(self._h, *[ptr(r[key]) for key in ("line_start", "flags", "nsf", "pos", "chrom_len",
+                                                                                "codes")]))
         return r
 
     @property

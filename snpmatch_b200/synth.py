@@ -250,13 +250,15 @@ def pl_table(max_pl):
 
 
 # ---- multi-sample VCF text (tests and measurement of parsers.read_vcf_many) -----------------------------------------------
-def multi_sample_vcf(n_records, n_samples, seed=7, line_end="\n", info_dp_header=True, late_info_dp=False, edge_cases=True):
+def multi_sample_vcf(n_records, n_samples, seed=7, line_end="\n", info_dp_header=True, late_info_dp=False, edge_cases=True,
+                     hash_lines=True):
     """Seeded text of a VCF with n_samples sample columns.  With edge_cases, the records mix every GT form read_vcf_minimal
     renders (phased, single alleles, '.', empty, multi-digit, more than two alleles, GT missing from FORMAT or from the cell,
     PL before GT), PL forms (missing key, '.', fewer or more than three values, 3.5, 1e2), INFO DP forms (present, absent,
     DP=x, DP=1_0, ADP=, an empty DP= before a real one), cells with fewer subfields than FORMAT, records with fewer sample
     columns than the header (one with exactly 32), '##' and '#' lines, blank and short lines among the records and a non-ASCII chromosome name.
-    late_info_dp puts a '##INFO=<ID=DP,' line among the records.  line_end may also be a list of line ends to cycle through.  Returns (text, fallback): fallback = the 0-based indices of
+    late_info_dp puts a '##INFO=<ID=DP,' line among the records; without hash_lines its '#' lines among the records become '##'
+    lines (the same text otherwise).  line_end may also be a list of line ends to cycle through.  Returns (text, fallback): fallback = the 0-based indices of
     the records the device parser cannot reproduce (lib.VcfParser.FLAG_FALLBACK), i.e. the ones it hands to the Python code."""
     rng = np.random.default_rng(seed)
     ends = line_end if isinstance(line_end, (list, tuple)) else [line_end]
@@ -273,7 +275,8 @@ def multi_sample_vcf(n_records, n_samples, seed=7, line_end="\n", info_dp_header
         if late_info_dp and r == n_records // 2:
             lines.append('##INFO=<ID=DP,Number=1,Type=Integer,Description="depth">')
         if edge_cases and rng.random() < 0.03:
-            lines.append(["##INFO=<ID=XX,Number=1>", "#comment", "", "Chr1\t5\t.\tA\tT", "##contig=<ID=Chr1>"][rng.integers(0, 5)])
+            extra = ["##INFO=<ID=XX,Number=1>", "#comment", "", "Chr1\t5\t.\tA\tT", "##contig=<ID=Chr1>"][rng.integers(0, 5)]
+            lines.append(extra if hash_lines or extra != "#comment" else "#" + extra)
         chrom = chroms[min(r * len(chroms) // max(n_records, 1), len(chroms) - 1)]
         if edge_cases and r % 97 == 13:
             chrom, fb = "Chrü", True
@@ -366,3 +369,28 @@ def panel_vcf(fh, n_rows, n_acc, seed=SEED_PANEL, block=4096):
         fh.write(b"".join(b"%s\t%d\t.\tA\tT\t.\tPASS\t.\tGT\t" % (TAIR10_CHRS[c].encode(), p) + line.tobytes()
                           for c, p, line in zip(chrom[rows].tolist(), positions[rows].tolist(), cells)))
     return positions, regions
+
+
+POPULATION_GT = ["0/0", "1/1", "0/1", "1/0", "./.", "0|1", "1|1", ".", "0", "1/.", "./1", "2/2", "1/1/0", "", "1|", "10/1", "A/1"]
+
+
+def population_vcf(fh, chrs, positions, n_samples, seed=11, edge_forms=True, block=4096):
+    """A seeded population VCF for `genotype_cross`, written to the binary file fh: record r at chrs[r], positions[r], FORMAT GT
+    or GT:DP, n_samples columns whose GT is drawn from POPULATION_GT (edge_forms) or from 0/0, 1/1, 0/1, ./. alone."""
+    rng = np.random.default_rng(seed)
+    forms = POPULATION_GT if edge_forms else POPULATION_GT[:3] + POPULATION_GT[4:5]
+    fh.write(b"##fileformat=VCFv4.2\n")
+    fh.write(b"#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\t" + "\t".join("p%d" % i for i in range(n_samples)).encode() + b"\n")
+    gts = np.array([g.encode() for g in forms], dtype=object)
+    for r0 in range(0, len(positions), block):
+        rows = range(r0, min(r0 + block, len(positions)))
+        pick = rng.integers(0, len(forms), size=(len(rows), n_samples))
+        dp = rng.random(len(rows)) < 0.3
+        out = []
+        for k, r in enumerate(rows):
+            cells = gts[pick[k]]
+            if dp[k]:
+                out.append(b"%s\t%d\t.\tA\tT\t.\tPASS\t.\tGT:DP\t" % (str(chrs[r]).encode(), positions[r]) + b"\t".join(c + b":5" for c in cells))
+            else:
+                out.append(b"%s\t%d\t.\tA\tT\t.\tPASS\t.\tGT\t" % (str(chrs[r]).encode(), positions[r]) + b"\t".join(cells))
+        fh.write(b"\n".join(out) + b"\n")
