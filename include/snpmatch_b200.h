@@ -480,6 +480,35 @@ int snpm_vcf_fetch_gt_codes(snpm_vcf *h, int32_t *line_start, int32_t *flags, in
                             int8_t *codes);
 void snpm_vcf_destroy(snpm_vcf *h);
 
+/* ---- BGZF-compressed VCFs inflated on the device (the `.vcf.gz` input of the device VCF readers) --------------------------
+ * No reference symbol: the reference reads `.vcf.gz` through scikit-allel and zlib on the host.  BGZF (bgzip, `bcftools -Oz`)
+ * is a series of independent gzip members, each with FLG = FEXTRA, a `BC` extra subfield holding its size - 1, and at most
+ * 65536 bytes of text (ISIZE); the file may end with the empty 28-byte EOF member.
+ * snpm_bgzf_scan (host only, no device): walks the member headers of data[0..n_bytes).  *n_members = the number of members
+ * when the file is all BGZF -- every member has ID1 ID2 = 1f 8b, CM 8, FLG exactly 4, an extra field with a BC subfield and
+ * ISIZE <= 65536, and the members tile the data to its last byte -- or -1 otherwise (no member at all counts as not BGZF).
+ * The first min(n, cap) members' byte offsets go to member_off (and member_off[n] = n_bytes when n <= cap; cap + 1 entries)
+ * and their ISIZE to isize (cap entries).  Call again with cap >= n when n > cap.
+ * snpm_bgzf_create: a handle with pinned staging for up to max_in_bytes of members and max_out_bytes of text per call
+ * (each at most SNPM_BGZF_MAX_BYTES) and the device buffers.
+ * snpm_bgzf_inflate: members i = comp[member_off[i] .. member_off[i+1]) for i < n (member_off int64 [n+1], offsets into comp;
+ * comp_bytes <= max_in_bytes; each must have a BGZF header with FLG 4 and ISIZE <= 65536, and their ISIZEs must sum to at most
+ * max_out_bytes: SNPM_E_ARG otherwise) go up in one copy; k_bgzf_inflate decodes each member's DEFLATE stream with one warp
+ * into its place (the exclusive sum of the ISIZEs) and checks its length and CRC-32 against the trailer; the text comes back in
+ * one copy.  info int64[3] = bytes of text, the index of the first refused member or -1, and its reason (1 invalid DEFLATE
+ * stream, 2 length other than ISIZE, 3 CRC-32 mismatch).  The text goes to out (info[0] bytes) unless out is NULL; either way
+ * it stays in the pinned staging that snpm_bgzf_text returns until the next call.  Nothing is copied back when a member is
+ * refused.  ms (optional) float[3] = device time of the copy up, of the kernel alone, of the copy down of the text (the
+ * per-member status copy in between is in none of the three). */
+#define SNPM_BGZF_MAX_BYTES (int64_t(1) << 31)
+typedef struct snpm_bgzf snpm_bgzf;
+int snpm_bgzf_scan(const uint8_t *data, int64_t n_bytes, int64_t *member_off, int32_t *isize, int64_t cap, int64_t *n_members);
+int snpm_bgzf_create(int device, int64_t max_in_bytes, int64_t max_out_bytes, snpm_bgzf **out);
+int snpm_bgzf_inflate(snpm_bgzf *h, const uint8_t *comp, int64_t comp_bytes, const int64_t *member_off, int64_t n, uint8_t *out,
+                      int64_t *info, float *ms);
+const uint8_t *snpm_bgzf_text(snpm_bgzf *h);
+void snpm_bgzf_destroy(snpm_bgzf *h);
+
 #ifdef __cplusplus
 }
 #endif

@@ -179,7 +179,8 @@ def makeDB_from_vcf(inVCF, outFile, device=0, chunk_bytes=parsers.VCF_CHUNK_BYTE
     CHROM or sample name holding ',' or '"', a non-ASCII sample name, no sample columns, no #CHROM line or a record before it;
     so does a line longer than chunk_bytes.  timings (optional dict) receives seconds of the stages (read_s: read and gunzip,
     device_s with h2d_ms / kernel_ms, host_chunk_s, assemble_s, write_s), h2d_bytes, and under "flagged" the indices of the
-    records whose POS text the host converted.  Returns the open Genotype."""
+    records whose POS text the host converted; a BGZF .vcf.gz is inflated on the device (parsers.BgzfReader) and the route
+    goes to timings as parsers._inflate_timings records it.  Returns the open Genotype."""
     import time
     from .. import lib
     chunk_bytes = int(chunk_bytes)
@@ -189,7 +190,7 @@ def makeDB_from_vcf(inVCF, outFile, device=0, chunk_bytes=parsers.VCF_CHUNK_BYTE
         tm[k] = 0
     tm["flagged"] = []
     t0 = time.perf_counter()
-    fh = parsers._open_binary(inVCF)
+    fh = parsers._open_binary(inVCF, device)
     try:
         meta = []
         try:
@@ -276,6 +277,7 @@ def makeDB_from_vcf(inVCF, outFile, device=0, chunk_bytes=parsers.VCF_CHUNK_BYTE
         finally:
             parser.close()
     finally:
+        parsers._inflate_timings(fh, tm)
         fh.close()
     t0 = time.perf_counter()
     ids = np.concatenate(ids) if ids else np.zeros(0, np.int32)

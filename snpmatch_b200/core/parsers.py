@@ -18,6 +18,7 @@ import gzip
 import json
 import locale
 import logging
+import mmap
 import os
 import re
 import sys
@@ -344,8 +345,128 @@ VCF_GT_LEN = np.array([len(t) for t in VCF_GT_TEXT.tolist()])
 _LINE_END = re.compile(rb"\r\n|\r|\n")
 
 
-def _open_binary(path):
-    return gzip.open(path, "rb") if str(path).endswith(".gz") else open(path, "rb")
+# text per device call of BgzfReader, chosen end to end: makeDB_from_vcf of 4.57 GB of text (NVIDIA B200, three alternating runs
+# of each size; DESIGN.md section 6) took 5.5-6.4 s at 64 MB, 7.0-8.4 s at 256 MB and 5.7-6.6 s at 512 MB.  The kernel alone
+# favours larger batches (111 / 42 / 35 ms: 1000 members do not fill the GPU); the host's reading of the text out of the pinned
+# buffer favours smaller ones (read_s 2.7-3.0 / 4.0-4.8 / 3.2-3.8 s)
+BGZF_BATCH_BYTES = 64 << 20
+
+
+class BgzfReader(object):
+    """A BGZF file read as its text, its members inflated on CUDA device `device` (lib.BgzfInflater), in batches of consecutive
+    members of at most batch_bytes of text and batch_bytes // 4 compressed bytes whatever the caller's n.  read(n) returns at
+    most n bytes of the current batch (b"" only at the end of the text).  A refused member raises gzip.BadGzipFile naming the
+    path, its byte offset and the reason.  Counters: comp_bytes (compressed bytes inflated), inflate_s (wall time of the device
+    calls, copies of the compressed bytes into pinned staging included) and ms (device ms of the copies up, the kernel and the
+    copies down).  Made by BgzfReader.open."""
+
+    def __init__(self, path, mm, member_off, isize, device, batch_bytes):
+        from .. import lib
+        self.path, self._mm, self._data = path, mm, np.frombuffer(mm, np.uint8)
+        self._off = member_off
+        text_end = np.concatenate([[0], np.cumsum(isize)])
+        in_cap = max(batch_bytes // 4, 1 << 17)
+        self._bounds, i, n = [], 0, len(isize)
+        while i < n:
+            j = min(int(np.searchsorted(text_end, text_end[i] + batch_bytes, "right")),
+                    int(np.searchsorted(member_off, member_off[i] + in_cap, "right"))) - 1
+            j = max(j, i + 1)
+            self._bounds.append((i, j))
+            i = j
+        max_out = max(int(max(text_end[j] - text_end[i] for i, j in self._bounds)), 1)
+        max_in = max(int(max(member_off[j] - member_off[i] for i, j in self._bounds)), 1)
+        self._inf = lib.BgzfInflater(device, max_in, max_out)
+        self._batch, self._at, self._end = 0, 0, 0
+        self.comp_bytes, self.inflate_s = 0, 0.0
+
+    @classmethod
+    def open(cls, path, device, batch_bytes=None):
+        """A reader of path when it is all BGZF (lib.bgzf_scan), else None; batch_bytes defaults to BGZF_BATCH_BYTES."""
+        from .. import lib
+        with open(path, "rb") as f:
+            if os.fstat(f.fileno()).st_size == 0:
+                return None
+            mm = mmap.mmap(f.fileno(), 0, access=mmap.ACCESS_READ)
+        table = lib.bgzf_scan(np.frombuffer(mm, np.uint8))
+        if table is None:
+            mm.close()
+            return None
+        return cls(path, mm, table[0], table[1], device, batch_bytes or BGZF_BATCH_BYTES)
+
+    @property
+    def ms(self):
+        return self._inf.ms
+
+    def _next(self):
+        while self._batch < len(self._bounds):
+            i, j = self._bounds[self._batch]
+            self._batch += 1
+            a = int(self._off[i])
+            t0 = time.perf_counter()
+            self._end = self._inf.inflate(self._data[a:int(self._off[j])], self._off[i:j + 1] - a, path=self.path, base=a)
+            self.inflate_s += time.perf_counter() - t0
+            self.comp_bytes += int(self._off[j]) - a
+            self._at = 0
+            if self._end:
+                return True
+        return False
+
+    def read(self, n=-1):
+        if n is None or n < 0:
+            parts = []
+            while self._at < self._end or self._next():
+                parts.append(self.read(self._end - self._at))
+            return b"".join(parts)
+        if n == 0 or (self._at == self._end and not self._next()):
+            return b""
+        k = min(n, self._end - self._at)
+        out = self._inf.text(self._at, self._at + k)
+        self._at += k
+        return out
+
+    def readable(self):
+        return True
+
+    def close(self):
+        if self._mm is not None:
+            self._inf.close()
+            self._data = None
+            try:
+                self._mm.close()
+            except BufferError:               # a traceback still holds a view of the mapping: it is unmapped when that goes
+                pass
+            self._mm = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+def _open_binary(path, device=None):
+    """path opened for binary reading of its text: a BgzfReader inflating on CUDA device `device` when device is given, the
+    name ends in .gz and the file is all BGZF; gzip.open for any other .gz; open otherwise."""
+    if not str(path).endswith(".gz"):
+        return open(path, "rb")
+    if device is not None:
+        reader = BgzfReader.open(path, device)
+        if reader is not None:
+            return reader
+    return gzip.open(path, "rb")
+
+
+def _inflate_timings(fh, tm):
+    """The decompression route of fh into tm: inflate = "device" (BgzfReader), "host" (gzip) or None (plain text); for .gz,
+    gz_bytes = compressed bytes read; for the device route, inflate_s (wall time of the device calls, inside read_s) and the
+    device times inflate_h2d_ms, inflate_ms (k_bgzf_inflate) and d2h_ms."""
+    if isinstance(fh, BgzfReader):
+        tm.update(inflate="device", gz_bytes=fh.comp_bytes, inflate_s=fh.inflate_s, inflate_h2d_ms=float(fh.ms[0]),
+                  inflate_ms=float(fh.ms[1]), d2h_ms=float(fh.ms[2]))
+    elif isinstance(fh, gzip.GzipFile):
+        tm.update(inflate="host", gz_bytes=fh.fileobj.tell() if fh.fileobj is not None else 0)
+    else:
+        tm["inflate"] = None
 
 
 def read_vcf_header(fh, block=1 << 20, meta_lines=None):
@@ -438,8 +559,9 @@ def read_vcf_many(path, device=0, chunk_bytes=VCF_CHUNK_BYTES, timings=None):
     the #CHROM line in chunks of whole lines of at most chunk_bytes; the genotype columns are parsed on CUDA device `device`
     (lib.VcfParser); records the device flags are re-parsed with vcf_record.  Nothing is written next to the VCF and no parser
     dump is loaded.  A line longer than chunk_bytes, a record before the #CHROM line and a VCF without sample columns raise
-    ValueError.  timings (optional dict) receives seconds and bytes of the stages and, under "fallback", the indices of the
-    records the Python code parsed."""
+    ValueError.  A BGZF .vcf.gz is inflated on the same device (BgzfReader).  timings (optional dict) receives seconds and
+    bytes of the stages, the decompression route (_inflate_timings) and, under "fallback", the indices of the records the
+    Python code parsed."""
     from .. import lib
     enc = locale.getpreferredencoding(False)
     tm = timings if timings is not None else {}
@@ -447,7 +569,7 @@ def read_vcf_many(path, device=0, chunk_bytes=VCF_CHUNK_BYTES, timings=None):
         tm[k] = 0
     tm["fallback"] = []
     t0 = time.perf_counter()
-    fh = _open_binary(path)
+    fh = _open_binary(path, device)
     try:
         names, has_info_dp, line_no, head = read_vcf_header(fh)
         if not names:
@@ -502,6 +624,7 @@ def read_vcf_many(path, device=0, chunk_bytes=VCF_CHUNK_BYTES, timings=None):
         finally:
             parser.close()
     finally:
+        _inflate_timings(fh, tm)
         fh.close()
     t0 = time.perf_counter()
     rec = {k: (np.concatenate(v) if v else np.zeros(0)) for k, v in rec.items()}
@@ -572,7 +695,8 @@ def read_vcf_gt_codes(path, device=0, chunk_bytes=VCF_CHUNK_BYTES, timings=None)
     CHROM only where it may change and converts a POS that is not 1-9 plain digits with int().  Raises ValueError naming the line
     or value on the inputs read_vcf_samples gives no usable result for: a '#' line after the #CHROM line, a POS that int()
     rejects; and on no #CHROM line, a record before it, no sample columns and a line longer than chunk_bytes.  timings (optional
-    dict) receives read_s, device_s, h2d_ms, kernel_ms, host_chunk_s, assemble_s (seconds, ms) and h2d_bytes."""
+    dict) receives read_s, device_s, h2d_ms, kernel_ms, host_chunk_s, assemble_s (seconds, ms) and h2d_bytes, and the
+    decompression route (_inflate_timings): a BGZF .vcf.gz is inflated on the same device (BgzfReader)."""
     from .. import lib
     chunk_bytes = int(chunk_bytes)
     enc = locale.getpreferredencoding(False)
@@ -580,7 +704,7 @@ def read_vcf_gt_codes(path, device=0, chunk_bytes=VCF_CHUNK_BYTES, timings=None)
     for k in ("read_s", "device_s", "host_chunk_s", "assemble_s", "h2d_ms", "kernel_ms", "h2d_bytes"):
         tm[k] = 0
     t0 = time.perf_counter()
-    fh = _open_binary(path)
+    fh = _open_binary(path, device)
     try:
         names, line_no, head = _population_header(fh, path)
         S = len(names)
@@ -635,6 +759,7 @@ def read_vcf_gt_codes(path, device=0, chunk_bytes=VCF_CHUNK_BYTES, timings=None)
         finally:
             parser.close()
     finally:
+        _inflate_timings(fh, tm)
         fh.close()
     t0 = time.perf_counter()
     cid = np.concatenate(cids) if cids else np.zeros(0, np.int32)

@@ -18,6 +18,7 @@
 #include "acc_pairs.cuh"
 #include "cross_geno.cuh"
 #include "vcf.cuh"
+#include "inflate.cuh"
 #include <unordered_map>
 
 namespace snpm {
@@ -2926,6 +2927,176 @@ int snpm_vcf_fetch_gt_codes(snpm_vcf *h, int32_t *line_start, int32_t *flags, in
         for (const auto &c : per_line) SNPM_CUDA(cudaMemcpyAsync(c.first, c.second->p, nl * 4, cudaMemcpyDeviceToHost, st));
     if (nc) SNPM_CUDA(cudaMemcpyAsync(codes, h->d_codes.p, nc, cudaMemcpyDeviceToHost, st));
     SNPM_CUDA(cudaStreamSynchronize(st));
+    return SNPM_OK;
+}
+
+}  // extern "C"
+
+// ---- BGZF members inflated on the device (inflate.cuh) ----------------------------------------------------------------------
+struct snpm_bgzf {
+    int device = 0;
+    int64_t max_in = 0, max_out = 0, max_members = 0;
+    cudaStream_t st = nullptr;
+    uint8_t *h_in = nullptr;             // pinned: member descriptors, then the compressed bytes; one copy up
+    uint8_t *h_out = nullptr;            // pinned: the text of the last batch
+    DevBuf d_in, d_out, d_status;
+    std::vector<int32_t> status;
+    cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};  // copy up, kernel, copy down of the text
+    ~snpm_bgzf() {
+        for (cudaEvent_t e : ev)
+            if (e) cudaEventDestroy(e);
+        if (h_in) cudaFreeHost(h_in);
+        if (h_out) cudaFreeHost(h_out);
+        if (st) cudaStreamDestroy(st);
+    }
+};
+
+static inline uint32_t bgzf_le32(const uint8_t *p) { return uint32_t(p[0]) | uint32_t(p[1]) << 8 | uint32_t(p[2]) << 16 | uint32_t(p[3]) << 24; }
+
+extern "C" {
+
+int snpm_bgzf_scan(const uint8_t *data, int64_t n_bytes, int64_t *member_off, int32_t *isize, int64_t cap, int64_t *n_members) {
+    if (!n_members || (n_bytes > 0 && !data) || n_bytes < 0 || cap < 0 || (cap > 0 && (!member_off || !isize)))
+        return fail(SNPM_E_ARG, "snpm_bgzf_scan: bad arguments");
+    *n_members = -1;
+    int64_t at = 0, m = 0;
+    while (at < n_bytes) {
+        const uint8_t *h = data + at;
+        const int64_t left = n_bytes - at;
+        if (left < 18 || h[0] != 0x1f || h[1] != 0x8b || h[2] != 8 || h[3] != 4) return SNPM_OK;
+        const int64_t xlen = int64_t(h[10]) | int64_t(h[11]) << 8;
+        if (12 + xlen > left) return SNPM_OK;
+        int64_t bsize = -1;
+        for (int64_t x = 12; x + 4 <= 12 + xlen;) {          // subfields: SI1 SI2 SLEN(2) data
+            const int64_t slen = int64_t(h[x + 2]) | int64_t(h[x + 3]) << 8;
+            if (x + 4 + slen > 12 + xlen) return SNPM_OK;
+            if (h[x] == 'B' && h[x + 1] == 'C' && slen == 2) bsize = int64_t(h[x + 4]) | int64_t(h[x + 5]) << 8;
+            x += 4 + slen;
+        }
+        if (bsize < 0) return SNPM_OK;
+        const int64_t size = bsize + 1;
+        if (size < 12 + xlen + 8 || size > left) return SNPM_OK;
+        const uint32_t is = bgzf_le32(h + size - 4);
+        if (is > 65536) return SNPM_OK;
+        if (m < cap) {
+            member_off[m] = at;
+            isize[m] = int32_t(is);
+        }
+        ++m;
+        at += size;
+    }
+    if (m == 0) return SNPM_OK;
+    if (m <= cap) member_off[m] = at;
+    *n_members = m;
+    return SNPM_OK;
+}
+
+int snpm_bgzf_create(int device, int64_t max_in_bytes, int64_t max_out_bytes, snpm_bgzf **out) {
+    if (!out) return fail(SNPM_E_ARG, "snpm_bgzf_create: out is NULL");
+    *out = nullptr;
+    if (max_in_bytes < 1 || max_in_bytes > SNPM_BGZF_MAX_BYTES || max_out_bytes < 1 || max_out_bytes > SNPM_BGZF_MAX_BYTES)
+        return fail(SNPM_E_ARG, "snpm_bgzf_create: max_in_bytes = %lld, max_out_bytes = %lld, each must be in 1..%lld",
+                    (long long)max_in_bytes, (long long)max_out_bytes, (long long)SNPM_BGZF_MAX_BYTES);
+    SNPM_CUDA(cudaSetDevice(device));
+    std::unique_ptr<snpm_bgzf> h(new (std::nothrow) snpm_bgzf);
+    if (!h) return fail(SNPM_E_NOMEM, "snpm_bgzf_create: out of host memory");
+    h->device = device;
+    h->max_in = max_in_bytes;
+    h->max_out = max_out_bytes;
+    h->max_members = max_in_bytes / 20 + 1;                 // a member holds at least a 12-byte header and an 8-byte trailer
+    const size_t in_cap = size_t(h->max_members) * sizeof(BgzfMember) + 16 + size_t(max_in_bytes);
+    SNPM_CUDA(cudaStreamCreateWithFlags(&h->st, cudaStreamNonBlocking));
+    for (cudaEvent_t &e : h->ev) SNPM_CUDA(cudaEventCreate(&e));
+    if (cudaMallocHost(&h->h_in, in_cap) != cudaSuccess) {
+        h->h_in = nullptr;
+        return fail(SNPM_E_NOMEM, "snpm_bgzf_create: cannot pin %zu bytes of host memory", in_cap);
+    }
+    if (cudaMallocHost(&h->h_out, size_t(max_out_bytes)) != cudaSuccess) {
+        h->h_out = nullptr;
+        return fail(SNPM_E_NOMEM, "snpm_bgzf_create: cannot pin %lld bytes of host memory", (long long)max_out_bytes);
+    }
+    SNPM_TRY(h->d_in.ensure(in_cap));
+    SNPM_TRY(h->d_out.ensure(size_t(max_out_bytes)));
+    *out = h.release();
+    return SNPM_OK;
+}
+
+void snpm_bgzf_destroy(snpm_bgzf *h) {
+    if (!h) return;
+    cudaSetDevice(h->device);
+    if (h->st) cudaStreamSynchronize(h->st);
+    delete h;
+}
+
+const uint8_t *snpm_bgzf_text(snpm_bgzf *h) { return h ? h->h_out : nullptr; }
+
+int snpm_bgzf_inflate(snpm_bgzf *h, const uint8_t *comp, int64_t comp_bytes, const int64_t *member_off, int64_t n, uint8_t *out,
+                      int64_t *info, float *ms) {
+    if (!h) return fail(SNPM_E_ARG, "snpm_bgzf_inflate: h is NULL");
+    if (!member_off || !info || (comp_bytes > 0 && !comp)) return fail(SNPM_E_ARG, "snpm_bgzf_inflate: comp, member_off or info is NULL");
+    if (comp_bytes < 0 || comp_bytes > h->max_in)
+        return fail(SNPM_E_ARG, "snpm_bgzf_inflate: comp_bytes = %lld outside 0..%lld", (long long)comp_bytes, (long long)h->max_in);
+    if (n < 0 || n > h->max_members)
+        return fail(SNPM_E_ARG, "snpm_bgzf_inflate: n = %lld outside 0..%lld", (long long)n, (long long)h->max_members);
+    // the member table, checked on the host: each member lies in comp, has a BGZF header and ISIZE <= 64 KiB, and the texts fit
+    BgzfMember *mem = reinterpret_cast<BgzfMember *>(h->h_in);
+    const size_t desc_bytes = (size_t(n) * sizeof(BgzfMember) + 15) & ~size_t(15);
+    uint64_t total = 0;
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t a = member_off[i], b = member_off[i + 1];
+        if (a < 0 || b < a || b > comp_bytes)
+            return fail(SNPM_E_ARG, "snpm_bgzf_inflate: member %lld spans bytes %lld..%lld of %lld", (long long)i, (long long)a, (long long)b,
+                        (long long)comp_bytes);
+        const uint8_t *m = comp + a;
+        if (b - a < 20 || m[0] != 0x1f || m[1] != 0x8b || m[2] != 8 || m[3] != 4)
+            return fail(SNPM_E_ARG, "snpm_bgzf_inflate: member %lld at byte %lld has no BGZF header", (long long)i, (long long)a);
+        const int64_t hdr = 12 + (int64_t(m[10]) | int64_t(m[11]) << 8);
+        if (hdr + 8 > b - a)
+            return fail(SNPM_E_ARG, "snpm_bgzf_inflate: member %lld at byte %lld: its extra field runs past its end", (long long)i, (long long)a);
+        const uint32_t is = bgzf_le32(comp + b - 4);
+        if (is > 65536)
+            return fail(SNPM_E_ARG, "snpm_bgzf_inflate: member %lld at byte %lld has ISIZE %u > 65536", (long long)i, (long long)a, is);
+        mem[i] = BgzfMember{uint32_t(desc_bytes + a + hdr), uint32_t(b - a - hdr - 8), uint32_t(total), is, bgzf_le32(comp + b - 8)};
+        total += is;
+        if (total > uint64_t(h->max_out))
+            return fail(SNPM_E_ARG, "snpm_bgzf_inflate: the members hold more than max_out_bytes = %lld of text", (long long)h->max_out);
+    }
+    SNPM_CUDA(cudaSetDevice(h->device));
+    cudaStream_t st = h->st;
+    if (comp_bytes) memcpy(h->h_in + desc_bytes, comp, size_t(comp_bytes));
+    h->status.assign(size_t(n), 0);
+    SNPM_TRY(h->d_status.ensure(size_t(std::max<int64_t>(n, 1)) * 4));
+    SNPM_CUDA(cudaEventRecord(h->ev[0], st));
+    SNPM_CUDA(cudaMemcpyAsync(h->d_in.p, h->h_in, desc_bytes + size_t(comp_bytes), cudaMemcpyHostToDevice, st));
+    SNPM_CUDA(cudaEventRecord(h->ev[1], st));
+    if (n) {
+        k_bgzf_inflate<<<unsigned(ceil_div64(n, BGZF_WARPS)), BGZF_WARPS * 32, 0, st>>>(h->d_in.as<uint8_t>(), h->d_in.as<BgzfMember>(), int(n),
+                                                                                       h->d_out.as<uint8_t>(), h->d_status.as<int32_t>());
+        SNPM_KERNEL_CHECK();
+    }
+    SNPM_CUDA(cudaEventRecord(h->ev[2], st));
+    if (n) SNPM_CUDA(cudaMemcpyAsync(h->status.data(), h->d_status.p, size_t(n) * 4, cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaStreamSynchronize(st));
+    info[0] = int64_t(total);
+    info[1] = -1;
+    info[2] = 0;
+    for (int64_t i = 0; i < n; ++i)
+        if (h->status[size_t(i)]) {
+            info[1] = i;
+            info[2] = h->status[size_t(i)];
+            break;
+        }
+    SNPM_CUDA(cudaEventRecord(h->ev[3], st));
+    if (info[1] < 0 && total) SNPM_CUDA(cudaMemcpyAsync(h->h_out, h->d_out.p, size_t(total), cudaMemcpyDeviceToHost, st));
+    SNPM_CUDA(cudaEventRecord(h->ev[4], st));
+    SNPM_CUDA(cudaStreamSynchronize(st));
+    if (info[1] < 0 && out && total) memcpy(out, h->h_out, size_t(total));
+    if (ms) {
+        ms[0] = ms[1] = ms[2] = 0.f;
+        cudaEventElapsedTime(&ms[0], h->ev[0], h->ev[1]);
+        cudaEventElapsedTime(&ms[1], h->ev[1], h->ev[2]);
+        cudaEventElapsedTime(&ms[2], h->ev[3], h->ev[4]);
+    }
     return SNPM_OK;
 }
 

@@ -278,6 +278,11 @@ SIGNATURES = {
     "snpm_vcf_parse_gt_codes": (C.c_int, [_p, C.c_char_p, _i64, _p, _p]),
     "snpm_vcf_fetch_gt_codes": (C.c_int, [_p, _p, _p, _p, _p, _p, _p]),
     "snpm_vcf_destroy": (None, [_p]),
+    "snpm_bgzf_scan": (C.c_int, [_p, _i64, _p, _p, _i64, _p]),
+    "snpm_bgzf_create": (C.c_int, [C.c_int, _i64, _i64, _p]),
+    "snpm_bgzf_inflate": (C.c_int, [_p, _p, _i64, _p, _i64, _p, _p, _p]),
+    "snpm_bgzf_text": (_p, [_p]),
+    "snpm_bgzf_destroy": (None, [_p]),
 }
 
 
@@ -609,6 +614,67 @@ class VcfParser(object):
     def close(self):
         if getattr(self, "_h", None):
             load().snpm_vcf_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def bgzf_scan(data):
+    """Member table of a BGZF file held in data (a buffer of uint8, e.g. an mmap viewed by NumPy): (member_off int64 [n+1],
+    isize int64 [n]) when the file is all BGZF (snpm_bgzf_scan: every member a BGZF member with ISIZE <= 65536, the members
+    tiling the data to its last byte), else None.  Host code; needs no device."""
+    data = np.frombuffer(data, np.uint8) if not isinstance(data, np.ndarray) else data
+    n_bytes = len(data)
+    cap = n_bytes // 8192 + 16
+    while True:
+        off, isize, n = np.empty(cap + 1, np.int64), np.empty(cap, np.int32), C.c_int64(0)
+        check(load().snpm_bgzf_scan(ptr(data) if n_bytes else None, n_bytes, ptr(off), ptr(isize), cap, C.byref(n)))
+        if n.value < 0:
+            return None
+        if n.value <= cap:
+            return off[:n.value + 1], isize[:n.value].astype(np.int64)
+        cap = n.value
+
+
+class BgzfInflater(object):
+    """BGZF members inflated on CUDA device `device` (snpm_bgzf_*): up to max_in_bytes of members and max_out_bytes of text
+    per call.  inflate() raises gzip.BadGzipFile naming the path, the refused member's byte offset in the file and the reason."""
+
+    REASONS = {1: "invalid DEFLATE stream", 2: "text length differs from ISIZE", 3: "CRC-32 mismatch"}
+
+    def __init__(self, device, max_in_bytes, max_out_bytes):
+        self.max_in_bytes, self.max_out_bytes = int(max_in_bytes), int(max_out_bytes)
+        h = C.c_void_p()
+        check(load().snpm_bgzf_create(int(device), self.max_in_bytes, self.max_out_bytes, C.byref(h)))
+        self._h = h
+        self.ms = np.zeros(3)                   # device ms summed over the calls: copy up, kernel, copy down
+
+    def inflate(self, comp, member_off, path="<bytes>", base=0, out=None):
+        """comp: uint8 array holding the members, member_off int64 [n+1] their offsets in it; base = the byte offset of
+        comp[0] in the file (for the error).  Returns the number of bytes of text.  The text goes to out (uint8 array) when
+        given; it stays in the handle's pinned staging (text()) until the next call either way."""
+        member_off = as_c(member_off, np.int64)
+        info = np.zeros(3, np.int64)
+        ms = (C.c_float * 3)()
+        check(load().snpm_bgzf_inflate(self._h, ptr(comp), len(comp), ptr(member_off), len(member_off) - 1, ptr(out), ptr(info), ms))
+        self.ms += np.array(ms[:3])
+        if info[1] >= 0:
+            import gzip
+            raise gzip.BadGzipFile("%s: BGZF member at byte %d: %s" % (path, base + int(member_off[info[1]]),
+                                                                       self.REASONS.get(int(info[2]), "reason %d" % info[2])))
+        return int(info[0])
+
+    def text(self, start, stop):
+        """bytes start..stop of the last call's text, copied once out of the pinned staging."""
+        return C.string_at(load().snpm_bgzf_text(self._h) + start, stop - start)
+
+    def close(self):
+        if getattr(self, "_h", None):
+            load().snpm_bgzf_destroy(self._h)
             self._h = None
 
     def __del__(self):

@@ -13,6 +13,8 @@ The sample recipe follows the reference's simulator (simulate.py:10-31) and the 
 sample_files/701_501.filter.vcf (e.g. `0,9,87` at DP 3).
 """
 import io
+import struct
+import zlib
 
 import numpy as np
 
@@ -394,3 +396,34 @@ def population_vcf(fh, chrs, positions, n_samples, seed=11, edge_forms=True, blo
             else:
                 out.append(b"%s\t%d\t.\tA\tT\t.\tPASS\t.\tGT\t" % (str(chrs[r]).encode(), positions[r]) + b"\t".join(cells))
         fh.write(b"\n".join(out) + b"\n")
+
+
+BGZF_EOF = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
+
+
+def write_bgzf(path, data, level=6, strategy=zlib.Z_DEFAULT_STRATEGY, member_bytes=65280, eof=True):
+    """Write data as BGZF (bgzip's format: gzip members with a BC extra subfield holding the member's size - 1), each member
+    the raw DEFLATE stream of zlib.compressobj(level, wbits=-15, strategy).  member_bytes: text per member (65280, bgzip's
+    default), or a list of the sizes of the members in order (they must sum to len(data); 0 gives an empty member).  eof
+    appends the 28-byte EOF member.  Raises ValueError when a member would exceed 65536 bytes."""
+    data = bytes(data)
+    if isinstance(member_bytes, int):
+        sizes = [min(member_bytes, len(data) - a) for a in range(0, len(data), member_bytes)]
+    else:
+        sizes = list(member_bytes)
+        if sum(sizes) != len(data):
+            raise ValueError("member sizes sum to %d, not %d" % (sum(sizes), len(data)))
+    with open(path, "wb") as fh:
+        at = 0
+        for n in sizes:
+            piece = data[at:at + n]
+            at += n
+            c = zlib.compressobj(level, zlib.DEFLATED, -15, 8, strategy)
+            payload = c.compress(piece) + c.flush()
+            size = 26 + len(payload)
+            if n > 65536 or size > 65536:
+                raise ValueError("a member of %d bytes of text takes %d bytes" % (n, size))
+            fh.write(b"\x1f\x8b\x08\x04\0\0\0\0\0\xff\x06\0BC\x02\0" + struct.pack("<H", size - 1) + payload
+                     + struct.pack("<II", zlib.crc32(piece), n))
+        if eof:
+            fh.write(BGZF_EOF)
